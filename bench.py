@@ -338,6 +338,9 @@ def run_single_process(args):
         toks += st["target_tokens"]
     sampler.mark_end()
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {f"{args.math}_tokens": out_tokens[:int(out_offsets[-1])].astype(np.float32),
+                                         f"{args.math}_offsets": out_offsets.astype(np.float64)})
     cfg = workload_config()
     cfg["sentences_per_gpu"] = None
     cfg["sentences"] = int(n_sent)
@@ -356,6 +359,21 @@ def run_single_process(args):
            "input_generation_s": round(gen_s, 2)}
     os.write(json_fd, (json.dumps(out) + "\n").encode())
     return 0
+
+
+DUMP_CAP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy.  Beyond DUMP_CAP_BYTES in all, every array is replaced by a fixed, seeded
+    sample of its elements (in order), so two builds run with the same arguments still compare element for element."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_CAP_BYTES:
+            a = a.ravel()[np.sort(np.random.RandomState(0).choice(a.size, a.size * DUMP_CAP_BYTES // total, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    print(f"bench: wrote {len(arrays)} arrays to {out_dir}" + (" (sampled)" if total > DUMP_CAP_BYTES else ""), file=sys.stderr)
 
 
 def workload_config():
@@ -383,7 +401,14 @@ def main():
     ap.add_argument("--sentences", type=int, default=0, help="with --single-process: sentences in the request (default: the workload's)")
     ap.add_argument("--profiler-range", action="store_true",
                     help="bracket the timed steps with cudaProfilerStart/Stop (for ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned to the caller as DIR/<name>.npy "
+                         "(token ids as float32, offsets as float64; rank 0; at most 64 MiB, a seeded sample beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this project's GPU path, not of --impl reference")
     global WL
     WL = dict(WORKLOADS[args.workload])
     if _MW:
@@ -439,7 +464,7 @@ def main():
     def resident_pass():
         toks = 0
         for b in resident:
-            _, t = model.forward_resident(b["tok"], b["lens"], b["B"], b["T"], b["steps"], LIMIT, b["sl"], b["nsl"])
+            b["decode_steps"], t = model.forward_resident(b["tok"], b["lens"], b["B"], b["T"], b["steps"], LIMIT, b["sl"], b["nsl"])
             toks += t
         return toks
 
@@ -502,6 +527,10 @@ def main():
             sampler.mark_end()
         total_ms = sum(step_ms)
         tokens = [step_tokens_of(e) for e in resident]
+        outputs = {}
+        if args.dump_outputs:  # per batch of the plan: step tokens [decode steps, sentences of the batch]
+            outputs = {f"{mode}_step_tokens_{i:03d}": t[:e["decode_steps"]].astype(np.float32)
+                       for i, (e, t) in enumerate(zip(resident, tokens))}
 
         # ---- end-to-end arm through the public C-ABI call with host buffers (ragged tokens/offsets in, ragged targets
         # out; Batcher, shortlist generation, H2D and D2H all inside the timed call)
@@ -516,6 +545,9 @@ def main():
             e2e_tokens += st["target_tokens"]
             e2e_stats = st
         barrier()
+        if args.dump_outputs:
+            outputs[f"{mode}_e2e_tokens"] = h_out_tokens[:int(h_out_offsets[-1])].astype(np.float32)
+            outputs[f"{mode}_e2e_offsets"] = h_out_offsets.astype(np.float64)
 
         # ---- per-kernel event timing: one extra profiled pass (not part of the timed region)
         ctx.profile(True)
@@ -569,7 +601,7 @@ def main():
                                   "achieved_tops": round(gemm_ops / max(gemm_ms, 1e-9) / 1e9, 1), "peak_tops": int8_peak_tops,
                                   "frac": round(gemm_ops / max(gemm_ms, 1e-9) / 1e9 / int8_peak_tops, 4),
                                   "note": "all kernels that issue tcgen05 MMAs, fused epilogues included in their time"},
-            "target_tokens_per_step_per_gpu": tokens_per_step, "_tokens": tokens,
+            "target_tokens_per_step_per_gpu": tokens_per_step, "_tokens": tokens, "_outputs": outputs,
         }
 
     sampler = ClockSampler(local_rank)
@@ -586,6 +618,8 @@ def main():
         dist.destroy_process_group()
     if rank != 0:
         return 0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: v for m in modes for k, v in res[m]["_outputs"].items()})
 
     head = res[modes[0]]
     out = {

@@ -41,6 +41,25 @@ def test_mixed_workload_batches_respect_max_words():
     assert widths == sorted(widths)
 
 
+def test_dump_outputs_whole_below_the_cap_and_a_fixed_sample_above(tmp_path, monkeypatch):
+    arrays = {"exact_step_tokens_000": np.arange(3000, dtype=np.float32).reshape(60, 50),
+              "exact_e2e_offsets": np.arange(1001, dtype=np.float64)}
+    bench.dump_outputs(str(tmp_path / "whole"), arrays)
+    for name, a in arrays.items():
+        got = np.load(tmp_path / "whole" / f"{name}.npy")
+        assert got.dtype == a.dtype and np.array_equal(got, a)
+    monkeypatch.setattr(bench, "DUMP_CAP_BYTES", 4096)
+    bench.dump_outputs(str(tmp_path / "a"), arrays)
+    bench.dump_outputs(str(tmp_path / "b"), arrays)
+    total = 0
+    for name, a in arrays.items():
+        x, y = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert x.dtype == a.dtype and np.array_equal(x, y) and 0 < x.size < a.size
+        assert np.all(np.diff(x) > 0)  # elements of the original, in their original order
+        total += x.nbytes
+    assert total <= 4096
+
+
 def test_headline_is_one_batch_of_4096_by_32():
     wl = bench.WORKLOADS["tiny_shortlist"]
     plan = capi.batcher_plan([wl["length"]] * wl["sentences"], wl["max_words"])

@@ -5,9 +5,10 @@ splitter, TextProcessor, AnnotatedText, Response / combine.
    TextProcessor.cc, Splitter.cc, Regex.cc, Annotation.cc, Response.cc, Request.cc with the vendored sentencepiece
    0.2.00, compiled in place; tests/golden/make_text_golden.py) -- is replayed through the product's host code behind the
    same driver (tests/cpp/text_front_driver.cc) and must be answered byte for byte the same.
-2. Vocabulary::encode / decode against the sentencepiece wheel of this image on seeded random strings.
+2. Vocabulary::encode / decode against the sentencepiece wheel's stored answers on seeded random strings.
 3. Where the reference sources exist (this container), the freshly built reference driver and the product driver are
    compared live on further random inputs."""
+import hashlib
 import json
 import os
 import random
@@ -62,12 +63,8 @@ def _random_text(rng, lo=0, hi=40):
     return "".join(rng.choice(ALPHABET) for _ in range(rng.randint(lo, hi)))
 
 
-@pytest.mark.parametrize("model", ["spm_unigram.model", "spm_bytes.model"])
-def test_vocabulary_against_the_sentencepiece_wheel(driver, model):
-    """Encode: ids and the byte range of every piece (SentencePieceText.pieces[].begin / end); Decode: text and ranges.
-    Includes malformed UTF-8."""
-    spm = pytest.importorskip("sentencepiece")
-    sp = spm.SentencePieceProcessor(model_file=os.path.join(GOLD, model))
+def vocabulary_commands(model, pieces):
+    """Seeded random strings (malformed UTF-8 included) to encode and id lists to decode, as driver commands."""
     rng = random.Random(31337 if model.startswith("spm_u") else 271828)
     texts = [_random_text(rng).encode("utf-8") for _ in range(400)]
     for _ in range(60):  # random byte damage
@@ -75,34 +72,25 @@ def test_vocabulary_against_the_sentencepiece_wheel(driver, model):
         for _ in range(rng.randint(1, 3)):
             b[rng.randrange(len(b))] = rng.randrange(256)
         texts.append(bytes(b))
-    V = sp.get_piece_size()
-    id_lists = [[rng.randrange(V) for _ in range(rng.randint(0, 25))] for _ in range(300)]
+    id_lists = [[rng.randrange(pieces) for _ in range(rng.randint(0, 25))] for _ in range(300)]
     cmds = [f"vocab {os.path.join('tests', 'golden', 'text', model)}"] + [f"encode {_hx(t)}" for t in texts] + \
         ["decode " + " ".join(map(str, ids)) for ids in id_lists]
+    return texts, id_lists, cmds
+
+
+@pytest.mark.parametrize("model", ["spm_unigram.model", "spm_bytes.model"])
+def test_vocabulary_against_the_sentencepiece_wheel(driver, model):
+    """Encode: ids and the byte range of every piece (SentencePieceText.pieces[].begin / end); Decode: text and ranges.
+    Includes malformed UTF-8, where only the ids are compared (offsets are pinned by the reference goldens).  The
+    wheel's answers are stored in tests/golden/text/wheel.json (tests/golden/make_wheel_golden.py)."""
+    g = json.load(open(os.path.join(GOLD, "wheel.json")))["vocabulary"][model]
+    _, _, cmds = vocabulary_commands(model, g["pieces"])
+    assert hashlib.sha256("\n".join(cmds).encode("utf-8")).hexdigest() == g["commands_sha256"], "inputs drifted"
     got = _run(driver, cmds)[1:]
-    def byte_offsets(text):  # the wheel reports offsets in code points (its ConvertToUnicodeAlignment); the C++ API in bytes
-        at = [0]
-        for ch in text:
-            at.append(at[-1] + len(ch.encode("utf-8")))
-        return at
-    for t, line in zip(texts, got[:len(texts)]):
-        try:
-            s = t.decode("utf-8")
-        except UnicodeDecodeError:  # malformed input: ids only here, offsets are pinned by the reference goldens
-            assert line.split(" |")[0] == "ids" + "".join(f" {i}" for i in sp.encode(t, out_type=int)), t
-            continue
-        proto = sp.encode(s, out_type="immutable_proto")
-        at = byte_offsets(s)
-        want = "ids" + "".join(f" {p.id}" for p in proto.pieces) + " |" + "".join(f" {at[p.begin]}:{at[p.end]}" for p in proto.pieces)
-        assert line == want, t
-    for ids, line in zip(id_lists, got[len(texts):]):
-        if not ids:
-            assert line == "text - |"
-            continue
-        proto = sp.decode_ids_as_immutable_proto(ids)
-        at = byte_offsets(proto.text)
-        want = "text " + _hx(proto.text) + " |" + "".join(f" {at[p.begin]}:{at[p.end]}" for p in proto.pieces)
-        assert line == want, ids
+    assert len(got) == len(g["answers"])
+    bad = [(c, want, have) for c, want, have in zip(cmds[1:], g["answers"], got)
+           if (have if " |" in want else have.split(" |")[0]) != want]
+    assert not bad, f"{len(bad)} of {len(got)} answers differ; first: {bad[0][0][:120]!r}\n want {bad[0][1][:300]}\n have {bad[0][2][:300]}"
 
 
 @pytest.mark.skipif(not os.path.isdir("/root/reference/slimt"), reason="the reference sources only exist in the build container")

@@ -97,6 +97,15 @@ void slimt_b200_model_destroy(slimt_b200_model* model);
 /* embedding dim, ffn dim, vocabulary rows */
 int slimt_b200_model_dims(const slimt_b200_model* model, int32_t* emb, int32_t* ffn, int32_t* vocab);
 
+/* Longest sentence (source tokens, EOS included) the model accepts in slimt_b200_model_forward and in every
+ * translate call; a longer one is an error ("exceeds the supported maximum of N"), never a truncation.  The reference
+ * bounds segments only through the caller's wrap_length (TextProcessor::wrap, TextProcessor.cc:123-157).
+ * `current` starts at 256; set_max_length raises or lowers it within [1, supported], where `supported` = 1024 is the
+ * positional table's length.  n outside that range is an error and leaves the model unchanged.  Decoding runs up to
+ * limit_factor x T steps, and an alignment request holds 4 * steps * B * T bytes of device workspace. */
+int slimt_b200_model_set_max_length(slimt_b200_model* model, int32_t n);
+int slimt_b200_model_max_length(const slimt_b200_model* model, int32_t* current, int32_t* supported);
+
 typedef struct slimt_b200_forward_io {
   /* inputs: the padded batch of slimt::Input (Input.cc:13-63) */
   const uint32_t* tokens;   /* [B][T] row-major, padded with pad id */
@@ -163,7 +172,8 @@ int slimt_b200_translate(slimt_b200_model* model, slimt_b200_translate_io* io);
  * one Batcher forms the batches, and every replica's worker thread takes the next unserved batch as soon as it is
  * free -- Async's workers pulling from the batcher queue (Frontend.cc:207-227, Batcher.hh:203-259).  Sentences are
  * independent and every batch is the one the Batcher would have formed anyway, so the output is identical to
- * slimt_b200_translate's; there is no collective on the data path.  device_ms = the longest replica's time. */
+ * slimt_b200_translate's; there is no collective on the data path.  device_ms = the longest replica's time.
+ * The length bound is the smallest slimt_b200_model_max_length current over the replicas. */
 int slimt_b200_translate_multi(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_translate_io* io);
 
 /* Host-only pieces of the same path, callable without a GPU (used by the CPU test-suite):

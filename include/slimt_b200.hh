@@ -388,6 +388,10 @@ class Model {
       detail::check(slimt_b200_model_create(detail::context(device), package.model.data, package.model.size, &c, &m),
                     "slimt_b200_model_create");
       replicas_.push_back(m);
+      // as in the reference, only the caller's wrap_length bounds a segment: admit every length the model can encode
+      int32_t current = 0, supported = 0;
+      slimt_b200_model_max_length(m, &current, &supported);
+      detail::check(slimt_b200_model_set_max_length(m, supported), "slimt_b200_model_set_max_length");
     }
     int32_t e = 0, f = 0, v = 0;
     slimt_b200_model_dims(replicas_[0], &e, &f, &v);

@@ -26,6 +26,7 @@ EXPORTS = [
     "slimt_b200_model_dims", "slimt_b200_model_forward", "slimt_b200_translate", "slimt_b200_kernel_launches",
     "slimt_b200_shortlist_generate", "slimt_b200_batcher_plan", "slimt_b200_profile_enable", "slimt_b200_profile_read",
     "slimt_b200_translate_multi", "slimt_b200_shortlist_check", "slimt_b200_ctx_set_math", "slimt_b200_ctx_get_math",
+    "slimt_b200_model_set_max_length", "slimt_b200_model_max_length",
 ]
 
 
@@ -92,6 +93,8 @@ def lib() -> C.CDLL:
                                               C.POINTER(C.c_void_p)]
         L.slimt_b200_model_destroy.argtypes = [C.c_void_p]
         L.slimt_b200_model_dims.argtypes = [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
+        L.slimt_b200_model_set_max_length.argtypes = [C.c_void_p, C.c_int32]
+        L.slimt_b200_model_max_length.argtypes = [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
         L.slimt_b200_model_forward.argtypes = [C.c_void_p, C.POINTER(ForwardIO)]
         L.slimt_b200_translate.argtypes = [C.c_void_p, C.POINTER(TranslateIO)]
         L.slimt_b200_translate_multi.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.POINTER(TranslateIO)]
@@ -250,6 +253,16 @@ class Model:
         if self.h:
             lib().slimt_b200_model_destroy(self.h)
             self.h = C.c_void_p()
+
+    def set_max_length(self, n: int):
+        """Longest sentence the model accepts, within [1, max_length()[1]] (default 256)."""
+        _check(lib().slimt_b200_model_set_max_length(self.h, int(n)), "slimt_b200_model_set_max_length")
+
+    def max_length(self):
+        """(current bound, largest bound the model supports)."""
+        cur, sup = C.c_int32(), C.c_int32()
+        _check(lib().slimt_b200_model_max_length(self.h, C.byref(cur), C.byref(sup)), "slimt_b200_model_max_length")
+        return cur.value, sup.value
 
     def forward(self, tokens: np.ndarray, lengths: np.ndarray, limit_factor: float = 1.5,
                 shortlist: Optional[np.ndarray] = None, forced: Optional[np.ndarray] = None,

@@ -156,6 +156,21 @@ int slimt_b200_model_dims(const slimt_b200_model* model, int32_t* emb, int32_t* 
   return 0;
 }
 
+int slimt_b200_model_set_max_length(slimt_b200_model* model, int32_t n) {
+  if (n < 1 || n > model->m.max_pos) {
+    sb::set_error("max length " + std::to_string(n) + " is outside [1, " + std::to_string(model->m.max_pos) +
+                  "] (the positional table's rows)");
+    return 1;
+  }
+  model->m.len_bound = n;
+  return 0;
+}
+
+int slimt_b200_model_max_length(const slimt_b200_model* model, int32_t* current, int32_t* supported) {
+  *current = model->m.max_len(), *supported = model->m.max_pos;
+  return 0;
+}
+
 int slimt_b200_model_forward(slimt_b200_model* model, slimt_b200_forward_io* io) {
   sb::ForwardArgs a;
   a.tokens = io->tokens, a.lengths = io->lengths, a.B = io->batch, a.T = io->seq;

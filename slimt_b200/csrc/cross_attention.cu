@@ -18,9 +18,12 @@ namespace sb {
 
 namespace {
 
-constexpr int kMaxKeyChunks = 8;  // S <= 256
+constexpr int kRegKeyChunks = 8;   // S <= 256: every lane keeps its keys' scores in registers
+constexpr int kMaxKeyChunks = 32;  // S <= 1024: the scores are parked in the warp's shared memory instead
 
-// NC = compile-time bound on 32-key chunks per sentence (ceil(S / 32) rounded up to 1, 2, 4 or 8)
+// NC = compile-time bound on 32-key chunks per sentence (ceil(S / 32) rounded up to 1, 2, 4, 8 or 32).  Above 8 chunks
+// the score array would spill; each lane then keeps score c of key 32 c + lane at sc_smem[32 c + lane] of its warp's
+// block (written and read back by the same lane only), and the chunk loops are not unrolled.
 template <int DH, int H, int NC>
 __global__ void __launch_bounds__((H + 1) * 32, 3)
     cross_attention_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_constant__ CUtensorMap mapV,
@@ -37,6 +40,8 @@ __global__ void __launch_bounds__((H + 1) * 32, 3)
   uint64_t* empty_bar = full_bar + stages;
   uint64_t* exp_tab = empty_bar + stages;
   float* sq_all = reinterpret_cast<float*>(exp_tab + 32);
+  constexpr bool kSmemScores = NC > kRegKeyChunks;
+  constexpr int kUnroll = kSmemScores ? 1 : NC;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (threadIdx.x >= 32 && threadIdx.x < 64) exp_tab[threadIdx.x - 32] = kExp2fTab[threadIdx.x - 32];
@@ -81,6 +86,7 @@ __global__ void __launch_bounds__((H + 1) * 32, 3)
   const int h = warp;
   float* sq = sq_all + h * DH;
   float* sp = sq_all + H * DH + h * 32;  // this warp's probabilities of the current 32-key chunk
+  float* sc_smem = sq_all + H * (DH + 32) + h * (kSmemScores ? NC * 32 : 0);
   // Per-lane byte offsets inside a swizzled [rows][128 B] tile.  Score pass: lane = key row, 16-byte
   // chunk g sits at ((g ^ (row & 7)) << 4).  Value pass: lane = head dimension, row l of the tile holds
   // it at (((lane >> 2) ^ (l & 7)) << 4) + (lane & 3) * 4.
@@ -94,11 +100,15 @@ __global__ void __launch_bounds__((H + 1) * 32, 3)
     __syncwarp();
     for (int d = lane; d < DH; d += 32) sq[d] = Qr[static_cast<size_t>(b) * E + h * DH + d];
     __syncwarp();
-    float sc[NC];
+    float sc_reg[kSmemScores ? 1 : NC];
+    auto sc = [&](int c) -> float& {
+      if constexpr (kSmemScores) return sc_smem[c * 32 + lane];
+      else return sc_reg[c];
+    };
     float mx = -3.402823466e+38f;
-#pragma unroll
+#pragma unroll kUnroll
     for (int c = 0; c < NC; c++) {
-      sc[c] = 0.0f;
+      sc(c) = 0.0f;
       if (c < nc) {
         const uint32_t s = it % stages;
         const uint32_t ph = (it / stages) & 1;
@@ -122,7 +132,7 @@ __global__ void __launch_bounds__((H + 1) * 32, 3)
         if (lane == 0) mbar_arrive(&empty_bar[s]);
         if (c * 32 + lane < len) {
           acc = __fmul_rn(dk, acc);
-          sc[c] = acc;
+          sc(c) = acc;
           mx = fmaxf(mx, acc);
         }
       }
@@ -130,14 +140,14 @@ __global__ void __launch_bounds__((H + 1) * 32, 3)
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
     float sum = 0.0f;
-#pragma unroll
+#pragma unroll kUnroll
     for (int c = 0; c < NC; c++) {
       if (c < nc) {
         const int j = c * 32 + lane;
-        sc[c] = (j < len) ? expf_glibc_nonpos_tab(__fsub_rn(sc[c], mx), exp_tab) : 0.0f;
+        sc(c) = (j < len) ? expf_glibc_nonpos_tab(__fsub_rn(sc(c), mx), exp_tab) : 0.0f;
         // sum in key order (slimt/TensorOps.cc:296-314): exp of a masked key is +0 and adding it is exact
         __syncwarp();
-        sp[lane] = sc[c];
+        sp[lane] = sc(c);
         __syncwarp();
 #pragma unroll
         for (int l = 0; l < 32; l += 4) {
@@ -149,29 +159,29 @@ __global__ void __launch_bounds__((H + 1) * 32, 3)
         }
       }
     }
-#pragma unroll
+#pragma unroll kUnroll
     for (int c = 0; c < NC; c++) {
-      if (c < nc) sc[c] = __fdiv_rn(sc[c], sum);
+      if (c < nc) sc(c) = __fdiv_rn(sc(c), sum);
     }
     if (attn_head0 != nullptr && h == 0) {
-#pragma unroll
+#pragma unroll kUnroll
       for (int c = 0; c < NC; c++) {
         const int j = c * 32 + lane;
-        if (j < S) attn_head0[static_cast<size_t>(b) * S + j] = (j < len) ? sc[c] : 0.0f;
+        if (j < S) attn_head0[static_cast<size_t>(b) * S + j] = (j < len) ? sc(c) : 0.0f;
       }
     }
 
     float acc[kSub];
 #pragma unroll
     for (int u = 0; u < kSub; u++) acc[u] = 0.0f;
-#pragma unroll
+#pragma unroll kUnroll
     for (int c = 0; c < NC; c++) {
       if (c < nc) {
         const uint32_t s = it % stages;
         const uint32_t ph = (it / stages) & 1;
         it++;
         __syncwarp();
-        sp[lane] = sc[c];
+        sp[lane] = sc(c);
         __syncwarp();
         mbar_wait(&full_bar[s], ph);
         const uint8_t* tile = smem + static_cast<size_t>(s) * chunk_bytes + (h * kSub) * tile_bytes;
@@ -216,15 +226,11 @@ __global__ void __launch_bounds__((H + 1) * 32, 3)
 
 int cross_attention_box_rows(int S) { return S >= 32 ? 32 : ((S + 7) & ~7); }
 
-void launch_cross_attention(const CUtensorMap& mapK, const CUtensorMap& mapV, const float* Qr, const uint32_t* lengths,
-                            int B, int S, int H, int dh, int num_sms, float* out_f32, QuantOuts q, float* attn_head0,
-                            cudaStream_t stream) {
-  if (B == 0) return;
-  if (S > 32 * kMaxKeyChunks || H != 8 || (dh != 32 && dh != 64)) {
-    fprintf(stderr, "slimt_b200: cross attention supports S <= %d, 8 heads of 32 or 64 (got S=%d H=%d dh=%d)\n",
-            32 * kMaxKeyChunks, S, H, dh);
-    abort();
-  }
+int launch_cross_attention(const CUtensorMap& mapK, const CUtensorMap& mapV, const float* Qr, const uint32_t* lengths,
+                           int B, int S, int H, int dh, int num_sms, float* out_f32, QuantOuts q, float* attn_head0,
+                           cudaStream_t stream) {
+  if (B == 0) return 0;
+  if (S > 32 * kMaxKeyChunks || H != 8 || (dh != 32 && dh != 64)) return 1;
   const float dk = static_cast<float>(1.0 / std::sqrt(static_cast<double>(dh)));
   const int box_rows = cross_attention_box_rows(S);
   const size_t chunk = static_cast<size_t>(box_rows) * 128 * H * (dh / 32);
@@ -233,17 +239,18 @@ void launch_cross_attention(const CUtensorMap& mapK, const CUtensorMap& mapV, co
   // flight come from co-resident CTAs.
   int stages = 2;
   if (chunk <= 8 * 1024) stages = 4;
-  const size_t smem = 1024 + stages * chunk + stages * 16 + 256 + static_cast<size_t>(H) * (dh + 32) * sizeof(float);
+  const int nc = (S + 31) / 32;
+  const size_t sc_park = nc > kRegKeyChunks ? static_cast<size_t>(H) * kMaxKeyChunks * 32 * sizeof(float) : 0;
+  const size_t smem = 1024 + stages * chunk + stages * 16 + 256 + static_cast<size_t>(H) * (dh + 32) * sizeof(float) + sc_park;
   int per_sm = static_cast<int>((220 * 1024) / (smem + 1024));
   if (per_sm < 1) per_sm = 1;
   if (per_sm > 3) per_sm = 3;
   const int grid = B < num_sms * per_sm ? B : num_sms * per_sm;
   const int threads = (H + 1) * 32;
-  const int nc = (S + 31) / 32;
 #define SB_CA_LAUNCH(DH_, NC_)                                                                                   \
   do {                                                                                                           \
     auto kern = cross_attention_kernel<DH_, 8, NC_>;                                                             \
-    ensure_dyn_smem(kern, smem);             \
+    if (ensure_dyn_smem(kern, smem) != cudaSuccess) return 1;                                                    \
     kern<<<grid, threads, smem, stream>>>(mapK, mapV, Qr, lengths, B, S, box_rows, stages, dk, out_f32, q,      \
                                           attn_head0);                                                           \
   } while (0)
@@ -251,14 +258,17 @@ void launch_cross_attention(const CUtensorMap& mapK, const CUtensorMap& mapV, co
     if (nc <= 1) SB_CA_LAUNCH(32, 1);
     else if (nc <= 2) SB_CA_LAUNCH(32, 2);
     else if (nc <= 4) SB_CA_LAUNCH(32, 4);
-    else SB_CA_LAUNCH(32, 8);
+    else if (nc <= 8) SB_CA_LAUNCH(32, 8);
+    else SB_CA_LAUNCH(32, 32);
   } else {
     if (nc <= 1) SB_CA_LAUNCH(64, 1);
     else if (nc <= 2) SB_CA_LAUNCH(64, 2);
     else if (nc <= 4) SB_CA_LAUNCH(64, 4);
-    else SB_CA_LAUNCH(64, 8);
+    else if (nc <= 8) SB_CA_LAUNCH(64, 8);
+    else SB_CA_LAUNCH(64, 32);
   }
 #undef SB_CA_LAUNCH
+  return 0;
 }
 
 }  // namespace sb

@@ -128,7 +128,13 @@ int Context::reserve(size_t bytes) {
   arena = nullptr;
   arena_bytes = 0;
   size_t want = bytes + (bytes >> 3);
-  SB_CUDA(cudaMalloc(&arena, want));
+  if (cudaMalloc(&arena, want) != cudaSuccess) {
+    (void)cudaGetLastError();
+    arena = nullptr;
+    set_error("workspace of " + std::to_string(want) + " bytes could not be allocated on the device (a smaller batch, or "
+              "no alignment output, needs less)");
+    return 1;
+  }
   arena_bytes = want;
   return 0;
 }
@@ -639,8 +645,8 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
   a.steps = 0;
   a.target_tokens = 0;
   if (B == 0 || T == 0) return 0;
-  if (T > m.max_pos || T > 256) {
-    set_error("sequence length " + std::to_string(T) + " exceeds the supported maximum of 256");
+  if (T > m.max_len()) {
+    set_error("sequence length " + std::to_string(T) + " exceeds the supported maximum of " + std::to_string(m.max_len()));
     return 1;
   }
   if (Ld < 1 || 2 * Ld > kMaxQuantOut) {
@@ -733,9 +739,19 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
   // the tiled kernel's 64-query x 128-key tiles pay off from T > 64 (mixed lengths: 15.9 -> 8.5 ms per layer of a
   // 1M-word batch); at T <= 64 with head size 64 (base) half of every tile is idle and the row-wise kernel is faster
   // (666 vs 1149 us per layer at 4096 x 32); SLIMT_B200_SELFATTN=tiled forces the tiled kernel (parity cross-check)
-  const bool attn_rowwise = (sa_env && strcmp(sa_env, "rowwise") == 0) || (T <= 64 && !(sa_env && strcmp(sa_env, "tiled") == 0));
+  const bool sa_long = sa_env && strcmp(sa_env, "long") == 0;
+  const bool attn_rowwise = (sa_env && strcmp(sa_env, "rowwise") == 0) ||
+                            (T <= 64 && !(sa_env && (strcmp(sa_env, "tiled") == 0 || sa_long)));
+  // The long kernel (self_attention_long.cu) takes what the tiled kernel cannot hold (T > 556 at head size 32, T > 400
+  // at 64) and 257 .. 384 tokens, where its 32-row score block lets two or three blocks share an SM against the tiled
+  // kernel's one: 16.5 vs 19.9 ms for the six layers of 455 x 288, 20.1 vs 22.3 ms at 341 x 384; at 256 x 512 the
+  // tiled kernel's 64-row reuse wins, 29.3 vs 30.4 ms (B200, 1000 W; profiles/r4_long_bench.jsonl).  T <= 256 routes as
+  // before.  SLIMT_B200_SELFATTN=long forces the long kernel (parity cross-check).
+  const bool attn_long = sa_long || (!attn_rowwise && !(sa_env && strcmp(sa_env, "tiled") == 0) &&
+                                     ((T > 256 && T <= 384) || !self_attention_tiled_supported(T, dh)));
   const bool attn_fused = enc_attention_supported(E, H, dh, T) &&
-                          !(sa_env && (strcmp(sa_env, "split") == 0 || strcmp(sa_env, "rowwise") == 0 || strcmp(sa_env, "tiled") == 0));
+                          !(sa_env && (strcmp(sa_env, "split") == 0 || strcmp(sa_env, "rowwise") == 0 ||
+                                       strcmp(sa_env, "tiled") == 0 || sa_long));
   CUtensorMap map_qa[3], map_qa32[3];
   if (attn_fused)
     for (int i = 0; i < 3; i++)
@@ -797,9 +813,12 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
       QuantOuts q = qouts();
       qadd(q, attn_q, L.self.o.aq);
       LaunchScope ls(c, "enc_self_attention", 0, 13.0 * R * E);
-      if (attn_rowwise ? launch_self_attention(Qb, Kb, Vb, d_lengths, B, T, H, dh, nullptr, q, s)
-                       : launch_self_attention_tiled(Qb, Kb, Vb, d_lengths, B, T, H, dh, nullptr, q, s)) {
-        set_error("self-attention: unsupported head size " + std::to_string(dh));
+      const int rc = attn_long      ? launch_self_attention_long(Qb, Kb, Vb, d_lengths, B, T, H, dh, nullptr, q, s)
+                     : attn_rowwise ? launch_self_attention(Qb, Kb, Vb, d_lengths, B, T, H, dh, nullptr, q, s)
+                                    : launch_self_attention_tiled(Qb, Kb, Vb, d_lengths, B, T, H, dh, nullptr, q, s);
+      if (rc) {
+        set_error(std::string("self-attention: the ") + (attn_long ? "long" : attn_rowwise ? "row-wise" : "tiled") +
+                  " kernel does not take head size " + std::to_string(dh) + " at sequence length " + std::to_string(T));
         return 1;
       }
     }
@@ -1095,8 +1114,12 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
         QuantOuts q = qouts();
         qadd(q, caq, L.ctx.o.aq);
         LaunchScope ls(c, "dec_cross_attention", 0, 8.0 * src_tokens * E + 5.0 * B * E);
-        launch_cross_attention(mapKc[l], mapVc[l], qd, d_lengths, B, T, H, dh, c.num_sms, nullptr, q,
-                               last ? d_align : nullptr, s);
+        if (launch_cross_attention(mapKc[l], mapVc[l], qd, d_lengths, B, T, H, dh, c.num_sms, nullptr, q,
+                                   last ? d_align : nullptr, s)) {
+          set_error("cross-attention: no kernel for " + std::to_string(H) + " heads of " + std::to_string(dh) +
+                    " over " + std::to_string(T) + " source tokens");
+          return 1;
+        }
       }
       {  // Wo + residual + LN, FFN1 + ReLU, FFN2 + residual + LN in one row-tile kernel (Modules.cc:308-316, 251-257)
         RowsFfnArgs k{};

@@ -173,7 +173,9 @@ struct Model {
   std::vector<std::unique_ptr<Context>> lanes;
   std::mutex lanes_mu;
   Context* lane(size_t i);  // lane 0 is the model's own context
-  int max_len() const { return max_pos < 256 ? max_pos : 256; }  // longest sentence a batch may hold
+  // Longest sentence a batch may hold: starts at 256 and may be raised up to max_pos (slimt_b200_model_set_max_length).
+  int len_bound = 256;
+  int max_len() const { return len_bound < max_pos ? len_bound : max_pos; }
 
   int load(Context* c, const void* bin, size_t bytes, int enc_layers, int dec_layers, int heads);
   void destroy();

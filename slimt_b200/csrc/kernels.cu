@@ -382,6 +382,7 @@ int launch_self_attention(const float* Q, const float* K, const float* V, const 
     threads -= 32;
     smem = (static_cast<size_t>(2) * T * dh + static_cast<size_t>(threads) * Tp) * sizeof(float);
   }
+  if (smem > 200 * 1024) return 1;  // K, V and one warp's score rows no longer fit: T > 533 (head size 32), T > 319 (64)
   if (dh == 32) {
     ensure_dyn_smem(self_attention_kernel<32>, smem);
     self_attention_kernel<32><<<B * H, threads, smem, stream>>>(Q, K, V, lengths, T, H, dk, out_f32, q);

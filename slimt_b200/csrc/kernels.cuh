@@ -32,14 +32,24 @@ int launch_self_attention(const float* Q, const float* K, const float* V, const 
 
 // The same operation as a register-tiled kernel (self_attention_tiled.cu): 64 query rows of one (sentence, head) per
 // block, every output still one sequential chain.  The default for every shape the fused encoder kernel does not take.
+// Returns nonzero when the shape does not fit: head sizes 32 and 64, T up to 556 (head size 32) or 400 (64), which
+// self_attention_tiled_supported tells without launching.
 int launch_self_attention_tiled(const float* Q, const float* K, const float* V, const uint32_t* lengths, int B, int T,
                                 int H, int dh, float* out_f32, QuantOuts q, cudaStream_t stream);
+bool self_attention_tiled_supported(int T, int dh);
+
+// The same operation for sentences the tiled kernel cannot hold (self_attention_long.cu): 32 query rows per block, K
+// and V streamed in 128-key tiles, the same chains and so the same bits.  Head sizes 32 and 64, T up to 1024.
+int launch_self_attention_long(const float* Q, const float* K, const float* V, const uint32_t* lengths, int B, int T,
+                               int H, int dh, float* out_f32, QuantOuts q, cudaStream_t stream);
+bool self_attention_long_supported(int T, int dh);
 
 // Decoder cross-attention for one query row per sentence over cached K,V [B][S][E] (cross_attention.cu).
 // mapK/mapV: f32 tensor maps over [B*S][E] with box {32 floats, cross_attention_box_rows(S)}, 128B swizzle.
 // attn_head0 (optional) receives head 0's probabilities [B][S] (alignment, slimt/Model.cc:84-108).
+// S <= 1024; returns nonzero for a shape it does not take (S beyond that, heads other than 8 of 32 or 64).
 int cross_attention_box_rows(int S);
-void launch_cross_attention(const CUtensorMap& mapK, const CUtensorMap& mapV, const float* Qr,
+int launch_cross_attention(const CUtensorMap& mapK, const CUtensorMap& mapV, const float* Qr,
                             const uint32_t* lengths, int B, int S, int H, int dh, int num_sms, float* out_f32,
                             QuantOuts q, float* attn_head0, cudaStream_t stream);
 

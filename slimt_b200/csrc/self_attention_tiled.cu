@@ -215,17 +215,27 @@ __global__ void __launch_bounds__(kTThreads) self_attention_tiled_kernel(
 
 }  // namespace
 
+namespace {
+size_t tiled_smem_bytes(int T, int dh) {
+  const int Tk = (T + 3) & ~3, SK = Tk + 4;
+  const size_t kv = static_cast<size_t>(std::max(dh * SK, Tk * dh));
+  return (static_cast<size_t>(dh) * (kQB + 4) + kv + static_cast<size_t>(kQB) * SK + 2 * kQB) * sizeof(float);
+}
+}  // namespace
+
+bool self_attention_tiled_supported(int T, int dh) {
+  return (dh == 32 || dh == 64) && T >= 1 && tiled_smem_bytes(T, dh) <= 220 * 1024;
+}
+
 int launch_self_attention_tiled(const float* Q, const float* K, const float* V, const uint32_t* lengths, int B, int T, int H,
                                 int dh, float* out_f32, QuantOuts q, cudaStream_t stream) {
   if (B == 0) return 0;
   // 1/sqrt(dim_head) evaluated in double then narrowed, as `1.0F / std::sqrt(size_t)` does (Modules.cc:43)
   const float dk = static_cast<float>(1.0 / std::sqrt(static_cast<double>(dh)));
   const int n_qb = (T + kQB - 1) / kQB;
-  const int Tk = (T + 3) & ~3, SK = Tk + 4;
-  const size_t kv = static_cast<size_t>(std::max(dh * SK, Tk * dh));
-  const size_t smem = (static_cast<size_t>(dh) * (kQB + 4) + kv + static_cast<size_t>(kQB) * SK + 2 * kQB) * sizeof(float);
+  const size_t smem = tiled_smem_bytes(T, dh);
   const long blocks = static_cast<long>(B) * H * n_qb;
-  if (smem > 220 * 1024 || blocks > 0x7fffffffL) return 1;
+  if (!self_attention_tiled_supported(T, dh) || blocks > 0x7fffffffL) return 1;
   if (dh == 32) {
     if (ensure_dyn_smem(self_attention_tiled_kernel<32>, smem) != cudaSuccess) return 1;
     self_attention_tiled_kernel<32><<<static_cast<unsigned>(blocks), kTThreads, smem, stream>>>(Q, K, V, lengths, T, H, n_qb, dk, out_f32, q);

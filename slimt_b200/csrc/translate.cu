@@ -117,11 +117,14 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
       plan.push_back(std::move(p));
     }
   }
-  // nothing has touched a GPU yet: a sentence no kernel can take fails the request as a whole, before any batch ran
+  // nothing has touched a GPU yet: a sentence no kernel can take fails the request as a whole, before any batch ran.
+  // Any replica may serve any batch, so the smallest bound of them all applies.
+  int max_len = m0.max_len();
+  for (size_t r = 1; r < n_rep; r++) max_len = std::min(max_len, models[r]->max_len());
   for (const Plan& p : plan) {
-    if (p.width > static_cast<size_t>(m0.max_len())) {
+    if (p.width > static_cast<size_t>(max_len)) {
       set_error("translate: a sentence of " + std::to_string(p.width) + " tokens exceeds the supported maximum of " +
-                std::to_string(m0.max_len()) + " (wrap longer input first: TextProcessor's wrap_length)");
+                std::to_string(max_len) + " (wrap longer input first: TextProcessor's wrap_length)");
       return 1;
     }
   }

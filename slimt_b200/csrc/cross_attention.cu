@@ -28,7 +28,7 @@ template <int DH, int H, int NC>
 __global__ void __launch_bounds__((H + 1) * 32, 3)
     cross_attention_kernel(const __grid_constant__ CUtensorMap mapK, const __grid_constant__ CUtensorMap mapV,
                            const float* __restrict__ Qr, const uint32_t* __restrict__ lengths, int B, int S,
-                           int box_rows, int stages, float dk, float* __restrict__ out_f32, QuantOuts q,
+                           int box_rows, int stages, float dk, QuantOuts q,
                            float* __restrict__ attn_head0) {
   constexpr int E = H * DH;
   constexpr int kSub = DH / 32;  // 128-byte column tiles per head
@@ -216,7 +216,6 @@ __global__ void __launch_bounds__((H + 1) * 32, 3)
     const size_t off = static_cast<size_t>(b) * E + h * DH;
 #pragma unroll
     for (int u = 0; u < kSub; u++) {
-      if (out_f32) out_f32[off + u * 32 + lane] = acc[u];
       for (int k = 0; k < q.n; k++) q.ptr[k][off + u * 32 + lane] = static_cast<int8_t>(quantize1(acc[u], q.aq[k]));
     }
   }
@@ -227,7 +226,7 @@ __global__ void __launch_bounds__((H + 1) * 32, 3)
 int cross_attention_box_rows(int S) { return S >= 32 ? 32 : ((S + 7) & ~7); }
 
 int launch_cross_attention(const CUtensorMap& mapK, const CUtensorMap& mapV, const float* Qr, const uint32_t* lengths,
-                           int B, int S, int H, int dh, int num_sms, float* out_f32, QuantOuts q, float* attn_head0,
+                           int B, int S, int H, int dh, int num_sms, QuantOuts q, float* attn_head0,
                            cudaStream_t stream) {
   if (B == 0) return 0;
   if (S > 32 * kMaxKeyChunks || H != 8 || (dh != 32 && dh != 64)) return 1;
@@ -251,7 +250,7 @@ int launch_cross_attention(const CUtensorMap& mapK, const CUtensorMap& mapV, con
   do {                                                                                                           \
     auto kern = cross_attention_kernel<DH_, 8, NC_>;                                                             \
     if (ensure_dyn_smem(kern, smem) != cudaSuccess) return 1;                                                    \
-    kern<<<grid, threads, smem, stream>>>(mapK, mapV, Qr, lengths, B, S, box_rows, stages, dk, out_f32, q,      \
+    kern<<<grid, threads, smem, stream>>>(mapK, mapV, Qr, lengths, B, S, box_rows, stages, dk, q,               \
                                           attn_head0);                                                           \
   } while (0)
   if (dh == 32) {

@@ -118,16 +118,6 @@ __global__ void __launch_bounds__(kThreadsRc, 1) cross_attention_rc_kernel(const
   __syncthreads();
   tc_fence_after();
   pdl_launch_dependents();
-  // Wk and Wv never change: request them before waiting for the preceding kernel, so that the 128 KB arrive while
-  // it drains.
-  if (SB_PRE_CROSS && warp == 0 && elect_one()) {
-    mbar_expect_tx(w_full, 128 * 1024);
-    for (int kb = 0; kb < 2; kb++)
-      for (int half = 0; half < 2; half++) {
-        tma_load_2d(s_wk + kb * 32768 + half * 16384, &a.map_wk, w_full, kb * 128, half * 128);
-        tma_load_2d(s_wv + kb * 32768 + half * 16384, &a.map_wv, w_full, kb * 128, half * 128);
-      }
-  }
   pdl_wait();  // everything above overlapped the previous kernel's tail; its outputs are visible from here on
   const uint32_t tmem = *tmem_slot;
   const uint32_t tmem_k = tmem;         // 256 columns: features
@@ -138,14 +128,12 @@ __global__ void __launch_bounds__(kThreadsRc, 1) cross_attention_rc_kernel(const
   if (warp == 0) {
     // ===== TMA producer
     if (elect_one()) {
-      if (!SB_PRE_CROSS) {
-        mbar_expect_tx(w_full, 128 * 1024);
-        for (int kb = 0; kb < 2; kb++)
-          for (int half = 0; half < 2; half++) {
-            tma_load_2d(s_wk + kb * 32768 + half * 16384, &a.map_wk, w_full, kb * 128, half * 128);
-            tma_load_2d(s_wv + kb * 32768 + half * 16384, &a.map_wv, w_full, kb * 128, half * 128);
-          }
-      }
+      mbar_expect_tx(w_full, 128 * 1024);
+      for (int kb = 0; kb < 2; kb++)
+        for (int half = 0; half < 2; half++) {
+          tma_load_2d(s_wk + kb * 32768 + half * 16384, &a.map_wk, w_full, kb * 128, half * 128);
+          tma_load_2d(s_wv + kb * 32768 + half * 16384, &a.map_wv, w_full, kb * 128, half * 128);
+        }
       uint32_t it = 0;
       for (int g = blockIdx.x; g < n_groups; g += gridDim.x, it++) {
         const uint32_t ph = it & 1;
@@ -464,7 +452,6 @@ __global__ void __launch_bounds__(kThreadsRc, 1) cross_attention_rc_kernel(const
         if (lane == 0) mbar_arrive(v_drained);
         auto emit = [&](int b, float acc) {
           const size_t off = static_cast<size_t>(b) * kE + v_feat;
-          if (a.out_f32) a.out_f32[off] = acc;
           // the usual case is one consumer (Wo): constant indices keep its multiplier and pointer in the constant bank
           if (a.qo.n == 1) a.qo.ptr[0][off] = static_cast<int8_t>(quantize<kFast>(acc, a.qo.aq[0]));
           else

@@ -367,7 +367,6 @@ __global__ void __launch_bounds__(kThreadsL, 1) cross_attention_rcl_kernel(const
           }
         }
         const size_t off = static_cast<size_t>(b) * kE + v_feat;
-        if (a.out_f32) a.out_f32[off] = acc;
         if (a.qo.n == 1) a.qo.ptr[0][off] = static_cast<int8_t>(quantize<false>(acc, a.qo.aq[0]));
         else
           for (int k = 0; k < a.qo.n; k++) a.qo.ptr[k][off] = static_cast<int8_t>(quantize<false>(acc, a.qo.aq[k]));

@@ -15,8 +15,8 @@
 // accumulators are in registers, so the projections of the next heads overlap the attention arithmetic.
 //
 // Supported: E = 256, 8 heads of 32, T <= 64 (scores are kept in registers).  Everything else takes the split path.
+// enc_attention_kernel below takes 33 <= T <= 64; enc_attention_warp_kernel, further down, takes T <= 32.
 #include <stdio.h>
-#include <string.h>
 
 #include "exact_math.cuh"
 #include "kernels.cuh"
@@ -32,6 +32,7 @@ constexpr int kWStages = 2;
 constexpr int kSlots = 2;
 constexpr int kConsWarps = 4 * kSlots;
 constexpr int kThreadsEa = 128 + 32 * kConsWarps;  // warp0 TMA, warp1 MMA, warp2 TMEM alloc, warp3 tables, 4.. consumers
+constexpr int kTMax = 64;                          // longest sentence enc_attention_kernel holds
 constexpr int kStride = 36;                        // floats per staged K / V row: 16-byte aligned, conflict-free
 constexpr int kStageRows = kTileRows + 4;          // the score loop reads keys in groups of four
 constexpr int kStageBytes = kStageRows * kStride * 4;
@@ -50,7 +51,6 @@ struct Smem {
 };
 static_assert(Smem::total <= 227 * 1024, "shared memory budget");
 
-template <int TMAX>
 __global__ void __launch_bounds__(kThreadsEa, 1) enc_attention_kernel(const __grid_constant__ EncAttnArgs a) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = smem_align1024(smem_raw);
@@ -218,10 +218,10 @@ __global__ void __launch_bounds__(kThreadsEa, 1) enc_attention_kernel(const __gr
         }
 
         // scores: four keys at a time (independent chains); each chain is the reference's sequential fma order
-        float S[TMAX];
+        float S[kTMax];
         float mx = ninf;
 #pragma unroll
-        for (int j0 = 0; j0 < TMAX; j0 += 4) {
+        for (int j0 = 0; j0 < kTMax; j0 += 4) {
           if (j0 < wmax) {
             const float* kp = Ks + (krow0 + j0) * kStride;
             float s0 = 0.0f, s1 = 0.0f, s2 = 0.0f, s3 = 0.0f;
@@ -248,7 +248,7 @@ __global__ void __launch_bounds__(kThreadsEa, 1) enc_attention_kernel(const __gr
         // softmax (TensorOps.cc:282-315): exp(s - max), sum in key order; masked keys contribute exactly +0
         float sum = 0.0f;
 #pragma unroll
-        for (int j0 = 0; j0 < TMAX; j0 += 4) {
+        for (int j0 = 0; j0 < kTMax; j0 += 4) {
           if (j0 < wmax) {
 #pragma unroll
             for (int u = 0; u < 4; u++) {
@@ -265,7 +265,7 @@ __global__ void __launch_bounds__(kThreadsEa, 1) enc_attention_kernel(const __gr
         const float sum_rcp = rcp_refined(sum);
         const float sum_lo = div_guard_lo(sum);
 #pragma unroll
-        for (int j0 = 0; j0 < TMAX; j0 += 4) {
+        for (int j0 = 0; j0 < kTMax; j0 += 4) {
           if (j0 < wmax) {
 #pragma unroll
             for (int u = 0; u < 4; u++) {
@@ -305,291 +305,11 @@ __global__ void __launch_bounds__(kThreadsEa, 1) enc_attention_kernel(const __gr
   if (warp == 2) tmem_dealloc<512>(tmem);
 }
 
-
 // ---------------------------------------------------------------------------------------------------------------------
-// Second generation for T <= 32: TWO threads per query row.  The kernel above gives a query row to one thread, which
-// then holds q[32], the row's 32 scores and 32 accumulators (159 registers): two consumer warps per scheduler, too few
-// to hide the latency of the broadcast shared-memory loads the inner loops live on.  Here the pair (same TMEM lane, warps
-// w and w + 4 of an eight-warp slot) splits the KEYS for the scores (16 each) and the head's DIMS for the weighted sum
-// (16 each): half the per-thread state, sixteen consumer warps.  No chain is reordered -- a score is still one thread's
-// fma chain over d, an output still one thread's chain over the keys in order, the row sum is formed by both threads
-// over ALL keys in key order (masked keys add exactly +0, as in the reference) -- so the result is bit-identical.
-// What the pair exchanges goes through shared memory: the two partial maxima, and the exponentials, which take the
-// place of the K tile once every score of the head is formed.
-constexpr int kPairWarps = 16;
-constexpr int kThreadsPair = 128 + 32 * kPairWarps;
-
-struct SmemPair {
-  static constexpr int mx = Smem::tmem_slot + 16;                  // f32 [2 slots][128 rows][2 halves]
-  static constexpr int total = mx + kSlots * kTileRows * 2 * 4 + 1024;
-};
-static_assert(SmemPair::total <= 227 * 1024, "shared memory budget");
-
-__global__ void __launch_bounds__(kThreadsPair, 1) enc_attention_pair_kernel(const __grid_constant__ EncAttnArgs a) {
-  constexpr int TH = 16;  // keys per thread of a pair
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = smem_align1024(smem_raw);
-  uint8_t* s_a = smem + Smem::a;
-  uint8_t* s_w = smem + Smem::w;
-  float* s_pb = reinterpret_cast<float*>(smem + Smem::pb);
-  uint64_t* exp_tab = reinterpret_cast<uint64_t*>(smem + Smem::exp_tab);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Smem::bars);
-  uint64_t* a_full = bars;
-  uint64_t* a_free = bars + 1;
-  uint64_t* w_full = bars + 2;
-  uint64_t* w_free = w_full + kWStages;
-  uint64_t* acc_full = w_free + kWStages;
-  uint64_t* acc_free = acc_full + 4;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + Smem::tmem_slot);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&a.map_aq), tma_prefetch_desc(&a.map_ak), tma_prefetch_desc(&a.map_av);
-    tma_prefetch_desc(&a.map_wq), tma_prefetch_desc(&a.map_wk), tma_prefetch_desc(&a.map_wv);
-  }
-  if (warp == 1 && lane == 0) {
-    mbar_init(a_full, 1), mbar_init(a_free, 1);
-    for (int i = 0; i < kWStages; i++) mbar_init(&w_full[i], 1), mbar_init(&w_free[i], 1);
-    for (int i = 0; i < 4; i++) mbar_init(&acc_full[i], 1), mbar_init(&acc_free[i], 8);
-    fence_barrier_init();
-  }
-  if (warp == 2) tmem_alloc<512>(tmem_slot);
-  if (warp == 3) {
-    exp_tab[lane] = kExp2fTab[lane];
-    for (int i = lane; i < kE; i += 32) {
-      s_pb[i] = a.pb_q[i];
-      s_pb[kE + i] = a.pb_k[i];
-      s_pb[2 * kE + i] = a.pb_v[i];
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  pdl_launch_dependents();
-  pdl_wait();  // the previous kernel's outputs (the quantised x copies) are visible from here on
-  const uint32_t tmem = *tmem_slot;
-
-  const int T = a.T;
-  const int G = kTileRows / T;  // whole sentences per tile
-  const int n_tiles = (a.B + G - 1) / G;
-
-  if (warp == 0) {
-    // ===== TMA producer (as in enc_attention_kernel)
-    if (elect_one()) {
-      const CUtensorMap* map_a[3] = {&a.map_aq, &a.map_ak, &a.map_av};
-      const CUtensorMap* map_w[3] = {&a.map_wq, &a.map_wk, &a.map_wv};
-      uint32_t hc = 0, it = 0;
-      for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, it++) {
-        const int row0 = tile * G * T;
-        mbar_wait(a_free, (it & 1) ^ 1);
-        mbar_expect_tx(a_full, 3 * 32768);
-        for (int m = 0; m < 3; m++)
-          for (int kb = 0; kb < 2; kb++) tma_load_2d(s_a + m * 32768 + kb * 16384, map_a[m], a_full, kb * 128, row0);
-        for (int h = 0; h < kH; h++, hc++) {
-          const uint32_t s = hc % kWStages, ph = (hc / kWStages) & 1;
-          mbar_wait(&w_free[s], ph ^ 1);
-          mbar_expect_tx(&w_full[s], 24576);
-          for (int m = 0; m < 3; m++)
-            for (int kb = 0; kb < 2; kb++)
-              tma_load_2d(s_w + s * 24576 + m * 8192 + kb * 4096, map_w[m], &w_full[s], kb * 128, h * kDH);
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ===== MMA issuer (as in enc_attention_kernel)
-    if (elect_one()) {
-      constexpr uint32_t idesc = make_idesc_i8(kTileRows, kDH);
-      uint32_t hc = 0, it = 0;
-      for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, it++) {
-        mbar_wait(a_full, it & 1);
-        for (int h = 0; h < kH; h++, hc++) {
-          const uint32_t s = hc % kWStages;
-          const uint32_t reg = hc & 3;
-          mbar_wait(&w_full[s], (hc / kWStages) & 1);
-          mbar_wait(&acc_free[reg], ((hc >> 2) & 1) ^ 1);
-          tc_fence_after();
-#pragma unroll
-          for (int m = 0; m < 3; m++) {
-#pragma unroll
-            for (int kb = 0; kb < 2; kb++) {
-              const uint64_t da = make_kmajor_sw128_desc(smem_u32(s_a + m * 32768 + kb * 16384));
-              const uint64_t db = make_kmajor_sw128_desc(smem_u32(s_w + s * 24576 + m * 8192 + kb * 4096));
-#pragma unroll
-              for (int k = 0; k < 4; k++) umma_i8(tmem + reg * 128 + m * 32, da + 2 * k, db + 2 * k, idesc, (kb | k) ? 1u : 0u);
-            }
-          }
-          umma_commit(&w_free[s]);
-          umma_commit(&acc_full[reg]);
-        }
-        umma_commit(a_free);
-      }
-    }
-  } else if (warp >= 4) {
-    // ===== consumers: (query row, half) per thread
-    const int cw = warp - 4;
-    const int slot = cw >> 3;
-    const int half = (cw >> 2) & 1;
-    const int qd = warp & 3;
-    const int r = qd * 32 + lane;
-    const uint32_t lane_sel = static_cast<uint32_t>(qd * 32) << 16;
-    float* Ks = reinterpret_cast<float*>(smem + Smem::kv + slot * 2 * kStageBytes);
-    float* Vs = Ks + kStageRows * kStride;
-    float* prow = Ks + r * kStride;  // the row's exponentials take the K tile's place once the head's scores are formed
-    float* s_mx = reinterpret_cast<float*>(smem + SmemPair::mx) + (slot * kTileRows + r) * 2;
-    const uint32_t slot_bar = 1 + slot, pair_bar = 3 + slot * 4 + qd;
-    const float ninf = -3.402823466e+38f;
-    const int kbase = half * TH, d0 = half * 16;
-    uint32_t it = 0;
-    for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, it++) {
-      const int j = r / T, i = r - j * T;
-      const int b = tile * G + j;
-      const bool sent_ok = j < G && b < a.B;
-      const int len = sent_ok ? min(static_cast<int>(__ldg(a.lengths + b)), T) : 0;
-      const int krow0 = sent_ok ? j * T : 0;
-      int wmax = len;
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) wmax = max(wmax, __shfl_xor_sync(0xffffffffu, wmax, o));
-      const bool row_live = sent_ok && i < len;
-      uint8_t* out_row = a.out_q + (static_cast<size_t>(tile) * G * T + r) * kE;
-
-#pragma unroll 1
-      for (int hh = 0; hh < kH / kSlots; hh++) {
-        const int h = hh * kSlots + slot;
-        const uint32_t reg = h & 3;
-        const uint32_t use = it * 2 + (h >> 2);
-        float q[kDH];
-        {
-          uint32_t vq[32], vx[32];
-          mbar_wait(&acc_full[reg], use & 1);
-          tc_fence_after();
-          const uint32_t taddr = tmem + lane_sel + reg * 128;
-          tmem_ld32_nowait(taddr + (half ? 64 : 32), vx);  // half 0 stages the K rows, half 1 the V rows
-          tmem_ld32_nowait(taddr, vq);
-          tmem_ld_wait();
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&acc_free[reg]);
-          named_bar_sync(slot_bar, 256);  // the slot is done reading the previous head's V and probabilities
-          const float* pbx = s_pb + (half ? 2 * kE : kE) + h * kDH;
-          const float umx = half ? a.um_v : a.um_k;
-          float* xr = (half ? Vs : Ks) + r * kStride;
-#pragma unroll
-          for (int d = 0; d < kDH; d += 4) {
-            const float4 px = *reinterpret_cast<const float4*>(pbx + d);
-            *reinterpret_cast<float4*>(xr + d) =
-                make_float4(dequant1(static_cast<int>(vx[d]), umx, px.x), dequant1(static_cast<int>(vx[d + 1]), umx, px.y),
-                            dequant1(static_cast<int>(vx[d + 2]), umx, px.z), dequant1(static_cast<int>(vx[d + 3]), umx, px.w));
-          }
-          const float* pbq = s_pb + h * kDH;
-#pragma unroll
-          for (int d = 0; d < kDH; d += 4) {
-            const float4 pq = *reinterpret_cast<const float4*>(pbq + d);
-            q[d] = dequant1(static_cast<int>(vq[d]), a.um_q, pq.x);
-            q[d + 1] = dequant1(static_cast<int>(vq[d + 1]), a.um_q, pq.y);
-            q[d + 2] = dequant1(static_cast<int>(vq[d + 2]), a.um_q, pq.z);
-            q[d + 3] = dequant1(static_cast<int>(vq[d + 3]), a.um_q, pq.w);
-          }
-          named_bar_sync(slot_bar, 256);  // K and V of every row of the tile are staged
-        }
-
-        // scores of this half's keys: four keys at a time (independent chains), each the reference's fma order
-        float S[TH];
-        float mx = ninf;
-#pragma unroll
-        for (int j0 = 0; j0 < TH; j0 += 4) {
-          const int jk = kbase + j0;
-          if (jk < wmax) {
-            const float* kp = Ks + (krow0 + jk) * kStride;
-            float s0 = 0.0f, s1 = 0.0f, s2 = 0.0f, s3 = 0.0f;
-#pragma unroll
-            for (int d = 0; d < kDH; d += 4) {
-              const float4 k0 = *reinterpret_cast<const float4*>(kp + d);
-              const float4 k1 = *reinterpret_cast<const float4*>(kp + kStride + d);
-              const float4 k2 = *reinterpret_cast<const float4*>(kp + 2 * kStride + d);
-              const float4 k3 = *reinterpret_cast<const float4*>(kp + 3 * kStride + d);
-              s0 = fmaf(q[d], k0.x, s0), s1 = fmaf(q[d], k1.x, s1), s2 = fmaf(q[d], k2.x, s2), s3 = fmaf(q[d], k3.x, s3);
-              s0 = fmaf(q[d + 1], k0.y, s0), s1 = fmaf(q[d + 1], k1.y, s1), s2 = fmaf(q[d + 1], k2.y, s2), s3 = fmaf(q[d + 1], k3.y, s3);
-              s0 = fmaf(q[d + 2], k0.z, s0), s1 = fmaf(q[d + 2], k1.z, s1), s2 = fmaf(q[d + 2], k2.z, s2), s3 = fmaf(q[d + 2], k3.z, s3);
-              s0 = fmaf(q[d + 3], k0.w, s0), s1 = fmaf(q[d + 3], k1.w, s1), s2 = fmaf(q[d + 3], k2.w, s2), s3 = fmaf(q[d + 3], k3.w, s3);
-            }
-            S[j0] = jk < len ? __fmul_rn(a.dk, s0) : ninf;
-            S[j0 + 1] = jk + 1 < len ? __fmul_rn(a.dk, s1) : ninf;
-            S[j0 + 2] = jk + 2 < len ? __fmul_rn(a.dk, s2) : ninf;
-            S[j0 + 3] = jk + 3 < len ? __fmul_rn(a.dk, s3) : ninf;
-            mx = fmaxf(fmaxf(fmaxf(mx, S[j0]), fmaxf(S[j0 + 1], S[j0 + 2])), S[j0 + 3]);
-          } else {
-            S[j0] = S[j0 + 1] = S[j0 + 2] = S[j0 + 3] = ninf;
-          }
-        }
-        // the row maximum is the larger of the pair's two
-        s_mx[half] = mx;
-        named_bar_sync(pair_bar, 64);
-        mx = fmaxf(s_mx[0], s_mx[1]);
-        // exp(s - max) of this half's keys; masked keys contribute exactly +0 (TensorOps.cc:282-315)
-#pragma unroll
-        for (int u = 0; u < TH; u++) S[u] = kbase + u < len ? expf_glibc_nonpos_tab(__fsub_rn(S[u], mx), exp_tab) : 0.0f;
-        named_bar_sync(slot_bar, 256);  // every score of the head is formed: the K tile may be overwritten
-#pragma unroll
-        for (int u = 0; u < TH; u += 4) *reinterpret_cast<float4*>(prow + kbase + u) = make_float4(S[u], S[u + 1], S[u + 2], S[u + 3]);
-        named_bar_sync(pair_bar, 64);
-        // the row sum over ALL keys in key order, by both threads of the pair
-        float sum = 0.0f;
-#pragma unroll
-        for (int j0 = 0; j0 < 2 * TH; j0 += 4) {
-          const float4 e4 = *reinterpret_cast<const float4*>(prow + j0);
-          sum = __fadd_rn(__fadd_rn(__fadd_rn(__fadd_rn(sum, e4.x), e4.y), e4.z), e4.w);
-        }
-        // weighted sum of V over the keys in order, this half's sixteen dims
-        float acc[16];
-#pragma unroll
-        for (int d = 0; d < 16; d++) acc[d] = 0.0f;
-        const float sum_rcp = rcp_refined(sum);
-        const float sum_lo = div_guard_lo(sum);
-#pragma unroll
-        for (int j0 = 0; j0 < 2 * TH; j0 += 4) {
-          if (j0 < wmax) {
-            const float4 e4 = *reinterpret_cast<const float4*>(prow + j0);
-            const float ev[4] = {e4.x, e4.y, e4.z, e4.w};
-#pragma unroll
-            for (int u = 0; u < 4; u++) {
-              if (j0 + u < wmax) {
-                const float p = j0 + u < len ? div_by_rcp(ev[u], sum, sum_rcp, sum_lo) : 0.0f;
-                const float* vp = Vs + (krow0 + j0 + u) * kStride + d0;
-#pragma unroll
-                for (int d = 0; d < 16; d += 4) {
-                  const float4 v4 = *reinterpret_cast<const float4*>(vp + d);
-                  acc[d] = fmaf(p, v4.x, acc[d]);
-                  acc[d + 1] = fmaf(p, v4.y, acc[d + 1]);
-                  acc[d + 2] = fmaf(p, v4.z, acc[d + 2]);
-                  acc[d + 3] = fmaf(p, v4.w, acc[d + 3]);
-                }
-              }
-            }
-          }
-        }
-        if (sent_ok) {
-          // padded query rows never reach a valid output; like the split path they carry quantize(0)
-          uint32_t wq[4];
-#pragma unroll
-          for (int d = 0; d < 16; d += 4)
-            wq[d >> 2] = row_live ? pack4(quantize1(acc[d], a.aq_out), quantize1(acc[d + 1], a.aq_out),
-                                          quantize1(acc[d + 2], a.aq_out), quantize1(acc[d + 3], a.aq_out))
-                                  : 0x7f7f7f7fu;
-          *reinterpret_cast<uint4*>(out_row + h * kDH + d0) = make_uint4(wq[0], wq[1], wq[2], wq[3]);
-        }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  if (warp == 2) tmem_dealloc<512>(tmem);
-}
-
-// ---------------------------------------------------------------------------------------------------------------------
-// Third generation for T <= 32: one WARP per (sentence, head), register-tiled.  In the kernels above every K and V
-// element reaches a thread as a broadcast 16-byte shared-memory load that feeds four FMAs, and that load -- eight issue
-// cycles per scheduler -- is what the inner loops cost.  Here a tile is four sentences, each in its own 32-row slot of
+// T <= 32: one WARP per (sentence, head), register-tiled.  In the kernel above every K and V element reaches a thread
+// as a broadcast 16-byte shared-memory load that feeds four FMAs, and that load -- eight issue cycles per scheduler --
+// is what the inner loops cost.  At T <= 32 this kernel takes 241 us per layer, where one thread per query row took 347
+// and two threads per row 313 (DESIGN.md 4.3).  Here a tile is four sentences, each in its own 32-row slot of
 // the A operands (its own TMA box), so TMEM lane quadrant qd = sentence qd and the warp that drains a quadrant owns the
 // whole attention of that sentence for the head: no barrier wider than the warp.  The warp parks Q and K transposed
 // ([d][row], conflict-free scalar stores), then works like a register-tiled SGEMM whose every output is still ONE
@@ -599,7 +319,7 @@ __global__ void __launch_bounds__(kThreadsPair, 1) enc_attention_pair_kernel(con
 //            elementwise, the row sum handed from lane to lane so that it is one chain in key order, p = e / sum;
 //   P V      P parked transposed in K's place, V (drained from TMEM only now) in Q's place; thread = 4 queries x 8 dims,
 //            three loads per 32 FMAs, chains over the valid keys in order (a masked key adds exactly +0: skipped).
-// Bit-identical to the kernels above and to the split path (test_fused_encoder_attention_equals_split_path).
+// Bit-identical to the kernel above and to the split path (test_fused_encoder_attention_equals_split_path).
 // Twelve consumer warps (three per scheduler: the phases of a unit are latency chains, the third warp fills their gaps)
 // take the CTA's (tile, head) units round-robin.  That many staging tiles only fit because they are unpadded
 // ([32][32] floats with XOR-swizzled 16-byte chunks where a padded row used to avoid the bank conflicts) and the weight
@@ -918,38 +638,23 @@ __global__ void __launch_bounds__(kThreadsW, 1) enc_attention_warp_kernel(const 
   if (warp == 2) tmem_dealloc<512>(tmem);
 }
 
-template <int TMAX>
-int launch_t(const EncAttnArgs& a, int grid, cudaStream_t stream) {
-  auto kern = enc_attention_kernel<TMAX>;
-  if (ensure_dyn_smem(kern, Smem::total) != cudaSuccess) return 1;
-  return launch_pdl(kern, dim3(grid), dim3(kThreadsEa), Smem::total, stream, a) != cudaSuccess;
-}
-
 }  // namespace
 
-bool enc_attention_supported(int E, int H, int dh, int T) { return E == kE && H == kH && dh == kDH && T >= 1 && T <= 64; }
+bool enc_attention_supported(int E, int H, int dh, int T) { return E == kE && H == kH && dh == kDH && T >= 1 && T <= kTMax; }
 
 int launch_enc_attention(const EncAttnArgs& a, int num_sms, cudaStream_t stream) {
   if (a.B == 0) return 0;
-  const int G = kTileRows / a.T;
-  const int tiles = (a.B + G - 1) / G;
-  const int grid = tiles < num_sms ? tiles : num_sms;
-  static const int variant = [] {
-    const char* e = getenv("SLIMT_B200_ENCATTN");  // =single / =pair keep the earlier T <= 32 kernels (A/B, cross-check)
-    return e && strcmp(e, "single") == 0 ? 1 : e && strcmp(e, "pair") == 0 ? 2 : 0;
-  }();
-  const bool single = variant == 1;
-  if (a.T <= 32 && variant == 0) {
-    const int tiles4 = (a.B + 3) / 4;
+  if (a.T <= 32) {
+    const int tiles = (a.B + 3) / 4;
     if (ensure_dyn_smem(enc_attention_warp_kernel, SmemW::total) != cudaSuccess) return 1;
-    return launch_pdl(enc_attention_warp_kernel, dim3(tiles4 < num_sms ? tiles4 : num_sms), dim3(kThreadsW), SmemW::total, stream,
+    return launch_pdl(enc_attention_warp_kernel, dim3(tiles < num_sms ? tiles : num_sms), dim3(kThreadsW), SmemW::total, stream,
                       a) != cudaSuccess;
   }
-  if (a.T <= 32 && !single) {
-    if (ensure_dyn_smem(enc_attention_pair_kernel, SmemPair::total) != cudaSuccess) return 1;
-    return launch_pdl(enc_attention_pair_kernel, dim3(grid), dim3(kThreadsPair), SmemPair::total, stream, a) != cudaSuccess;
-  }
-  return a.T <= 32 ? launch_t<32>(a, grid, stream) : launch_t<64>(a, grid, stream);
+  const int G = kTileRows / a.T;
+  const int tiles = (a.B + G - 1) / G;
+  if (ensure_dyn_smem(enc_attention_kernel, Smem::total) != cudaSuccess) return 1;
+  return launch_pdl(enc_attention_kernel, dim3(tiles < num_sms ? tiles : num_sms), dim3(kThreadsEa), Smem::total, stream, a) !=
+         cudaSuccess;
 }
 
 }  // namespace sb

@@ -524,7 +524,6 @@ struct GemmCall {
       if (epi == EPI_F32 || epi == EPI_ACC) out_bytes += 4 * M * N;
       if (epi == EPI_QUANT) out_bytes += M * N;
       if (epi == EPI_RES_LN) out_bytes += 4 * M * N + (p.out ? 4 * M * N : 0) + p.n_qout * M * N;
-      if (epi == EPI_ARGMAX) out_bytes += 8 * M;
     }
     LaunchScope ls(*c, tag, 2.0 * M * N * K * n, n * (M * K + N * K) + out_bytes);
     launch_gemm_i8(b, n, epi, bn, c->stream);
@@ -627,6 +626,67 @@ int qmm_affine_host(Context& c, const float* x, size_t M, size_t K, const int8_t
   }
   return 0;
 }
+
+// ------------------------------------------------------------------ kernel routes
+namespace {
+
+enum class SelfAttn { Fused, Rowwise, Tiled, Long };
+enum class Cross { Cached, Rc, Rcl };
+
+const char* route_name(SelfAttn r) {
+  switch (r) {
+    case SelfAttn::Fused: return "Fused";
+    case SelfAttn::Rowwise: return "Rowwise";
+    case SelfAttn::Tiled: return "Tiled";
+    case SelfAttn::Long: return "Long";
+  }
+  return "?";
+}
+
+struct Routes {
+  SelfAttn self;
+  Cross cross;
+};
+
+// Which kernel runs the encoder's self-attention and the decoder's cross-attention for one forward call.  The two
+// environment variables are read on every call, so that tests can switch kernels between calls; a value not listed
+// below means the default.
+Routes choose_routes(int E, int H, int dh, int T, int B, bool fast) {
+  auto env_is = [](const char* env, const char* v) { return env != nullptr && strcmp(env, v) == 0; };
+  Routes r{};
+  // SLIMT_B200_SELFATTN = split keeps the projections and the attention as separate kernels; rowwise | tiled | long
+  // also force that attention kernel (parity cross-checks)
+  const char* sa = getenv("SLIMT_B200_SELFATTN");
+  if (env_is(sa, "rowwise")) r.self = SelfAttn::Rowwise;
+  else if (env_is(sa, "tiled")) r.self = SelfAttn::Tiled;
+  else if (env_is(sa, "long")) r.self = SelfAttn::Long;
+  else if (!env_is(sa, "split") && enc_attention_supported(E, H, dh, T)) r.self = SelfAttn::Fused;
+  // the tiled kernel's 64-query x 128-key tiles pay off from T > 64 (mixed lengths: 15.9 -> 8.5 ms per layer of a
+  // 1M-word batch); at T <= 64 with head size 64 (base) half of every tile is idle and the row-wise kernel is faster
+  // (666 vs 1149 us per layer at 4096 x 32)
+  else if (T <= 64) r.self = SelfAttn::Rowwise;
+  // The long kernel (self_attention_long.cu) takes what the tiled kernel cannot hold (T > 556 at head size 32, T > 400
+  // at 64) and 257 .. 384 tokens, where its 32-row score block lets two or three blocks share an SM against the tiled
+  // kernel's one: 16.5 vs 19.9 ms for the six layers of 455 x 288, 20.1 vs 22.3 ms at 341 x 384; at 256 x 512 the
+  // tiled kernel's 64-row reuse wins, 29.3 vs 30.4 ms (B200, 1000 W; profiles/r4_long_bench.jsonl).
+  else if ((T > 256 && T <= 384) || !self_attention_tiled_supported(T, dh)) r.self = SelfAttn::Long;
+  else r.self = SelfAttn::Tiled;
+
+  // Cross-attention K/V: the reference re-projects them every step (Modules.cc:244-249); so do the recompute kernels
+  // (tensor cores, from the u8 encoder output); the cached kernel reads them projected once.  Small batches take the
+  // cached kernel: below ~4 k source tokens the recompute kernel has fewer sentence groups than SMs and its launch is
+  // all latency (64 x 32: 8.6 us cached against 12.8 us recomputed per launch, 5.40 -> 5.13 ms per batch; the two are
+  // bit-identical).  SLIMT_B200_CROSS = cached | rc overrides the choice (tests, A/B runs).
+  const char* ca = getenv("SLIMT_B200_CROSS");
+  if (env_is(ca, "cached") || (!env_is(ca, "rc") && static_cast<long>(B) * T <= 4096)) r.cross = Cross::Cached;
+  else if (cross_attention_rc_supported(E, H, dh, T)) r.cross = Cross::Rc;
+  // long sentences (65 .. 256 tokens) take the sentence-at-a-time recompute kernel (cross_attention_rcl.cu; bit-exact mode)
+  else if (!fast && cross_attention_rcl_supported(E, H, dh, T)) r.cross = Cross::Rcl;
+  else r.cross = Cross::Cached;
+  return r;
+}
+
+}  // namespace
 
 // ------------------------------------------------------------------ Model::forward
 int model_forward(Model& m, ForwardArgs& a) { return model_forward_on(m, *m.ctx, a); }
@@ -733,27 +793,9 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
   CUtensorMap map_attn_q;  // u8 [R][E], box {128 B, 128 rows}: operand of the encoder's row-tile kernel
   if (c.make_map(&map_attn_q, attn_q, R, E, 128)) return 1;
 
-  // SLIMT_B200_SELFATTN=split keeps the projections and the attention as separate kernels (parity cross-check);
-  // =rowwise additionally takes the first-generation one-thread-per-query kernel instead of the tiled one
-  const char* sa_env = getenv("SLIMT_B200_SELFATTN");
-  // the tiled kernel's 64-query x 128-key tiles pay off from T > 64 (mixed lengths: 15.9 -> 8.5 ms per layer of a
-  // 1M-word batch); at T <= 64 with head size 64 (base) half of every tile is idle and the row-wise kernel is faster
-  // (666 vs 1149 us per layer at 4096 x 32); SLIMT_B200_SELFATTN=tiled forces the tiled kernel (parity cross-check)
-  const bool sa_long = sa_env && strcmp(sa_env, "long") == 0;
-  const bool attn_rowwise = (sa_env && strcmp(sa_env, "rowwise") == 0) ||
-                            (T <= 64 && !(sa_env && (strcmp(sa_env, "tiled") == 0 || sa_long)));
-  // The long kernel (self_attention_long.cu) takes what the tiled kernel cannot hold (T > 556 at head size 32, T > 400
-  // at 64) and 257 .. 384 tokens, where its 32-row score block lets two or three blocks share an SM against the tiled
-  // kernel's one: 16.5 vs 19.9 ms for the six layers of 455 x 288, 20.1 vs 22.3 ms at 341 x 384; at 256 x 512 the
-  // tiled kernel's 64-row reuse wins, 29.3 vs 30.4 ms (B200, 1000 W; profiles/r4_long_bench.jsonl).  T <= 256 routes as
-  // before.  SLIMT_B200_SELFATTN=long forces the long kernel (parity cross-check).
-  const bool attn_long = sa_long || (!attn_rowwise && !(sa_env && strcmp(sa_env, "tiled") == 0) &&
-                                     ((T > 256 && T <= 384) || !self_attention_tiled_supported(T, dh)));
-  const bool attn_fused = enc_attention_supported(E, H, dh, T) &&
-                          !(sa_env && (strcmp(sa_env, "split") == 0 || strcmp(sa_env, "rowwise") == 0 ||
-                                       strcmp(sa_env, "tiled") == 0 || sa_long));
+  const Routes route = choose_routes(E, H, dh, T, B, c.fast);
   CUtensorMap map_qa[3], map_qa32[3];
-  if (attn_fused)
+  if (route.self == SelfAttn::Fused)
     for (int i = 0; i < 3; i++)
       if (c.make_map(&map_qa[i], qa[i], R, E, 128) || c.make_map(&map_qa32[i], qa[i], R, E, 32)) return 1;
 
@@ -780,7 +822,7 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
   // ---- encoder (Transformer.cc:57-69; EncoderLayer::forward Modules.cc:321-334)
   for (int i = 0; i < Le; i++) {
     const EncLayerW& L = m.enc[i];
-    if (attn_fused) {
+    if (route.self == SelfAttn::Fused) {
       // q/k/v projections + scaled dot-product attention in one kernel: Q, K, V stay on the SM (enc_attention.cu)
       EncAttnArgs k{};
       k.map_aq = map_qa[0], k.map_ak = map_qa[1], k.map_av = map_qa[2];
@@ -813,12 +855,16 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
       QuantOuts q = qouts();
       qadd(q, attn_q, L.self.o.aq);
       LaunchScope ls(c, "enc_self_attention", 0, 13.0 * R * E);
-      const int rc = attn_long      ? launch_self_attention_long(Qb, Kb, Vb, d_lengths, B, T, H, dh, nullptr, q, s)
-                     : attn_rowwise ? launch_self_attention(Qb, Kb, Vb, d_lengths, B, T, H, dh, nullptr, q, s)
-                                    : launch_self_attention_tiled(Qb, Kb, Vb, d_lengths, B, T, H, dh, nullptr, q, s);
+      int rc = 1;
+      switch (route.self) {
+        case SelfAttn::Rowwise: rc = launch_self_attention(Qb, Kb, Vb, d_lengths, B, T, H, dh, q, s); break;
+        case SelfAttn::Tiled: rc = launch_self_attention_tiled(Qb, Kb, Vb, d_lengths, B, T, H, dh, q, s); break;
+        case SelfAttn::Long: rc = launch_self_attention_long(Qb, Kb, Vb, d_lengths, B, T, H, dh, q, s); break;
+        case SelfAttn::Fused: break;
+      }
       if (rc) {
-        set_error(std::string("self-attention: the ") + (attn_long ? "long" : attn_rowwise ? "row-wise" : "tiled") +
-                  " kernel does not take head size " + std::to_string(dh) + " at sequence length " + std::to_string(T));
+        set_error(std::string("self-attention: the ") + route_name(route.self) + " kernel does not take head size " +
+                  std::to_string(dh) + " at sequence length " + std::to_string(T));
         return 1;
       }
     }
@@ -902,23 +948,13 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
     c.d2h_bytes += 4ul * R * E;
   }
 
-  // ---- cross-attention K/V.  The reference re-projects them every step (Modules.cc:244-249); so does the
-  // recompute kernel (tensor cores, from the u8 encoder output); otherwise they are projected once and cached.
-  // Small batches take the cached kernel: below ~4 k source tokens the recompute kernel has fewer sentence groups than
-  // SMs and its launch is all latency (64 x 32: 8.6 us cached against 12.8 us recomputed per launch, 5.40 -> 5.13 ms per
-  // batch; the two are bit-identical).  SLIMT_B200_CROSS = cached | rc overrides the choice (tests, A/B runs).
-  const char* ca_env = getenv("SLIMT_B200_CROSS");
-  const bool ca_force_rc = ca_env && strcmp(ca_env, "rc") == 0;
-  const bool ca_cached = (ca_env && strcmp(ca_env, "cached") == 0) || (!ca_force_rc && static_cast<long>(B) * T <= 4096);
-  // long sentences (65 .. 256 tokens) take the sentence-at-a-time recompute kernel (cross_attention_rcl.cu; bit-exact mode)
-  const bool cross_rcl = !ca_cached && !c.fast && !cross_attention_rc_supported(E, H, dh, T) && cross_attention_rcl_supported(E, H, dh, T);
-  const bool cross_rc = cross_rcl || (cross_attention_rc_supported(E, H, dh, T) && !ca_cached);
+  // ---- cross-attention K/V: the recompute kernels read the u8 encoder output, the cached kernel K and V projected here
   std::vector<CUtensorMap> mapAk(Ld), mapAv(Ld);
-  if (cross_rc) {
+  if (route.cross != Cross::Cached) {
     for (int l = 0; l < Ld; l++)
       if (c.make_map(&mapAk[l], qa[2 * l], R, E, 32) || c.make_map(&mapAv[l], qa[2 * l + 1], R, E, 32)) return 1;
   }
-  for (int l = 0; l < Ld && !cross_rc; l++) {
+  for (int l = 0; l < Ld && route.cross == Cross::Cached; l++) {
     GemmCall g(&c, "dec_gemm_cross_kv_f32", R, E, E, EPI_F32, 2);
     GemmProblem* pk = g.add(qa[2 * l], m.dec[l].ctx.k);
     GemmProblem* pv = g.add(qa[2 * l + 1], m.dec[l].ctx.v);
@@ -988,11 +1024,7 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
   const int32_t* ipb6_out = m.out.ipb6;
   const int32_t* dshift_out = m.out.dshift;
   CUtensorMap map_ext = m.out.map_ext;
-  static const bool out_legacy = [] {
-    const char* e = getenv("SLIMT_B200_OUT");  // SLIMT_B200_OUT=legacy keeps gemm_out.cu (A/B measurements, cross-checks)
-    return e && strcmp(e, "legacy") == 0;
-  }();
-  const bool out_ext = m.out.ext_ok && !out_legacy;
+  const bool out_ext = m.out.ext_ok;
   if (use_sl) {
     if (a.device_io) {
       d_sl = a.shortlist;
@@ -1090,7 +1122,7 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
           return 1;
         }
       }
-      if (cross_rc) {
+      if (route.cross != Cross::Cached) {
         CrossRcArgs k{};
         k.map_ak = mapAk[l], k.map_av = mapAv[l];
         k.map_wk = L.ctx.k.map128, k.map_wv = L.ctx.v.map128;
@@ -1098,15 +1130,15 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
         k.um_k = L.ctx.k.um, k.um_v = L.ctx.v.um;
         k.q = qd, k.lengths = d_lengths, k.B = B, k.T = T;
         k.dk = static_cast<float>(1.0 / std::sqrt(static_cast<double>(dh)));
-        k.out_f32 = nullptr;
         k.qo = qouts();
         qadd(k.qo, caq, L.ctx.o.aq);
         k.attn_head0 = last ? d_align : nullptr;
         if (trace_buf && step == 3 && l == 0) k.trace = trace_buf + 3 * trace_n;
         const double Bd = B, Ed = E;
-        LaunchScope ls(c, "dec_cross_attention_rc", 2.0 * (cross_rcl ? src_tokens : Bd * (T > 32 ? 64.0 : 32.0)) * Ed * 2.0 * Ed,
+        const bool rcl = route.cross == Cross::Rcl;
+        LaunchScope ls(c, "dec_cross_attention_rc", 2.0 * (rcl ? src_tokens : Bd * (T > 32 ? 64.0 : 32.0)) * Ed * 2.0 * Ed,
                        2.0 * src_tokens * Ed + 2.0 * Ed * Ed + 5.0 * Bd * Ed);  // valid keys only
-        if (cross_rcl ? launch_cross_attention_rcl(k, c.num_sms, s) : launch_cross_attention_rc(k, c.num_sms, c.fast, s)) {
+        if (rcl ? launch_cross_attention_rcl(k, c.num_sms, s) : launch_cross_attention_rc(k, c.num_sms, c.fast, s)) {
           set_error("recompute cross-attention launch failed");
           return 1;
         }
@@ -1114,7 +1146,7 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
         QuantOuts q = qouts();
         qadd(q, caq, L.ctx.o.aq);
         LaunchScope ls(c, "dec_cross_attention", 0, 8.0 * src_tokens * E + 5.0 * B * E);
-        if (launch_cross_attention(mapKc[l], mapVc[l], qd, d_lengths, B, T, H, dh, c.num_sms, nullptr, q,
+        if (launch_cross_attention(mapKc[l], mapVc[l], qd, d_lengths, B, T, H, dh, c.num_sms, q,
                                    last ? d_align : nullptr, s)) {
           set_error("cross-attention: no kernel for " + std::to_string(H) + " heads of " + std::to_string(dh) +
                     " over " + std::to_string(T) + " source tokens");

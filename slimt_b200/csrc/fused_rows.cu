@@ -94,22 +94,6 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
   // descriptors and addresses stay in uniform registers: no per-MMA waterfall loop as with `lane == 0`).  The ring
   // positions live in the leader's registers across tiles, hence a single election.
   const bool leader = elect_one();
-  // The weight stream of one tile in consumption order: tiles [from, to) are requested, the others stepped over.
-  auto load_weights = [&](int from, int to) {
-    int i = 0;
-    for (int mb = 0; mb < EM; mb++)
-      for (int kb = 0; kb < EK; kb++, i++)
-        if (i >= from && i < to) prod.load(&a.map_wf, kb, mb);
-    for (int mb = 0; mb < EM; mb++)
-      for (int kb = 0; kb < EK; kb++, i++)
-        if (i >= from && i < to) prod.load(&a.map_w, kb, mb);
-    for (int mb = 0; mb < EM; mb++)
-      for (int kb = 0; kb < EK; kb++, i++)
-        if (i >= from && i < to) prod.load(&a.map_wq, kb, mb);
-  };
-  // Weights are never written by a kernel, so the first ring-ful is requested before waiting for the preceding
-  // kernel: its L2 latency hides behind that kernel's tail.
-  if (SB_PRE_SSRU && warp == 0 && leader && static_cast<int>(blockIdx.x) < n_tiles) load_weights(0, L::kStages);
   pdl_wait();  // everything above overlapped the previous kernel's tail; its outputs are visible from here on
   if (threadIdx.x == 0) SB_TRACE(a, 1);
   for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, iter++) {
@@ -124,7 +108,13 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
             tma_load_2d(opnd_xw + kb * kOpK, &a.map_xw, x_full, kb * 128, row0);
           }
         }
-        load_weights(iter == 0 && SB_PRE_SSRU ? L::kStages : 0, 1 << 30);
+        // the weight stream of one tile in consumption order
+        for (int mb = 0; mb < EM; mb++)
+          for (int kb = 0; kb < EK; kb++) prod.load(&a.map_wf, kb, mb);
+        for (int mb = 0; mb < EM; mb++)
+          for (int kb = 0; kb < EK; kb++) prod.load(&a.map_w, kb, mb);
+        for (int mb = 0; mb < EM; mb++)
+          for (int kb = 0; kb < EK; kb++) prod.load(&a.map_wq, kb, mb);
       }
     } else if (warp == 1) {
       if (leader) {

@@ -22,13 +22,6 @@ struct TileCfg {
   static constexpr uint32_t kTmemCols = BN < 32 ? 32 : BN;
 };
 
-__device__ __forceinline__ unsigned long long pack_best(float v, uint32_t idx) {
-  if (v == 0.0f) v = 0.0f;  // canonicalise -0 so equal values compare equal
-  uint32_t b = __float_as_uint(v);
-  uint32_t key = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-  return (static_cast<unsigned long long>(key) << 32) | static_cast<unsigned long long>(0xFFFFFFFFu - idx);
-}
-
 template <int BN, int STAGES, int EPI>
 __global__ void __launch_bounds__(kThreads) gemm_i8_kernel(const __grid_constant__ GemmBatch batch) {
   using Cfg = TileCfg<BN>;
@@ -261,28 +254,6 @@ __global__ void __launch_bounds__(kThreads) gemm_i8_kernel(const __grid_constant
           }
         }
       }
-    } else if constexpr (EPI == EPI_ARGMAX) {
-      // greedy_sample: first strict maximum (slimt/Transformer.cc:279-339).  Columns ascend within the
-      // tile; across tiles the packed key breaks value ties towards the lower index.
-      float best = 0.0f;
-      uint32_t best_idx = 0;
-      bool have = false;
-#pragma unroll 1
-      for (int c = 0; c < BN / 32; c++) {
-        tmem_ld32(taddr + c * 32, v);
-        const int nb = n0 + c * 32;
-#pragma unroll
-        for (int j = 0; j < 32; j++) {
-          float y = dequant1((int)v[j], um, s_pb[c * 32 + j]);
-          bool valid = nb + j < N;
-          if (valid && (!have || y > best)) {
-            best = y;
-            best_idx = nb + j;
-            have = true;
-          }
-        }
-      }
-      if (row_ok && have) atomicMax(P.best + row, pack_best(best, best_idx));
     }
   }
 
@@ -336,8 +307,6 @@ void launch_gemm_i8(const GemmBatch& batch, int n_problems, int epilogue, int BN
       return dispatch_bn<EPI_QUANT>(batch, n_problems, BN, stream);
     case EPI_RES_LN:
       return dispatch_bn<EPI_RES_LN>(batch, n_problems, BN, stream);
-    case EPI_ARGMAX:
-      return dispatch_bn<EPI_ARGMAX>(batch, n_problems, BN, stream);
     case EPI_ACC:
       return dispatch_bn<EPI_ACC>(batch, n_problems, BN, stream);
     default:

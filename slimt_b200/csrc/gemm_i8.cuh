@@ -5,8 +5,8 @@
 // affine_with_select (reference slimt/QMM.cc:37-75, qmm/Intgemm.inl.cc:8-243 ==
 // qmm/Gemmology.inl.cc:33-281): PrepareA is done by the PRODUCER of the
 // activation (it emits int8), PrepareBias is precomputed at load, Multiply is the
-// MMA, UnquantizeAndAddBiasAndWrite (+ReLU / +requantize / +residual+LayerNorm /
-// +argmax) is the epilogue.
+// MMA, UnquantizeAndAddBiasAndWrite (+ReLU / +requantize / +residual+LayerNorm)
+// is the epilogue; the output projection's fused argmax is gemm_out*.cu.
 //
 // Layouts: A = quantized activations as the reference's PrepareA emits them, u8 = qa + 127, [M][K] row-major
 // (K contiguous), so the u8 x s8 MMA forms Int8Shift::Multiply's shifted accumulator directly;
@@ -29,7 +29,6 @@ enum Epilogue : int {
   EPI_F32 = 0,     // y (optionally ReLU) -> f32 [M][N]
   EPI_QUANT = 1,   // relu?(y) -> requantize with aq_out[0] -> int8 [M][N]
   EPI_RES_LN = 2,  // LayerNorm(y + residual) -> f32 (optional) + up to 4 int8 copies; needs BN == N
-  EPI_ARGMAX = 3,  // per-row first-max over this tile's columns -> atomicMax on packed (value,index)
   EPI_ACC = 4,     // raw shifted int32 accumulators -> s32 [M][N] (parity/debug tap)
 };
 
@@ -52,8 +51,6 @@ struct GemmProblem {
   const float* ln_scale;  // [N]
   const float* ln_bias;   // [N]
   float ln_eps;
-  // EPI_ARGMAX
-  unsigned long long* best;  // [M] packed (ordered value << 32 | ~index), pre-zeroed
 };
 
 struct GemmBatch {

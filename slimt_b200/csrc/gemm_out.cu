@@ -97,15 +97,6 @@ __global__ void __launch_bounds__(kOutThreads, 1)
   __syncthreads();
   tc_fence_after();
   pdl_launch_dependents();
-  // The weight tile of the first run does not depend on the preceding kernel (the model's weights, or the shortlist
-  // gather that ran before the decode loop behind an ordinary launch): request it before waiting, so that its 64 KB
-  // arrive while the predecessor drains.
-  const int pre_n = (SB_PRE_OUT && t_begin < t_end) ? t_begin / m_tiles : -1;
-  if (warp == 0 && pre_n >= 0 && elect_one()) {
-    mbar_expect_tx(b_full, KB * kBBytes);
-#pragma unroll
-    for (int kb = 0; kb < KB; kb++) tma_load_2d(smem_b + kb * kBBytes, &tma_b, b_full, kb * kBK, pre_n * kOutBN);
-  }
   pdl_wait();  // everything above overlapped the previous kernel's tail; its outputs are visible from here on
   const uint32_t tmem_base = *tmem_slot;
 
@@ -113,8 +104,8 @@ __global__ void __launch_bounds__(kOutThreads, 1)
     // ===== TMA producer =====
     if (elect_one()) {
       uint32_t kbc = 0;  // running k-block counter (ring position)
-      uint32_t run = pre_n >= 0 ? 1 : 0;  // running count of column-tile runs (the first one is already in flight)
-      int cur_n = pre_n;
+      uint32_t run = 0;  // running count of column-tile runs
+      int cur_n = -1;
       for (int t = t_begin; t < t_end; t++) {
         const int n = t / m_tiles, m = t % m_tiles;
         if (n != cur_n) {

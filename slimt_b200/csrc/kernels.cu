@@ -65,7 +65,7 @@ __global__ void quantize_kernel(const float* __restrict__ x, size_t n4, QuantOut
 template <int DH>
 __global__ void self_attention_kernel(const float* __restrict__ Q, const float* __restrict__ K,
                                       const float* __restrict__ V, const uint32_t* __restrict__ lengths, int T,
-                                      int H, float dk, float* __restrict__ out_f32, QuantOuts q) {
+                                      int H, float dk, QuantOuts q) {
   extern __shared__ float smem_f[];
   const int b = blockIdx.x / H;
   const int h = blockIdx.x % H;
@@ -154,56 +154,11 @@ __global__ void self_attention_kernel(const float* __restrict__ Q, const float* 
 #pragma unroll
       for (int d = 0; d < DH; d++) acc[d] = 0.0f;  // padded query rows never reach a valid output
     }
-    if (out_f32) {
-#pragma unroll
-      for (int d = 0; d < DH; d += 4) *reinterpret_cast<float4*>(out_f32 + off + d) = make_float4(acc[d], acc[d + 1], acc[d + 2], acc[d + 3]);
-    }
 #pragma unroll
     for (int d = 0; d < DH; d += 4) {
       const float y[4] = {acc[d], acc[d + 1], acc[d + 2], acc[d + 3]};
       store_quant4(q, off + d, y);
     }
-  }
-}
-
-// ------------------------------------------------------------------ SSRU tail
-// Warp = one sentence row.  Elementwise part is lane-parallel and coalesced; the two LayerNorm sums
-// run in element order over the row parked in shared memory (every lane walks the same chain).
-__global__ void ssru_ln_kernel(const float* __restrict__ f, const float* __restrict__ wx, float* __restrict__ state,
-                               const float* __restrict__ x, const float* __restrict__ ln_scale,
-                               const float* __restrict__ ln_bias, float eps, int B, int E, float* __restrict__ h,
-                               QuantOuts q) {
-  extern __shared__ float smem_f[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int row = blockIdx.x * (blockDim.x >> 5) + warp;
-  if (row >= B) return;
-  float* t = smem_f + static_cast<size_t>(warp) * E;
-  const size_t base = static_cast<size_t>(row) * E;
-  for (int e = lane; e < E; e += 32) {
-    const float sg = sigmoid_ref(f[base + e]);
-    const float a = __fmul_rn(sg, state[base + e]);
-    const float bb = __fmul_rn(__fsub_rn(1.0f, sg), wx[base + e]);
-    const float c = __fadd_rn(a, bb);  // highway(c_prev, Wx, f), slimt/TensorOps.cc:662-682
-    state[base + e] = c;
-    const float y = c > 0.0f ? c : 0.0f;
-    t[e] = __fadd_rn(x[base + e], y);
-  }
-  __syncwarp();
-  float sum = 0.0f;
-  for (int e = 0; e < E; e++) sum = __fadd_rn(sum, t[e]);
-  const float cols = static_cast<float>(E);
-  const float mean = __fdiv_rn(sum, cols);
-  float sq = 0.0f;
-  for (int e = 0; e < E; e++) {
-    const float d = __fsub_rn(t[e], mean);
-    sq = __fadd_rn(sq, __fmul_rn(d, d));
-  }
-  const float sigma = __fsqrt_rn(__fadd_rn(__fdiv_rn(sq, cols), eps));
-  for (int e = lane; e < E; e += 32) {
-    const float n = __fdiv_rn(__fsub_rn(t[e], mean), sigma);
-    const float y = __fadd_rn(__fmul_rn(ln_scale[e], n), ln_bias[e]);
-    if (h) h[base + e] = y;
-    for (int k = 0; k < q.n; k++) q.ptr[k][base + e] = static_cast<int8_t>(quantize1(y, q.aq[k]));
   }
 }
 
@@ -370,7 +325,7 @@ void launch_quantize(const float* x, size_t n, QuantOuts q, cudaStream_t stream)
 }
 
 int launch_self_attention(const float* Q, const float* K, const float* V, const uint32_t* lengths, int B, int T, int H,
-                          int dh, float* out_f32, QuantOuts q, cudaStream_t stream) {
+                          int dh, QuantOuts q, cudaStream_t stream) {
   if (B == 0) return 0;
   // 1/sqrt(dim_head) evaluated in double then narrowed, as `1.0F / std::sqrt(size_t)` does (Modules.cc:43).
   const float dk = static_cast<float>(1.0 / std::sqrt(static_cast<double>(dh)));
@@ -385,22 +340,14 @@ int launch_self_attention(const float* Q, const float* K, const float* V, const 
   if (smem > 200 * 1024) return 1;  // K, V and one warp's score rows no longer fit: T > 533 (head size 32), T > 319 (64)
   if (dh == 32) {
     ensure_dyn_smem(self_attention_kernel<32>, smem);
-    self_attention_kernel<32><<<B * H, threads, smem, stream>>>(Q, K, V, lengths, T, H, dk, out_f32, q);
+    self_attention_kernel<32><<<B * H, threads, smem, stream>>>(Q, K, V, lengths, T, H, dk, q);
   } else if (dh == 64) {
     ensure_dyn_smem(self_attention_kernel<64>, smem);
-    self_attention_kernel<64><<<B * H, threads, smem, stream>>>(Q, K, V, lengths, T, H, dk, out_f32, q);
+    self_attention_kernel<64><<<B * H, threads, smem, stream>>>(Q, K, V, lengths, T, H, dk, q);
   } else {
     return 1;  // the model loader only admits head sizes 32 and 64; reported through the error convention by the caller
   }
   return 0;
-}
-
-void launch_ssru_ln(const float* f, const float* wx, float* state, const float* x, const float* ln_scale,
-                    const float* ln_bias, float eps, int B, int E, float* h, QuantOuts q, cudaStream_t stream) {
-  if (B == 0) return;
-  const int wpb = 4;
-  const size_t smem = static_cast<size_t>(wpb) * E * sizeof(float);
-  ssru_ln_kernel<<<(B + wpb - 1) / wpb, wpb * 32, smem, stream>>>(f, wx, state, x, ln_scale, ln_bias, eps, B, E, h, q);
 }
 
 void launch_finalize_step(unsigned long long* best, const uint32_t* shortlist, const uint32_t* forced, int step,

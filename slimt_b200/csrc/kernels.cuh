@@ -1,4 +1,4 @@
-// Non-GEMM kernels of the hot path (embedding, attention, SSRU, step bookkeeping).
+// Non-GEMM kernels of the hot path (embedding, attention, step bookkeeping).
 // Each one reproduces the reference's f32 arithmetic bit for bit (see
 // exact_math.cuh) while emitting the int8 operands of the GEMMs that consume it.
 #pragma once
@@ -26,22 +26,23 @@ void launch_embed(const uint32_t* tokens, const int8_t* emb_q, float inv_qm, flo
 void launch_quantize(const float* x, size_t n, QuantOuts q, cudaStream_t stream);
 
 // Encoder self-attention on unsplit [B*T][E] Q,K,V (scaled_dot_product_attention, slimt/Modules.cc:24-86,
-// with split_heads/join_heads folded into the addressing).  Emits the Wo operand (int8) and/or f32.
+// with split_heads/join_heads folded into the addressing).  Emits the Wo operand (int8).
 int launch_self_attention(const float* Q, const float* K, const float* V, const uint32_t* lengths, int B, int T,
-                           int H, int dh, float* out_f32, QuantOuts q, cudaStream_t stream);
+                           int H, int dh, QuantOuts q, cudaStream_t stream);
 
 // The same operation as a register-tiled kernel (self_attention_tiled.cu): 64 query rows of one (sentence, head) per
-// block, every output still one sequential chain.  The default for every shape the fused encoder kernel does not take.
+// block, every output still one sequential chain.  Which of the self-attention kernels runs for a shape is decided in
+// one place, choose_routes in engine.cu.
 // Returns nonzero when the shape does not fit: head sizes 32 and 64, T up to 556 (head size 32) or 400 (64), which
 // self_attention_tiled_supported tells without launching.
 int launch_self_attention_tiled(const float* Q, const float* K, const float* V, const uint32_t* lengths, int B, int T,
-                                int H, int dh, float* out_f32, QuantOuts q, cudaStream_t stream);
+                                int H, int dh, QuantOuts q, cudaStream_t stream);
 bool self_attention_tiled_supported(int T, int dh);
 
 // The same operation for sentences the tiled kernel cannot hold (self_attention_long.cu): 32 query rows per block, K
 // and V streamed in 128-key tiles, the same chains and so the same bits.  Head sizes 32 and 64, T up to 1024.
 int launch_self_attention_long(const float* Q, const float* K, const float* V, const uint32_t* lengths, int B, int T,
-                               int H, int dh, float* out_f32, QuantOuts q, cudaStream_t stream);
+                               int H, int dh, QuantOuts q, cudaStream_t stream);
 bool self_attention_long_supported(int T, int dh);
 
 // Decoder cross-attention for one query row per sentence over cached K,V [B][S][E] (cross_attention.cu).
@@ -50,8 +51,8 @@ bool self_attention_long_supported(int T, int dh);
 // S <= 1024; returns nonzero for a shape it does not take (S beyond that, heads other than 8 of 32 or 64).
 int cross_attention_box_rows(int S);
 int launch_cross_attention(const CUtensorMap& mapK, const CUtensorMap& mapV, const float* Qr,
-                            const uint32_t* lengths, int B, int S, int H, int dh, int num_sms, float* out_f32,
-                            QuantOuts q, float* attn_head0, cudaStream_t stream);
+                            const uint32_t* lengths, int B, int S, int H, int dh, int num_sms, QuantOuts q,
+                            float* attn_head0, cudaStream_t stream);
 
 // The same attention with K and V re-projected from the quantised encoder output on the tensor cores every step
 // instead of read from an f32 cache (cross_attention_rc.cu): 4x less HBM traffic, bit-identical results.
@@ -65,7 +66,6 @@ struct CrossRcArgs {
   const uint32_t* lengths;
   int B, T;
   float dk;                    // 1 / sqrt(head size)
-  float* out_f32;              // optional f32 [B][E]
   QuantOuts qo;                // int8 copies of the output (Wo's operand)
   float* attn_head0;           // optional [B][T]
   long long* trace;            // optional phase stamps (clock64) of consumer thread 0, 128 slots per CTA (SLIMT_B200_TRACE)
@@ -94,10 +94,6 @@ struct EncAttnArgs {
 };
 bool enc_attention_supported(int E, int H, int dh, int T);
 int launch_enc_attention(const EncAttnArgs& a, int num_sms, cudaStream_t stream);
-
-// SSRU cell tail (slimt/Modules.cc:190-235): c = highway(c_prev, Wx, f); h = LN(x + relu(c)); state <- c.
-void launch_ssru_ln(const float* f, const float* wx, float* state, const float* x, const float* ln_scale,
-                    const float* ln_bias, float eps, int B, int E, float* h, QuantOuts q, cudaStream_t stream);
 
 // Per decode step: packed argmax -> word id (through the shortlist when given), record into
 // step_tokens[step][B], EOS bookkeeping, re-arm `best`, and build the next step's decoder input

@@ -220,28 +220,11 @@ __host__ __device__ constexpr uint32_t make_idesc_i8(uint32_t M, uint32_t N) {
 // thread of a PDL-launched kernel calls pdl_wait() before touching global memory, which also keeps the chain
 // transitive.  pdl_launch_dependents() lets the NEXT kernel's CTAs be scheduled as soon as resources free up.
 // Both are no-ops for ordinary launches.
-// SB_PREWAIT_LOADS: request constant data (weights) before griddepcontrol.wait.  Build-time switch for A/B runs.
-#ifndef SB_PREWAIT_LOADS
-#define SB_PREWAIT_LOADS 0
-#endif
-#ifndef SB_PRE_SSRU
-#define SB_PRE_SSRU SB_PREWAIT_LOADS
-#endif
-#ifndef SB_PRE_FFN
-#define SB_PRE_FFN SB_PREWAIT_LOADS
-#endif
-#ifndef SB_PRE_OUT
-#define SB_PRE_OUT SB_PREWAIT_LOADS
-#endif
-#ifndef SB_PRE_CROSS
-#define SB_PRE_CROSS SB_PREWAIT_LOADS
-#endif
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
 }  // namespace sb
 
-#include <cstdlib>
 #include <mutex>
 #include <unordered_map>
 #include <utility>
@@ -267,15 +250,6 @@ inline cudaError_t ensure_dyn_smem(Kern kern, size_t bytes) {
   return e;
 }
 
-// SLIMT_B200_PDL=0 turns the attribute off (plain stream order) for A/B measurements.
-inline bool pdl_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("SLIMT_B200_PDL");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
                               Args&&... args) {
@@ -285,7 +259,7 @@ inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, siz
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
 }
 

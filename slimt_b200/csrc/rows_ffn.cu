@@ -120,38 +120,25 @@ __global__ void __launch_bounds__(kThreads, 1) rows_ffn_kernel(const __grid_cons
   // descriptors and addresses stay in uniform registers: no per-MMA waterfall loop as with `lane == 0`).  The ring
   // positions live in the leader's registers across tiles, hence a single election.
   const bool leader = elect_one();
-  // The weight stream of one tile in consumption order; tiles [from_a, to_a) of ring A's sequence and [from_b, to_b)
-  // of ring B's are requested, the others stepped over.
-  auto load_weights = [&](int from_a, int from_b, int to_a, int to_b) {
-    int ia = 0, ib = 0;
-    for (int mb = 0; mb < EM; mb++)
-      for (int kb = 0; kb < EK; kb++, ia++)
-        if (ia >= from_a && ia < to_a) prod_a.load(&a.map_wo, kb, mb);
-    for (int st = 0; st < FM + kLook; st++) {
-      if (st < FM)
-        for (int kb = 0; kb < EK; kb++, ia++)
-          if (ia >= from_a && ia < to_a) prod_a.load(&a.map_w1, kb, st);
-      if (st >= kLook)
-        for (int mb = 0; mb < EM; mb++, ib++)
-          if (ib >= from_b && ib < to_b) prod_b.load(&a.map_w2, st - kLook, mb);
-    }
-  };
-  // Weights are never written by a kernel, so the first ring-fuls are requested before waiting for the preceding
-  // kernel: their L2 latency hides behind its tail.
-  const int pre_a = L::kStagesA, pre_b = L::kStagesB;
-  if (SB_PRE_FFN && warp == 0 && leader && static_cast<int>(blockIdx.x) < n_tiles) load_weights(0, 0, pre_a, pre_b);
   pdl_wait();  // everything above overlapped the previous kernel's tail; its outputs are visible from here on
   if (threadIdx.x == 0) SB_TRACE(a, 1);
   for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, iter++) {
     const int row0 = tile * R;
     const uint32_t tph = iter & 1;
     if (warp == 0) {
-      // ===== TMA producer: the tile's input operand, then every weight tile in consumption order.  The weight
-      // tiles that fit the rings at kernel start were already requested before griddepcontrol.wait (above).
+      // ===== TMA producer: the tile's input operand, then every weight tile in consumption order (Wo and W1 through
+      // ring A, W2 through ring B)
       if (leader) {
         mbar_expect_tx(a_full, EK * kOpK);
         for (int kb = 0; kb < EK; kb++) tma_load_2d(opnd_a + kb * kOpK, &a.map_a, a_full, kb * 128, row0);
-        load_weights(iter == 0 && SB_PRE_FFN ? pre_a : 0, iter == 0 && SB_PRE_FFN ? pre_b : 0, 1 << 30, 1 << 30);
+        for (int mb = 0; mb < EM; mb++)
+          for (int kb = 0; kb < EK; kb++) prod_a.load(&a.map_wo, kb, mb);
+        for (int st = 0; st < FM + kLook; st++) {
+          if (st < FM)
+            for (int kb = 0; kb < EK; kb++) prod_a.load(&a.map_w1, kb, st);
+          if (st >= kLook)
+            for (int mb = 0; mb < EM; mb++) prod_b.load(&a.map_w2, st - kLook, mb);
+        }
       }
     } else if (warp == 1) {
       // ===== MMA issuer A: the Wo GEMM and the FFN1 feature blocks.  The FFN2 k-steps are issued by warp 3, so that

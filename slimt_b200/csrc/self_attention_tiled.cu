@@ -34,7 +34,7 @@ constexpr int kTThreads = 256;
 template <int DH>
 __global__ void __launch_bounds__(kTThreads) self_attention_tiled_kernel(
     const float* __restrict__ Q, const float* __restrict__ K, const float* __restrict__ V,
-    const uint32_t* __restrict__ lengths, int T, int H, int n_qb, float dk, float* __restrict__ out_f32, QuantOuts qo) {
+    const uint32_t* __restrict__ lengths, int T, int H, int n_qb, float dk, QuantOuts qo) {
   extern __shared__ __align__(16) float sm[];
   __shared__ uint64_t exp_tab[32];
   const int tid = threadIdx.x, lane = tid & 31;
@@ -201,7 +201,6 @@ __global__ void __launch_bounds__(kTThreads) self_attention_tiled_kernel(
         float y[4];
 #pragma unroll
         for (int k = 0; k < 4; k++) y[k] = live ? acc[u][w + k] : 0.0f;
-        if (out_f32) *reinterpret_cast<float4*>(out_f32 + off + w) = make_float4(y[0], y[1], y[2], y[3]);
         for (int k = 0; k < qo.n; k++) {
           const float aq = qo.aq[k];
           *reinterpret_cast<uint32_t*>(qo.ptr[k] + off + w) =
@@ -228,7 +227,7 @@ bool self_attention_tiled_supported(int T, int dh) {
 }
 
 int launch_self_attention_tiled(const float* Q, const float* K, const float* V, const uint32_t* lengths, int B, int T, int H,
-                                int dh, float* out_f32, QuantOuts q, cudaStream_t stream) {
+                                int dh, QuantOuts q, cudaStream_t stream) {
   if (B == 0) return 0;
   // 1/sqrt(dim_head) evaluated in double then narrowed, as `1.0F / std::sqrt(size_t)` does (Modules.cc:43)
   const float dk = static_cast<float>(1.0 / std::sqrt(static_cast<double>(dh)));
@@ -238,10 +237,10 @@ int launch_self_attention_tiled(const float* Q, const float* K, const float* V, 
   if (!self_attention_tiled_supported(T, dh) || blocks > 0x7fffffffL) return 1;
   if (dh == 32) {
     if (ensure_dyn_smem(self_attention_tiled_kernel<32>, smem) != cudaSuccess) return 1;
-    self_attention_tiled_kernel<32><<<static_cast<unsigned>(blocks), kTThreads, smem, stream>>>(Q, K, V, lengths, T, H, n_qb, dk, out_f32, q);
+    self_attention_tiled_kernel<32><<<static_cast<unsigned>(blocks), kTThreads, smem, stream>>>(Q, K, V, lengths, T, H, n_qb, dk, q);
   } else if (dh == 64) {
     if (ensure_dyn_smem(self_attention_tiled_kernel<64>, smem) != cudaSuccess) return 1;
-    self_attention_tiled_kernel<64><<<static_cast<unsigned>(blocks), kTThreads, smem, stream>>>(Q, K, V, lengths, T, H, n_qb, dk, out_f32, q);
+    self_attention_tiled_kernel<64><<<static_cast<unsigned>(blocks), kTThreads, smem, stream>>>(Q, K, V, lengths, T, H, n_qb, dk, q);
   } else {
     return 1;
   }

@@ -47,8 +47,7 @@ WANT = ["gpu__time_duration.sum", "dram__bytes_read.sum", "dram__bytes_write.sum
 TAGS = {"cross_attention_kernel": "dec_cross_attention", "out_argmax_kernel": "dec_gemm_out_argmax", "dec_ssru_kernel": "dec_ssru_q_fused",
         "self_attention_kernel": "enc_self_attention",
         "cross_attention_rc_kernel": "dec_cross_attention_rc", "cross_attention_rcl_kernel": "dec_cross_attention_rc",
-        "enc_attention_kernel": "enc_qkv_attention_fused", "enc_attention_pair_kernel": "enc_qkv_attention_fused",
-        "enc_attention_warp_kernel": "enc_qkv_attention_fused"}
+        "enc_attention_kernel": "enc_qkv_attention_fused", "enc_attention_warp_kernel": "enc_qkv_attention_fused"}
 traffic = {}
 tpath = os.path.join(out_dir, "roofline_traffic.json")
 if os.path.exists(tpath):

@@ -121,7 +121,6 @@ cudaEvent_t Context::pooled_event() {
 }
 
 int Context::reserve(size_t bytes) {
-  arena_used = 0;
   if (bytes <= arena_bytes) return 0;
   SB_CUDA(cudaStreamSynchronize(stream));
   if (arena) SB_CUDA(cudaFree(arena));
@@ -398,7 +397,7 @@ int Model::load(Context* c, const void* bin, size_t bytes, int enc_layers, int d
     std::vector<int8_t> req(deq.size());
     host_quantize(deq.data(), req.data(), emb_qm, deq.size());
     if (weight("Wemb", "decoder_ff_logit_out_b", out, req.data(), "none_QuantMultA")) return 1;
-    // bound filter of the fused output GEMM: 127 * colsum per column, per-chunk dmax, rounding slack eta
+    // 127 * colsum per column, then the digit rows of gemm_out_ext.cu
     std::vector<int32_t> c127(V);
     for (int n = 0; n < V; n++) {
       int32_t cs = 0;
@@ -406,29 +405,29 @@ int Model::load(Context* c, const void* bin, size_t bytes, int enc_layers, int d
       c127[n] = 127 * cs;
     }
     if (upload(c127.data(), 4ul * V, reinterpret_cast<void**>(&out.c127))) return 1;
+    const size_t vpad = static_cast<size_t>((V + 255) / 256 * 256);
+    int* d_flag = nullptr;
+    SB_CUDA(cudaMalloc(&out.ext, vpad * 128));
+    owned.push_back(out.ext);
+    SB_CUDA(cudaMalloc(&out.dshift, vpad * 4));
+    owned.push_back(out.dshift);
+    SB_CUDA(cudaMalloc(&d_flag, 4));
+    SB_CUDA(cudaMemsetAsync(d_flag, 0, 4, c->stream));
+    launch_out_ext(out.c127, out.pb, out.um, V, out.ext, out.dshift, d_flag, c->stream);
+    int flag = 0;
+    SB_CUDA(cudaMemcpyAsync(&flag, d_flag, 4, cudaMemcpyDeviceToHost, c->stream));
+    SB_CUDA(cudaStreamSynchronize(c->stream));
+    SB_CUDA(cudaFree(d_flag));
+    out.ext_ok = flag == 0;
+    if (ctx->make_map(&out.map_ext, out.ext, vpad, 128, 256)) return 1;
+  }
+  if (!out.ext_ok) {  // gemm_out.cu's bound filter: per-chunk dmax, proxy offsets, rounding slack eta
     SB_CUDA(cudaMalloc(&out.dmax, 4ul * ((V + 31) / 32)));
     owned.push_back(out.dmax);
     launch_out_bounds(out.c127, out.pb, out.um, V, out.dmax, c->stream);
     SB_CUDA(cudaMalloc(&out.ipb6, 4ul * ((V + 255) / 256 * 256)));
     owned.push_back(out.ipb6);
     launch_out_ipb(out.c127, out.pb, out.um, V, out.ipb6, c->stream);
-    {
-      const size_t vpad = static_cast<size_t>((V + 255) / 256 * 256);
-      int* d_flag = nullptr;
-      SB_CUDA(cudaMalloc(&out.ext, vpad * 128));
-      owned.push_back(out.ext);
-      SB_CUDA(cudaMalloc(&out.dshift, vpad * 4));
-      owned.push_back(out.dshift);
-      SB_CUDA(cudaMalloc(&d_flag, 4));
-      SB_CUDA(cudaMemsetAsync(d_flag, 0, 4, c->stream));
-      launch_out_ext(out.c127, out.pb, out.um, V, out.ext, out.dshift, d_flag, c->stream);
-      int flag = 0;
-      SB_CUDA(cudaMemcpyAsync(&flag, d_flag, 4, cudaMemcpyDeviceToHost, c->stream));
-      SB_CUDA(cudaStreamSynchronize(c->stream));
-      SB_CUDA(cudaFree(d_flag));
-      out.ext_ok = flag == 0;
-      if (ctx->make_map(&out.map_ext, out.ext, vpad, 128, 256)) return 1;
-    }
     SB_CUDA(cudaStreamSynchronize(c->stream));
     std::vector<float> pbh(V);
     SB_CUDA(cudaMemcpy(pbh.data(), out.pb, 4ul * V, cudaMemcpyDeviceToHost));
@@ -478,6 +477,34 @@ void Model::destroy() {
   owned.clear();
 }
 
+// ------------------------------------------------------------------ workspace
+namespace {
+
+// The device buffers of one call, each listed once: add() records where a buffer's pointer goes and how many elements
+// it holds; carve() reserves the sum in the context's arena and hands out the pointers in list order, each buffer
+// starting on a 256-byte boundary.
+// Margin behind the last buffer: not every kernel has been shown to keep its loads inside its buffer (the output GEMMs
+// index per-column arrays by 256-column tile), so the arena keeps ending with 16 KB that no buffer owns.
+constexpr size_t kTailPad = 64 * 256;
+
+struct Workspace {
+  size_t bytes = kTailPad;
+  std::vector<std::pair<void**, size_t>> bufs;
+  template <class T>
+  void add(T*& slot, size_t count) {
+    bufs.emplace_back(reinterpret_cast<void**>(&slot), (count * sizeof(T) + 255) & ~size_t(255));
+    bytes += bufs.back().second;
+  }
+  int carve(Context& c) const {
+    if (c.reserve(bytes)) return 1;
+    char* p = c.arena;
+    for (const auto& b : bufs) *b.first = p, p += b.second;
+    return 0;
+  }
+};
+
+}  // namespace
+
 // ------------------------------------------------------------------ GEMM helpers
 namespace {
 
@@ -497,7 +524,6 @@ struct GemmCall {
   int epi = EPI_F32;
   int bn = 256;
   const char* tag = "gemm";
-  double extra_bytes = 0;  // epilogue traffic beyond A, W and the primary output (residual reads, int8 copies)
   GemmCall(Context* ctx, const char* tag_, int M, int N, int K, int epilogue, int n_prob_hint = 1)
       : c(ctx), epi(epilogue), tag(tag_) {
     b.M = M, b.N = N, b.K = K;
@@ -569,14 +595,15 @@ int qmm_affine_host(Context& c, const float* x, size_t M, size_t K, const int8_t
   std::vector<float> pb(N);
   host_prepare_bias(W, bias, aq, bq, K, N, pb.data());
   const size_t Nout = indices ? n_idx : N;
-  const size_t need = M * K * 5 + N * K + N * 8 + Nout * K + Nout * 8 + n_idx * 4 + M * Nout * 8 + 16 * 256;
-  if (c.reserve(need)) return 1;
-  float* dx = c.take<float>(M * K);
-  int8_t* dqa = c.take<int8_t>(M * K);
-  int8_t* dW = c.take<int8_t>(N * K);
-  float* dpb = c.take<float>(N);
-  float* dy = c.take<float>(M * Nout);
-  int32_t* dacc = c.take<int32_t>(M * Nout);
+  float *dx = nullptr, *dpb = nullptr, *dy = nullptr, *dpbs = nullptr;
+  int8_t *dqa = nullptr, *dW = nullptr, *dWs = nullptr;
+  int32_t* dacc = nullptr;
+  uint32_t* didx = nullptr;
+  Workspace ws;
+  ws.add(dx, M * K), ws.add(dqa, M * K), ws.add(dW, N * K), ws.add(dpb, N), ws.add(dy, M * Nout);
+  if (acc_out) ws.add(dacc, M * Nout);
+  if (indices) ws.add(didx, n_idx), ws.add(dWs, n_idx * K), ws.add(dpbs, n_idx);
+  if (ws.carve(c)) return 1;
   cudaStream_t s = c.stream;
   SB_CUDA(cudaMemcpyAsync(dx, x, M * K * 4, cudaMemcpyHostToDevice, s));
   SB_CUDA(cudaMemcpyAsync(dW, W, N * K, cudaMemcpyHostToDevice, s));
@@ -585,9 +612,6 @@ int qmm_affine_host(Context& c, const float* x, size_t M, size_t K, const int8_t
   const int8_t* Wuse = dW;
   const float* pbuse = dpb;
   if (indices) {
-    uint32_t* didx = c.take<uint32_t>(n_idx);
-    int8_t* dWs = c.take<int8_t>(n_idx * K);
-    float* dpbs = c.take<float>(n_idx);
     SB_CUDA(cudaMemcpyAsync(didx, indices, n_idx * 4, cudaMemcpyHostToDevice, s));
     {
       LaunchScope ls(c, "gather_rows", 0, 2.0 * n_idx * K);
@@ -633,25 +657,23 @@ namespace {
 enum class SelfAttn { Fused, Rowwise, Tiled, Long };
 enum class Cross { Cached, Rc, Rcl };
 
-const char* route_name(SelfAttn r) {
-  switch (r) {
-    case SelfAttn::Fused: return "Fused";
-    case SelfAttn::Rowwise: return "Rowwise";
-    case SelfAttn::Tiled: return "Tiled";
-    case SelfAttn::Long: return "Long";
-  }
-  return "?";
-}
+const char* const kSelfAttnName[] = {"Fused", "Rowwise", "Tiled", "Long"};  // indexed by SelfAttn
+
+enum class EncFfn { Rows, Gemm };
+// output: digit argmax GEMM (gemm_out_ext.cu), bound-filter argmax GEMM (gemm_out.cu), or logits tap + argmax_rows
+enum class Out { Digits, Bounds, Logits };
 
 struct Routes {
   SelfAttn self;
   Cross cross;
+  EncFfn ffn;
+  Out out;
 };
 
-// Which kernel runs the encoder's self-attention and the decoder's cross-attention for one forward call.  The two
-// environment variables are read on every call, so that tests can switch kernels between calls; a value not listed
-// below means the default.
-Routes choose_routes(int E, int H, int dh, int T, int B, bool fast) {
+// Which kernel runs each stage of one forward call that has more than one.  The two environment variables are read on
+// every call, so that tests can switch kernels between calls; a value not listed below means the default.
+Routes choose_routes(const Model& m, int T, int B, bool fast, bool logits) {
+  const int E = m.E, H = m.H, dh = m.dh;
   auto env_is = [](const char* env, const char* v) { return env != nullptr && strcmp(env, v) == 0; };
   Routes r{};
   // SLIMT_B200_SELFATTN = split keeps the projections and the attention as separate kernels; rowwise | tiled | long
@@ -683,28 +705,61 @@ Routes choose_routes(int E, int H, int dh, int T, int B, bool fast) {
   // long sentences (65 .. 256 tokens) take the sentence-at-a-time recompute kernel (cross_attention_rcl.cu; bit-exact mode)
   else if (!fast && cross_attention_rcl_supported(E, H, dh, T)) r.cross = Cross::Rcl;
   else r.cross = Cross::Cached;
+
+  // Wo + residual + LN, FFN1 + ReLU, FFN2 + residual + LN in one row-tile kernel, 128 rows per CTA
+  r.ffn = E == 256 && m.F == 1536 ? EncFfn::Rows : EncFfn::Gemm;
+
+  // a caller that wants the logits gets them from the tap; otherwise the fused argmax GEMM, with the digits wherever
+  // every column's offset fits them (Model::load sets ext_ok)
+  if (logits) r.out = Out::Logits;
+  else if (m.out.ext_ok) r.out = Out::Digits;
+  else r.out = Out::Bounds;
   return r;
 }
 
-}  // namespace
-
 // ------------------------------------------------------------------ Model::forward
-int model_forward(Model& m, ForwardArgs& a) { return model_forward_on(m, *m.ctx, a); }
+// What the stages of one forward call share: its shape, its routes, its workspace buffers and their tensor maps.
+// Built as Pass{m, c, a, c.stream}, which value-initialises the rest: a buffer no chosen route reads stays null.
+struct Pass {
+  Model& m;
+  Context& c;
+  ForwardArgs& a;
+  cudaStream_t s;
+  int B, T, R, E, F, H, dh, Le, Ld, max_steps, Nout;  // Nout: with a lazy shortlist the vocabulary until its callback
+  double src_tokens;
+  bool lazy_sl, use_sl;
+  Routes route;
+  // batch inputs and outputs: workspace copies with host buffers, the caller's buffers with device_io
+  uint32_t *d_tokens, *d_lengths, *d_steps, *d_forced, *d_sl, *d_rows, *tgt_len;
+  // encoder; Kc/Vc: the cross K/V projected once per decoder layer (Cross::Cached)
+  float *x0, *x1, *Qb, *Kb, *Vb, *Kc[2], *Vc[2];
+  int8_t *qa[4], *attn_q, *ffn_q;
+  // decoder state (Model.cc:111-185); counters: [0] n_done, [1] step counter, [2] ticket
+  float *xd, *hb, *qd, *zb, *state[2], *d_logits, *d_align_all;  // zb: the first of two decoder layers' output
+  int8_t *xq[2], *zq[2], *caq, *oq;
+  unsigned long long* best;
+  uint8_t *done, *exts;
+  int *counters, *flag;
+  // the output layer's columns: the model's, or the shortlist's (gathered, with what the output route reads of them)
+  int8_t* Wout;
+  float *pb_out, *dmax_out;
+  int32_t *c127_out, *ipb6_out, *dshift_out;
+  CUtensorMap map_attn_q;  // u8 [R][E], box {128 B, 128 rows}: operand of the encoder's row-tile kernel
+  CUtensorMap map_qa[3], map_qa32[3], mapK[2], mapV[2];
+  CUtensorMap map_xq[2], map_zq[2], map_caq;  // u8 activation operands of the row-tile kernels, box {128 B, 32 rows}
+  CUtensorMap map_oq, map_wout, map_ext;
+  const char* trace_path;  // SLIMT_B200_TRACE
+  long long* trace_buf;
+  size_t trace_n;
+  int plan(), encode(), prepare_cross(), prepare_output(), decode_step(int step), decode();
+};
 
-int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
-  std::lock_guard<std::recursive_mutex> ctx_lock(c.mu);
-  if (c.device != m.ctx->device) {
-    set_error("model_forward: the lane context and the model live on different devices");
-    return 1;
-  }
-  SB_CUDA(cudaSetDevice(c.device));
-  cudaStream_t s = c.stream;
-  const int B = static_cast<int>(a.B), T = static_cast<int>(a.T), E = m.E, F = m.F, H = m.H, dh = m.dh;
-  const int R = B * T;
-  const int Le = static_cast<int>(m.enc.size()), Ld = static_cast<int>(m.dec.size());
-  a.steps = 0;
-  a.target_tokens = 0;
-  if (B == 0 || T == 0) return 0;
+// Checks the request, chooses the routes and plans the workspace: each buffer is listed once, under the condition in
+// which the chosen routes read it.
+int Pass::plan() {
+  B = static_cast<int>(a.B), T = static_cast<int>(a.T), E = m.E, F = m.F, H = m.H, dh = m.dh;
+  R = B * T;
+  Le = static_cast<int>(m.enc.size()), Ld = static_cast<int>(m.dec.size());
   if (T > m.max_len()) {
     set_error("sequence length " + std::to_string(T) + " exceeds the supported maximum of " + std::to_string(m.max_len()));
     return 1;
@@ -715,8 +770,8 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
   }
   // Model.cc:160: size_t max_seq_length = limit_factor * source_sequence_length (float product, truncated).  The first
   // decoder step runs before that loop (Model.cc:145-157), so at least one step is always executed and recorded.
-  const int max_steps = forward_max_steps(a.limit_factor, a.T);
-  double src_tokens = static_cast<double>(R);  // cross-attention reads only valid keys; exact count when lengths are on the host
+  max_steps = forward_max_steps(a.limit_factor, a.T);
+  src_tokens = static_cast<double>(R);  // cross-attention reads only valid keys; exact count when lengths are on the host
   if (!a.device_io || c.profiling) {
     // per-kernel accounting only (profiling passes are never timed): with device-resident input the lengths are fetched
     std::vector<uint32_t> lens_h(B);
@@ -729,86 +784,85 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
     src_tokens = 0;
     for (int b = 0; b < B; b++) src_tokens += std::min<uint32_t>(lp[b], T);
   }
-  const bool lazy_sl = a.shortlist == nullptr && a.shortlist_cb != nullptr && !a.device_io;
-  const bool use_sl = lazy_sl || (a.shortlist != nullptr && a.n_shortlist > 0);
-  int Nout = use_sl && !lazy_sl ? static_cast<int>(a.n_shortlist) : m.V;  // lazy: upper bound until the callback ran
+  lazy_sl = a.shortlist == nullptr && a.shortlist_cb != nullptr && !a.device_io;
+  use_sl = lazy_sl || (a.shortlist != nullptr && a.n_shortlist > 0);
+  Nout = use_sl && !lazy_sl ? static_cast<int>(a.n_shortlist) : m.V;  // lazy: upper bound until the callback ran
   if (use_sl && !lazy_sl && a.n_shortlist % 8 != 0) {
     set_error("shortlist size must be a multiple of 8");
     return 1;
   }
+  route = choose_routes(m, T, B, c.fast, a.logits != nullptr);
 
-  // ---- workspace
-  size_t need = 0;
-  auto acc = [&need](size_t bytes) { need += (bytes + 255) & ~size_t(255); };
-  acc(4ul * R), acc(4ul * B);                                   // tokens, lengths
-  acc(4ul * R * E), acc(4ul * R * E);                           // x0, x1
-  for (int i = 0; i < 4; i++) acc(1ul * R * E);                 // qa[4]
-  for (int i = 0; i < 3; i++) acc(4ul * R * E);                 // Q K V
-  acc(1ul * R * E), acc(1ul * R * F);                           // attn_q, ffn_q
-  for (int i = 0; i < 2 * Ld; i++) acc(4ul * R * E);            // cross K/V caches
-  for (int i = 0; i < 9 + Ld; i++) acc(4ul * B * E);            // decode f32 rows
-  for (int i = 0; i < 8; i++) acc(1ul * B * E);                 // decode int8 rows
-  acc(1ul * B * F);
-  acc(8ul * B), acc(B), acc(4ul * B), acc(256);                 // best, done, tgt_len, counters
-  acc(4ul * max_steps * B);                        // step tokens
-  if (a.forced) acc(4ul * max_steps * B);
-  if (a.sentence_tokens) acc(4ul * max_steps * B);
-  if (use_sl) acc(4ul * Nout), acc(1ul * Nout * E), acc(4ul * Nout), acc(4ul * Nout), acc(4ul * (Nout / 32 + 1)), acc(4ul * (Nout + 256)), acc(128ul * (Nout + 256)), acc(4ul * (Nout + 256)), acc(256);
-  if (a.logits) acc(4ul * B * Nout);
-  if (a.alignment) acc(4ul * max_steps * B * T);
-  need += 64 * 256;
-  if (c.reserve(need)) return 1;
-
-  uint32_t* d_tokens = nullptr;
-  uint32_t* d_lengths = nullptr;
+  const size_t RE = static_cast<size_t>(R) * E, BE = static_cast<size_t>(B) * E;
+  const size_t SB = static_cast<size_t>(max_steps) * B, N = static_cast<size_t>(Nout);
+  // the output layer's columns are the model's unless the shortlist's are listed below
+  Wout = m.out.w, pb_out = m.out.pb, c127_out = m.out.c127, dmax_out = m.out.dmax, ipb6_out = m.out.ipb6;
+  dshift_out = m.out.dshift, map_ext = m.out.map_ext;
+  Workspace ws;
+  if (!a.device_io) ws.add(d_tokens, R), ws.add(d_lengths, B);
+  ws.add(x0, RE), ws.add(x1, RE);
+  for (int i = 0; i < std::max(3, 2 * Ld); i++) ws.add(qa[i], RE);  // encoder q/k/v inputs, decoder layers' K/V inputs
+  if (route.self != SelfAttn::Fused) ws.add(Qb, RE), ws.add(Kb, RE), ws.add(Vb, RE);
+  ws.add(attn_q, RE);
+  if (route.ffn == EncFfn::Gemm) ws.add(ffn_q, static_cast<size_t>(R) * F);
+  for (int l = 0; l < Ld && route.cross == Cross::Cached; l++) ws.add(Kc[l], RE), ws.add(Vc[l], RE);
+  ws.add(xd, BE), ws.add(hb, BE), ws.add(qd, BE), ws.add(zb, BE);
+  for (int l = 0; l < Ld; l++) ws.add(state[l], BE);
+  ws.add(xq[0], BE), ws.add(xq[1], BE), ws.add(zq[0], BE), ws.add(zq[1], BE), ws.add(caq, BE), ws.add(oq, BE);
+  ws.add(best, B), ws.add(done, B), ws.add(tgt_len, B), ws.add(counters, 64);
+  if (!a.device_io) {
+    ws.add(d_steps, SB);
+    if (a.forced) ws.add(d_forced, SB);
+  }
+  if (use_sl) {
+    if (!a.device_io) ws.add(d_sl, N);
+    ws.add(Wout, N * E), ws.add(pb_out, N), ws.add(c127_out, N);
+    if (route.out == Out::Bounds && !c.fast) ws.add(dmax_out, N / 32 + 1);
+    if (route.out == Out::Bounds && c.fast) ws.add(ipb6_out, N + 256);  // read by 256-column tiles
+    if (route.out == Out::Digits) ws.add(exts, 128 * (N + 256)), ws.add(dshift_out, N + 256), ws.add(flag, 64);
+  }
+  if (route.out == Out::Logits) ws.add(d_logits, static_cast<size_t>(B) * N);
+  // head-0 probabilities of every step stay on the device and come back in one copy after the loop
+  if (a.alignment) ws.add(d_align_all, SB * T);
+  if (!a.device_io && a.sentence_tokens) ws.add(d_rows, SB);
+  if (ws.carve(c)) return 1;
   if (a.device_io) {
-    d_tokens = const_cast<uint32_t*>(a.tokens);
-    d_lengths = const_cast<uint32_t*>(a.lengths);
-    c.take<uint32_t>(R), c.take<uint32_t>(B);
-  } else {
-    d_tokens = c.take<uint32_t>(R);
-    d_lengths = c.take<uint32_t>(B);
-    SB_CUDA(cudaMemcpyAsync(d_tokens, a.tokens, 4ul * R, cudaMemcpyHostToDevice, s));
-    SB_CUDA(cudaMemcpyAsync(d_lengths, a.lengths, 4ul * B, cudaMemcpyHostToDevice, s));
-    c.h2d_bytes += 4ul * R + 4ul * B;
-  }
-  float* x0 = c.take<float>(static_cast<size_t>(R) * E);
-  float* x1 = c.take<float>(static_cast<size_t>(R) * E);
-  int8_t* qa[4];
-  for (auto& p : qa) p = c.take<int8_t>(static_cast<size_t>(R) * E);
-  float* Qb = c.take<float>(static_cast<size_t>(R) * E);
-  float* Kb = c.take<float>(static_cast<size_t>(R) * E);
-  float* Vb = c.take<float>(static_cast<size_t>(R) * E);
-  int8_t* attn_q = c.take<int8_t>(static_cast<size_t>(R) * E);
-  int8_t* ffn_q = c.take<int8_t>(static_cast<size_t>(R) * F);
-  std::vector<float*> Kc(Ld), Vc(Ld);
-  std::vector<CUtensorMap> mapKc(Ld), mapVc(Ld);
-  for (int l = 0; l < Ld; l++) {
-    Kc[l] = c.take<float>(static_cast<size_t>(R) * E);
-    Vc[l] = c.take<float>(static_cast<size_t>(R) * E);
-    const uint32_t box_rows = static_cast<uint32_t>(cross_attention_box_rows(T));
-    if (c.make_map_f32(&mapKc[l], Kc[l], R, E, box_rows) || c.make_map_f32(&mapVc[l], Vc[l], R, E, box_rows)) return 1;
+    d_tokens = const_cast<uint32_t*>(a.tokens), d_lengths = const_cast<uint32_t*>(a.lengths), d_steps = a.step_tokens;
+    d_forced = const_cast<uint32_t*>(a.forced), d_sl = use_sl ? const_cast<uint32_t*>(a.shortlist) : nullptr;
   }
 
-  CUtensorMap map_attn_q;  // u8 [R][E], box {128 B, 128 rows}: operand of the encoder's row-tile kernel
-  if (c.make_map(&map_attn_q, attn_q, R, E, 128)) return 1;
-
-  const Routes route = choose_routes(E, H, dh, T, B, c.fast);
-  CUtensorMap map_qa[3], map_qa32[3];
+  // cross-attention K/V operands: projected once (Cross::Cached), or the u8 encoder output the recompute kernels read
+  const uint32_t box_rows = static_cast<uint32_t>(cross_attention_box_rows(T));
+  for (int l = 0; l < Ld; l++)
+    if (route.cross == Cross::Cached
+            ? c.make_map_f32(&mapK[l], Kc[l], R, E, box_rows) || c.make_map_f32(&mapV[l], Vc[l], R, E, box_rows)
+            : c.make_map(&mapK[l], qa[2 * l], R, E, 32) || c.make_map(&mapV[l], qa[2 * l + 1], R, E, 32))
+      return 1;
+  if (route.ffn == EncFfn::Rows && c.make_map(&map_attn_q, attn_q, R, E, 128)) return 1;
   if (route.self == SelfAttn::Fused)
     for (int i = 0; i < 3; i++)
       if (c.make_map(&map_qa[i], qa[i], R, E, 128) || c.make_map(&map_qa32[i], qa[i], R, E, 32)) return 1;
+  for (int i = 0; i < 2; i++)
+    if (c.make_map(&map_xq[i], xq[i], B, E, kRowTile) || c.make_map(&map_zq[i], zq[i], B, E, kRowTile)) return 1;
+  if (c.make_map(&map_caq, caq, B, E, kRowTile) || c.make_map(&map_oq, oq, B, E, kBM)) return 1;
 
   // debugging aid: SLIMT_B200_TRACE=<file> records the phase stamps of the row-tile kernels: the encoder's first FFN
   // launch (first tile of every CTA) and the two decoder kernels of layer 0 in decode step 3
-  const char* trace_path = getenv("SLIMT_B200_TRACE");
-  long long* trace_buf = nullptr;
-  const size_t trace_n = static_cast<size_t>(c.num_sms) * kTraceSlots;
+  trace_path = getenv("SLIMT_B200_TRACE");
+  trace_n = static_cast<size_t>(c.num_sms) * kTraceSlots;
   if (trace_path) {
     SB_CUDA(cudaMallocManaged(&trace_buf, 5 * trace_n * sizeof(long long)));
     SB_CUDA(cudaMemsetAsync(trace_buf, 0, 5 * trace_n * sizeof(long long), s));
   }
+  return 0;
+}
 
+int Pass::encode() {
+  if (!a.device_io) {
+    SB_CUDA(cudaMemcpyAsync(d_tokens, a.tokens, 4ul * R, cudaMemcpyHostToDevice, s));
+    SB_CUDA(cudaMemcpyAsync(d_lengths, a.lengths, 4ul * B, cudaMemcpyHostToDevice, s));
+    c.h2d_bytes += 4ul * R + 4ul * B;
+  }
   // ---- embedding (Model.cc:195-197)
   {
     QuantOuts q = qouts();
@@ -842,16 +896,15 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
       }
     } else {
       {
-      GemmCall g(&c, "enc_gemm_qkv_f32", R, E, E, EPI_F32, 3);
-      GemmProblem* pq = g.add(qa[0], L.self.q);
-      GemmProblem* pk = g.add(qa[1], L.self.k);
-      GemmProblem* pv = g.add(qa[2], L.self.v);
-      if (!pq || !pk || !pv) return 1;
-      pq->out = Qb, pk->out = Kb, pv->out = Vb;
-      pq->ldo = pk->ldo = pv->ldo = E;
-      if (g.launch()) return 1;
-    }
-    {
+        GemmCall g(&c, "enc_gemm_qkv_f32", R, E, E, EPI_F32, 3);
+        GemmProblem* pq = g.add(qa[0], L.self.q);
+        GemmProblem* pk = g.add(qa[1], L.self.k);
+        GemmProblem* pv = g.add(qa[2], L.self.v);
+        if (!pq || !pk || !pv) return 1;
+        pq->out = Qb, pk->out = Kb, pv->out = Vb;
+        pq->ldo = pk->ldo = pv->ldo = E;
+        if (g.launch()) return 1;
+      }
       QuantOuts q = qouts();
       qadd(q, attn_q, L.self.o.aq);
       LaunchScope ls(c, "enc_self_attention", 0, 13.0 * R * E);
@@ -863,14 +916,12 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
         case SelfAttn::Fused: break;
       }
       if (rc) {
-        set_error(std::string("self-attention: the ") + route_name(route.self) + " kernel does not take head size " +
-                  std::to_string(dh) + " at sequence length " + std::to_string(T));
+        set_error(std::string("self-attention: the ") + kSelfAttnName[static_cast<int>(route.self)] +
+                  " kernel does not take head size " + std::to_string(dh) + " at sequence length " + std::to_string(T));
         return 1;
       }
     }
-    }
-    if (E == 256 && F == 1536) {
-      // Wo + residual + LN, FFN1 + ReLU, FFN2 + residual + LN in one row-tile kernel, 128 rows per CTA
+    if (route.ffn == EncFfn::Rows) {
       RowsFfnArgs k{};
       k.map_a = map_attn_q;
       k.map_wo = L.self.o.map128, k.map_w1 = L.ffn.w1.map128, k.map_w2 = L.ffn.w2.map128;
@@ -947,13 +998,11 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
     SB_CUDA(cudaMemcpyAsync(a.encoder_out, x0, 4ul * R * E, cudaMemcpyDeviceToHost, s));
     c.d2h_bytes += 4ul * R * E;
   }
+  return 0;
+}
 
-  // ---- cross-attention K/V: the recompute kernels read the u8 encoder output, the cached kernel K and V projected here
-  std::vector<CUtensorMap> mapAk(Ld), mapAv(Ld);
-  if (route.cross != Cross::Cached) {
-    for (int l = 0; l < Ld; l++)
-      if (c.make_map(&mapAk[l], qa[2 * l], R, E, 32) || c.make_map(&mapAv[l], qa[2 * l + 1], R, E, 32)) return 1;
-  }
+// Cross-attention K/V for the cached kernel, projected once here (the recompute kernels read the u8 encoder output).
+int Pass::prepare_cross() {
   for (int l = 0; l < Ld && route.cross == Cross::Cached; l++) {
     GemmCall g(&c, "dec_gemm_cross_kv_f32", R, E, E, EPI_F32, 2);
     GemmProblem* pk = g.add(qa[2 * l], m.dec[l].ctx.k);
@@ -963,46 +1012,14 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
     pk->ldo = pv->ldo = E;
     if (g.launch()) return 1;
   }
+  return 0;
+}
 
-  // ---- decoder state (Model.cc:111-185)
-  float* xd = c.take<float>(static_cast<size_t>(B) * E);
-  float* fb = c.take<float>(static_cast<size_t>(B) * E);
-  float* wxb = c.take<float>(static_cast<size_t>(B) * E);
-  float* hb = c.take<float>(static_cast<size_t>(B) * E);
-  float* qd = c.take<float>(static_cast<size_t>(B) * E);
-  float* yb = c.take<float>(static_cast<size_t>(B) * E);
-  float* zb[2] = {c.take<float>(static_cast<size_t>(B) * E), c.take<float>(static_cast<size_t>(B) * E)};
-  c.take<float>(static_cast<size_t>(B) * E);
-  std::vector<float*> state(Ld);
-  for (int l = 0; l < Ld; l++) state[l] = c.take<float>(static_cast<size_t>(B) * E);
-  int8_t* xq[2] = {c.take<int8_t>(static_cast<size_t>(B) * E), c.take<int8_t>(static_cast<size_t>(B) * E)};
-  int8_t* zq[2] = {c.take<int8_t>(static_cast<size_t>(B) * E), c.take<int8_t>(static_cast<size_t>(B) * E)};
-  int8_t* hq = c.take<int8_t>(static_cast<size_t>(B) * E);
-  int8_t* caq = c.take<int8_t>(static_cast<size_t>(B) * E);
-  int8_t* yq = c.take<int8_t>(static_cast<size_t>(B) * E);
-  int8_t* oq = c.take<int8_t>(static_cast<size_t>(B) * E);
-  int8_t* fq = c.take<int8_t>(static_cast<size_t>(B) * F);
-  unsigned long long* best = c.take<unsigned long long>(B);
-  uint8_t* done = c.take<uint8_t>(B);
-  uint32_t* tgt_len = c.take<uint32_t>(B);
-  int* counters = c.take<int>(64);  // [0] n_done, [1] step counter, [2] ticket
-  uint32_t* d_steps = nullptr;
-  if (a.device_io) {
-    d_steps = a.step_tokens;
-    c.take<uint32_t>(static_cast<size_t>(max_steps) * B);
-  } else {
-    d_steps = c.take<uint32_t>(static_cast<size_t>(max_steps) * B);
-  }
-  const uint32_t* d_forced = nullptr;
-  if (a.forced) {
-    if (a.device_io) {
-      d_forced = a.forced;
-    } else {
-      uint32_t* t = c.take<uint32_t>(static_cast<size_t>(max_steps) * B);
-      SB_CUDA(cudaMemcpyAsync(t, a.forced, 4ul * max_steps * B, cudaMemcpyHostToDevice, s));
-      c.h2d_bytes += 4ul * max_steps * B;
-      d_forced = t;
-    }
+// The output layer's columns: the model's, or the shortlist's gathered once per batch with what the route reads.
+int Pass::prepare_output() {
+  if (a.forced && !a.device_io) {
+    SB_CUDA(cudaMemcpyAsync(d_forced, a.forced, 4ul * max_steps * B, cudaMemcpyHostToDevice, s));
+    c.h2d_bytes += 4ul * max_steps * B;
   }
   if (lazy_sl) {
     // the encoder and the cross K/V projections are already queued: build the candidate set meanwhile
@@ -1016,64 +1033,161 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
     a.shortlist = words, a.n_shortlist = n;
     Nout = static_cast<int>(n);
   }
-  const uint32_t* d_sl = nullptr;
-  const int8_t* Wout = m.out.w;
-  const float* pb_out = m.out.pb;
-  const int32_t* c127_out = m.out.c127;
-  const float* dmax_out = m.out.dmax;
-  const int32_t* ipb6_out = m.out.ipb6;
-  const int32_t* dshift_out = m.out.dshift;
-  CUtensorMap map_ext = m.out.map_ext;
-  const bool out_ext = m.out.ext_ok;
   if (use_sl) {
-    if (a.device_io) {
-      d_sl = a.shortlist;
-      c.take<uint32_t>(Nout);
-    } else {
-      uint32_t* t = c.take<uint32_t>(Nout);
-      SB_CUDA(cudaMemcpyAsync(t, a.shortlist, 4ul * Nout, cudaMemcpyHostToDevice, s));
+    if (!a.device_io) {
+      SB_CUDA(cudaMemcpyAsync(d_sl, a.shortlist, 4ul * Nout, cudaMemcpyHostToDevice, s));
       c.h2d_bytes += 4ul * Nout;
-      d_sl = t;
     }
     // SelectColumnsB + bias gather, once per batch (qmm/Intgemm.inl.cc:49-66)
-    int8_t* Ws = c.take<int8_t>(static_cast<size_t>(Nout) * E);
-    float* pbs = c.take<float>(Nout);
-    int32_t* cs = c.take<int32_t>(Nout);
-    float* dms = c.take<float>(Nout / 32 + 1);
     {
       LaunchScope ls(c, "gather_rows", 0, 2.0 * Nout * E);
-      launch_gather_rows(m.out.w, m.out.pb, m.out.c127, d_sl, Nout, E, Ws, pbs, cs, s);
+      launch_gather_rows(m.out.w, m.out.pb, m.out.c127, d_sl, Nout, E, Wout, pb_out, c127_out, s);
     }
-    {
-      LaunchScope ls(c, "out_bounds", 0, 8.0 * Nout);
-      launch_out_bounds(cs, pbs, m.out.um, Nout, dms, s);
-    }
-    int32_t* ips = c.take<int32_t>(static_cast<size_t>(Nout) + 256);
-    uint8_t* exts = c.take<uint8_t>(128ul * (static_cast<size_t>(Nout) + 256));
-    int32_t* dss = c.take<int32_t>(static_cast<size_t>(Nout) + 256);
-    int* flag = c.take<int>(64);
-    if (out_ext) {
+    if (route.out == Out::Digits) {
       // a subset of columns whose offsets all fit the digits fits them too: the flag is not read back
       LaunchScope ls(c, "out_bounds", 0, 140.0 * Nout);
-      launch_out_ext(cs, pbs, m.out.um, Nout, exts, dss, flag, s);
+      launch_out_ext(c127_out, pb_out, m.out.um, Nout, exts, dshift_out, flag, s);
       if (c.make_map(&map_ext, exts, static_cast<uint64_t>((Nout + 255) / 256 * 256), 128, 256)) return 1;
-    } else if (c.fast) {
+    } else if (route.out == Out::Bounds && c.fast) {
       LaunchScope ls(c, "out_bounds", 0, 12.0 * Nout);
-      launch_out_ipb(cs, pbs, m.out.um, Nout, ips, s);
+      launch_out_ipb(c127_out, pb_out, m.out.um, Nout, ipb6_out, s);
+    } else if (route.out == Out::Bounds) {
+      LaunchScope ls(c, "out_bounds", 0, 8.0 * Nout);
+      launch_out_bounds(c127_out, pb_out, m.out.um, Nout, dmax_out, s);
     }
-    Wout = Ws, pb_out = pbs, c127_out = cs, dmax_out = dms, ipb6_out = ips, dshift_out = dss;
   }
-  CUtensorMap map_xq[2], map_zq[2], map_caq;  // u8 activation operands of the row-tile kernels, box {128 B, 32 rows}
-  for (int i = 0; i < 2; i++) {
-    if (c.make_map(&map_xq[i], xq[i], B, E, kRowTile) || c.make_map(&map_zq[i], zq[i], B, E, kRowTile)) return 1;
-  }
-  if (c.make_map(&map_caq, caq, B, E, kRowTile)) return 1;
-  CUtensorMap map_oq, map_wout;
-  if (c.make_map(&map_oq, oq, B, E, kBM) || c.make_map(&map_wout, Wout, Nout, E, 256)) return 1;
-  float* d_logits = a.logits ? c.take<float>(static_cast<size_t>(B) * Nout) : nullptr;
-  // head-0 probabilities of every step stay on the device and come back in one copy after the loop
-  float* d_align_all = a.alignment ? c.take<float>(static_cast<size_t>(max_steps) * B * T) : nullptr;
+  return c.make_map(&map_wout, Wout, Nout, E, 256);
+}
 
+// One decoder step: the decoder layers and the output projection with the greedy choice.
+int Pass::decode_step(int step) {
+  float* d_align = d_align_all ? d_align_all + static_cast<size_t>(step) * B * T : nullptr;
+  for (int l = 0; l < Ld; l++) {
+    const DecLayerW& L = m.dec[l];
+    const bool last = (l + 1 == Ld);
+    {  // SSRU cell + query projection in one row-tile kernel (Modules.cc:190-235, 291)
+      DecSsruArgs k{};
+      k.map_xf = l == 0 ? map_xq[0] : map_zq[0];
+      k.map_xw = l == 0 ? map_xq[1] : map_zq[1];
+      k.map_wf = L.rnn_wf.map128, k.map_w = L.rnn_w.map128, k.map_wq = L.ctx.q.map128;
+      k.pb_f = L.rnn_wf.pb, k.pb_w = L.rnn_w.pb, k.pb_q = L.ctx.q.pb;
+      k.um_f = L.rnn_wf.um, k.um_w = L.rnn_w.um, k.um_q = L.ctx.q.um;
+      k.aq_q = L.ctx.q.aq;
+      k.x = l == 0 ? xd : zb, k.state = state[l];
+      if (l == 0 && step > 0) {  // close the previous step and embed its words in this kernel's front
+        k.embed = 1, k.prev_step = step - 1;
+        k.best = best, k.shortlist = d_sl, k.forced = d_forced, k.step_tokens = d_steps;
+        k.done = done, k.tgt_len = tgt_len, k.n_done = counters, k.eos_id = m.eos_id;
+        k.emb_q = m.emb_q, k.inv_qm = m.inv_qm, k.sqrt_e = m.sqrt_e, k.pos0 = m.pos;
+        k.aq_xf = L.rnn_wf.aq, k.aq_xw = L.rnn_w.aq;
+      }
+      k.ln_scale = L.rnn_ln.scale, k.ln_bias = L.rnn_ln.bias, k.eps = 1e-6f;
+      k.h_out = hb, k.q_out = qd, k.M = B;
+      if (trace_buf && step == 3 && l == 0) k.trace = trace_buf;
+      const double Bd = B, Ed = E;
+      LaunchScope ls(c, "dec_ssru_q_fused", 2.0 * Bd * 3.0 * Ed * Ed, 3.0 * Ed * Ed + Bd * Ed * (2.0 + 4.0 * 5.0));
+      if (launch_dec_ssru(k, E, c.fast, s)) {
+        set_error("fused SSRU kernel: unsupported embedding size " + std::to_string(E));
+        return 1;
+      }
+    }
+    if (route.cross != Cross::Cached) {
+      CrossRcArgs k{};
+      k.map_ak = mapK[l], k.map_av = mapV[l];
+      k.map_wk = L.ctx.k.map128, k.map_wv = L.ctx.v.map128;
+      k.pb_k = L.ctx.k.pb, k.pb_v = L.ctx.v.pb;
+      k.um_k = L.ctx.k.um, k.um_v = L.ctx.v.um;
+      k.q = qd, k.lengths = d_lengths, k.B = B, k.T = T;
+      k.dk = static_cast<float>(1.0 / std::sqrt(static_cast<double>(dh)));
+      k.qo = qouts();
+      qadd(k.qo, caq, L.ctx.o.aq);
+      k.attn_head0 = last ? d_align : nullptr;
+      if (trace_buf && step == 3 && l == 0) k.trace = trace_buf + 3 * trace_n;
+      const double Bd = B, Ed = E;
+      const bool rcl = route.cross == Cross::Rcl;
+      LaunchScope ls(c, "dec_cross_attention_rc", 2.0 * (rcl ? src_tokens : Bd * (T > 32 ? 64.0 : 32.0)) * Ed * 2.0 * Ed,
+                     2.0 * src_tokens * Ed + 2.0 * Ed * Ed + 5.0 * Bd * Ed);  // valid keys only
+      if (rcl ? launch_cross_attention_rcl(k, c.num_sms, s) : launch_cross_attention_rc(k, c.num_sms, c.fast, s)) {
+        set_error("recompute cross-attention launch failed");
+        return 1;
+      }
+    } else {
+      QuantOuts q = qouts();
+      qadd(q, caq, L.ctx.o.aq);
+      LaunchScope ls(c, "dec_cross_attention", 0, 8.0 * src_tokens * E + 5.0 * B * E);
+      if (launch_cross_attention(mapK[l], mapV[l], qd, d_lengths, B, T, H, dh, c.num_sms, q,
+                                 last ? d_align : nullptr, s)) {
+        set_error("cross-attention: no kernel for " + std::to_string(H) + " heads of " + std::to_string(dh) +
+                  " over " + std::to_string(T) + " source tokens");
+        return 1;
+      }
+    }
+    {  // Wo + residual + LN, FFN1 + ReLU, FFN2 + residual + LN in one row-tile kernel (Modules.cc:308-316, 251-257)
+      RowsFfnArgs k{};
+      k.map_a = map_caq;
+      k.map_wo = L.ctx.o.map128, k.map_w1 = L.ffn.w1.map128, k.map_w2 = L.ffn.w2.map128;
+      k.pb_o = L.ctx.o.pb, k.pb_1 = L.ffn.w1.pb, k.pb_2 = L.ffn.w2.pb;
+      k.um_o = L.ctx.o.um, k.um_1 = L.ffn.w1.um, k.um_2 = L.ffn.w2.um;
+      k.aq_1 = L.ffn.w1.aq, k.aq_2 = L.ffn.w2.aq;
+      k.res = hb;
+      k.ln1_scale = L.ctx.ln.scale, k.ln1_bias = L.ctx.ln.bias;
+      k.ln2_scale = L.ffn.ln.scale, k.ln2_bias = L.ffn.ln.bias, k.eps = 1e-6f;
+      if (last) {
+        k.z_out = nullptr;
+        k.zq[0] = reinterpret_cast<uint8_t*>(oq), k.zaq[0] = m.out.aq, k.n_zq = 1;
+        k.zq_signed = route.out == Out::Logits ? 0 : 1;  // the fused argmax GEMMs take the signed qa
+      } else {
+        k.z_out = zb;
+        k.zq[0] = reinterpret_cast<uint8_t*>(zq[0]), k.zaq[0] = m.dec[l + 1].rnn_wf.aq;
+        k.zq[1] = reinterpret_cast<uint8_t*>(zq[1]), k.zaq[1] = m.dec[l + 1].rnn_w.aq;
+        k.n_zq = 2;
+      }
+      k.M = B;
+      if (trace_buf && step == 3 && l == 0) k.trace = trace_buf + trace_n;
+      const double Bd = B, Ed = E, Fd = F;
+      LaunchScope ls(c, "dec_wo_ffn_fused", 2.0 * Bd * (Ed * Ed + 2.0 * Ed * Fd),
+                     Ed * Ed + 2.0 * Ed * Fd + Bd * Ed * (1.0 + 4.0 + (last ? 1.0 : 6.0)));
+      if (launch_rows_ffn(k, E, F, kRowTile, c.fast, s)) {
+        set_error("fused FFN kernel: unsupported sizes E=" + std::to_string(E) + " F=" + std::to_string(F));
+        return 1;
+      }
+    }
+  }
+  // output projection (+ shortlist) and greedy choice (Transformer.cc:176-182, 279-339)
+  if (route.out == Out::Logits) {
+    GemmCall g(&c, "dec_gemm_out_logits", B, Nout, E, EPI_F32);
+    GemmProblem* p = g.add(oq, Wout, pb_out, m.out.um);
+    if (!p) return 1;
+    p->out = d_logits, p->ldo = Nout;
+    if (g.launch()) return 1;
+    {
+      LaunchScope ls(c, "argmax_rows", 0, 4.0 * B * Nout);
+      launch_argmax_rows(d_logits, B, Nout, best, s);
+    }
+    SB_CUDA(cudaMemcpyAsync(a.logits + static_cast<size_t>(step) * B * Nout, d_logits, 4ul * B * Nout,
+                            cudaMemcpyDeviceToHost, s));
+    c.d2h_bytes += 4ul * B * Nout;
+  } else {
+    const double Md = B, Nd = Nout, Kd = E;
+    LaunchScope ls(c, "dec_gemm_out_argmax", 2.0 * Md * Nd * Kd, Md * Kd + Nd * Kd + 4.0 * Nd + 8.0 * Md);
+    const int rc = route.out == Out::Digits
+                       ? launch_gemm_out_argmax_ext(map_oq, map_wout, map_ext, pb_out, dshift_out, m.out.um,
+                                                    c.fast, B, Nout, E, best, c.num_sms, s,
+                                                    (trace_buf && step == 3) ? trace_buf + 4 * trace_n : nullptr)
+                       : launch_gemm_out_argmax(map_oq, map_wout, pb_out, c127_out, dmax_out,
+                                                c.fast ? ipb6_out : nullptr, m.out.um, m.out.eta, B, Nout, E, best,
+                                                c.num_sms, s);
+    if (rc) {
+      set_error("output GEMM: unsupported K " + std::to_string(E));
+      return 1;
+    }
+  }
+  return 0;
+}
+
+// The decode loop (Model.cc:111-185) with its early exit, the kernel that closes the last step, and the result copies.
+int Pass::decode() {
+  int executed = 0, host_done = 0;
   for (int l = 0; l < Ld; l++) SB_CUDA(cudaMemsetAsync(state[l], 0, 4ul * B * E, s));  // Decoder::start_states
   SB_CUDA(cudaMemsetAsync(best, 0, 8ul * B, s));
   SB_CUDA(cudaMemsetAsync(done, 0, B, s));
@@ -1081,138 +1195,15 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
   SB_CUDA(cudaMemsetAsync(counters, 0, 256, s));
 
   // step 0 input: zero embedding + position-0 signal (Transformer.cc:133-160)
+  QuantOuts q = qouts();
+  qadd(q, xq[0], m.dec[0].rnn_wf.aq), qadd(q, xq[1], m.dec[0].rnn_w.aq);
   {
-    QuantOuts q = qouts();
-    qadd(q, xq[0], m.dec[0].rnn_wf.aq), qadd(q, xq[1], m.dec[0].rnn_w.aq);
     LaunchScope ls(c, "dec_embed0", 0, 6.0 * B * E);
     launch_embed(nullptr, m.emb_q, m.inv_qm, m.sqrt_e, m.pos, B, 1, E, 0, 1, xd, q, s);
   }
 
-  int executed = 0;
-  int host_done = 0;
   for (int step = 0; step < max_steps; step++) {
-    float* d_align = d_align_all ? d_align_all + static_cast<size_t>(step) * B * T : nullptr;
-    const float* in_f = xd;
-    for (int l = 0; l < Ld; l++) {
-      const DecLayerW& L = m.dec[l];
-      const bool last = (l + 1 == Ld);
-      {  // SSRU cell + query projection in one row-tile kernel (Modules.cc:190-235, 291)
-        DecSsruArgs k{};
-        k.map_xf = l == 0 ? map_xq[0] : map_zq[0];
-        k.map_xw = l == 0 ? map_xq[1] : map_zq[1];
-        k.map_wf = L.rnn_wf.map128, k.map_w = L.rnn_w.map128, k.map_wq = L.ctx.q.map128;
-        k.pb_f = L.rnn_wf.pb, k.pb_w = L.rnn_w.pb, k.pb_q = L.ctx.q.pb;
-        k.um_f = L.rnn_wf.um, k.um_w = L.rnn_w.um, k.um_q = L.ctx.q.um;
-        k.aq_q = L.ctx.q.aq;
-        k.x = in_f, k.state = state[l];
-        if (l == 0 && step > 0) {  // close the previous step and embed its words in this kernel's front
-          k.embed = 1, k.prev_step = step - 1;
-          k.best = best, k.shortlist = d_sl, k.forced = d_forced, k.step_tokens = d_steps;
-          k.done = done, k.tgt_len = tgt_len, k.n_done = counters, k.eos_id = m.eos_id;
-          k.emb_q = m.emb_q, k.inv_qm = m.inv_qm, k.sqrt_e = m.sqrt_e, k.pos0 = m.pos;
-          k.aq_xf = L.rnn_wf.aq, k.aq_xw = L.rnn_w.aq;
-        }
-        k.ln_scale = L.rnn_ln.scale, k.ln_bias = L.rnn_ln.bias, k.eps = 1e-6f;
-        k.h_out = hb, k.q_out = qd, k.M = B;
-        if (trace_buf && step == 3 && l == 0) k.trace = trace_buf;
-        const double Bd = B, Ed = E;
-        LaunchScope ls(c, "dec_ssru_q_fused", 2.0 * Bd * 3.0 * Ed * Ed, 3.0 * Ed * Ed + Bd * Ed * (2.0 + 4.0 * 5.0));
-        if (launch_dec_ssru(k, E, c.fast, s)) {
-          set_error("fused SSRU kernel: unsupported embedding size " + std::to_string(E));
-          return 1;
-        }
-      }
-      if (route.cross != Cross::Cached) {
-        CrossRcArgs k{};
-        k.map_ak = mapAk[l], k.map_av = mapAv[l];
-        k.map_wk = L.ctx.k.map128, k.map_wv = L.ctx.v.map128;
-        k.pb_k = L.ctx.k.pb, k.pb_v = L.ctx.v.pb;
-        k.um_k = L.ctx.k.um, k.um_v = L.ctx.v.um;
-        k.q = qd, k.lengths = d_lengths, k.B = B, k.T = T;
-        k.dk = static_cast<float>(1.0 / std::sqrt(static_cast<double>(dh)));
-        k.qo = qouts();
-        qadd(k.qo, caq, L.ctx.o.aq);
-        k.attn_head0 = last ? d_align : nullptr;
-        if (trace_buf && step == 3 && l == 0) k.trace = trace_buf + 3 * trace_n;
-        const double Bd = B, Ed = E;
-        const bool rcl = route.cross == Cross::Rcl;
-        LaunchScope ls(c, "dec_cross_attention_rc", 2.0 * (rcl ? src_tokens : Bd * (T > 32 ? 64.0 : 32.0)) * Ed * 2.0 * Ed,
-                       2.0 * src_tokens * Ed + 2.0 * Ed * Ed + 5.0 * Bd * Ed);  // valid keys only
-        if (rcl ? launch_cross_attention_rcl(k, c.num_sms, s) : launch_cross_attention_rc(k, c.num_sms, c.fast, s)) {
-          set_error("recompute cross-attention launch failed");
-          return 1;
-        }
-      } else {
-        QuantOuts q = qouts();
-        qadd(q, caq, L.ctx.o.aq);
-        LaunchScope ls(c, "dec_cross_attention", 0, 8.0 * src_tokens * E + 5.0 * B * E);
-        if (launch_cross_attention(mapKc[l], mapVc[l], qd, d_lengths, B, T, H, dh, c.num_sms, q,
-                                   last ? d_align : nullptr, s)) {
-          set_error("cross-attention: no kernel for " + std::to_string(H) + " heads of " + std::to_string(dh) +
-                    " over " + std::to_string(T) + " source tokens");
-          return 1;
-        }
-      }
-      {  // Wo + residual + LN, FFN1 + ReLU, FFN2 + residual + LN in one row-tile kernel (Modules.cc:308-316, 251-257)
-        RowsFfnArgs k{};
-        k.map_a = map_caq;
-        k.map_wo = L.ctx.o.map128, k.map_w1 = L.ffn.w1.map128, k.map_w2 = L.ffn.w2.map128;
-        k.pb_o = L.ctx.o.pb, k.pb_1 = L.ffn.w1.pb, k.pb_2 = L.ffn.w2.pb;
-        k.um_o = L.ctx.o.um, k.um_1 = L.ffn.w1.um, k.um_2 = L.ffn.w2.um;
-        k.aq_1 = L.ffn.w1.aq, k.aq_2 = L.ffn.w2.aq;
-        k.res = hb;
-        k.ln1_scale = L.ctx.ln.scale, k.ln1_bias = L.ctx.ln.bias;
-        k.ln2_scale = L.ffn.ln.scale, k.ln2_bias = L.ffn.ln.bias, k.eps = 1e-6f;
-        if (last) {
-          k.z_out = nullptr;
-          k.zq[0] = reinterpret_cast<uint8_t*>(oq), k.zaq[0] = m.out.aq, k.n_zq = 1;
-          k.zq_signed = a.logits ? 0 : 1;  // the fused argmax GEMM takes the signed qa (gemm_out.cu)
-        } else {
-          k.z_out = zb[l & 1];
-          k.zq[0] = reinterpret_cast<uint8_t*>(zq[0]), k.zaq[0] = m.dec[l + 1].rnn_wf.aq;
-          k.zq[1] = reinterpret_cast<uint8_t*>(zq[1]), k.zaq[1] = m.dec[l + 1].rnn_w.aq;
-          k.n_zq = 2;
-        }
-        k.M = B;
-        if (trace_buf && step == 3 && l == 0) k.trace = trace_buf + trace_n;
-        const double Bd = B, Ed = E, Fd = F;
-        LaunchScope ls(c, "dec_wo_ffn_fused", 2.0 * Bd * (Ed * Ed + 2.0 * Ed * Fd),
-                       Ed * Ed + 2.0 * Ed * Fd + Bd * Ed * (1.0 + 4.0 + (last ? 1.0 : 6.0)));
-        if (launch_rows_ffn(k, E, F, kRowTile, c.fast, s)) {
-          set_error("fused FFN kernel: unsupported sizes E=" + std::to_string(E) + " F=" + std::to_string(F));
-          return 1;
-        }
-      }
-      in_f = zb[l & 1];
-    }
-    // output projection (+ shortlist) and greedy choice (Transformer.cc:176-182, 279-339)
-    if (d_logits) {
-      GemmCall g(&c, "dec_gemm_out_logits", B, Nout, E, EPI_F32);
-      GemmProblem* p = g.add(oq, Wout, pb_out, m.out.um);
-      if (!p) return 1;
-      p->out = d_logits, p->ldo = Nout;
-      if (g.launch()) return 1;
-      {
-        LaunchScope ls(c, "argmax_rows", 0, 4.0 * B * Nout);
-        launch_argmax_rows(d_logits, B, Nout, best, s);
-      }
-      SB_CUDA(cudaMemcpyAsync(a.logits + static_cast<size_t>(step) * B * Nout, d_logits, 4ul * B * Nout,
-                              cudaMemcpyDeviceToHost, s));
-      c.d2h_bytes += 4ul * B * Nout;
-    } else {
-      const double Md = B, Nd = Nout, Kd = E;
-      LaunchScope ls(c, "dec_gemm_out_argmax", 2.0 * Md * Nd * Kd, Md * Kd + Nd * Kd + 4.0 * Nd + 8.0 * Md);
-      const int rc = out_ext ? launch_gemm_out_argmax_ext(map_oq, map_wout, map_ext, pb_out, dshift_out, m.out.um, c.fast, B,
-                                                          Nout, E, best, c.num_sms, s,
-                                                          (trace_buf && step == 3) ? trace_buf + 4 * trace_n : nullptr)
-                             : launch_gemm_out_argmax(map_oq, map_wout, pb_out, c127_out, dmax_out,
-                                                      c.fast ? ipb6_out : nullptr, m.out.um, m.out.eta, B, Nout, E, best,
-                                                      c.num_sms, s);
-      if (rc) {
-        set_error("output GEMM: unsupported K " + std::to_string(E));
-        return 1;
-      }
-    }
+    if (decode_step(step)) return 1;
     // The step's bookkeeping (argmax -> word, record(), EOS flags) and the next step's input embedding are done by the
     // FRONT of the next step's first kernel (dec_ssru_kernel with embed set); the last executed step is closed by the
     // stand-alone kernel after the loop.
@@ -1235,8 +1226,6 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
     }
   }
   if (executed > 0) {
-    QuantOuts q = qouts();
-    qadd(q, xq[0], m.dec[0].rnn_wf.aq), qadd(q, xq[1], m.dec[0].rnn_w.aq);
     {
       LaunchScope ls(c, "dec_finalize_embed", 0, 7.0 * B * E + 20.0 * B);
       launch_finalize_step(best, d_sl, d_forced, executed - 1, d_steps, done, tgt_len, counters, m.eos_id, m.emb_q, m.inv_qm,
@@ -1248,6 +1237,7 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
     host_done = c.done_slots[0];
   }
 
+  // ---- SLIMT_B200_TRACE file and results
   if (trace_buf) {
     SB_CUDA(cudaStreamSynchronize(s));
     if (FILE* f = fopen(trace_path, "w")) {
@@ -1265,7 +1255,6 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
     cudaFree(trace_buf);
   }
 
-  // ---- results
   std::vector<uint32_t> lens(B);
   SB_CUDA(cudaMemcpyAsync(lens.data(), tgt_len, 4ul * B, cudaMemcpyDeviceToHost, s));
   if (d_align_all && executed > 0) {
@@ -1282,7 +1271,6 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
       return 1;
     }
     // one row per sentence: the host then copies each sentence's recorded prefix without striding through the matrix
-    uint32_t* d_rows = c.take<uint32_t>(static_cast<size_t>(max_steps) * B);
     {
       LaunchScope ls(c, "transpose_steps", 0, 8.0 * executed * B);
       launch_transpose_u32(d_steps, executed, B, d_rows, executed, s);
@@ -1310,6 +1298,24 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
     return 1;
   }
   return 0;
+}
+
+}  // namespace
+
+int model_forward(Model& m, ForwardArgs& a) { return model_forward_on(m, *m.ctx, a); }
+
+int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
+  std::lock_guard<std::recursive_mutex> ctx_lock(c.mu);
+  if (c.device != m.ctx->device) {
+    set_error("model_forward: the lane context and the model live on different devices");
+    return 1;
+  }
+  SB_CUDA(cudaSetDevice(c.device));
+  a.steps = 0;
+  a.target_tokens = 0;
+  if (a.B == 0 || a.T == 0) return 0;
+  Pass p{m, c, a, c.stream};
+  return p.plan() || p.encode() || p.prepare_cross() || p.prepare_output() || p.decode() ? 1 : 0;
 }
 
 }  // namespace sb

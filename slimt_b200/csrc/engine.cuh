@@ -10,7 +10,6 @@
 #include <memory>
 #include <mutex>
 #include <string>
-#include <tuple>
 #include <vector>
 
 #include "fused_rows.cuh"
@@ -51,10 +50,9 @@ struct Context {
   CUresult (*encode_tiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                            const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                            CUtensorMapL2promotion, CUtensorMapFloatOOBfill) = nullptr;
-  // workspace arena (grown on demand, reused across calls)
+  // workspace arena (grown on demand, reused across calls; engine.cu's Workspace cuts it into buffers)
   char* arena = nullptr;
   size_t arena_bytes = 0;
-  size_t arena_used = 0;
   char* flush_buf = nullptr;
   size_t flush_bytes = 0;
   // pinned host staging of the service path (padded batch in, step tokens out): grown on demand, reused across calls
@@ -80,13 +78,6 @@ struct Context {
   int init(int dev);
   void destroy();
   int reserve(size_t bytes);
-  template <class T>
-  T* take(size_t count) {
-    size_t bytes = (count * sizeof(T) + 255) & ~size_t(255);
-    T* p = reinterpret_cast<T*>(arena + arena_used);
-    arena_used += bytes;
-    return p;
-  }
   // int8 row-major [rows][cols] -> 2D tensor map, box = {128 bytes, box_rows}, 128B swizzle
   int make_map(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows);
   // f32 row-major [rows][cols] -> 2D tensor map, box = {32 floats (128 bytes), box_rows}, 128B swizzle
@@ -120,7 +111,7 @@ struct DevWeight {
   CUtensorMap map128;       // TMA view of w with box {128 B, 128 rows}: the A operand of the row-tile kernels
   CUtensorMap map32;        // box {128 B, 32 rows}: one head's features, the B operand of the fused encoder attention
   float* pb = nullptr;      // [N]
-  // output layer only: inputs of the fused argmax GEMM's bound filter (gemm_out.cu)
+  // output layer only: inputs of the fused argmax GEMM's bound filter (gemm_out.cu); all but c127 only when !ext_ok
   int32_t* c127 = nullptr;  // [N] 127 * colsum
   float* dmax = nullptr;    // [ceil(N/32)]
   float eta = 0;            // slack covering the float roundings of the exact epilogue

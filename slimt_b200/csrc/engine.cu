@@ -271,6 +271,12 @@ int parse_items(const void* bin, size_t bytes, std::map<std::string, Item>& out)
   return 0;
 }
 
+// The tensor maps of o's weights and, on the digits, of its digit rows.
+int out_maps(Context& c, OutColumns& o, int K) {
+  if (o.digits && c.make_map(&o.map_ext, o.ext, OutColumns::pad(o.N), 128, kOutBN)) return 1;
+  return c.make_map(&o.map_w, o.w, o.N, K, kOutBN);
+}
+
 }  // namespace
 
 int Model::load(Context* c, const void* bin, size_t bytes, int enc_layers, int dec_layers, int heads) {
@@ -288,9 +294,13 @@ int Model::load(Context* c, const void* bin, size_t bytes, int enc_layers, int d
     }
     return &it->second;
   };
-  auto upload = [this](const void* src, size_t nbytes, void** dst) -> int {
+  auto alloc = [this](void** dst, size_t nbytes) -> int {
     SB_CUDA(cudaMalloc(dst, nbytes));
     owned.push_back(*dst);
+    return 0;
+  };
+  auto upload = [&](const void* src, size_t nbytes, void** dst) -> int {
+    if (alloc(dst, nbytes)) return 1;
     SB_CUDA(cudaMemcpy(*dst, src, nbytes, cudaMemcpyHostToDevice));
     ctx->h2d_bytes += nbytes;
     return 0;
@@ -397,44 +407,45 @@ int Model::load(Context* c, const void* bin, size_t bytes, int enc_layers, int d
     std::vector<int8_t> req(deq.size());
     host_quantize(deq.data(), req.data(), emb_qm, deq.size());
     if (weight("Wemb", "decoder_ff_logit_out_b", out, req.data(), "none_QuantMultA")) return 1;
-    // 127 * colsum per column, then the digit rows of gemm_out_ext.cu
-    std::vector<int32_t> c127(V);
+    std::vector<int32_t> c127(V);  // 127 * colsum per column
     for (int n = 0; n < V; n++) {
       int32_t cs = 0;
       for (int k = 0; k < E; k++) cs += req[static_cast<size_t>(n) * E + k];
       c127[n] = 127 * cs;
     }
-    if (upload(c127.data(), 4ul * V, reinterpret_cast<void**>(&out.c127))) return 1;
-    const size_t vpad = static_cast<size_t>((V + 255) / 256 * 256);
+    vocab.N = V, vocab.um = out.um, vocab.w = out.w, vocab.pb = out.pb;
+    if (upload(c127.data(), 4ul * V, reinterpret_cast<void**>(&vocab.c127))) return 1;
+  }
+  // The fused argmax takes the digits when every column's offset fits them (their build reports one that does not),
+  // otherwise the bound filter, whose slack eta covers the float roundings of the exact formula.
+  {
+    int bad = 0;
+    auto alloc_tables = [&] {
+      vocab.tables([&](auto*& p, size_t n) { bad = bad || alloc(reinterpret_cast<void**>(&p), n * sizeof(*p)); });
+      return bad;
+    };
+    vocab.digits = true;
     int* d_flag = nullptr;
-    SB_CUDA(cudaMalloc(&out.ext, vpad * 128));
-    owned.push_back(out.ext);
-    SB_CUDA(cudaMalloc(&out.dshift, vpad * 4));
-    owned.push_back(out.dshift);
+    int flag = 0;
+    if (alloc_tables()) return 1;
     SB_CUDA(cudaMalloc(&d_flag, 4));
     SB_CUDA(cudaMemsetAsync(d_flag, 0, 4, c->stream));
-    launch_out_ext(out.c127, out.pb, out.um, V, out.ext, out.dshift, d_flag, c->stream);
-    int flag = 0;
+    launch_out_tables(vocab, d_flag, c->stream);
     SB_CUDA(cudaMemcpyAsync(&flag, d_flag, 4, cudaMemcpyDeviceToHost, c->stream));
     SB_CUDA(cudaStreamSynchronize(c->stream));
     SB_CUDA(cudaFree(d_flag));
-    out.ext_ok = flag == 0;
-    if (ctx->make_map(&out.map_ext, out.ext, vpad, 128, 256)) return 1;
-  }
-  if (!out.ext_ok) {  // gemm_out.cu's bound filter: per-chunk dmax, proxy offsets, rounding slack eta
-    SB_CUDA(cudaMalloc(&out.dmax, 4ul * ((V + 31) / 32)));
-    owned.push_back(out.dmax);
-    launch_out_bounds(out.c127, out.pb, out.um, V, out.dmax, c->stream);
-    SB_CUDA(cudaMalloc(&out.ipb6, 4ul * ((V + 255) / 256 * 256)));
-    owned.push_back(out.ipb6);
-    launch_out_ipb(out.c127, out.pb, out.um, V, out.ipb6, c->stream);
-    SB_CUDA(cudaStreamSynchronize(c->stream));
-    std::vector<float> pbh(V);
-    SB_CUDA(cudaMemcpy(pbh.data(), out.pb, 4ul * V, cudaMemcpyDeviceToHost));
-    double pbabs = 0;
-    for (float v : pbh) pbabs = std::max(pbabs, static_cast<double>(fabsf(v)));
-    const double vmax = static_cast<double>(E) * 254.0 * 128.0;
-    out.eta = static_cast<float>((2.0 * vmax * out.um + pbabs) * ldexp(1.0, -22));
+    if (flag) {
+      vocab.digits = false;
+      if (alloc_tables()) return 1;
+      launch_out_tables(vocab, nullptr, c->stream);
+      std::vector<float> pbh(V);
+      SB_CUDA(cudaMemcpy(pbh.data(), vocab.pb, 4ul * V, cudaMemcpyDeviceToHost));
+      double pbabs = 0;
+      for (float v : pbh) pbabs = std::max(pbabs, static_cast<double>(fabsf(v)));
+      const double vmax = static_cast<double>(E) * 254.0 * 128.0;
+      vocab.eta = static_cast<float>((2.0 * vmax * vocab.um + pbabs) * ldexp(1.0, -22));
+    }
+    if (out_maps(*ctx, vocab, E)) return 1;
   }
 
   enc.resize(enc_layers);
@@ -660,8 +671,8 @@ enum class Cross { Cached, Rc, Rcl };
 const char* const kSelfAttnName[] = {"Fused", "Rowwise", "Tiled", "Long"};  // indexed by SelfAttn
 
 enum class EncFfn { Rows, Gemm };
-// output: digit argmax GEMM (gemm_out_ext.cu), bound-filter argmax GEMM (gemm_out.cu), or logits tap + argmax_rows
-enum class Out { Digits, Bounds, Logits };
+// output: the fused argmax GEMM (out_argmax.cu, in the encoding Model::load chose), or logits tap + argmax_rows
+enum class Out { Argmax, Logits };
 
 struct Routes {
   SelfAttn self;
@@ -709,11 +720,8 @@ Routes choose_routes(const Model& m, int T, int B, bool fast, bool logits) {
   // Wo + residual + LN, FFN1 + ReLU, FFN2 + residual + LN in one row-tile kernel, 128 rows per CTA
   r.ffn = E == 256 && m.F == 1536 ? EncFfn::Rows : EncFfn::Gemm;
 
-  // a caller that wants the logits gets them from the tap; otherwise the fused argmax GEMM, with the digits wherever
-  // every column's offset fits them (Model::load sets ext_ok)
-  if (logits) r.out = Out::Logits;
-  else if (m.out.ext_ok) r.out = Out::Digits;
-  else r.out = Out::Bounds;
+  // a caller that wants the logits gets them from the tap
+  r.out = logits ? Out::Logits : Out::Argmax;
   return r;
 }
 
@@ -738,16 +746,13 @@ struct Pass {
   float *xd, *hb, *qd, *zb, *state[2], *d_logits, *d_align_all;  // zb: the first of two decoder layers' output
   int8_t *xq[2], *zq[2], *caq, *oq;
   unsigned long long* best;
-  uint8_t *done, *exts;
-  int *counters, *flag;
-  // the output layer's columns: the model's, or the shortlist's (gathered, with what the output route reads of them)
-  int8_t* Wout;
-  float *pb_out, *dmax_out;
-  int32_t *c127_out, *ipb6_out, *dshift_out;
+  uint8_t* done;
+  int* counters;
+  OutColumns out;  // the output layer's columns: the model's, or the shortlist's gathered copy
   CUtensorMap map_attn_q;  // u8 [R][E], box {128 B, 128 rows}: operand of the encoder's row-tile kernel
   CUtensorMap map_qa[3], map_qa32[3], mapK[2], mapV[2];
   CUtensorMap map_xq[2], map_zq[2], map_caq;  // u8 activation operands of the row-tile kernels, box {128 B, 32 rows}
-  CUtensorMap map_oq, map_wout, map_ext;
+  CUtensorMap map_oq;
   const char* trace_path;  // SLIMT_B200_TRACE
   long long* trace_buf;
   size_t trace_n;
@@ -795,9 +800,9 @@ int Pass::plan() {
 
   const size_t RE = static_cast<size_t>(R) * E, BE = static_cast<size_t>(B) * E;
   const size_t SB = static_cast<size_t>(max_steps) * B, N = static_cast<size_t>(Nout);
-  // the output layer's columns are the model's unless the shortlist's are listed below
-  Wout = m.out.w, pb_out = m.out.pb, c127_out = m.out.c127, dmax_out = m.out.dmax, ipb6_out = m.out.ipb6;
-  dshift_out = m.out.dshift, map_ext = m.out.map_ext;
+  // the output layer's columns are the model's unless the shortlist's are listed below; a subset of the columns fits
+  // the model's encoding and its eta
+  out = m.vocab;
   Workspace ws;
   if (!a.device_io) ws.add(d_tokens, R), ws.add(d_lengths, B);
   ws.add(x0, RE), ws.add(x1, RE);
@@ -816,10 +821,9 @@ int Pass::plan() {
   }
   if (use_sl) {
     if (!a.device_io) ws.add(d_sl, N);
-    ws.add(Wout, N * E), ws.add(pb_out, N), ws.add(c127_out, N);
-    if (route.out == Out::Bounds && !c.fast) ws.add(dmax_out, N / 32 + 1);
-    if (route.out == Out::Bounds && c.fast) ws.add(ipb6_out, N + 256);  // read by 256-column tiles
-    if (route.out == Out::Digits) ws.add(exts, 128 * (N + 256)), ws.add(dshift_out, N + 256), ws.add(flag, 64);
+    out.N = Nout;
+    ws.add(out.w, N * E), ws.add(out.pb, N), ws.add(out.c127, N);
+    if (route.out == Out::Argmax) out.tables([&ws](auto*& p, size_t n) { ws.add(p, n); });
   }
   if (route.out == Out::Logits) ws.add(d_logits, static_cast<size_t>(B) * N);
   // head-0 probabilities of every step stay on the device and come back in one copy after the loop
@@ -1039,24 +1043,18 @@ int Pass::prepare_output() {
       c.h2d_bytes += 4ul * Nout;
     }
     // SelectColumnsB + bias gather, once per batch (qmm/Intgemm.inl.cc:49-66)
+    out.N = Nout;
     {
       LaunchScope ls(c, "gather_rows", 0, 2.0 * Nout * E);
-      launch_gather_rows(m.out.w, m.out.pb, m.out.c127, d_sl, Nout, E, Wout, pb_out, c127_out, s);
+      launch_gather_rows(m.vocab.w, m.vocab.pb, m.vocab.c127, d_sl, Nout, E, out.w, out.pb, out.c127, s);
     }
-    if (route.out == Out::Digits) {
-      // a subset of columns whose offsets all fit the digits fits them too: the flag is not read back
-      LaunchScope ls(c, "out_bounds", 0, 140.0 * Nout);
-      launch_out_ext(c127_out, pb_out, m.out.um, Nout, exts, dshift_out, flag, s);
-      if (c.make_map(&map_ext, exts, static_cast<uint64_t>((Nout + 255) / 256 * 256), 128, 256)) return 1;
-    } else if (route.out == Out::Bounds && c.fast) {
-      LaunchScope ls(c, "out_bounds", 0, 12.0 * Nout);
-      launch_out_ipb(c127_out, pb_out, m.out.um, Nout, ipb6_out, s);
-    } else if (route.out == Out::Bounds) {
-      LaunchScope ls(c, "out_bounds", 0, 8.0 * Nout);
-      launch_out_bounds(c127_out, pb_out, m.out.um, Nout, dmax_out, s);
+    if (route.out == Out::Argmax) {
+      LaunchScope ls(c, "out_bounds", 0, (out.digits ? 140.0 : 8.0) * Nout);
+      launch_out_tables(out, nullptr, s);
+      if (out_maps(c, out, E)) return 1;
     }
   }
-  return c.make_map(&map_wout, Wout, Nout, E, 256);
+  return 0;
 }
 
 // One decoder step: the decoder layers and the output projection with the greedy choice.
@@ -1156,7 +1154,7 @@ int Pass::decode_step(int step) {
   // output projection (+ shortlist) and greedy choice (Transformer.cc:176-182, 279-339)
   if (route.out == Out::Logits) {
     GemmCall g(&c, "dec_gemm_out_logits", B, Nout, E, EPI_F32);
-    GemmProblem* p = g.add(oq, Wout, pb_out, m.out.um);
+    GemmProblem* p = g.add(oq, out.w, out.pb, out.um);
     if (!p) return 1;
     p->out = d_logits, p->ldo = Nout;
     if (g.launch()) return 1;
@@ -1170,14 +1168,8 @@ int Pass::decode_step(int step) {
   } else {
     const double Md = B, Nd = Nout, Kd = E;
     LaunchScope ls(c, "dec_gemm_out_argmax", 2.0 * Md * Nd * Kd, Md * Kd + Nd * Kd + 4.0 * Nd + 8.0 * Md);
-    const int rc = route.out == Out::Digits
-                       ? launch_gemm_out_argmax_ext(map_oq, map_wout, map_ext, pb_out, dshift_out, m.out.um,
-                                                    c.fast, B, Nout, E, best, c.num_sms, s,
-                                                    (trace_buf && step == 3) ? trace_buf + 4 * trace_n : nullptr)
-                       : launch_gemm_out_argmax(map_oq, map_wout, pb_out, c127_out, dmax_out,
-                                                c.fast ? ipb6_out : nullptr, m.out.um, m.out.eta, B, Nout, E, best,
-                                                c.num_sms, s);
-    if (rc) {
+    if (launch_out_argmax(out, map_oq, c.fast, B, E, best, c.num_sms, s,
+                          (trace_buf && step == 3) ? trace_buf + 4 * trace_n : nullptr)) {
       set_error("output GEMM: unsupported K " + std::to_string(E));
       return 1;
     }

@@ -15,6 +15,7 @@
 #include "fused_rows.cuh"
 #include "gemm_i8.cuh"
 #include "kernels.cuh"
+#include "out_argmax.cuh"
 
 namespace sb {
 
@@ -111,17 +112,6 @@ struct DevWeight {
   CUtensorMap map128;       // TMA view of w with box {128 B, 128 rows}: the A operand of the row-tile kernels
   CUtensorMap map32;        // box {128 B, 32 rows}: one head's features, the B operand of the fused encoder attention
   float* pb = nullptr;      // [N]
-  // output layer only: inputs of the fused argmax GEMM's bound filter (gemm_out.cu); all but c127 only when !ext_ok
-  int32_t* c127 = nullptr;  // [N] 127 * colsum
-  float* dmax = nullptr;    // [ceil(N/32)]
-  float eta = 0;            // slack covering the float roundings of the exact epilogue
-  int32_t* ipb6 = nullptr;  // [ceil(N/256)*256] integer logit-proxy offsets (tolerance mode, gemm_out.cu)
-  // second-generation output GEMM (gemm_out_ext.cu): digit rows [ceil(N/256)*256][128], proxy -> accumulator shifts,
-  // and whether every column's offset fits the digits (otherwise gemm_out.cu is used)
-  uint8_t* ext = nullptr;
-  int32_t* dshift = nullptr;
-  CUtensorMap map_ext;
-  bool ext_ok = false;
 };
 
 struct DevLN {
@@ -156,6 +146,7 @@ struct Model {
   int8_t* emb_q = nullptr;  // [V][E] stored embedding (lookup: float(q) * (1/qm), Io.cc:275-283)
   float emb_qm = 0, inv_qm = 0, sqrt_e = 0;
   DevWeight out;            // Wemb_intgemm8 (re-quantised embedding) + decoder_ff_logit_out_b + none_QuantMultA
+  OutColumns vocab;         // out's columns as the fused argmax reads them, with the encoding chosen at load
   float* pos = nullptr;     // sinusoidal table [max_pos][E]
   int max_pos = 0;
   uint32_t eos_id = 0, pad_id = 0;  // Vocabulary::eos_id() / pad_id() (Vocabulary.hh:22-23); both 0 for browsermt vocabularies

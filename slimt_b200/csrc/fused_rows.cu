@@ -3,6 +3,7 @@
 
 #include <stdio.h>
 
+#include "packed_best.cuh"
 #include "rows_common.cuh"
 
 namespace sb {
@@ -164,7 +165,7 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
               was_done = a.done[bk];
               len_before = a.tgt_len[bk];
               const uint32_t forced = a.forced ? a.forced[static_cast<size_t>(a.prev_step) * a.M + bk] : 0u;
-              const uint32_t idx = 0xFFFFFFFFu - static_cast<uint32_t>(packed & 0xFFFFFFFFull);
+              const uint32_t idx = best_index(packed);
               word = a.shortlist ? a.shortlist[idx] : idx;
               tok = a.forced ? forced : word;
             }

@@ -6,7 +6,7 @@
 // qmm/Gemmology.inl.cc:33-281): PrepareA is done by the PRODUCER of the
 // activation (it emits int8), PrepareBias is precomputed at load, Multiply is the
 // MMA, UnquantizeAndAddBiasAndWrite (+ReLU / +requantize / +residual+LayerNorm)
-// is the epilogue; the output projection's fused argmax is gemm_out*.cu.
+// is the epilogue; the output projection's fused argmax is out_argmax.cu.
 //
 // Layouts: A = quantized activations as the reference's PrepareA emits them, u8 = qa + 127, [M][K] row-major
 // (K contiguous), so the u8 x s8 MMA forms Int8Shift::Multiply's shifted accumulator directly;
@@ -62,23 +62,5 @@ size_t gemm_smem_bytes(int BN, int stages);
 
 // Launches grid (ceil(N/BN), ceil(M/128), n_problems).
 void launch_gemm_i8(const GemmBatch& batch, int n_problems, int epilogue, int BN, cudaStream_t stream);
-
-// Output projection fused with greedy argmax (gemm_out.cu).  tma_a: SIGNED s8 activations [M][K] with box
-// {128 B, 128 rows}; tma_b: s8 [N][K] with box {128 B, 256 rows}; c127 [N] = 127 * colsum(B); dmax
-// [ceil(N/32)] and eta from launch_out_bounds; best [M] packed (ordered value << 32 | ~index), pre-zeroed.
-// Returns nonzero for an unsupported K (128 * {2, 4} are built).
-// ipb6 != nullptr selects the tolerance-mode epilogue (integer proxy argmax, see gemm_out.cu): ipb6 [ceil(N/256)*256]
-// from launch_out_ipb; pb / c127 / dmax / eta are then unused.
-int launch_gemm_out_argmax(const CUtensorMap& tma_a, const CUtensorMap& tma_b, const float* pb, const int32_t* c127,
-                           const float* dmax, const int32_t* ipb6, float um, float eta, int M, int N, int K,
-                           unsigned long long* best, int num_sms, cudaStream_t stream);
-
-// Second generation (gemm_out_ext.cu): the column offsets ride through the tensor core as an extra K = 32 block.
-// tma_e: the digit rows from launch_out_ext, u8 [ceil(N/256)*256][128] with box {128 B, 256 rows}; dshift from the
-// same call.  fast selects the tolerance-mode choice (integer proxy); otherwise the result is the exact first strict
-// maximum of the float logits.
-int launch_gemm_out_argmax_ext(const CUtensorMap& tma_a, const CUtensorMap& tma_b, const CUtensorMap& tma_e, const float* pb,
-                               const int32_t* dshift, float um, bool fast, int M, int N, int K, unsigned long long* best,
-                               int num_sms, cudaStream_t stream, long long* trace = nullptr);
 
 }  // namespace sb

@@ -2,10 +2,10 @@
 // round-to-nearest intrinsics in the reference's evaluation order.
 #include "kernels.cuh"
 
-#include <limits.h>
 #include <stdio.h>
 
 #include "exact_math.cuh"
+#include "packed_best.cuh"
 #include "ptx.cuh"
 
 namespace sb {
@@ -179,7 +179,7 @@ __global__ void __launch_bounds__(256) finalize_step_kernel(
   uint32_t tok = 0;
   if (lane == 0) {
     const unsigned long long packed = best[b];
-    const uint32_t idx = 0xFFFFFFFFu - static_cast<uint32_t>(packed & 0xFFFFFFFFull);
+    const uint32_t idx = best_index(packed);
     const uint32_t word = shortlist ? shortlist[idx] : idx;
     step_tokens[static_cast<size_t>(step) * B + b] = word;
     if (!done[b]) {  // record(), slimt/Model.cc:127-137: append unless already finished
@@ -222,87 +222,12 @@ __global__ void gather_rows_kernel(const int8_t* __restrict__ W, const float* __
   }
 }
 
-// dmax[chunk] = max over the chunk's 32 columns of (c127[n] * um + pb[n]), rounded up to float: the
-// column-dependent part of the logit upper bound used by the fused output GEMM (gemm_out.cu).
-__global__ void out_bounds_kernel(const int32_t* __restrict__ c127, const float* __restrict__ pb, float um, int N,
-                                  float* __restrict__ dmax) {
-  const int chunk = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  const int lane = threadIdx.x & 31;
-  if (chunk * 32 >= N) return;
-  const int n = chunk * 32 + lane;
-  double d = -1.0e300;
-  if (n < N) d = static_cast<double>(c127[n]) * static_cast<double>(um) + static_cast<double>(pb[n]);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) d = fmax(d, __shfl_xor_sync(0xffffffffu, d, o));
-  if (lane == 0) dmax[chunk] = __double2float_ru(d);
-}
-
-// ipb6[n] = (round(c127[n] + pb[n] / um) << 6) + (63 - n % 64): the per-column offset of the tolerance-mode output
-// GEMM's integer logit proxy (gemm_out.cu), evaluated in double.  Entries from N up to the end of the last 256-column
-// tile get the most negative value that cannot overflow when a zero accumulator is added.
-__global__ void out_ipb_kernel(const int32_t* __restrict__ c127, const float* __restrict__ pb, float um, int N, int n_pad,
-                               int32_t* __restrict__ ipb6) {
-  const int n = blockIdx.x * blockDim.x + threadIdx.x;
-  if (n >= n_pad) return;
-  if (n >= N) {
-    ipb6[n] = INT_MIN + 64;
-    return;
-  }
-  double t = rint(static_cast<double>(c127[n]) + static_cast<double>(pb[n]) / static_cast<double>(um));
-  t = fmin(fmax(t, -16777216.0), 16777216.0);  // |accumulator| < 2^22, so (v' + ipb) << 6 stays inside int32
-  ipb6[n] = (static_cast<int32_t>(t) << 6) + (63 - (n & 63));
-}
-
-// Per output column n (gemm_out_ext.cu): ipb[n] = round(c127[n] + pb[n] / um) in double, written as 32 int8 digits
-// e[n][0..31] with sum_k a_k * e[n][k] = ipb[n] for a = (127 x 31, 1), one 128-byte row per column (the layout the
-// weight tile's TMA box uses; bytes 32..127 stay zero); dshift[n] = c127[n] - ipb[n] turns a proxy back into the
-// shifted accumulator of the exact formula.  Columns N .. n_pad - 1 are zero.  *overflow is set when some |ipb|
-// exceeds what the digits can hold (31 * 127 * 127 + 63).
-__global__ void out_ext_kernel(const int32_t* __restrict__ c127, const float* __restrict__ pb, float um, int N, int n_pad,
-                               uint8_t* __restrict__ ext, int32_t* __restrict__ dshift, int* __restrict__ overflow) {
-  const int n = blockIdx.x * blockDim.x + threadIdx.x;
-  if (n >= n_pad) return;
-  uint4* row = reinterpret_cast<uint4*>(ext + static_cast<size_t>(n) * 128);
-  uint32_t w[8] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
-  int ds = 0;
-  if (n < N) {
-    double t = rint(static_cast<double>(c127[n]) + static_cast<double>(pb[n]) / static_cast<double>(um));
-    if (fabs(t) > 500093.0) {
-      atomicOr(overflow, 1);
-      t = fmin(fmax(t, -500093.0), 500093.0);
-    }
-    const int ipb = static_cast<int>(t);
-    int Q = static_cast<int>(rint(static_cast<double>(ipb) / 127.0));
-    if (Q > 3937) Q = 3937;
-    if (Q < -3937) Q = -3937;
-    const int r = ipb - 127 * Q;  // |r| <= 63 (<= 126 at the clamped ends, still an int8)
-    const int base = Q / 31, rem = Q - 31 * base;
-    const int step = rem > 0 ? 1 : -1, cnt = rem > 0 ? rem : -rem;
-    for (int k = 0; k < 32; k++) {
-      const int d = k < 31 ? base + (k < cnt ? step : 0) : r;
-      w[k >> 2] |= static_cast<uint32_t>(d & 0xff) << (8 * (k & 3));
-    }
-    ds = c127[n] - ipb;
-  }
-  row[0] = make_uint4(w[0], w[1], w[2], w[3]);
-  row[1] = make_uint4(w[4], w[5], w[6], w[7]);
-  for (int i = 2; i < 8; i++) row[i] = make_uint4(0u, 0u, 0u, 0u);
-  dshift[n] = ds;
-}
-
-__device__ __forceinline__ unsigned long long pack_best_k(float v, uint32_t idx) {
-  if (v == 0.0f) v = 0.0f;
-  uint32_t bits = __float_as_uint(v);
-  uint32_t key = (bits & 0x80000000u) ? ~bits : (bits | 0x80000000u);
-  return (static_cast<unsigned long long>(key) << 32) | static_cast<unsigned long long>(0xFFFFFFFFu - idx);
-}
-
 __global__ void argmax_rows_kernel(const float* __restrict__ logits, int cols, unsigned long long* __restrict__ best) {
   const int row = blockIdx.x;
   const float* p = logits + static_cast<size_t>(row) * cols;
   unsigned long long loc = 0ull;
   for (int c = threadIdx.x; c < cols; c += blockDim.x) {
-    const unsigned long long k = pack_best_k(p[c], c);
+    const unsigned long long k = pack_best(p[c], c);
     loc = k > loc ? k : loc;
   }
   atomicMax(best + row, loc);
@@ -363,25 +288,6 @@ void launch_gather_rows(const int8_t* W, const float* pb, const int32_t* c127, c
                         int8_t* W_sel, float* pb_sel, int32_t* c127_sel, cudaStream_t stream) {
   if (n_idx == 0) return;
   gather_rows_kernel<<<n_idx, 32, 0, stream>>>(W, pb, c127, idx, K, W_sel, pb_sel, c127_sel);
-}
-
-void launch_out_bounds(const int32_t* c127, const float* pb, float um, int N, float* dmax, cudaStream_t stream) {
-  const int chunks = (N + 31) / 32;
-  if (chunks == 0) return;
-  out_bounds_kernel<<<(chunks + 7) / 8, 256, 0, stream>>>(c127, pb, um, N, dmax);
-}
-
-void launch_out_ipb(const int32_t* c127, const float* pb, float um, int N, int32_t* ipb6, cudaStream_t stream) {
-  const int n_pad = (N + 255) / 256 * 256;
-  if (n_pad == 0) return;
-  out_ipb_kernel<<<(n_pad + 255) / 256, 256, 0, stream>>>(c127, pb, um, N, n_pad, ipb6);
-}
-
-void launch_out_ext(const int32_t* c127, const float* pb, float um, int N, uint8_t* ext, int32_t* dshift, int* overflow,
-                    cudaStream_t stream) {
-  const int n_pad = (N + 255) / 256 * 256;
-  if (n_pad == 0) return;
-  out_ext_kernel<<<(n_pad + 127) / 128, 128, 0, stream>>>(c127, pb, um, N, n_pad, ext, dshift, overflow);
 }
 
 __global__ void transpose_u32_kernel(const uint32_t* __restrict__ src, int rows, int cols, uint32_t* __restrict__ dst,

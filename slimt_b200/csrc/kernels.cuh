@@ -108,17 +108,6 @@ void launch_finalize_step(unsigned long long* best, const uint32_t* shortlist, c
 void launch_gather_rows(const int8_t* W, const float* pb, const int32_t* c127, const uint32_t* idx, int n_idx, int K,
                         int8_t* W_sel, float* pb_sel, int32_t* c127_sel, cudaStream_t stream);
 
-// dmax[ceil(N/32)]: per 32-column chunk, max_n(c127[n] * um + pb[n]) rounded up (see gemm_out.cu).
-void launch_out_bounds(const int32_t* c127, const float* pb, float um, int N, float* dmax, cudaStream_t stream);
-
-// ipb6[ceil(N/256)*256]: integer logit-proxy offsets of the tolerance-mode output GEMM (see gemm_out.cu).
-void launch_out_ipb(const int32_t* c127, const float* pb, float um, int N, int32_t* ipb6, cudaStream_t stream);
-
-// Digit rows ext [ceil(N/256)*256][128] and dshift [same] of the second-generation output GEMM (gemm_out_ext.cu);
-// *overflow (device int, pre-zeroed) is set when a column's offset does not fit the digits.
-void launch_out_ext(const int32_t* c127, const float* pb, float um, int N, uint8_t* ext, int32_t* dshift, int* overflow,
-                    cudaStream_t stream);
-
 // Row-wise first-max over f32 logits (used when logits are materialised for parity taps).
 void launch_argmax_rows(const float* logits, int rows, int cols, unsigned long long* best, cudaStream_t stream);
 // dst[c][r] = src[r][c] for r < rows, c < cols (dst rows are dst_stride apart): step-major token matrix -> sentence-major

@@ -1,8 +1,9 @@
 """GPU: the forward pass through every reachable combination of its kernel routes.  The workspace holds only the
 buffers the chosen routes read, so a route that lost one of its buffers would read a null or short one: each
 combination of self-attention kernel (SLIMT_B200_SELFATTN), cross-attention kernel (SLIMT_B200_CROSS and the batch
-shape), encoder FFN (tiny: row-tile kernel, base: gemm_i8), output route (digit GEMM, bound-filter GEMM on the model
-of test_gpu_out_fallback.py, logits tap), shortlist on and off, host and device I/O runs in both arithmetic modes.
+shape), encoder FFN (tiny: row-tile kernel, base: gemm_i8), output route (the fused argmax on the digits, the fused
+argmax on the bound filter with the models of test_gpu_out_fallback.py at K = 256 and 512, logits tap), shortlist on
+and off, host and device I/O runs in both arithmetic modes.
 Exact mode must give the oracle's tokens."""
 import numpy as np
 import pytest
@@ -10,7 +11,7 @@ import pytest
 import sb_testutil as util
 from oracle import slimt_oracle as so
 from slimt_b200 import capi, synth
-from test_gpu_out_fallback import fallback_model  # noqa: F401  (fixture)
+from test_gpu_out_fallback import fallback_base_model, fallback_model  # noqa: F401  (fixtures)
 
 pytestmark = pytest.mark.gpu
 
@@ -23,11 +24,12 @@ _oracle_cache = {}
 
 
 @pytest.fixture(scope="module")
-def models(gpu_ctx, tiny_model, fallback_model, tmp_path_factory):  # noqa: F811
+def models(gpu_ctx, tiny_model, fallback_model, fallback_base_model, tmp_path_factory):  # noqa: F811
     base_path = str(tmp_path_factory.mktemp("model") / "base.bin")
     synth.write_model(base_path, synth.make_params(synth.BASE, seed=77))
     out = {}
-    for name, path in (("tiny", tiny_model[0]), ("fallback", fallback_model[0]), ("base", base_path)):
+    for name, path in (("tiny", tiny_model[0]), ("fallback", fallback_model[0]), ("base", base_path),
+                       ("fallback_base", fallback_base_model[0])):
         out[name] = (capi.Model(gpu_ctx, open(path, "rb").read()), so.Oracle(synth.read_model(path)))
     yield out
     for m, _ in out.values():
@@ -69,7 +71,7 @@ def _device_forward(ctx, m, tokens, lengths, sl):
 @pytest.mark.parametrize("cross", CROSS)
 @pytest.mark.parametrize("selfattn", SELF)
 @pytest.mark.parametrize("name,shape", [("tiny", "short"), ("tiny", "long"), ("fallback", "short"),
-                                        ("fallback", "long"), ("base", "short")])
+                                        ("fallback", "long"), ("base", "short"), ("fallback_base", "short")])
 def test_route_combination(gpu_ctx, models, shortlist_assets, monkeypatch, name, shape, selfattn, cross):
     m, orc = models[name]
     tokens, lengths, sl_words = _batch(shape, shortlist_assets)
@@ -89,8 +91,8 @@ def test_route_combination(gpu_ctx, models, shortlist_assets, monkeypatch, name,
                         assert np.array_equal(out["step_tokens"], ref), f"{what} logits={logits}"
                     host = out["step_tokens"]
                 else:
-                    # teacher forcing keeps the histories equal: the fused integer-proxy argmax agrees with the argmax of
-                    # the same mode's float logits except at near-ties (the bar of test_gpu_fast_mode.py)
+                    # teacher forcing keeps the histories equal: the fused argmax agrees with the argmax of the same
+                    # mode's float logits except at near-ties (the bar of test_gpu_fast_mode.py)
                     steps = int(np.float32(1.5) * np.float32(tokens.shape[1]))
                     forced = np.random.RandomState(3).randint(1, 32000, size=(steps, len(lengths))).astype(np.uint32)
                     tap = m.forward(tokens, lengths, shortlist=sl, forced=forced, want_logits=True)["step_tokens"]

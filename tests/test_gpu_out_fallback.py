@@ -1,6 +1,6 @@
-"""GPU: the output GEMM's fallback kernel (gemm_out.cu).  The default kernel (gemm_out_ext.cu) adds every column's
+"""GPU: the output GEMM's bound-filter encoding (out_argmax.cu).  By default the fused argmax adds every column's
 offset round(bias * aq * bq) on the tensor core as 32 int8 digits, which hold at most 500 093 in magnitude.  A model
-with an output bias beyond that range decodes through gemm_out.cu instead, with the full vocabulary and with a
+with an output bias beyond that range decodes through the bound filter instead, with the full vocabulary and with a
 shortlist, in both arithmetic modes."""
 import struct
 
@@ -12,15 +12,14 @@ from oracle import slimt_oracle as so
 from slimt_b200 import capi, synth
 
 pytestmark = pytest.mark.gpu
-DIGIT_RANGE = 500093  # largest |offset| the digits of gemm_out_ext.cu represent (kernels.cu, out_ext_kernel)
+DIGIT_RANGE = 500093  # largest |offset| the digits represent (out_argmax.cu, out_ext_kernel)
 BIASED_COLUMN = 5     # not EOS (synth.EOS_ID)
 
 
-@pytest.fixture(scope="module")
-def fallback_model(tmp_path_factory):
-    """tiny11 with one output column biased so far below the others that it never wins, and whose offset is four
-    times what the digits hold."""
-    items = synth.make_params(synth.TINY, seed=1234)
+def _write_fallback_model(tmp_path_factory, cfg, name):
+    """The synthetic model `cfg` with one output column biased so far below the others that it never wins, and whose
+    offset is four times what the digits hold."""
+    items = synth.make_params(cfg, seed=1234)
     typ, shape, blob = items["Wemb"]
     V, E = shape
     bq = struct.unpack("<f", blob[V * E:V * E + 4])[0]
@@ -30,12 +29,24 @@ def fallback_model(tmp_path_factory):
     b[BIASED_COLUMN] = np.float32(-4.0 * DIGIT_RANGE / (aq * bq))
     items["decoder_ff_logit_out_b"] = (typ, shape, b.tobytes())
     offset = abs(float(b[BIASED_COLUMN]) * aq * bq)
-    # past the digits (so gemm_out.cu runs), inside the fallback's exact-integer range
+    # past the digits (so the bound filter runs), inside the bound filter's exact-integer range
     assert 2 * DIGIT_RANGE < offset < 2 ** 23, offset
     assert BIASED_COLUMN != synth.EOS_ID
-    path = str(tmp_path_factory.mktemp("model") / "tiny11_out_fallback.bin")
+    path = str(tmp_path_factory.mktemp("model") / f"{name}_out_fallback.bin")
     synth.write_model(path, items)
     return path, synth.read_model(path)
+
+
+@pytest.fixture(scope="module")
+def fallback_model(tmp_path_factory):
+    """tiny11 (E = 256: the bound filter at K = 256) with the biased column."""
+    return _write_fallback_model(tmp_path_factory, synth.TINY, "tiny11")
+
+
+@pytest.fixture(scope="module")
+def fallback_base_model(tmp_path_factory):
+    """The base model (E = 512: the bound filter at K = 512) with the same biased column."""
+    return _write_fallback_model(tmp_path_factory, synth.BASE, "base")
 
 
 def test_exact_greedy_tokens_equal_oracle(gpu_ctx, fallback_model):
@@ -59,8 +70,9 @@ def test_exact_greedy_tokens_equal_oracle(gpu_ctx, fallback_model):
 
 
 def test_tolerance_mode_fused_argmax_agrees_with_logits(fallback_model):
-    """Teacher forcing keeps the histories equal; the fused integer-proxy argmax must agree with the argmax of the
-    same mode's float logits except at near-ties (the bar of test_teacher_forced_logits_within_rtol)."""
+    """Teacher forcing keeps the histories equal; the fused argmax (the bound filter's exact first maximum of the
+    accumulators, in tolerance mode too) must agree with the argmax of the same mode's float logits except at
+    near-ties (the bar of test_teacher_forced_logits_within_rtol)."""
     path, _ = fallback_model
     ctx = capi.Context(0)
     ctx.set_math(True)

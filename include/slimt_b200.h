@@ -127,6 +127,10 @@ typedef struct slimt_b200_forward_io {
   float* encoder_out;       /* [B][T][E] */
   float* logits;            /* [max_steps][B][Nout] where Nout = n_shortlist or vocab */
   float* alignment;         /* [max_steps][B][T]: head 0 of the last layer's cross attention (Model.cc:84-108) */
+  /* optional result (NULL = not wanted): log-probability of each step's word, y[c] - log sum_n exp(y[n]) over the step's
+   * logits y (the shortlist's columns, or the vocabulary's), c the greedy choice or the forced word's column (-inf when
+   * the shortlist does not hold it).  Every executed step has one, like step_tokens.  A DEVICE pointer with device_io. */
+  float* token_scores;      /* [max_steps][B] */
 } slimt_b200_forward_io;
 
 /* Model::forward (Model.cc:187-204): embedding -> encoder -> greedy decode. */
@@ -164,6 +168,9 @@ typedef struct slimt_b200_translate_io {
   uint64_t kernel_launches;  /* out: kernels this library launched during the call */
   uint64_t h2d_bytes;        /* out */
   uint64_t d2h_bytes;        /* out */
+  /* optional (NULL = not wanted): the log-probability of every recorded target token, EOS included (token_scores of
+   * slimt_b200_forward_io).  Ragged exactly like out_tokens: indexed by out_offsets, capacity out_capacity. */
+  float* out_scores;
 } slimt_b200_translate_io;
 
 int slimt_b200_translate(slimt_b200_model* model, slimt_b200_translate_io* io);

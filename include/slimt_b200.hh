@@ -559,12 +559,14 @@ struct Config {
 
 // Response (Response.hh:20-43) at the WORD-ID level of this path: the reference's AnnotatedText source / target are the
 // sentences' word ids here; alignments[i][t][s] = p(source token s | target token t) of sentence i (head 0 of the last
-// decoder layer's cross-attention, Model.cc:84-108), empty unless Options::alignment.  The text-level slimt::Response
+// decoder layer's cross-attention, Model.cc:84-108), empty unless Options::alignment; scores[i][t] = log-probability of
+// target token t of sentence i (EOS included), empty unless Options::scores.  The text-level slimt::Response
 // (AnnotatedText source / target) and Options are in slimt_b200_text.hh.
 struct WordsResponse {
   Sentences source;  // one entry per SEGMENT (a sentence longer than Config::wrap_length is several, TextProcessor.cc:123)
   Sentences target;
   std::vector<Alignment> alignments;
+  std::vector<std::vector<float>> scores;
   // segments [sentence_begin[i], sentence_begin[i + 1]) came from input sentence i (the reference keeps this relation
   // in the byte ranges of its AnnotatedText); the identity while nothing was wrapped
   std::vector<size_t> sentence_begin;
@@ -573,9 +575,11 @@ struct WordsResponse {
 
 // remap_alignments + combine (Response.cc:126-175) for pivoting on word ids: the pivot sentence is handed to the second
 // model as produced, so the character-overlap transfer between two tokenisations of the pivot text is the identity and
-// what remains is the marginalisation p(s | t) = sum_q p(s | q) p(q | t).
+// what remains is the marginalisation p(s | t) = sum_q p(s | q) p(q | t).  The scores are the second leg's: they score
+// the target tokens the combined response returns.
 inline WordsResponse combine(WordsResponse &&first, WordsResponse &&second) {
   WordsResponse out;
+  out.scores = std::move(second.scores);
   // (a pivot sentence the second service had to wrap again has no one-to-one segment any more: no combined alignment)
   if (!first.alignments.empty() && second.alignments.size() == first.alignments.size()) {
     for (size_t i = 0; i < first.source.size(); i++) {
@@ -650,6 +654,8 @@ class Blocking {
     for (const History &h : histories) response.target.push_back(h->target);
     if (options.alignment)
       for (const History &h : histories) response.alignments.push_back(h->alignment);
+    if (options.scores)
+      for (const History &h : histories) response.scores.push_back(h->scores);
     return response;
   }
   // Blocking::pivot on word ids: the two models must share the pivot-language vocabulary; the pivot sentences are
@@ -701,19 +707,21 @@ class Blocking {
       Histories mine(histories.begin() + first[i], histories.begin() + first[i + 1]);
       responses[i] = make_response(std::move(annotated[i]), mine, model->vocabulary());
       if (!options.alignment) responses[i].alignments.clear();
+      if (!options.scores) responses[i].scores.clear();
     });
     return responses;
   }
 
   // cache prefill (Request.cc:58-78): a segment this model has translated before is not batched again.  A record
-  // stored by a request that did not ask for alignments cannot answer one that does.  The rest: run().
+  // stored by a request that did not ask for alignments (or scores) cannot answer one that does.  The rest: run().
   Histories serve(const Ptr<Model> &model, const Sentences &segments, const Options &options) {
     Histories histories(segments.size());
     std::vector<size_t> todo;
     for (size_t i = 0; i < segments.size(); i++) {
       if (cache_) {
         auto [found, history] = cache_->find(cache_key(model->id(), segments[i]));
-        if (found && history && (!options.alignment || history->alignment.size() == history->target.size())) {
+        if (found && history && (!options.alignment || history->alignment.size() == history->target.size()) &&
+            (!options.scores || history->scores.size() == history->target.size())) {
           histories[i] = history;
           cache_hits_++;
           continue;
@@ -745,6 +753,7 @@ class Blocking {
     std::vector<uint64_t> out_offsets(todo.size() + 1, 0);
     std::vector<float> align;
     std::vector<uint64_t> align_offsets(todo.size() + 1, 0);
+    std::vector<float> scores;
     slimt_b200_translate_io io;
     std::memset(&io, 0, sizeof(io));
     io.tokens = tokens.data(), io.offsets = offsets.data(), io.n_sentences = todo.size();
@@ -756,6 +765,10 @@ class Blocking {
       align.resize(std::max<size_t>(1, per * tokens.size()));
       io.out_alignments = align.data(), io.align_capacity = align.size(), io.out_align_offsets = align_offsets.data();
     }
+    if (options.scores) {  // ragged like out: one score per target token
+      scores.resize(out.size());
+      io.out_scores = scores.data();
+    }
     const std::vector<slimt_b200_model *> &replicas = model->replicas();
     detail::check(slimt_b200_translate_multi(replicas.data(), replicas.size(), &io), "slimt_b200_translate_multi");
     for (size_t k = 0; k < todo.size(); k++) {
@@ -766,6 +779,7 @@ class Blocking {
         const float *p = align.data() + align_offsets[k];
         for (size_t t = 0; t < h->target.size(); t++) h->alignment.emplace_back(p + t * S, p + (t + 1) * S);
       }
+      if (options.scores) h->scores.assign(scores.begin() + out_offsets[k], scores.begin() + out_offsets[k + 1]);
       histories[todo[k]] = std::move(h);
     }
   }
@@ -878,7 +892,7 @@ class Async {
   // depend on who shared the batch (the candidate set is the union over the batch, Model.cc:116-120).
   static bool poolable(const Job &a, const Job &b) {
     return !a.second && !b.second && a.first == b.first && a.is_text == b.is_text && a.options.alignment == b.options.alignment &&
-           a.options.html == b.options.html;
+           a.options.html == b.options.html && a.options.scores == b.options.scores;
   }
   void work() {
     Config one = config_;
@@ -934,6 +948,7 @@ class Async {
             mine.source.assign(all.source.begin() + g0, all.source.begin() + g1);
             mine.target.assign(all.target.begin() + g0, all.target.begin() + g1);
             if (!all.alignments.empty()) mine.alignments.assign(all.alignments.begin() + g0, all.alignments.begin() + g1);
+            if (!all.scores.empty()) mine.scores.assign(all.scores.begin() + g0, all.scores.begin() + g1);
             for (size_t s = s0; s <= s1; s++) mine.sentence_begin.push_back(all.sentence_begin[s] - g0);
             jobs[k].promise.set_value(std::move(mine));
           }

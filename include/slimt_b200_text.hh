@@ -66,6 +66,7 @@ struct View {
 struct Hypothesis {
   Words target;
   Alignment alignment;
+  std::vector<float> scores;  // log-probability of each target token (Options::scores), empty otherwise
 };
 using History = Ptr<Hypothesis>;
 using Histories = std::vector<History>;
@@ -1303,6 +1304,7 @@ class TextProcessor {
 struct Options {
   bool alignment = false;  // include alignments or not
   bool html = false;       // markup handling is not carried (see the header comment): must be false
+  bool scores = false;     // include per-token log-probabilities or not (marian's --word-scores)
 };
 
 struct Response {
@@ -1310,6 +1312,9 @@ struct Response {
   AnnotatedText target;
   // alignments[sentence][t][s] = p(source token s | target token t)
   std::vector<Alignment> alignments;
+  // scores[sentence][t] = log p(target token t | source, tokens before t) under greedy decoding, EOS included: one per
+  // token of the sentence's translation, empty unless Options::scores.  After a pivot: the second leg's scores.
+  std::vector<std::vector<float>> scores;
   size_t size() const { return source.sentence_count(); }
   void to(Encoding encoding) { source.to(encoding), target.to(encoding); }
 };
@@ -1376,9 +1381,12 @@ inline std::vector<Alignment> remap_alignments(const Response &first, const Resp
   return alignments;
 }
 
+// The scores of a pivot are the second leg's: they score the tokens the combined Response returns (the first leg's
+// scores are of the pivot text, which the caller does not see).
 inline Response combine(Response &&first, Response &&second) {  // Response.cc:165-175
   Response combined;
   if (!first.alignments.empty()) combined.alignments = remap_alignments(first, second);
+  combined.scores = std::move(second.scores);
   combined.source = std::move(first.source);
   combined.target = std::move(second.target);
   return combined;
@@ -1397,6 +1405,7 @@ inline Response make_response(AnnotatedText &&source, const Histories &histories
     response.target.append_sentence(response.source.gap(s), views.begin(), views.end());
     if (s + 1 == histories.size()) response.target.append_ending_whitespace(response.source.gap(s + 1));
     response.alignments.push_back(histories[s]->alignment);
+    response.scores.push_back(histories[s]->scores);
   }
   return response;
 }

@@ -40,7 +40,7 @@ class ForwardIO(C.Structure):
                 ("limit_factor", C.c_float), ("shortlist", C.c_void_p), ("n_shortlist", C.c_size_t),
                 ("forced", C.c_void_p), ("device_io", C.c_int32), ("step_tokens", C.c_void_p), ("steps", C.c_size_t),
                 ("target_tokens", C.c_uint64), ("encoder_out", C.c_void_p), ("logits", C.c_void_p),
-                ("alignment", C.c_void_p)]
+                ("alignment", C.c_void_p), ("token_scores", C.c_void_p)]
 
 
 class TranslateIO(C.Structure):
@@ -51,7 +51,7 @@ class TranslateIO(C.Structure):
                 ("out_alignments", C.c_void_p), ("align_capacity", C.c_size_t), ("out_align_offsets", C.c_void_p),
                 ("target_tokens", C.c_uint64), ("batches", C.c_uint64),
                 ("device_ms", C.c_double), ("kernel_launches", C.c_uint64), ("h2d_bytes", C.c_uint64),
-                ("d2h_bytes", C.c_uint64)]
+                ("d2h_bytes", C.c_uint64), ("out_scores", C.c_void_p)]
 
 
 class KernelStat(C.Structure):
@@ -266,8 +266,10 @@ class Model:
 
     def forward(self, tokens: np.ndarray, lengths: np.ndarray, limit_factor: float = 1.5,
                 shortlist: Optional[np.ndarray] = None, forced: Optional[np.ndarray] = None,
-                want_encoder: bool = False, want_logits: bool = False, want_alignment: bool = False):
-        """Model::forward on host buffers. Returns dict(step_tokens [steps,B], steps, target_tokens, ...)."""
+                want_encoder: bool = False, want_logits: bool = False, want_alignment: bool = False,
+                want_scores: bool = False):
+        """Model::forward on host buffers. Returns dict(step_tokens [steps,B], steps, target_tokens, ...); "scores"
+        [steps,B] holds each step's log-probability of its chosen (or forced) word when want_scores."""
         tokens = np.ascontiguousarray(tokens, dtype=np.uint32)
         lengths = np.ascontiguousarray(lengths, dtype=np.uint32)
         B, T = tokens.shape
@@ -279,28 +281,33 @@ class Model:
         enc = np.empty((B, T, self.E), dtype=np.float32) if want_encoder else None
         logits = np.zeros((max(1, max_steps), B, nout), dtype=np.float32) if want_logits else None
         align = np.zeros((max(1, max_steps), B, T), dtype=np.float32) if want_alignment else None
+        scores = np.zeros((max(1, max_steps), B), dtype=np.float32) if want_scores else None
         io = ForwardIO(_ptr(tokens), _ptr(lengths), B, T, limit_factor, _ptr(sl), 0 if sl is None else len(sl), _ptr(fo),
-                       0, _ptr(steps), 0, 0, _ptr(enc), _ptr(logits), _ptr(align))
+                       0, _ptr(steps), 0, 0, _ptr(enc), _ptr(logits), _ptr(align), _ptr(scores))
         _check(lib().slimt_b200_model_forward(self.h, C.byref(io)), "slimt_b200_model_forward")
         n = int(io.steps)
         return {"step_tokens": steps[:n], "steps": n, "target_tokens": int(io.target_tokens), "encoder_out": enc,
-                "logits": None if logits is None else logits[:n], "alignment": None if align is None else align[:n]}
+                "logits": None if logits is None else logits[:n], "alignment": None if align is None else align[:n],
+                "scores": None if scores is None else scores[:n]}
 
     def forward_resident(self, d_tokens: int, d_lengths: int, B: int, T: int, d_steps: int, limit_factor: float = 1.5,
-                         d_shortlist: int = 0, n_shortlist: int = 0):
-        """Model::forward with inputs/outputs already in HBM (no host<->device copies of the batch)."""
-        io = ForwardIO(d_tokens, d_lengths, B, T, limit_factor, d_shortlist or None, n_shortlist, None, 1, d_steps, 0, 0,
-                       None, None, None)
+                         d_shortlist: int = 0, n_shortlist: int = 0, d_scores: int = 0, d_forced: int = 0):
+        """Model::forward with inputs/outputs already in HBM (no host<->device copies of the batch); d_scores
+        (optional) receives the [max_steps][B] token scores on the device."""
+        io = ForwardIO(d_tokens, d_lengths, B, T, limit_factor, d_shortlist or None, n_shortlist, d_forced or None, 1,
+                       d_steps, 0, 0, None, None, None, d_scores or None)
         _check(lib().slimt_b200_model_forward(self.h, C.byref(io)), "slimt_b200_model_forward")
         return int(io.steps), int(io.target_tokens)
 
     def translate_flat(self, tokens: np.ndarray, offsets: np.ndarray, max_words: int, limit_factor: float = 1.5,
                        shortlist_bin: Optional[bytes] = None, out_tokens: Optional[np.ndarray] = None,
                        out_offsets: Optional[np.ndarray] = None, replicas=None, want_alignments: bool = False,
-                       shortlist_check: bool = False, shortlist_shared: bool = False):
+                       shortlist_check: bool = False, shortlist_shared: bool = False, want_scores: bool = False,
+                       out_scores: Optional[np.ndarray] = None):
         """slimt_b200_translate (or _translate_multi over `replicas`, a list of Models) on caller-owned host buffers:
         ragged sentences in (tokens, offsets), ragged targets out (out_tokens, out_offsets).  This is the C-ABI call a
-        host integration makes; nothing is repacked."""
+        host integration makes; nothing is repacked.  want_scores: stats["scores"] is ragged like out_tokens (one
+        log-probability per target token, EOS included); out_scores, when given, is that buffer."""
         n = len(offsets) - 1
         lens = np.diff(offsets.astype(np.int64))
         max_len = int(lens.max()) if n else 0
@@ -313,6 +320,8 @@ class Model:
         if want_alignments:
             align = np.zeros(max(1, per * int(lens.sum())), dtype=np.float32)  # upper bound: every sentence decoded to the limit
             align_offs = np.zeros(n + 1, dtype=np.uint64)
+        if want_scores and out_scores is None:
+            out_scores = np.zeros(len(out_tokens), dtype=np.float32)
         slbuf = None
         if shortlist_bin is not None:
             slbuf = shortlist_bin if isinstance(shortlist_bin, C.Array) else (C.c_char * len(shortlist_bin)).from_buffer_copy(shortlist_bin)
@@ -320,7 +329,8 @@ class Model:
                          C.cast(slbuf, C.c_void_p) if slbuf is not None else None,
                          0 if slbuf is None else len(slbuf), int(shortlist_check), int(shortlist_shared),
                          _ptr(out_tokens), len(out_tokens), _ptr(out_offsets),
-                         _ptr(align), 0 if align is None else len(align), _ptr(align_offs), 0, 0, 0.0, 0, 0, 0)
+                         _ptr(align), 0 if align is None else len(align), _ptr(align_offs), 0, 0, 0.0, 0, 0, 0,
+                         _ptr(out_scores) if want_scores else None)
         if replicas is None:
             _check(lib().slimt_b200_translate(self.h, C.byref(io)), "slimt_b200_translate")
         else:
@@ -331,19 +341,26 @@ class Model:
                  "d2h_bytes": int(io.d2h_bytes)}
         if want_alignments:
             stats["alignments"], stats["align_offsets"] = align, align_offs
+        if want_scores:
+            stats["scores"] = out_scores
         return out_tokens, out_offsets, stats
 
     def translate(self, sentences, max_words: int, limit_factor: float = 1.5, shortlist_bin: Optional[bytes] = None,
-                  replicas=None, want_alignments: bool = False, **kw):
-        """exhaust() over one request: Batcher + shortlist + forward per batch, host buffers in and out."""
+                  replicas=None, want_alignments: bool = False, want_scores: bool = False, **kw):
+        """exhaust() over one request: Batcher + shortlist + forward per batch, host buffers in and out.  want_scores:
+        stats["scores"][i] holds one log-probability per target token of sentence i."""
         offsets = np.zeros(len(sentences) + 1, dtype=np.uint64)
         offsets[1:] = np.cumsum([len(s) for s in sentences])
         tokens = np.concatenate([np.asarray(s, dtype=np.uint32) for s in sentences]) if sentences else np.zeros(0, np.uint32)
         out_tokens, out_offsets, stats = self.translate_flat(tokens, offsets, max_words, limit_factor, shortlist_bin,
-                                                             replicas=replicas, want_alignments=want_alignments, **kw)
+                                                             replicas=replicas, want_alignments=want_alignments,
+                                                             want_scores=want_scores, **kw)
         outs = [out_tokens[int(out_offsets[i]):int(out_offsets[i + 1])].copy() for i in range(len(sentences))]
         if want_alignments:
             al, ao = stats.pop("alignments"), stats.pop("align_offsets")
             stats["alignments"] = [al[int(ao[i]):int(ao[i + 1])].reshape(len(outs[i]), len(sentences[i])).copy()
                                    for i in range(len(sentences))]
+        if want_scores:
+            sc = stats.pop("scores")
+            stats["scores"] = [sc[int(out_offsets[i]):int(out_offsets[i + 1])].copy() for i in range(len(sentences))]
         return outs, stats

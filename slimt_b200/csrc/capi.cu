@@ -179,6 +179,7 @@ int slimt_b200_model_forward(slimt_b200_model* model, slimt_b200_forward_io* io)
   a.forced = io->forced, a.device_io = io->device_io != 0;
   a.step_tokens = io->step_tokens;
   a.encoder_out = io->encoder_out, a.logits = io->logits, a.alignment = io->alignment;
+  a.scores = io->token_scores;
   int rc = sb::model_forward(model->m, a);
   io->steps = a.steps;
   io->target_tokens = a.target_tokens;

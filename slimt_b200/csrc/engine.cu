@@ -1,6 +1,8 @@
 // See engine.cuh.
 #include "engine.cuh"
 
+#include "score_partial.cuh"
+
 #include <math.h>
 #include <stdio.h>
 #include <string.h>
@@ -671,8 +673,9 @@ enum class Cross { Cached, Rc, Rcl };
 const char* const kSelfAttnName[] = {"Fused", "Rowwise", "Tiled", "Long"};  // indexed by SelfAttn
 
 enum class EncFfn { Rows, Gemm };
-// output: the fused argmax GEMM (out_argmax.cu, in the encoding Model::load chose), or logits tap + argmax_rows
-enum class Out { Argmax, Logits };
+// output: the fused argmax GEMM (out_argmax.cu, in the encoding Model::load chose), logits tap + argmax_rows, or the
+// scores GEMM (the fused GEMM with every logit evaluated exactly) + score_step
+enum class Out { Argmax, Logits, Scores };
 
 struct Routes {
   SelfAttn self;
@@ -683,7 +686,7 @@ struct Routes {
 
 // Which kernel runs each stage of one forward call that has more than one.  The two environment variables are read on
 // every call, so that tests can switch kernels between calls; a value not listed below means the default.
-Routes choose_routes(const Model& m, int T, int B, bool fast, bool logits) {
+Routes choose_routes(const Model& m, int T, int B, bool fast, bool logits, bool scores) {
   const int E = m.E, H = m.H, dh = m.dh;
   auto env_is = [](const char* env, const char* v) { return env != nullptr && strcmp(env, v) == 0; };
   Routes r{};
@@ -720,8 +723,9 @@ Routes choose_routes(const Model& m, int T, int B, bool fast, bool logits) {
   // Wo + residual + LN, FFN1 + ReLU, FFN2 + residual + LN in one row-tile kernel, 128 rows per CTA
   r.ffn = E == 256 && m.F == 1536 ? EncFfn::Rows : EncFfn::Gemm;
 
-  // a caller that wants the logits gets them from the tap
-  r.out = logits ? Out::Logits : Out::Argmax;
+  // a caller that wants the logits gets them from the tap (and scores, when asked for, from them); scores alone come
+  // from the scores epilogue of the fused GEMM
+  r.out = logits ? Out::Logits : scores ? Out::Scores : Out::Argmax;
   return r;
 }
 
@@ -744,6 +748,8 @@ struct Pass {
   int8_t *qa[4], *attn_q, *ffn_q;
   // decoder state (Model.cc:111-185); counters: [0] n_done, [1] step counter, [2] ticket
   float *xd, *hb, *qd, *zb, *state[2], *d_logits, *d_align_all;  // zb: the first of two decoder layers' output
+  float* d_scores;    // [max_steps][B]
+  float2* partials;   // [ceil(Nout / 64)][B] strip partials of the step's scores
   int8_t *xq[2], *zq[2], *caq, *oq;
   unsigned long long* best;
   uint8_t* done;
@@ -796,7 +802,7 @@ int Pass::plan() {
     set_error("shortlist size must be a multiple of 8");
     return 1;
   }
-  route = choose_routes(m, T, B, c.fast, a.logits != nullptr);
+  route = choose_routes(m, T, B, c.fast, a.logits != nullptr, a.scores != nullptr);
 
   const size_t RE = static_cast<size_t>(R) * E, BE = static_cast<size_t>(B) * E;
   const size_t SB = static_cast<size_t>(max_steps) * B, N = static_cast<size_t>(Nout);
@@ -826,6 +832,10 @@ int Pass::plan() {
     if (route.out == Out::Argmax) out.tables([&ws](auto*& p, size_t n) { ws.add(p, n); });
   }
   if (route.out == Out::Logits) ws.add(d_logits, static_cast<size_t>(B) * N);
+  if (a.scores) {
+    if (!a.device_io) ws.add(d_scores, SB);
+    ws.add(partials, (N + kScoreStrip - 1) / kScoreStrip * static_cast<size_t>(B));
+  }
   // head-0 probabilities of every step stay on the device and come back in one copy after the loop
   if (a.alignment) ws.add(d_align_all, SB * T);
   if (!a.device_io && a.sentence_tokens) ws.add(d_rows, SB);
@@ -833,6 +843,7 @@ int Pass::plan() {
   if (a.device_io) {
     d_tokens = const_cast<uint32_t*>(a.tokens), d_lengths = const_cast<uint32_t*>(a.lengths), d_steps = a.step_tokens;
     d_forced = const_cast<uint32_t*>(a.forced), d_sl = use_sl ? const_cast<uint32_t*>(a.shortlist) : nullptr;
+    d_scores = a.scores;
   }
 
   // cross-attention K/V operands: projected once (Cross::Cached), or the u8 encoder output the recompute kernels read
@@ -1053,6 +1064,8 @@ int Pass::prepare_output() {
       launch_out_tables(out, nullptr, s);
       if (out_maps(c, out, E)) return 1;
     }
+    // the scores GEMM reads the weights alone: no table
+    if (route.out == Out::Scores && c.make_map(&out.map_w, out.w, out.N, E, kOutBN)) return 1;
   }
   return 0;
 }
@@ -1165,12 +1178,36 @@ int Pass::decode_step(int step) {
     SB_CUDA(cudaMemcpyAsync(a.logits + static_cast<size_t>(step) * B * Nout, d_logits, 4ul * B * Nout,
                             cudaMemcpyDeviceToHost, s));
     c.d2h_bytes += 4ul * B * Nout;
+    if (a.scores) {
+      LaunchScope ls(c, "score_rows", 0, 4.0 * B * Nout + 8.0 * B * ((Nout + kScoreStrip - 1) / kScoreStrip));
+      launch_score_rows(d_logits, B, Nout, partials, s);
+    }
+  } else if (route.out == Out::Scores) {
+    const double Md = B, Nd = Nout, Kd = E, strips = (Nout + kScoreStrip - 1) / kScoreStrip;
+    LaunchScope ls(c, "dec_gemm_out_scores", 2.0 * Md * Nd * Kd, Md * Kd + Nd * Kd + 8.0 * Nd + 8.0 * Md + 8.0 * Md * strips);
+    if (launch_out_scores(out, map_oq, B, E, best, partials, c.num_sms, s)) {
+      set_error("output GEMM (scores): unsupported K " + std::to_string(E));
+      return 1;
+    }
   } else {
     const double Md = B, Nd = Nout, Kd = E;
     LaunchScope ls(c, "dec_gemm_out_argmax", 2.0 * Md * Nd * Kd, Md * Kd + Nd * Kd + 4.0 * Nd + 8.0 * Md);
     if (launch_out_argmax(out, map_oq, c.fast, B, E, best, c.num_sms, s,
                           (trace_buf && step == 3) ? trace_buf + 4 * trace_n : nullptr)) {
       set_error("output GEMM: unsupported K " + std::to_string(E));
+      return 1;
+    }
+  }
+  if (a.scores) {
+    ScoreStepArgs k{};
+    k.partials = partials, k.best = best, k.forced = d_forced, k.shortlist = use_sl ? d_sl : nullptr;
+    k.oq = oq, k.w = out.w, k.c127 = out.c127, k.pb = out.pb, k.um = out.um;
+    k.logits = route.out == Out::Logits ? d_logits : nullptr;
+    k.B = B, k.N = Nout, k.K = E, k.step = step, k.scores = d_scores;
+    const double strips = (Nout + kScoreStrip - 1) / kScoreStrip;
+    LaunchScope ls(c, "score_step", 0, 8.0 * B * strips + 16.0 * B + (a.forced ? 2.0 * B * E : 0.0));
+    if (launch_score_step(k, s)) {
+      set_error("token scores: step kernel launch failed");
       return 1;
     }
   }
@@ -1252,6 +1289,10 @@ int Pass::decode() {
   if (d_align_all && executed > 0) {
     SB_CUDA(cudaMemcpyAsync(a.alignment, d_align_all, 4ul * executed * B * T, cudaMemcpyDeviceToHost, s));
     c.d2h_bytes += 4ul * executed * B * T;
+  }
+  if (!a.device_io && a.scores && executed > 0) {
+    SB_CUDA(cudaMemcpyAsync(a.scores, d_scores, 4ul * executed * B, cudaMemcpyDeviceToHost, s));
+    c.d2h_bytes += 4ul * executed * B;
   }
   if (!a.device_io && a.step_tokens && executed > 0) {
     SB_CUDA(cudaMemcpyAsync(a.step_tokens, d_steps, 4ul * executed * B, cudaMemcpyDeviceToHost, s));

@@ -188,6 +188,9 @@ struct ForwardArgs {
   float* encoder_out = nullptr;
   float* logits = nullptr;
   float* alignment = nullptr;
+  // [max_steps][B] log-probability of each step's chosen (or forced) word over the step's output columns; a device
+  // pointer with device_io (score_partial.cuh)
+  float* scores = nullptr;
 };
 
 int model_forward(Model& m, ForwardArgs& a);

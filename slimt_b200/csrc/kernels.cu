@@ -7,6 +7,7 @@
 #include "exact_math.cuh"
 #include "packed_best.cuh"
 #include "ptx.cuh"
+#include "score_partial.cuh"
 
 namespace sb {
 
@@ -233,6 +234,100 @@ __global__ void argmax_rows_kernel(const float* __restrict__ logits, int cols, u
   atomicMax(best + row, loc);
 }
 
+// ------------------------------------------------------------------ token scores
+// Logits tap: the partial (m, s) of every 64-column strip of every row, with the same strip_partial as the fused
+// scores epilogue.  Thread = (strip, row), rows fastest, so the partial stores are coalesced.
+__global__ void score_rows_kernel(const float* __restrict__ logits, int B, int N, float2* __restrict__ partials) {
+  const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  const int n_strips = (N + kScoreStrip - 1) / kScoreStrip;
+  if (i >= static_cast<size_t>(n_strips) * B) return;
+  const int t = static_cast<int>(i / B), b = static_cast<int>(i % B);
+  const float ninf = -__int_as_float(0x7f800000);
+  const float* p = logits + static_cast<size_t>(b) * N + t * kScoreStrip;
+  float y0[32], y1[32];
+#pragma unroll
+  for (int j = 0; j < 32; j += 4) {  // N % 8 == 0: groups of four are entirely inside or outside
+    const int n0 = t * kScoreStrip + j;
+    const float4 a = n0 < N ? *reinterpret_cast<const float4*>(p + j) : make_float4(ninf, ninf, ninf, ninf);
+    const float4 c = n0 + 32 < N ? *reinterpret_cast<const float4*>(p + 32 + j) : make_float4(ninf, ninf, ninf, ninf);
+    y0[j] = a.x, y0[j + 1] = a.y, y0[j + 2] = a.z, y0[j + 3] = a.w;
+    y1[j] = c.x, y1[j + 1] = c.y, y1[j + 2] = c.z, y1[j + 3] = c.w;
+  }
+  partials[i] = strip_partial(y0, y1);
+}
+
+// Block = 32 rows (lane = row) x 32 warps (warp = a contiguous group of strips).  LSE = M + log S with M = max_t m_t and
+// S = sum_t s_t * exp(m_t - M) summed in ascending strip order: each warp its group in double, the 32 group sums then
+// in ascending group order.  The chosen column's logit: the packed best word's value (greedy), or for a forced word its
+// column (binary search in the sorted shortlist) evaluated exactly from the int8 operands -- or read from the tap.
+constexpr int kScoreWarps = 32;
+__global__ void __launch_bounds__(32 * kScoreWarps) score_step_kernel(ScoreStepArgs a) {
+  __shared__ float mx[kScoreWarps][32];
+  __shared__ double sm[kScoreWarps][32];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int b = blockIdx.x * 32 + lane;
+  const int B = a.B;
+  pdl_launch_dependents();
+  pdl_wait();
+  const float ninf = -__int_as_float(0x7f800000);
+  const int n_strips = (a.N + kScoreStrip - 1) / kScoreStrip;
+  const int per = (n_strips + kScoreWarps - 1) / kScoreWarps;
+  const int t0 = min(n_strips, w * per), t1 = min(n_strips, t0 + per);
+  float m = ninf;
+  if (b < B)
+    for (int t = t0; t < t1; t++) m = fmaxf(m, a.partials[static_cast<size_t>(t) * B + b].x);
+  mx[w][lane] = m;
+  __syncthreads();
+  float M = ninf;
+#pragma unroll 8
+  for (int k = 0; k < kScoreWarps; k++) M = fmaxf(M, mx[k][lane]);
+  double s = 0.0;
+  if (b < B)
+    for (int t = t0; t < t1; t++) {
+      const float2 p = a.partials[static_cast<size_t>(t) * B + b];
+      s += static_cast<double>(p.y) * static_cast<double>(score_exp(__fsub_rn(p.x, M)));
+    }
+  sm[w][lane] = s;
+  __syncthreads();
+  if (w != 0 || b >= B) return;
+  double S = 0.0;
+  for (int k = 0; k < kScoreWarps; k++) S += sm[k][lane];
+  const double lse = static_cast<double>(M) + log(S);
+  float y;
+  if (a.forced == nullptr) {
+    y = best_value(a.best[b]);
+  } else {
+    const uint32_t word = a.forced[static_cast<size_t>(a.step) * B + b];
+    int col = -1;
+    if (a.shortlist) {
+      int lo = 0, hi = a.N;  // first entry >= word
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (a.shortlist[mid] < word) lo = mid + 1;
+        else hi = mid;
+      }
+      if (lo < a.N && a.shortlist[lo] == word) col = lo;
+    } else if (word < static_cast<uint32_t>(a.N)) {
+      col = static_cast<int>(word);
+    }
+    if (col < 0) {
+      y = ninf;  // not among the output columns: probability 0
+    } else if (a.logits) {
+      y = a.logits[static_cast<size_t>(b) * a.N + col];
+    } else {
+      const int4* q = reinterpret_cast<const int4*>(a.oq + static_cast<size_t>(b) * a.K);
+      const int4* wr = reinterpret_cast<const int4*>(a.w + static_cast<size_t>(col) * a.K);
+      int acc = 0;
+      for (int k = 0; k < a.K / 16; k++) {
+        const int4 x = q[k], v = wr[k];
+        acc = __dp4a(x.x, v.x, acc), acc = __dp4a(x.y, v.y, acc), acc = __dp4a(x.z, v.z, acc), acc = __dp4a(x.w, v.w, acc);
+      }
+      y = dequant1(acc + a.c127[col], a.um, a.pb[col]);
+    }
+  }
+  a.scores[static_cast<size_t>(a.step) * B + b] = static_cast<float>(static_cast<double>(y) - lse);
+}
+
 }  // namespace
 
 void launch_embed(const uint32_t* tokens, const int8_t* emb_q, float inv_qm, float sqrt_e, const float* pos, int rows,
@@ -313,6 +408,17 @@ void launch_transpose_u32(const uint32_t* src, int rows, int cols, uint32_t* dst
 void launch_argmax_rows(const float* logits, int rows, int cols, unsigned long long* best, cudaStream_t stream) {
   if (rows == 0) return;
   argmax_rows_kernel<<<rows, 256, 0, stream>>>(logits, cols, best);
+}
+
+void launch_score_rows(const float* logits, int B, int N, float2* partials, cudaStream_t stream) {
+  const size_t n = static_cast<size_t>((N + kScoreStrip - 1) / kScoreStrip) * B;
+  if (n == 0) return;
+  score_rows_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, stream>>>(logits, B, N, partials);
+}
+
+int launch_score_step(const ScoreStepArgs& a, cudaStream_t stream) {
+  if (a.B == 0) return 0;
+  return launch_pdl(score_step_kernel, dim3((a.B + 31) / 32), dim3(32 * kScoreWarps), 0, stream, a) != cudaSuccess ? 1 : 0;
 }
 
 }  // namespace sb

@@ -39,6 +39,7 @@
 #include "gemm_i8.cuh"
 #include "packed_best.cuh"
 #include "ptx.cuh"
+#include "score_partial.cuh"
 
 namespace sb {
 
@@ -163,11 +164,10 @@ __device__ __forceinline__ int int_max32(const uint32_t (&v)[32]) {
   return max(max(max(vt[0], vt[1]), max(vt[2], vt[3])), max(max(vt[4], vt[5]), max(vt[6], vt[7])));
 }
 
-// Bound filter: the exact logits of one 32-column chunk held in v[]; the chunk maximum and its first column.
-__device__ __forceinline__ void exact_chunk(const uint32_t (&v)[32], int nb, int N, const float* __restrict__ pb,
-                                            const int32_t* __restrict__ c127, float um, float floor_v, float& mx, int& idx) {
+// The exact logits of one 32-column chunk held in v[] (the logits tap's values); columns past N are -inf.
+__device__ __forceinline__ void exact_logits32(const uint32_t (&v)[32], int nb, int N, const float* __restrict__ pb,
+                                               const int32_t* __restrict__ c127, float um, float (&y)[32]) {
   const float ninf = -__int_as_float(0x7f800000);
-  float y[32];
 #pragma unroll
   for (int j = 0; j < 32; j += 4) {
     if (nb + j < N) {  // N % 8 == 0: groups of four are entirely inside or outside
@@ -181,6 +181,13 @@ __device__ __forceinline__ void exact_chunk(const uint32_t (&v)[32], int nb, int
       y[j] = y[j + 1] = y[j + 2] = y[j + 3] = ninf;
     }
   }
+}
+
+// Bound filter: the exact logits of one 32-column chunk held in v[]; the chunk maximum and its first column.
+__device__ __forceinline__ void exact_chunk(const uint32_t (&v)[32], int nb, int N, const float* __restrict__ pb,
+                                            const int32_t* __restrict__ c127, float um, float floor_v, float& mx, int& idx) {
+  float y[32];
+  exact_logits32(v, nb, N, pb, c127, um, y);
   float t8[8];
 #pragma unroll
   for (int j = 0; j < 8; j++) t8[j] = fmaxf(fmaxf(y[4 * j], y[4 * j + 1]), fmaxf(y[4 * j + 2], y[4 * j + 3]));
@@ -230,16 +237,40 @@ __device__ __forceinline__ void bounds_exact(const uint32_t (&v0)[32], const uin
   }
 }
 
+// Scores (both arithmetic modes): every column's exact logit.  The strip's partial (m, s) (score_partial.cuh) goes to
+// partials[strip][M]; its first maximum is published like the bound filter's, so the choice is the reference's first
+// strict maximum.  seen only spares an atomic that cannot raise the word: it decides nothing that is summed.
+__device__ __forceinline__ void scores_exact(const uint32_t (&v0)[32], const uint32_t (&v1)[32], unsigned long long seen,
+                                             int row, int nb0, int M, int N, const float* __restrict__ pb,
+                                             const int32_t* __restrict__ c127, float um,
+                                             unsigned long long* __restrict__ best, float2* __restrict__ partials) {
+  if (nb0 >= N) return;  // the whole warp: a strip past the last column has no partial
+  float y0[32], y1[32];
+  exact_logits32(v0, nb0, N, pb, c127, um, y0);
+  exact_logits32(v1, nb0 + 32, N, pb, c127, um, y1);
+  const float2 p = strip_partial(y0, y1);
+  if (row >= M) return;
+  int idx = 63;
+#pragma unroll
+  for (int j = 62; j >= 0; j--) idx = ((j < 32 ? y0[j & 31] : y1[j & 31]) == p.x) ? j : idx;
+  partials[static_cast<size_t>(nb0 / kScoreStrip) * M + row] = p;
+  const unsigned long long packed = pack_best(p.x, static_cast<uint32_t>(nb0 + idx));
+  if (packed > seen) atomicMax(best + row, packed);
+}
+
 // ------------------------------------------------------------------ the kernel
-// kDigits: the encoding; kFast: tolerance mode (digits only); kTrace: the SLIMT_B200_TRACE build (exact digits, KB = 2).
-// tma_e / dshift / inv_um are read by the digits only, c127 / dmax / eta by the bound filter only.
-template <bool kDigits, int KB, bool kFast, bool kTrace>  // K = 128 * KB bytes per row
+// kDigits: the encoding; kFast: tolerance mode (digits only); kTrace: the SLIMT_B200_TRACE build (exact digits, KB = 2);
+// kScores: the scores epilogue (kDigits = false: the weights alone, no column table).
+// tma_e / dshift / inv_um are read by the digits only, c127 by the bound filter and the scores, dmax / eta by the bound
+// filter only, partials by the scores only.
+template <bool kDigits, int KB, bool kFast, bool kTrace, bool kScores = false>  // K = 128 * KB bytes per row
 __global__ void __launch_bounds__(kThreads, 1)
     out_argmax_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
                       const __grid_constant__ CUtensorMap tma_e, const float* __restrict__ pb,
                       const int32_t* __restrict__ dshift, float um, float inv_um, int M, int N,
                       unsigned long long* __restrict__ best, long long* __restrict__ trace,
-                      const int32_t* __restrict__ c127, const float* __restrict__ dmax, float eta) {
+                      const int32_t* __restrict__ c127, const float* __restrict__ dmax, float eta,
+                      float2* __restrict__ partials) {
   using L = Smem<kDigits, KB>;
   constexpr int kStages = L::kStages;
   constexpr int kABytes = kBM * kBK;
@@ -404,7 +435,7 @@ __global__ void __launch_bounds__(kThreads, 1)
     auto prefetch = [&](int n, int m) {
       const int row = m * kBM + row_in_tile;
       seen_next = row < M ? __ldcg(best + row) : ~0ull;
-      if constexpr (!kDigits) {
+      if constexpr (!kDigits && !kScores) {
         const int ch = (n * kBN + quarter * 64) >> 5;
         dm0_next = ch < nch ? __ldg(dmax + ch) : ninf;
         dm1_next = ch + 1 < nch ? __ldg(dmax + ch + 1) : ninf;
@@ -431,7 +462,9 @@ __global__ void __launch_bounds__(kThreads, 1)
       __syncwarp();
       if (lane == 0) mbar_arrive(&tmem_empty[buf]);  // accumulators are in registers: release the buffer
 
-      if constexpr (kDigits) {
+      if constexpr (kScores) {
+        scores_exact(v0, v1, seen, row, nb0, M, N, pb, c127, um, best, partials);
+      } else if constexpr (kDigits) {
         int g[8];
         const int mx = digit_groups(v0, v1, nb0, N, g);
         if constexpr (kFast)
@@ -528,7 +561,7 @@ int launch_out_argmax(const OutColumns& c, const CUtensorMap& tma_a, bool fast, 
   auto go = [&](auto kern, size_t smem) {
     if (ensure_dyn_smem(kern, smem) != cudaSuccess) return 1;
     return launch_pdl(kern, dim3(grid), dim3(kThreads), smem, stream, tma_a, c.map_w, c.map_ext, c.pb, c.dshift, c.um,
-                      inv_um, M, N, best, trace, c.c127, c.dmax, c.eta) != cudaSuccess ? 1 : 0;
+                      inv_um, M, N, best, trace, c.c127, c.dmax, c.eta, static_cast<float2*>(nullptr)) != cudaSuccess ? 1 : 0;
   };
   if (!c.digits) {
     if (KB == 2) return go(out_argmax_kernel<false, 2, false, false>, Smem<false, 2>::total);
@@ -538,6 +571,23 @@ int launch_out_argmax(const OutColumns& c, const CUtensorMap& tma_a, bool fast, 
   if (trace != nullptr && KB == 2 && !fast) return go(out_argmax_kernel<true, 2, false, true>, Smem<true, 2>::total);  // the profiled build
   if (KB == 2) return fast ? go(out_argmax_kernel<true, 2, true, false>, Smem<true, 2>::total) : go(out_argmax_kernel<true, 2, false, false>, Smem<true, 2>::total);
   if (KB == 4) return fast ? go(out_argmax_kernel<true, 4, true, false>, Smem<true, 4>::total) : go(out_argmax_kernel<true, 4, false, false>, Smem<true, 4>::total);
+  return 1;
+}
+
+int launch_out_scores(const OutColumns& c, const CUtensorMap& tma_a, int M, int K, unsigned long long* best,
+                      float2* partials, int num_sms, cudaStream_t stream) {
+  const int KB = K / kBK, N = c.N;
+  const long tiles = static_cast<long>((M + kBM - 1) / kBM) * ((N + kBN - 1) / kBN);
+  const int grid = static_cast<int>(tiles < num_sms ? tiles : num_sms);
+  if (grid == 0) return 0;
+  auto go = [&](auto kern, size_t smem) {
+    if (ensure_dyn_smem(kern, smem) != cudaSuccess) return 1;
+    return launch_pdl(kern, dim3(grid), dim3(kThreads), smem, stream, tma_a, c.map_w, c.map_w, c.pb,
+                      static_cast<const int32_t*>(nullptr), c.um, 0.0f, M, N, best, static_cast<long long*>(nullptr), c.c127,
+                      static_cast<const float*>(nullptr), 0.0f, partials) != cudaSuccess ? 1 : 0;
+  };
+  if (KB == 2) return go(out_argmax_kernel<false, 2, false, false, true>, Smem<false, 2>::total);
+  if (KB == 4) return go(out_argmax_kernel<false, 4, false, false, true>, Smem<false, 4>::total);
   return 1;
 }
 

@@ -47,6 +47,7 @@ int lazy_shortlist_cb(void* user, const uint32_t** words, size_t* n) {
 struct Done {
   std::vector<uint32_t> kept;
   std::vector<float> align;  // per sentence [target_len][source_len], back to back (only when asked for)
+  std::vector<float> scores;  // like kept (only when asked for)
 };
 
 struct LaneStats {
@@ -87,6 +88,7 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
   io->kernel_launches = 0, io->h2d_bytes = 0, io->d2h_bytes = 0;
   const size_t n_sent = io->n_sentences;
   const bool want_align = io->out_alignments != nullptr;
+  const bool want_scores = io->out_scores != nullptr;
 
   ShortlistGenerator gen;
   const bool use_sl = io->shortlist_bin != nullptr && io->shortlist_bytes > 0;
@@ -169,11 +171,13 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
       const Plan& p = plan[bi];
       const size_t B = p.ids.size(), width = p.width;
       const size_t stride = static_cast<size_t>(forward_max_steps(io->limit_factor, width));
-      // staging: [padded tokens][lengths] | [sentence-major step tokens][recorded lengths] | [alignment rows]
+      // staging: [padded tokens][lengths] | [sentence-major step tokens][recorded lengths] | [alignment rows] |
+      // [step-major scores]
       const size_t in_bytes = (4 * (B * width + B) + 255) & ~size_t(255);
       const size_t tok_bytes = (4 * (stride + 1) * B + 255) & ~size_t(255);
       const size_t al_bytes = want_align ? 4 * stride * B * width : 0;
-      char* stage = c.staging_reserve(in_bytes + tok_bytes + al_bytes + 256);
+      const size_t sc_bytes = want_scores ? 4 * stride * B : 0;
+      char* stage = c.staging_reserve(in_bytes + tok_bytes + al_bytes + sc_bytes + 256);
       if (!stage) {
         st.error = last_error();
         failed = true;
@@ -198,12 +202,14 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
       uint32_t* rows = reinterpret_cast<uint32_t*>(stage + in_bytes);
       uint32_t* lens = rows + stride * B;
       float* align = want_align ? reinterpret_cast<float*>(stage + in_bytes + tok_bytes) : nullptr;
+      float* scores = want_scores ? reinterpret_cast<float*>(stage + in_bytes + tok_bytes + al_bytes) : nullptr;
       ForwardArgs a;
       a.tokens = tokens, a.lengths = lengths, a.B = B, a.T = width;
       a.limit_factor = io->limit_factor;
       if (use_sl) a.shortlist_cb = lazy_shortlist_cb, a.shortlist_user = &lazy;
       a.sentence_tokens = rows, a.row_stride = stride, a.target_lengths = lens;
       a.alignment = align;
+      a.scores = scores;
       if (!timed) {
         cudaEventCreate(&e0), cudaEventCreate(&e1);
         cudaEventRecord(e0, c.stream);
@@ -235,6 +241,12 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
             memcpy(d.align.data() + ap, align + (s * B + r) * width, 4ul * lengths[r]);
             ap += lengths[r];
           }
+      }
+      if (want_scores) {  // the scores of the recorded steps, sentence by sentence in batch row order like kept
+        d.scores.resize(kept_total);
+        size_t sp = 0;
+        for (size_t r = 0; r < B; r++)
+          for (size_t s = 0; s < lens[r]; s++) d.scores[sp++] = scores[s * B + r];
       }
       st.target_tokens += a.target_tokens;
     }
@@ -270,8 +282,8 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
   // ---- ragged outputs
   std::vector<uint64_t> out_off(n_sent + 1, 0);
   for (size_t i = 0; i < n_sent; i++) out_off[i + 1] = out_off[i] + out_len[i];
-  if (io->out_tokens && out_off[n_sent] > io->out_capacity) {
-    set_error("out_tokens capacity too small");
+  if ((io->out_tokens || want_scores) && out_off[n_sent] > io->out_capacity) {
+    set_error(io->out_tokens ? "out_tokens capacity too small" : "out_scores capacity too small");
     return 1;
   }
   if (io->out_offsets) memcpy(io->out_offsets, out_off.data(), 8 * (n_sent + 1));
@@ -280,6 +292,15 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
       size_t pos = 0;
       for (size_t s : plan[bi].ids) {
         memcpy(io->out_tokens + out_off[s], done[bi].kept.data() + pos, 4ul * out_len[s]);
+        pos += out_len[s];
+      }
+    }
+  }
+  if (want_scores) {
+    for (size_t bi = 0; bi < plan.size(); bi++) {
+      size_t pos = 0;
+      for (size_t s : plan[bi].ids) {
+        memcpy(io->out_scores + out_off[s], done[bi].scores.data() + pos, 4ul * out_len[s]);
         pos += out_len[s];
       }
     }

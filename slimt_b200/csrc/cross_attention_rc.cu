@@ -27,12 +27,6 @@
 #include "kernels.cuh"
 #include "ptx.cuh"
 
-// phase stamp of consumer thread 0 into the CTA's trace slots (groups 0..5 of the CTA; no-op without a trace buffer)
-#define RC_TRACE(slot)                                                                         \
-  do {                                                                                         \
-    if (a.trace && ct == 0 && it < 6) a.trace[blockIdx.x * 128 + 8 + 16 * it + (slot)] = clock64(); \
-  } while (0)
-
 namespace sb {
 
 namespace {
@@ -230,7 +224,6 @@ __global__ void __launch_bounds__(kThreadsRc, 1) cross_attention_rc_kernel(const
       }
       cp_async_commit();
     };
-    if (a.trace && ct == 0) a.trace[blockIdx.x * 128] = clock64();
     fetch_group(blockIdx.x, 0);
     // Accumulators travel TMEM -> registers one phase ahead of their use: the V accumulators are requested as soon as the
     // scores are formed (the K registers are dead then) and arrive during the softmax; the next group's K accumulators are
@@ -262,9 +255,7 @@ __global__ void __launch_bounds__(kThreadsRc, 1) cross_attention_rc_kernel(const
       const int* s_len = s_len_all + (it & 1) * kGroup;
       cp_async_wait_all();
       fetch_group(g + gridDim.x, (it & 1) ^ 1);
-      RC_TRACE(0);
       named_bar_sync(1, kConsThreads);
-      RC_TRACE(1);
 
       // ---- K phase: quadrant = 32 keys of a sentence, lane = key, two heads per warp
       {
@@ -272,9 +263,7 @@ __global__ void __launch_bounds__(kThreadsRc, 1) cross_attention_rc_kernel(const
         const int b = b0 + j;
         const int len_k = min(s_len[kj], a.T);
         const bool valid = key < len_k;
-        RC_TRACE(2);
         tmem_ld_wait_dep(v0, v1);
-        RC_TRACE(3);
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(k_drained);
@@ -367,7 +356,6 @@ __global__ void __launch_bounds__(kThreadsRc, 1) cross_attention_rc_kernel(const
           sc[0] = __fmul_rn(a.dk, acc0);
           sc[1] = __fmul_rn(a.dk, acc1);
         }
-        RC_TRACE(4);
         request_v(ph);
         // softmax over the sentence's keys (slimt/TensorOps.cc:282-315): max, exp, sum in key order, divide.  Both
         // heads advance together: nothing is stored between the two expf evaluations (a store would pin the second
@@ -438,15 +426,11 @@ __global__ void __launch_bounds__(kThreadsRc, 1) cross_attention_rc_kernel(const
         }
         }  // exact K phase
       }
-      RC_TRACE(5);
       named_bar_sync(1, kConsThreads);
-      RC_TRACE(6);
 
       // ---- V phase: lane = output feature; KB = 1: two sentences per warp, KB = 2: one sentence of up to 64 keys
       {
-        RC_TRACE(7);
         tmem_ld_wait_dep(v0, v1);
-        RC_TRACE(8);
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(v_drained);
@@ -521,10 +505,8 @@ __global__ void __launch_bounds__(kThreadsRc, 1) cross_attention_rc_kernel(const
               acc0 = fmaf(p0.w, dequant1(static_cast<int>(v0[l + 3]), a.um_v, pbv), acc0);
               acc1 = fmaf(p1.w, dequant1(static_cast<int>(v1[l + 3]), a.um_v, pbv), acc1);
             }
-            RC_TRACE(9);
             emit(b0 + j0, acc0);
             emit(b0 + j0 + 1, acc1);
-            RC_TRACE(10);
           } else {
 #pragma unroll
             for (int jj = 0; jj < 2; jj++) {

@@ -4,7 +4,6 @@
 #include "score_partial.cuh"
 
 #include <math.h>
-#include <stdio.h>
 #include <string.h>
 
 #include <algorithm>
@@ -759,9 +758,6 @@ struct Pass {
   CUtensorMap map_qa[3], map_qa32[3], mapK[2], mapV[2];
   CUtensorMap map_xq[2], map_zq[2], map_caq;  // u8 activation operands of the row-tile kernels, box {128 B, 32 rows}
   CUtensorMap map_oq;
-  const char* trace_path;  // SLIMT_B200_TRACE
-  long long* trace_buf;
-  size_t trace_n;
   int plan(), encode(), prepare_cross(), prepare_output(), decode_step(int step), decode();
 };
 
@@ -860,15 +856,6 @@ int Pass::plan() {
   for (int i = 0; i < 2; i++)
     if (c.make_map(&map_xq[i], xq[i], B, E, kRowTile) || c.make_map(&map_zq[i], zq[i], B, E, kRowTile)) return 1;
   if (c.make_map(&map_caq, caq, B, E, kRowTile) || c.make_map(&map_oq, oq, B, E, kBM)) return 1;
-
-  // debugging aid: SLIMT_B200_TRACE=<file> records the phase stamps of the row-tile kernels: the encoder's first FFN
-  // launch (first tile of every CTA) and the two decoder kernels of layer 0 in decode step 3
-  trace_path = getenv("SLIMT_B200_TRACE");
-  trace_n = static_cast<size_t>(c.num_sms) * kTraceSlots;
-  if (trace_path) {
-    SB_CUDA(cudaMallocManaged(&trace_buf, 5 * trace_n * sizeof(long long)));
-    SB_CUDA(cudaMemsetAsync(trace_buf, 0, 5 * trace_n * sizeof(long long), s));
-  }
   return 0;
 }
 
@@ -960,7 +947,6 @@ int Pass::encode() {
         k.n_zq = 2 * Ld;
       }
       k.M = R;
-      if (trace_buf && i == 0) k.trace = trace_buf + 2 * trace_n;
       const double Rd = R, Ed = E, Fd = F;
       LaunchScope ls(c, "enc_wo_ffn_fused", 2.0 * Rd * (Ed * Ed + 2.0 * Ed * Fd),
                      Ed * Ed + 2.0 * Ed * Fd + Rd * Ed * (1.0 + 4.0 + 4.0 + k.n_zq));  // u8 in, residual, f32 out, u8 copies
@@ -1094,7 +1080,6 @@ int Pass::decode_step(int step) {
       }
       k.ln_scale = L.rnn_ln.scale, k.ln_bias = L.rnn_ln.bias, k.eps = 1e-6f;
       k.h_out = hb, k.q_out = qd, k.M = B;
-      if (trace_buf && step == 3 && l == 0) k.trace = trace_buf;
       const double Bd = B, Ed = E;
       LaunchScope ls(c, "dec_ssru_q_fused", 2.0 * Bd * 3.0 * Ed * Ed, 3.0 * Ed * Ed + Bd * Ed * (2.0 + 4.0 * 5.0));
       if (launch_dec_ssru(k, E, c.fast, s)) {
@@ -1113,7 +1098,6 @@ int Pass::decode_step(int step) {
       k.qo = qouts();
       qadd(k.qo, caq, L.ctx.o.aq);
       k.attn_head0 = last ? d_align : nullptr;
-      if (trace_buf && step == 3 && l == 0) k.trace = trace_buf + 3 * trace_n;
       const double Bd = B, Ed = E;
       const bool rcl = route.cross == Cross::Rcl;
       LaunchScope ls(c, "dec_cross_attention_rc", 2.0 * (rcl ? src_tokens : Bd * (T > 32 ? 64.0 : 32.0)) * Ed * 2.0 * Ed,
@@ -1154,7 +1138,6 @@ int Pass::decode_step(int step) {
         k.n_zq = 2;
       }
       k.M = B;
-      if (trace_buf && step == 3 && l == 0) k.trace = trace_buf + trace_n;
       const double Bd = B, Ed = E, Fd = F;
       LaunchScope ls(c, "dec_wo_ffn_fused", 2.0 * Bd * (Ed * Ed + 2.0 * Ed * Fd),
                      Ed * Ed + 2.0 * Ed * Fd + Bd * Ed * (1.0 + 4.0 + (last ? 1.0 : 6.0)));
@@ -1192,8 +1175,7 @@ int Pass::decode_step(int step) {
   } else {
     const double Md = B, Nd = Nout, Kd = E;
     LaunchScope ls(c, "dec_gemm_out_argmax", 2.0 * Md * Nd * Kd, Md * Kd + Nd * Kd + 4.0 * Nd + 8.0 * Md);
-    if (launch_out_argmax(out, map_oq, c.fast, B, E, best, c.num_sms, s,
-                          (trace_buf && step == 3) ? trace_buf + 4 * trace_n : nullptr)) {
+    if (launch_out_argmax(out, map_oq, c.fast, B, E, best, c.num_sms, s)) {
       set_error("output GEMM: unsupported K " + std::to_string(E));
       return 1;
     }
@@ -1266,24 +1248,7 @@ int Pass::decode() {
     host_done = c.done_slots[0];
   }
 
-  // ---- SLIMT_B200_TRACE file and results
-  if (trace_buf) {
-    SB_CUDA(cudaStreamSynchronize(s));
-    if (FILE* f = fopen(trace_path, "w")) {
-      for (int k = 0; k < 5; k++)
-        for (int cta = 0; cta < c.num_sms; cta++) {
-          const long long* t = trace_buf + k * trace_n + static_cast<size_t>(cta) * kTraceSlots;
-          if (t[0] == 0) continue;
-          fprintf(f, "%s %d", k == 0 ? "ssru" : k == 1 ? "ffn" : k == 2 ? "encffn" : k == 3 ? "cross" : "out", cta);
-          // (the output GEMM's slots 4.. are counts and accumulated waits, not stamps)
-          for (int i = 0; i < kTraceSlots; i++) fprintf(f, " %lld", (k == 4 && i >= 4) ? t[i] : (t[i] ? t[i] - t[0] : -1));
-          fprintf(f, "\n");
-        }
-      fclose(f);
-    }
-    cudaFree(trace_buf);
-  }
-
+  // ---- results
   std::vector<uint32_t> lens(B);
   SB_CUDA(cudaMemcpyAsync(lens.data(), tgt_len, 4ul * B, cudaMemcpyDeviceToHost, s));
   if (d_align_all && executed > 0) {

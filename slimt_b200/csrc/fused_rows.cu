@@ -59,7 +59,6 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + L::tmem_slot);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (threadIdx.x == 0) SB_TRACE(a, 0);
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&a.map_xf);
     tma_prefetch_desc(&a.map_xw);
@@ -96,7 +95,6 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
   // positions live in the leader's registers across tiles, hence a single election.
   const bool leader = elect_one();
   pdl_wait();  // everything above overlapped the previous kernel's tail; its outputs are visible from here on
-  if (threadIdx.x == 0) SB_TRACE(a, 1);
   for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, iter++) {
     const int row0 = tile * kR;
     const uint32_t tph = iter & 1;
@@ -121,20 +119,16 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
       if (leader) {
         mbar_wait(x_full, tph);
         if constexpr (kEmbed) tc_fence_after();
-        SB_TRACE(a, 2);
         for (int mb = 0; mb < EM; mb++)
           for (int kb = 0; kb < EK; kb++) cons.mma(tmem_f + mb * kR, opnd_xf + kb * kOpK, kb == 0);
         for (int mb = 0; mb < EM; mb++)
           for (int kb = 0; kb < EK; kb++) cons.mma(tmem_w + mb * kR, opnd_xw + kb * kOpK, kb == 0);
         umma_commit(g0_done);
-        SB_TRACE(a, 3);
         mbar_wait(hq_ready, tph);
         tc_fence_after();
-        SB_TRACE(a, 8);
         for (int mb = 0; mb < EM; mb++)
           for (int kb = 0; kb < EK; kb++) cons.mma(tmem_q + mb * kR, opnd_h + kb * kOpK, kb == 0);
         umma_commit(g1_done);
-        SB_TRACE(a, 9);
       }
     } else if (warp >= 4) {
       const int ew = warp - 4;
@@ -171,9 +165,7 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
             }
             s_tok[et] = tok;
           }
-          if (et == 0) SB_TRACE(a, 15);
           named_bar_sync(1, kEpiThreads);
-          if (et == 0) SB_TRACE(a, 16);
           // swizzled byte offset of (row, f) inside an operand k-block is row * 128 + xo[row & 7] (rows_common.cuh: opnd_off)
           uint32_t xo[8];
           {
@@ -199,7 +191,6 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
           fence_proxy_async();
           __syncwarp();
           if (lane == 0) mbar_arrive(x_full);
-          if (et == 0) SB_TRACE(a, 17);
           if (et < kR && bk < a.M) {  // record(): append unless already finished; re-arm the packed best
             a.step_tokens[static_cast<size_t>(a.prev_step) * a.M + bk] = word;
             if (!was_done) {
@@ -222,10 +213,8 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
             if constexpr (!kEmbed) xv[mb][r] = a.x[o];
           }
         }
-        if (et == 0) SB_TRACE(a, 14);
         mbar_wait(g0_done, tph);
         tc_fence_after();
-        if (et == 0) SB_TRACE(a, 4);
 #pragma unroll
         for (int mb = 0; mb < EM; mb++) {
           uint32_t vf[8], vw[8];
@@ -252,11 +241,9 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
         }
       }
       named_bar_sync(1, kEpiThreads);
-      if (et == 0) SB_TRACE(a, 5);
       if constexpr (kFast) ln_stats_fast<E, kR>(xs, stats, a.eps, ew, lane);
       else if (et < kR) ln_stats_row<E>(xs + et * XS, &stats[et], &stats[32 + et], a.eps);
       named_bar_sync(1, kEpiThreads);
-      if (et == 0) SB_TRACE(a, 6);
       {
         const float g = a.ln_scale[nf], b = a.ln_bias[nf];
 #pragma unroll 4
@@ -270,12 +257,10 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
       fence_proxy_async();
       __syncwarp();
       if (lane == 0) mbar_arrive(hq_ready);
-      if (et == 0) SB_TRACE(a, 7);
 
       // ---- q = Wq h + bq -> global
       mbar_wait(g1_done, tph);
       tc_fence_after();
-      if (et == 0) SB_TRACE(a, 10);
 #pragma unroll
       for (int mb = 0; mb < EM; mb++) {
         uint32_t v[8];
@@ -289,13 +274,11 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
           if (grow < a.M) a.q_out[static_cast<size_t>(grow) * E + f] = dequant<kFast>(static_cast<int>(v[r]), a.um_q, pb);
         }
       }
-      if (et == 0) SB_TRACE(a, 11);
     }
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
   }
-  if (threadIdx.x == 0) SB_TRACE(a, 13);
   if (warp == 2) tmem_dealloc<512>(tmem);
 }
 

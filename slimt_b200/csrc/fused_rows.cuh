@@ -16,7 +16,6 @@
 namespace sb {
 
 constexpr int kRowTile = 32;
-constexpr int kTraceSlots = 128;  // debugging aid: per-CTA clock64() stamps of a kernel's phase boundaries
 
 // Attention output projection + residual + LayerNorm, then the feed-forward block with its own residual +
 // LayerNorm (encoder and decoder layers):  y = LN1(res + Wo a + bo);  z = LN2(y + W2 relu(W1 y + b1) + b2).
@@ -41,7 +40,6 @@ struct RowsFfnArgs {
   int n_zq;
   int zq_signed;                       // bit k: zq[k] receives the signed value instead of u8 = q + 127
   int M;
-  long long* trace;                    // optional phase timestamps (clock64), kTraceSlots per CTA; see SLIMT_B200_TRACE
 };
 
 // SSRU cell + query projection:  c = sigmoid(Wf x + bf) * c_prev + (1 - sigmoid(.)) * (W x);
@@ -62,7 +60,6 @@ struct DecSsruArgs {
   float* h_out;                        // f32 [M][E]
   float* q_out;                        // f32 [M][E]
   int M;
-  long long* trace;                    // optional phase timestamps, as above
   // ---- layer 0 from the second step on (embed != 0): the kernel's front does what finalize_step_kernel does for the
   // PREVIOUS step -- packed argmax -> word id (through the shortlist), record into step_tokens[prev_step][M], EOS
   // bookkeeping (Model.cc:127-137), re-arm `best` -- and builds this step's input from the word's embedding row

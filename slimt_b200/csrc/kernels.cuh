@@ -68,7 +68,6 @@ struct CrossRcArgs {
   float dk;                    // 1 / sqrt(head size)
   QuantOuts qo;                // int8 copies of the output (Wo's operand)
   float* attn_head0;           // optional [B][T]
-  long long* trace;            // optional phase stamps (clock64) of consumer thread 0, 128 slots per CTA (SLIMT_B200_TRACE)
 };
 bool cross_attention_rc_supported(int E, int H, int dh, int S);
 int launch_cross_attention_rc(const CrossRcArgs& a, int num_sms, bool fast, cudaStream_t stream);

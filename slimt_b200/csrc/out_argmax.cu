@@ -117,25 +117,22 @@ __device__ __forceinline__ void digits_tolerance(const uint32_t (&v0)[32], const
 }
 
 // Digits, exact mode: the columns within kDelta proxy units of the strip's maximum and of the row's best so far, each
-// evaluated with the exact formula; the first strict maximum.  tr: SLIMT_B200_TRACE counters (slots 9 and 10).
-template <bool kTrace>
+// evaluated with the exact formula; the first strict maximum.
 __device__ __forceinline__ void digits_exact(const uint32_t (&v0)[32], const uint32_t (&v1)[32], const int (&g)[8],
                                              int mx, unsigned long long seen, int row, int nb0, int M, int N,
                                              const float* __restrict__ pb, const int32_t* __restrict__ dshift, float um,
-                                             float inv_um, unsigned long long* __restrict__ best, long long* tr, int lane) {
+                                             float inv_um, unsigned long long* __restrict__ best) {
   int floor_p = INT_MIN + 16;
   // proxy of the best column so far >= its logit / um - 1.25; the product itself is good to half a unit
   if (seen != 0ull) floor_p = __float2int_rd(best_value(seen) * inv_um) - 3;
   const bool trig = row < M && nb0 < N && mx >= floor_p - kDelta;
   const int thr = max(mx, floor_p) - kDelta;
   if (__any_sync(0xffffffffu, trig)) {
-    if (kTrace && tr && lane == 0) atomicAdd(reinterpret_cast<unsigned long long*>(tr + 9), 1ull);  // strips on the exact path, all warps
     int bi = -1;
     float bvf = 0.0f;
 #pragma unroll
     for (int k = 0; k < 8; k++) {
       if (__any_sync(0xffffffffu, trig && g[k] >= thr)) {
-        if (kTrace && tr && lane == 0) atomicAdd(reinterpret_cast<unsigned long long*>(tr + 10), 1ull);  // 8-column groups evaluated
 #pragma unroll
         for (int jj = 0; jj < 8; jj++) {
           const int j = 8 * k + jj;
@@ -259,18 +256,17 @@ __device__ __forceinline__ void scores_exact(const uint32_t (&v0)[32], const uin
 }
 
 // ------------------------------------------------------------------ the kernel
-// kDigits: the encoding; kFast: tolerance mode (digits only); kTrace: the SLIMT_B200_TRACE build (exact digits, KB = 2);
-// kScores: the scores epilogue (kDigits = false: the weights alone, no column table).
+// kDigits: the encoding; kFast: tolerance mode (digits only); kScores: the scores epilogue (kDigits = false: the weights
+// alone, no column table).
 // tma_e / dshift / inv_um are read by the digits only, c127 by the bound filter and the scores, dmax / eta by the bound
 // filter only, partials by the scores only.
-template <bool kDigits, int KB, bool kFast, bool kTrace, bool kScores = false>  // K = 128 * KB bytes per row
+template <bool kDigits, int KB, bool kFast, bool kScores = false>  // K = 128 * KB bytes per row
 __global__ void __launch_bounds__(kThreads, 1)
     out_argmax_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
                       const __grid_constant__ CUtensorMap tma_e, const float* __restrict__ pb,
                       const int32_t* __restrict__ dshift, float um, float inv_um, int M, int N,
-                      unsigned long long* __restrict__ best, long long* __restrict__ trace,
-                      const int32_t* __restrict__ c127, const float* __restrict__ dmax, float eta,
-                      float2* __restrict__ partials) {
+                      unsigned long long* __restrict__ best, const int32_t* __restrict__ c127,
+                      const float* __restrict__ dmax, float eta, float2* __restrict__ partials) {
   using L = Smem<kDigits, KB>;
   constexpr int kStages = L::kStages;
   constexpr int kABytes = kBM * kBK;
@@ -334,14 +330,7 @@ __global__ void __launch_bounds__(kThreads, 1)
   __syncthreads();
   tc_fence_after();
   pdl_launch_dependents();
-  // optional per-CTA profile (SLIMT_B200_TRACE): 0 entry, 1 released by the previous kernel, 2 last tile's epilogue done,
-  // 3 exit, 4 tiles, 5 weight tiles, 6-8 MMA thread waiting for weights / a free accumulator buffer / activation tiles,
-  // 9 strips that took the exact path, 10 eight-column groups evaluated exactly (all epilogue warps)
-  // (a template flag, not a run-time test: the test alone cost 3 us per launch in the single-thread MMA loop)
-  long long* tr = (kTrace && trace) ? trace + static_cast<size_t>(blockIdx.x) * 128 : nullptr;
-  if (kTrace && tr && threadIdx.x == 0) tr[0] = clock64();
   pdl_wait();  // everything above overlapped the previous kernel's tail; its outputs are visible from here on
-  if (kTrace && tr && threadIdx.x == 0) tr[1] = clock64(), tr[4] = t_end - t_begin;
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0) {
@@ -378,32 +367,21 @@ __global__ void __launch_bounds__(kThreads, 1)
       const uint64_t dbe = make_kmajor_sw128_desc(smem_u32(smem_be));
       uint32_t kbc = 0, run = 0, i = 0;
       int n = n_first, m = m_first, cur_n = -1;
-      long long w_b = 0, w_t = 0, w_a = 0;
       for (int t = t_begin; t < t_end; t++, i++) {
         if (n != cur_n) {
-          const long long c0 = (kTrace && tr) ? clock64() : 0;
           mbar_wait(b_full, run & 1);
-          if (kTrace && tr) w_b += clock64() - c0;
           cur_n = n;
           run++;
         }
         const uint32_t buf = i & 1;
         const uint32_t tmem_d = tmem_base + buf * kBN;
-        {
-          const long long c0 = (kTrace && tr) ? clock64() : 0;
-          mbar_wait(&tmem_empty[buf], ((i >> 1) & 1) ^ 1);
-          if (kTrace && tr) w_t += clock64() - c0;
-        }
+        mbar_wait(&tmem_empty[buf], ((i >> 1) & 1) ^ 1);
         tc_fence_after();
 #pragma unroll
         for (int kb = 0; kb < KB; kb++, kbc++) {
           const uint32_t s = kbc % kStages;
           const uint32_t ph = (kbc / kStages) & 1;
-          {
-            const long long c0 = (kTrace && tr) ? clock64() : 0;
-            mbar_wait(&full_bar[s], ph);
-            if (kTrace && tr) w_a += clock64() - c0;
-          }
+          mbar_wait(&full_bar[s], ph);
           tc_fence_after();
           const uint64_t da = make_kmajor_sw128_desc(smem_u32(smem_a + s * kABytes));
           const uint64_t db = make_kmajor_sw128_desc(smem_u32(smem_b + kb * kBBytes));
@@ -417,7 +395,6 @@ __global__ void __launch_bounds__(kThreads, 1)
         if (last_of_run) umma_commit(b_empty);
         if (++m == m_tiles) m = 0, n++;
       }
-      if (kTrace && tr) tr[5] = run, tr[6] = w_b, tr[7] = w_t, tr[8] = w_a;
     }
   } else if (warp >= 4) {
     // ===== epilogue: thread <-> TMEM lane <-> output row; warp = (lane quadrant, 64-column strip) =====
@@ -470,19 +447,17 @@ __global__ void __launch_bounds__(kThreads, 1)
         if constexpr (kFast)
           digits_tolerance(v0, v1, g, mx, seen, row, nb0, M, N, best);
         else
-          digits_exact<kTrace>(v0, v1, g, mx, seen, row, nb0, M, N, pb, dshift, um, inv_um, best, tr, lane);
+          digits_exact(v0, v1, g, mx, seen, row, nb0, M, N, pb, dshift, um, inv_um, best);
       } else {
         bounds_exact(v0, v1, dm0, dm1, seen, row, nb0, M, N, pb, c127, um, eta, best);
       }
       m = m_nx, n = n_nx;
     }
-    if (kTrace && tr && warp == 4 && lane == 0) tr[2] = clock64();
   }
 
   tc_fence_before();
   __syncthreads();
   if (warp == 2) tmem_dealloc<512>(tmem_base);
-  if (kTrace && tr && threadIdx.x == 0) tr[3] = clock64();
 }
 
 // ------------------------------------------------------------------ per-column tables
@@ -552,7 +527,7 @@ void launch_out_tables(const OutColumns& c, int* overflow, cudaStream_t stream) 
 }
 
 int launch_out_argmax(const OutColumns& c, const CUtensorMap& tma_a, bool fast, int M, int K, unsigned long long* best,
-                      int num_sms, cudaStream_t stream, long long* trace) {
+                      int num_sms, cudaStream_t stream) {
   const int KB = K / kBK, N = c.N;
   const long tiles = static_cast<long>((M + kBM - 1) / kBM) * ((N + kBN - 1) / kBN);
   const int grid = static_cast<int>(tiles < num_sms ? tiles : num_sms);
@@ -561,16 +536,15 @@ int launch_out_argmax(const OutColumns& c, const CUtensorMap& tma_a, bool fast, 
   auto go = [&](auto kern, size_t smem) {
     if (ensure_dyn_smem(kern, smem) != cudaSuccess) return 1;
     return launch_pdl(kern, dim3(grid), dim3(kThreads), smem, stream, tma_a, c.map_w, c.map_ext, c.pb, c.dshift, c.um,
-                      inv_um, M, N, best, trace, c.c127, c.dmax, c.eta, static_cast<float2*>(nullptr)) != cudaSuccess ? 1 : 0;
+                      inv_um, M, N, best, c.c127, c.dmax, c.eta, static_cast<float2*>(nullptr)) != cudaSuccess ? 1 : 0;
   };
   if (!c.digits) {
-    if (KB == 2) return go(out_argmax_kernel<false, 2, false, false>, Smem<false, 2>::total);
-    if (KB == 4) return go(out_argmax_kernel<false, 4, false, false>, Smem<false, 4>::total);
+    if (KB == 2) return go(out_argmax_kernel<false, 2, false>, Smem<false, 2>::total);
+    if (KB == 4) return go(out_argmax_kernel<false, 4, false>, Smem<false, 4>::total);
     return 1;
   }
-  if (trace != nullptr && KB == 2 && !fast) return go(out_argmax_kernel<true, 2, false, true>, Smem<true, 2>::total);  // the profiled build
-  if (KB == 2) return fast ? go(out_argmax_kernel<true, 2, true, false>, Smem<true, 2>::total) : go(out_argmax_kernel<true, 2, false, false>, Smem<true, 2>::total);
-  if (KB == 4) return fast ? go(out_argmax_kernel<true, 4, true, false>, Smem<true, 4>::total) : go(out_argmax_kernel<true, 4, false, false>, Smem<true, 4>::total);
+  if (KB == 2) return fast ? go(out_argmax_kernel<true, 2, true>, Smem<true, 2>::total) : go(out_argmax_kernel<true, 2, false>, Smem<true, 2>::total);
+  if (KB == 4) return fast ? go(out_argmax_kernel<true, 4, true>, Smem<true, 4>::total) : go(out_argmax_kernel<true, 4, false>, Smem<true, 4>::total);
   return 1;
 }
 
@@ -583,11 +557,11 @@ int launch_out_scores(const OutColumns& c, const CUtensorMap& tma_a, int M, int 
   auto go = [&](auto kern, size_t smem) {
     if (ensure_dyn_smem(kern, smem) != cudaSuccess) return 1;
     return launch_pdl(kern, dim3(grid), dim3(kThreads), smem, stream, tma_a, c.map_w, c.map_w, c.pb,
-                      static_cast<const int32_t*>(nullptr), c.um, 0.0f, M, N, best, static_cast<long long*>(nullptr), c.c127,
+                      static_cast<const int32_t*>(nullptr), c.um, 0.0f, M, N, best, c.c127,
                       static_cast<const float*>(nullptr), 0.0f, partials) != cudaSuccess ? 1 : 0;
   };
-  if (KB == 2) return go(out_argmax_kernel<false, 2, false, false, true>, Smem<false, 2>::total);
-  if (KB == 4) return go(out_argmax_kernel<false, 4, false, false, true>, Smem<false, 4>::total);
+  if (KB == 2) return go(out_argmax_kernel<false, 2, false, true>, Smem<false, 2>::total);
+  if (KB == 4) return go(out_argmax_kernel<false, 4, false, true>, Smem<false, 4>::total);
   return 1;
 }
 

@@ -53,11 +53,10 @@ void launch_out_tables(const OutColumns& c, int* overflow, cudaStream_t stream);
 
 // best[M] (pre-zeroed, packed_best.cuh) receives each row's first maximum over c's columns of the logits of the s8
 // activations in tma_a ([M][K], box {128 B, 128 rows}).  fast selects tolerance mode, which on the digits takes the
-// integer proxy as the score; the bound filter always gives the exact first maximum of the float logits.  trace
-// (optional, exact digits at K = 256 only): per-CTA profile, 128 slots per CTA.  Returns nonzero for an unsupported K
-// (128 * {2, 4} are built).
+// integer proxy as the score; the bound filter always gives the exact first maximum of the float logits.  Returns
+// nonzero for an unsupported K (128 * {2, 4} are built).
 int launch_out_argmax(const OutColumns& c, const CUtensorMap& tma_a, bool fast, int M, int K, unsigned long long* best,
-                      int num_sms, cudaStream_t stream, long long* trace);
+                      int num_sms, cudaStream_t stream);
 
 // The same GEMM with the scores epilogue, in either encoding and arithmetic mode (it reads c.w, c.pb, c.c127 and
 // c.map_w, none of the encoding's tables): every logit is evaluated exactly, best[M] (pre-zeroed) receives each row's

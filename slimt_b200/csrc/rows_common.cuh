@@ -9,13 +9,6 @@
 #include "fused_rows.cuh"
 #include "ptx.cuh"
 
-// phase stamp of the calling thread into the CTA's trace slots (no-op unless the launch carries a trace buffer)
-#define SB_TRACE(args, slot)                                                                  \
-  do {                                                                                        \
-    if ((args).trace && (args).trace[blockIdx.x * kTraceSlots + (slot)] == 0)                 \
-      (args).trace[blockIdx.x * kTraceSlots + (slot)] = clock64(); /* first tile of the CTA */ \
-  } while (0)
-
 namespace sb {
 namespace rows {
 
@@ -146,27 +139,16 @@ struct RingConsumer {
   uint64_t* empty;
   uint32_t it;
   int stages;
-  bool timing = false;     // tracing only: accumulate the cycles spent waiting for weight tiles
-  long long waited = 0;
-  long long* fine = nullptr;  // tracing only: 8 stamps of the next call (entry, tile landed, fence, 4 MMAs, commit)
   __device__ __forceinline__ void mma(uint32_t tmem_d, const uint8_t* opnd_kblock, bool first) {
     constexpr uint32_t idesc = make_idesc_i8_wa(128, R);
     const uint32_t s = it % stages, ph = (it / stages) & 1;
-    const long long t0 = timing ? clock64() : 0;
     mbar_wait(&full[s], ph);
-    if (timing) waited += clock64() - t0;
-    if (fine) fine[0] = t0, fine[1] = clock64();
     tc_fence_after();
-    if (fine) fine[2] = clock64();
     const uint64_t da = make_kmajor_sw128_desc(smem_u32(ring + s * kWTile));
     const uint64_t db = make_kmajor_sw128_desc(smem_u32(opnd_kblock));
 #pragma unroll
-    for (int k = 0; k < 4; k++) {
-      umma_i8(tmem_d, da + 2 * k, db + 2 * k, idesc, (first && k == 0) ? 0u : 1u);
-      if (fine) fine[3 + k] = clock64();
-    }
+    for (int k = 0; k < 4; k++) umma_i8(tmem_d, da + 2 * k, db + 2 * k, idesc, (first && k == 0) ? 0u : 1u);
     umma_commit(&empty[s]);
-    if (fine) fine[7] = clock64(), fine = nullptr;
     it++;
   }
 };

@@ -78,7 +78,6 @@ __global__ void __launch_bounds__(kThreads, 1) rows_ffn_kernel(const __grid_cons
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + L::tmem_slot);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (threadIdx.x == 0) SB_TRACE(a, 0);
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&a.map_a);
     tma_prefetch_desc(&a.map_wo);
@@ -113,15 +112,12 @@ __global__ void __launch_bounds__(kThreads, 1) rows_ffn_kernel(const __grid_cons
   RingProducer prod_b{ring_b, full + L::kStagesA, empty + L::kStagesA, 0, L::kStagesB};
   RingConsumer<R> cons = (warp == 3) ? RingConsumer<R>{ring_b, full + L::kStagesA, empty + L::kStagesA, 0, L::kStagesB}
                                      : RingConsumer<R>{ring, full, empty, 0, L::kStagesA};
-  cons.timing = a.trace != nullptr;
-  long long waited_fq = 0;
 
   // One leader lane per warp, elected once (elect.sync also tells the compiler the branch is single-threaded, so
   // descriptors and addresses stay in uniform registers: no per-MMA waterfall loop as with `lane == 0`).  The ring
   // positions live in the leader's registers across tiles, hence a single election.
   const bool leader = elect_one();
   pdl_wait();  // everything above overlapped the previous kernel's tail; its outputs are visible from here on
-  if (threadIdx.x == 0) SB_TRACE(a, 1);
   for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, iter++) {
     const int row0 = tile * R;
     const uint32_t tph = iter & 1;
@@ -146,30 +142,21 @@ __global__ void __launch_bounds__(kThreads, 1) rows_ffn_kernel(const __grid_cons
       // ~2200 cycles per block for ~700 cycles of tensor-pipe work).  Each has its own weight ring.
       if (leader) {
         mbar_wait(a_full, tph);
-        SB_TRACE(a, 2);
         for (int mb = 0; mb < EM; mb++)
           for (int kb = 0; kb < EK; kb++) cons.mma(tmem_acc + mb * R, opnd_a + kb * kOpK, kb == 0);
         umma_commit(g0_done);
-        SB_TRACE(a, 3);
         mbar_wait(yq_ready, tph);
         tc_fence_after();
-        SB_TRACE(a, 8);
         for (int st = 0; st < FM + kLook; st++) {
           if (st < FM) {  // FFN1 feature block st -> TMEM slot
             const uint32_t n = blocks + st;
             const uint32_t s = n % L::kTS, ph = (n / L::kTS) & 1;
             mbar_wait(&slot_empty[s], ph ^ 1);
             tc_fence_after();
-            for (int kb = 0; kb < EK; kb++) {
-              if (a.trace && st == 5 && kb < 2) cons.fine = a.trace + blockIdx.x * kTraceSlots + 64 + 8 * kb;
-              cons.mma(tmem_ring + s * R, opnd_y + kb * kOpK, kb == 0);
-            }
+            for (int kb = 0; kb < EK; kb++) cons.mma(tmem_ring + s * R, opnd_y + kb * kOpK, kb == 0);
             umma_commit(&slot_full[s]);
-            if (st < 12) SB_TRACE(a, 16 + st);
           }
         }
-        if (a.trace)  // slot 14: cycles this thread spent waiting for weight tiles
-          a.trace[blockIdx.x * kTraceSlots + 14] = a.trace[blockIdx.x * kTraceSlots] + cons.waited;
         blocks += FM;
       }
     } else if (warp == 3) {
@@ -181,21 +168,13 @@ __global__ void __launch_bounds__(kThreads, 1) rows_ffn_kernel(const __grid_cons
             const int kb2 = st - kLook;
             const uint32_t n = blocks + kb2;
             const uint32_t s = n % L::kFS, ph = (n / L::kFS) & 1;
-            const long long t0 = cons.timing ? clock64() : 0;
             mbar_wait(&fq_full[s], ph);
-            if (cons.timing) waited_fq += clock64() - t0;
             tc_fence_after();
-            for (int mb = 0; mb < EM; mb++) {
-              if (a.trace && kb2 == 3 && mb < 2) cons.fine = a.trace + blockIdx.x * kTraceSlots + 80 + 8 * mb;
-              cons.mma(tmem_acc + mb * R, opnd_f + s * kOpK, kb2 == 0);
-            }
+            for (int mb = 0; mb < EM; mb++) cons.mma(tmem_acc + mb * R, opnd_f + s * kOpK, kb2 == 0);
             umma_commit(&fq_free[s]);
-            if (kb2 < 12) SB_TRACE(a, 28 + kb2);
           }
         }
         umma_commit(g2_done);
-        if (a.trace)  // slot 15: cycles this thread spent waiting for requantised blocks
-          a.trace[blockIdx.x * kTraceSlots + 15] = a.trace[blockIdx.x * kTraceSlots] + waited_fq;
         blocks += FM;
       }
     } else if (warp >= 4) {
@@ -222,7 +201,6 @@ __global__ void __launch_bounds__(kThreads, 1) rows_ffn_kernel(const __grid_cons
       // ---- epilogue 0: x = (Wo a + bo) + res -> xs
       mbar_wait(g0_done, tph);
       tc_fence_after();
-      if (et == 0) SB_TRACE(a, 4);
 #pragma unroll 1
       for (int mb = 0; mb < EM; mb++) {
         uint32_t v[RPW];
@@ -241,11 +219,9 @@ __global__ void __launch_bounds__(kThreads, 1) rows_ffn_kernel(const __grid_cons
           xs[(cg * RPW + r) * XS + f] = __fadd_rn(dequant<kFast>(static_cast<int>(v[r]), a.um_o, pb), res[r]);
       }
       named_bar_sync(1, kEpiThreads);
-      if (et == 0) SB_TRACE(a, 5);
       if constexpr (kFast) ln_stats_fast<E, R>(xs, stats, a.eps, ew, lane);
       else if (et < R) ln_stats_row<E>(xs + et * XS, &stats[et], &stats[R + et], a.eps);
       named_bar_sync(1, kEpiThreads);
-      if (et == 0) SB_TRACE(a, 6);
       // y = LN1(x): residual of the FFN block (kept in xs, or parked in global when xs is about to be reused by
       // the operand ring) and the u8 operand of W1
       {
@@ -268,7 +244,6 @@ __global__ void __launch_bounds__(kThreads, 1) rows_ffn_kernel(const __grid_cons
       if constexpr (L::kParkY) named_bar_sync(1, kEpiThreads);  // xs is dead from here: the operand ring may overwrite it
       __syncwarp();
       if (lane == 0) mbar_arrive(yq_ready);
-      if (et == 0) SB_TRACE(a, 7);
 
       // ---- epilogue 1: per FFN1 feature block, relu + requantise -> operand ring slot
 #pragma unroll 1
@@ -278,7 +253,6 @@ __global__ void __launch_bounds__(kThreads, 1) rows_ffn_kernel(const __grid_cons
         const uint32_t fs = n % L::kFS, fph = (n / L::kFS) & 1;
         mbar_wait(&slot_full[ts], tph2);
         tc_fence_after();
-        if (et == 0 && j < 12) SB_TRACE(a, 40 + j);
         uint32_t v[RPW];
         tmem_ldn_nowait<RPW>(tmem_ring + lane_sel + ts * R + cg * RPW, v);
         const float pb = a.pb_1[j * 128 + kk];
@@ -297,14 +271,12 @@ __global__ void __launch_bounds__(kThreads, 1) rows_ffn_kernel(const __grid_cons
         fence_proxy_async();
         __syncwarp();
         if (lane == 0) mbar_arrive(&fq_full[fs]);
-        if (et == 0 && j < 12) SB_TRACE(a, 52 + j);
       }
       blocks += FM;
 
       // ---- epilogue 2: x = (W2 f + b2) + y -> xs; z = LN2(x) -> global
       mbar_wait(g2_done, tph);
       tc_fence_after();
-      if (et == 0) SB_TRACE(a, 9);
 #pragma unroll 1
       for (int mb = 0; mb < EM; mb++) {
         uint32_t v[RPW];
@@ -328,11 +300,9 @@ __global__ void __launch_bounds__(kThreads, 1) rows_ffn_kernel(const __grid_cons
       }
       tc_fence_before();
       named_bar_sync(1, kEpiThreads);
-      if (et == 0) SB_TRACE(a, 10);
       if constexpr (kFast) ln_stats_fast<E, R>(xs, stats, a.eps, ew, lane);
       else if (et < R) ln_stats_row<E>(xs + et * XS, &stats[et], &stats[R + et], a.eps);
       named_bar_sync(1, kEpiThreads);
-      if (et == 0) SB_TRACE(a, 11);
       {
         const float g = a.ln2_scale[nf], b = a.ln2_bias[nf];
         // consumers' quantised copies: pointers and multipliers in registers, sign handling decided once
@@ -358,14 +328,12 @@ __global__ void __launch_bounds__(kThreads, 1) rows_ffn_kernel(const __grid_cons
             if (zp[k]) zp[k][o] = static_cast<uint8_t>(quantize<kFast>(z, za[k]) - zsub[k]);
         }
       }
-      if (et == 0) SB_TRACE(a, 12);
     }
     // all roles meet before the tile's buffers and once-per-tile barriers are reused
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
   }
-  if (threadIdx.x == 0) SB_TRACE(a, 13);
   if (warp == 2) tmem_dealloc<512>(tmem);
 }
 

@@ -183,6 +183,33 @@ int slimt_b200_translate(slimt_b200_model* model, slimt_b200_translate_io* io);
  * The length bound is the smallest slimt_b200_model_max_length current over the replicas. */
 int slimt_b200_translate_multi(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_translate_io* io);
 
+/* ---- sampling: each step's word drawn from the model's distribution instead of chosen greedily ----
+ * For decode step s and row b, with y[n] the step's exact logits over the output columns (the shortlist's or the
+ * vocabulary's: the values of the logits tap):
+ *  - tempered logits z[n] = fl32(y[n] * inv_t), inv_t = (float)(1.0 / (double)temperature); at temperature 1, z = y.
+ *  - (x0, x1, x2, x3) = Philox4x32-10(counter = (s, key_lo, key_hi, 0), key = (seed_lo, seed_hi)) and
+ *    u = ((((uint64)x0 << 32) | x1) >> 11) * 2^-53 in [0, 1), with `key` the row's sampling key.
+ *  - the word is the first column c, in ascending order, whose cumulative probability sum_{j<=c} exp(z[j] - LSE(z))
+ *    exceeds u, summed in the order of the token scores (64-column strips, their groups, then the strip's columns); a
+ *    column whose term underflows to 0 is never chosen.
+ *  - the sampled word replaces the greedy choice: EOS handling, recorded tokens and alignments follow it unchanged.
+ *    token_scores / out_scores, when asked for, hold z[c] - LSE(z), the word's log-probability under the distribution
+ *    it was drawn from (at temperature 1 exactly the greedy call's score definition).
+ * Both arithmetic modes draw from the same exact logits.  A temperature that is not finite or lies outside [1e-3, 1e3],
+ * or sampling together with `forced`, is an error; the model stays usable. */
+typedef struct slimt_b200_sampling {
+  float temperature;     /* finite, in [1e-3, 1e3] */
+  uint64_t seed;
+  const uint64_t* keys;  /* one per row (forward; a DEVICE pointer with device_io) or per sentence (translate);
+                            NULL = the row's index in the batch (forward) or the sentence's index in the request
+                            (translate), so a translation never depends on which batch, lane or replica served it */
+} slimt_b200_sampling;
+/* slimt_b200_model_forward / slimt_b200_translate_multi with sampling; sampling = NULL is the greedy call. */
+int slimt_b200_model_forward_sampled(slimt_b200_model* model, slimt_b200_forward_io* io,
+                                     const slimt_b200_sampling* sampling);
+int slimt_b200_translate_sampled(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_translate_io* io,
+                                 const slimt_b200_sampling* sampling);
+
 /* Host-only pieces of the same path, callable without a GPU (used by the CPU test-suite):
  * ShortlistGenerator::generate (Shortlist.cc:115-175) and Batcher::generate (Batcher.cc:95-120). */
 int slimt_b200_shortlist_generate(const void* shortlist_bin, size_t shortlist_bytes, const uint32_t* words,

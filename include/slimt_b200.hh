@@ -525,6 +525,14 @@ inline size_t cache_key(size_t model_id, const Words &words) {
   for (size_t word : words) hash_combine<size_t>(seed, word);
   return seed;
 }
+// The sampling key of a segment: 64-bit FNV-1a over its words' little-endian bytes, so that a sampled translation depends
+// on the segment's words and not on where it sits in a request or a pooled batch.
+inline uint64_t sampling_key(const Words &words) {
+  uint64_t h = 0xcbf29ce484222325ull;
+  for (uint32_t word : words)
+    for (int b = 0; b < 4; b++) h = (h ^ ((word >> (8 * b)) & 0xffu)) * 0x100000001b3ull;
+  return h;
+}
 inline Ptr<TranslationCache> make_cache(size_t cache_size) {  // Frontend.cc:78-85
   constexpr size_t kCacheBucketSize = 16;
   return cache_size > 0 ? std::make_shared<TranslationCache>(cache_size, kCacheBucketSize) : nullptr;
@@ -713,12 +721,14 @@ class Blocking {
   }
 
   // cache prefill (Request.cc:58-78): a segment this model has translated before is not batched again.  A record
-  // stored by a request that did not ask for alignments (or scores) cannot answer one that does.  The rest: run().
+  // stored by a request that did not ask for alignments (or scores) cannot answer one that does.  A sampled segment is
+  // neither looked up nor stored: the cache holds greedy translations.  The rest: run().
   Histories serve(const Ptr<Model> &model, const Sentences &segments, const Options &options) {
     Histories histories(segments.size());
     std::vector<size_t> todo;
+    const bool cached = cache_ && !options.sample;
     for (size_t i = 0; i < segments.size(); i++) {
-      if (cache_) {
+      if (cached) {
         auto [found, history] = cache_->find(cache_key(model->id(), segments[i]));
         if (found && history && (!options.alignment || history->alignment.size() == history->target.size()) &&
             (!options.scores || history->scores.size() == history->target.size())) {
@@ -731,7 +741,7 @@ class Blocking {
     }
     if (!todo.empty()) run(model, segments, todo, options, histories);
     for (size_t i : todo)
-      if (cache_) cache_->store(cache_key(model->id(), segments[i]), histories[i]);  // Request.cc:120-125
+      if (cached) cache_->store(cache_key(model->id(), segments[i]), histories[i]);  // Request.cc:120-125
     return histories;
   }
 
@@ -769,8 +779,15 @@ class Blocking {
       scores.resize(out.size());
       io.out_scores = scores.data();
     }
+    std::vector<uint64_t> keys;
+    slimt_b200_sampling sampling{options.temperature, options.seed, nullptr};
+    if (options.sample) {
+      for (size_t i : todo) keys.push_back(sampling_key(segments[i]));
+      sampling.keys = keys.data();
+    }
     const std::vector<slimt_b200_model *> &replicas = model->replicas();
-    detail::check(slimt_b200_translate_multi(replicas.data(), replicas.size(), &io), "slimt_b200_translate_multi");
+    detail::check(slimt_b200_translate_sampled(replicas.data(), replicas.size(), &io, options.sample ? &sampling : nullptr),
+                  "slimt_b200_translate_sampled");
     for (size_t k = 0; k < todo.size(); k++) {
       auto h = std::make_shared<Hypothesis>();
       h->target.assign(out.begin() + out_offsets[k], out.begin() + out_offsets[k + 1]);
@@ -892,7 +909,8 @@ class Async {
   // depend on who shared the batch (the candidate set is the union over the batch, Model.cc:116-120).
   static bool poolable(const Job &a, const Job &b) {
     return !a.second && !b.second && a.first == b.first && a.is_text == b.is_text && a.options.alignment == b.options.alignment &&
-           a.options.html == b.options.html && a.options.scores == b.options.scores;
+           a.options.html == b.options.html && a.options.scores == b.options.scores && a.options.sample == b.options.sample &&
+           (!a.options.sample || (a.options.temperature == b.options.temperature && a.options.seed == b.options.seed));
   }
   void work() {
     Config one = config_;

@@ -1305,6 +1305,12 @@ struct Options {
   bool alignment = false;  // include alignments or not
   bool html = false;       // markup handling is not carried (see the header comment): must be false
   bool scores = false;     // include per-token log-probabilities or not (marian's --word-scores)
+  // Draw each word from the model's distribution at `temperature` instead of decoding greedily (marian's
+  // --output-sampling; slimt_b200_translate_sampled).  A segment's answer depends on (seed, temperature, segment) alone,
+  // not on the request or batch that carried it; sampled segments bypass the translation cache.
+  bool sample = false;
+  float temperature = 1.0f;  // finite, in [1e-3, 1e3]
+  uint64_t seed = 0;
 };
 
 struct Response {

@@ -26,7 +26,8 @@ EXPORTS = [
     "slimt_b200_model_dims", "slimt_b200_model_forward", "slimt_b200_translate", "slimt_b200_kernel_launches",
     "slimt_b200_shortlist_generate", "slimt_b200_batcher_plan", "slimt_b200_profile_enable", "slimt_b200_profile_read",
     "slimt_b200_translate_multi", "slimt_b200_shortlist_check", "slimt_b200_ctx_set_math", "slimt_b200_ctx_get_math",
-    "slimt_b200_model_set_max_length", "slimt_b200_model_max_length",
+    "slimt_b200_model_set_max_length", "slimt_b200_model_max_length", "slimt_b200_model_forward_sampled",
+    "slimt_b200_translate_sampled",
 ]
 
 
@@ -52,6 +53,10 @@ class TranslateIO(C.Structure):
                 ("target_tokens", C.c_uint64), ("batches", C.c_uint64),
                 ("device_ms", C.c_double), ("kernel_launches", C.c_uint64), ("h2d_bytes", C.c_uint64),
                 ("d2h_bytes", C.c_uint64), ("out_scores", C.c_void_p)]
+
+
+class Sampling(C.Structure):
+    _fields_ = [("temperature", C.c_float), ("seed", C.c_uint64), ("keys", C.c_void_p)]
 
 
 class KernelStat(C.Structure):
@@ -98,6 +103,9 @@ def lib() -> C.CDLL:
         L.slimt_b200_model_forward.argtypes = [C.c_void_p, C.POINTER(ForwardIO)]
         L.slimt_b200_translate.argtypes = [C.c_void_p, C.POINTER(TranslateIO)]
         L.slimt_b200_translate_multi.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.POINTER(TranslateIO)]
+        L.slimt_b200_model_forward_sampled.argtypes = [C.c_void_p, C.POINTER(ForwardIO), C.POINTER(Sampling)]
+        L.slimt_b200_translate_sampled.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.POINTER(TranslateIO),
+                                                   C.POINTER(Sampling)]
         L.slimt_b200_shortlist_check.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t]
         L.slimt_b200_shortlist_generate.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p,
                                                     C.c_size_t, C.POINTER(C.c_size_t)]
@@ -107,6 +115,18 @@ def lib() -> C.CDLL:
         L.slimt_b200_profile_read.argtypes = [C.c_void_p, C.POINTER(KernelStat), C.c_size_t, C.POINTER(C.c_size_t)]
         _lib = L
     return _lib
+
+
+def _sampling(sampling: Optional[dict], device_keys: bool = False):
+    """(Sampling, keys array to keep alive) for sampling = dict(temperature=1.0, seed=0, keys=None), or (None, None).
+    keys: one uint64 per row (forward) or per sentence (translate); a device pointer (int) when device_keys."""
+    if sampling is None:
+        return None, None
+    keys = sampling.get("keys")
+    if keys is not None and not device_keys:
+        keys = np.ascontiguousarray(keys, dtype=np.uint64)
+    ptr = (keys or None) if device_keys else _ptr(keys)
+    return Sampling(float(sampling.get("temperature", 1.0)), int(sampling.get("seed", 0)), ptr), keys
 
 
 def shortlist_generate(shortlist_bin: bytes, words: np.ndarray, vocab: int) -> np.ndarray:
@@ -267,9 +287,10 @@ class Model:
     def forward(self, tokens: np.ndarray, lengths: np.ndarray, limit_factor: float = 1.5,
                 shortlist: Optional[np.ndarray] = None, forced: Optional[np.ndarray] = None,
                 want_encoder: bool = False, want_logits: bool = False, want_alignment: bool = False,
-                want_scores: bool = False):
+                want_scores: bool = False, sampling: Optional[dict] = None):
         """Model::forward on host buffers. Returns dict(step_tokens [steps,B], steps, target_tokens, ...); "scores"
-        [steps,B] holds each step's log-probability of its chosen (or forced) word when want_scores."""
+        [steps,B] holds each step's log-probability of its chosen (or forced) word when want_scores.  sampling =
+        dict(temperature, seed, keys [B] or None) draws each word from the model's distribution (slimt_b200.h)."""
         tokens = np.ascontiguousarray(tokens, dtype=np.uint32)
         lengths = np.ascontiguousarray(lengths, dtype=np.uint32)
         B, T = tokens.shape
@@ -284,30 +305,41 @@ class Model:
         scores = np.zeros((max(1, max_steps), B), dtype=np.float32) if want_scores else None
         io = ForwardIO(_ptr(tokens), _ptr(lengths), B, T, limit_factor, _ptr(sl), 0 if sl is None else len(sl), _ptr(fo),
                        0, _ptr(steps), 0, 0, _ptr(enc), _ptr(logits), _ptr(align), _ptr(scores))
-        _check(lib().slimt_b200_model_forward(self.h, C.byref(io)), "slimt_b200_model_forward")
+        self._forward(io, sampling)
         n = int(io.steps)
         return {"step_tokens": steps[:n], "steps": n, "target_tokens": int(io.target_tokens), "encoder_out": enc,
                 "logits": None if logits is None else logits[:n], "alignment": None if align is None else align[:n],
                 "scores": None if scores is None else scores[:n]}
 
     def forward_resident(self, d_tokens: int, d_lengths: int, B: int, T: int, d_steps: int, limit_factor: float = 1.5,
-                         d_shortlist: int = 0, n_shortlist: int = 0, d_scores: int = 0, d_forced: int = 0):
+                         d_shortlist: int = 0, n_shortlist: int = 0, d_scores: int = 0, d_forced: int = 0,
+                         sampling: Optional[dict] = None):
         """Model::forward with inputs/outputs already in HBM (no host<->device copies of the batch); d_scores
-        (optional) receives the [max_steps][B] token scores on the device."""
+        (optional) receives the [max_steps][B] token scores on the device.  sampling: as forward's, with "keys" a
+        device pointer to [B] uint64 (or None)."""
         io = ForwardIO(d_tokens, d_lengths, B, T, limit_factor, d_shortlist or None, n_shortlist, d_forced or None, 1,
                        d_steps, 0, 0, None, None, None, d_scores or None)
-        _check(lib().slimt_b200_model_forward(self.h, C.byref(io)), "slimt_b200_model_forward")
+        self._forward(io, sampling, device_keys=True)
         return int(io.steps), int(io.target_tokens)
+
+    def _forward(self, io: ForwardIO, sampling: Optional[dict], device_keys: bool = False):
+        if sampling is None:
+            _check(lib().slimt_b200_model_forward(self.h, C.byref(io)), "slimt_b200_model_forward")
+        else:
+            sp, _keys = _sampling(sampling, device_keys)
+            _check(lib().slimt_b200_model_forward_sampled(self.h, C.byref(io), C.byref(sp)),
+                   "slimt_b200_model_forward_sampled")
 
     def translate_flat(self, tokens: np.ndarray, offsets: np.ndarray, max_words: int, limit_factor: float = 1.5,
                        shortlist_bin: Optional[bytes] = None, out_tokens: Optional[np.ndarray] = None,
                        out_offsets: Optional[np.ndarray] = None, replicas=None, want_alignments: bool = False,
                        shortlist_check: bool = False, shortlist_shared: bool = False, want_scores: bool = False,
-                       out_scores: Optional[np.ndarray] = None):
+                       out_scores: Optional[np.ndarray] = None, sampling: Optional[dict] = None):
         """slimt_b200_translate (or _translate_multi over `replicas`, a list of Models) on caller-owned host buffers:
         ragged sentences in (tokens, offsets), ragged targets out (out_tokens, out_offsets).  This is the C-ABI call a
         host integration makes; nothing is repacked.  want_scores: stats["scores"] is ragged like out_tokens (one
-        log-probability per target token, EOS included); out_scores, when given, is that buffer."""
+        log-probability per target token, EOS included); out_scores, when given, is that buffer.  sampling =
+        dict(temperature, seed, keys [n] or None): slimt_b200_translate_sampled, one key per sentence."""
         n = len(offsets) - 1
         lens = np.diff(offsets.astype(np.int64))
         max_len = int(lens.max()) if n else 0
@@ -331,7 +363,11 @@ class Model:
                          _ptr(out_tokens), len(out_tokens), _ptr(out_offsets),
                          _ptr(align), 0 if align is None else len(align), _ptr(align_offs), 0, 0, 0.0, 0, 0, 0,
                          _ptr(out_scores) if want_scores else None)
-        if replicas is None:
+        if sampling is not None:
+            sp, _keys = _sampling(sampling)
+            hs = (C.c_void_p * len(replicas or [self]))(*[r.h for r in (replicas or [self])])
+            _check(lib().slimt_b200_translate_sampled(hs, len(hs), C.byref(io), C.byref(sp)), "slimt_b200_translate_sampled")
+        elif replicas is None:
             _check(lib().slimt_b200_translate(self.h, C.byref(io)), "slimt_b200_translate")
         else:
             hs = (C.c_void_p * len(replicas))(*[r.h for r in replicas])
@@ -346,15 +382,16 @@ class Model:
         return out_tokens, out_offsets, stats
 
     def translate(self, sentences, max_words: int, limit_factor: float = 1.5, shortlist_bin: Optional[bytes] = None,
-                  replicas=None, want_alignments: bool = False, want_scores: bool = False, **kw):
+                  replicas=None, want_alignments: bool = False, want_scores: bool = False,
+                  sampling: Optional[dict] = None, **kw):
         """exhaust() over one request: Batcher + shortlist + forward per batch, host buffers in and out.  want_scores:
-        stats["scores"][i] holds one log-probability per target token of sentence i."""
+        stats["scores"][i] holds one log-probability per target token of sentence i.  sampling: translate_flat's."""
         offsets = np.zeros(len(sentences) + 1, dtype=np.uint64)
         offsets[1:] = np.cumsum([len(s) for s in sentences])
         tokens = np.concatenate([np.asarray(s, dtype=np.uint32) for s in sentences]) if sentences else np.zeros(0, np.uint32)
         out_tokens, out_offsets, stats = self.translate_flat(tokens, offsets, max_words, limit_factor, shortlist_bin,
                                                              replicas=replicas, want_alignments=want_alignments,
-                                                             want_scores=want_scores, **kw)
+                                                             want_scores=want_scores, sampling=sampling, **kw)
         outs = [out_tokens[int(out_offsets[i]):int(out_offsets[i + 1])].copy() for i in range(len(sentences))]
         if want_alignments:
             al, ao = stats.pop("alignments"), stats.pop("align_offsets")

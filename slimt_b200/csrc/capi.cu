@@ -172,6 +172,16 @@ int slimt_b200_model_max_length(const slimt_b200_model* model, int32_t* current,
 }
 
 int slimt_b200_model_forward(slimt_b200_model* model, slimt_b200_forward_io* io) {
+  return slimt_b200_model_forward_sampled(model, io, nullptr);
+}
+
+int slimt_b200_model_forward_sampled(slimt_b200_model* model, slimt_b200_forward_io* io,
+                                     const slimt_b200_sampling* sampling) {
+  if (sb::check_sampling(sampling)) return 1;
+  if (sampling && io->forced) {
+    sb::set_error("sampling: teacher forcing (forced) and sampling exclude each other");
+    return 1;
+  }
   sb::ForwardArgs a;
   a.tokens = io->tokens, a.lengths = io->lengths, a.B = io->batch, a.T = io->seq;
   a.limit_factor = io->limit_factor;
@@ -180,6 +190,7 @@ int slimt_b200_model_forward(slimt_b200_model* model, slimt_b200_forward_io* io)
   a.step_tokens = io->step_tokens;
   a.encoder_out = io->encoder_out, a.logits = io->logits, a.alignment = io->alignment;
   a.scores = io->token_scores;
+  if (sampling) a.sample = true, a.inv_t = sb::sampling_inv_t(sampling->temperature), a.seed = sampling->seed, a.keys = sampling->keys;
   int rc = sb::model_forward(model->m, a);
   io->steps = a.steps;
   io->target_tokens = a.target_tokens;
@@ -188,13 +199,19 @@ int slimt_b200_model_forward(slimt_b200_model* model, slimt_b200_forward_io* io)
 
 int slimt_b200_translate(slimt_b200_model* model, slimt_b200_translate_io* io) {
   sb::Model* m = &model->m;
-  return sb::translate_multi(&m, 1, io);
+  return sb::translate_multi(&m, 1, io, nullptr);
 }
 
 int slimt_b200_translate_multi(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_translate_io* io) {
+  return slimt_b200_translate_sampled(replicas, n_replicas, io, nullptr);
+}
+
+int slimt_b200_translate_sampled(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_translate_io* io,
+                                 const slimt_b200_sampling* sampling) {
+  if (sb::check_sampling(sampling)) return 1;
   std::vector<sb::Model*> ms(n_replicas);
-  for (size_t i = 0; i < n_replicas; i++) ms[i] = replicas[i] ? &replicas[i]->m : nullptr;
-  return sb::translate_multi(ms.data(), n_replicas, io);
+  for (size_t i = 0; i < n_replicas; i++) ms[i] = replicas && replicas[i] ? &replicas[i]->m : nullptr;
+  return sb::translate_multi(ms.data(), n_replicas, io, sampling);
 }
 
 uint64_t slimt_b200_kernel_launches(const slimt_b200_ctx* ctx) { return ctx->c.launches; }

@@ -673,7 +673,7 @@ const char* const kSelfAttnName[] = {"Fused", "Rowwise", "Tiled", "Long"};  // i
 
 enum class EncFfn { Rows, Gemm };
 // output: the fused argmax GEMM (out_argmax.cu, in the encoding Model::load chose), logits tap + argmax_rows, or the
-// scores GEMM (the fused GEMM with every logit evaluated exactly) + score_step
+// scores GEMM (the fused GEMM with every logit evaluated exactly) + score_step or sample_step
 enum class Out { Argmax, Logits, Scores };
 
 struct Routes {
@@ -722,8 +722,8 @@ Routes choose_routes(const Model& m, int T, int B, bool fast, bool logits, bool 
   // Wo + residual + LN, FFN1 + ReLU, FFN2 + residual + LN in one row-tile kernel, 128 rows per CTA
   r.ffn = E == 256 && m.F == 1536 ? EncFfn::Rows : EncFfn::Gemm;
 
-  // a caller that wants the logits gets them from the tap (and scores, when asked for, from them); scores alone come
-  // from the scores epilogue of the fused GEMM
+  // a caller that wants the logits gets them from the tap (and scores or samples, when asked for, from them); scores
+  // or samples alone come from the scores epilogue of the fused GEMM
   r.out = logits ? Out::Logits : scores ? Out::Scores : Out::Argmax;
   return r;
 }
@@ -742,6 +742,7 @@ struct Pass {
   Routes route;
   // batch inputs and outputs: workspace copies with host buffers, the caller's buffers with device_io
   uint32_t *d_tokens, *d_lengths, *d_steps, *d_forced, *d_sl, *d_rows, *tgt_len;
+  uint64_t* d_keys;  // [B] sampling keys (null: the row index)
   // encoder; Kc/Vc: the cross K/V projected once per decoder layer (Cross::Cached)
   float *x0, *x1, *Qb, *Kb, *Vb, *Kc[2], *Vc[2];
   int8_t *qa[4], *attn_q, *ffn_q;
@@ -798,7 +799,7 @@ int Pass::plan() {
     set_error("shortlist size must be a multiple of 8");
     return 1;
   }
-  route = choose_routes(m, T, B, c.fast, a.logits != nullptr, a.scores != nullptr);
+  route = choose_routes(m, T, B, c.fast, a.logits != nullptr, a.scores != nullptr || a.sample);
 
   const size_t RE = static_cast<size_t>(R) * E, BE = static_cast<size_t>(B) * E;
   const size_t SB = static_cast<size_t>(max_steps) * B, N = static_cast<size_t>(Nout);
@@ -828,10 +829,9 @@ int Pass::plan() {
     if (route.out == Out::Argmax) out.tables([&ws](auto*& p, size_t n) { ws.add(p, n); });
   }
   if (route.out == Out::Logits) ws.add(d_logits, static_cast<size_t>(B) * N);
-  if (a.scores) {
-    if (!a.device_io) ws.add(d_scores, SB);
-    ws.add(partials, (N + kScoreStrip - 1) / kScoreStrip * static_cast<size_t>(B));
-  }
+  if (a.scores && !a.device_io) ws.add(d_scores, SB);
+  if (a.scores || a.sample) ws.add(partials, (N + kScoreStrip - 1) / kScoreStrip * static_cast<size_t>(B));
+  if (a.sample && a.keys && !a.device_io) ws.add(d_keys, B);
   // head-0 probabilities of every step stay on the device and come back in one copy after the loop
   if (a.alignment) ws.add(d_align_all, SB * T);
   if (!a.device_io && a.sentence_tokens) ws.add(d_rows, SB);
@@ -840,6 +840,7 @@ int Pass::plan() {
     d_tokens = const_cast<uint32_t*>(a.tokens), d_lengths = const_cast<uint32_t*>(a.lengths), d_steps = a.step_tokens;
     d_forced = const_cast<uint32_t*>(a.forced), d_sl = use_sl ? const_cast<uint32_t*>(a.shortlist) : nullptr;
     d_scores = a.scores;
+    d_keys = const_cast<uint64_t*>(a.keys);
   }
 
   // cross-attention K/V operands: projected once (Cross::Cached), or the u8 encoder output the recompute kernels read
@@ -1022,6 +1023,10 @@ int Pass::prepare_output() {
     SB_CUDA(cudaMemcpyAsync(d_forced, a.forced, 4ul * max_steps * B, cudaMemcpyHostToDevice, s));
     c.h2d_bytes += 4ul * max_steps * B;
   }
+  if (d_keys && !a.device_io) {
+    SB_CUDA(cudaMemcpyAsync(d_keys, a.keys, 8ul * B, cudaMemcpyHostToDevice, s));
+    c.h2d_bytes += 8ul * B;
+  }
   if (lazy_sl) {
     // the encoder and the cross K/V projections are already queued: build the candidate set meanwhile
     const uint32_t* words = nullptr;
@@ -1161,14 +1166,14 @@ int Pass::decode_step(int step) {
     SB_CUDA(cudaMemcpyAsync(a.logits + static_cast<size_t>(step) * B * Nout, d_logits, 4ul * B * Nout,
                             cudaMemcpyDeviceToHost, s));
     c.d2h_bytes += 4ul * B * Nout;
-    if (a.scores) {
+    if (a.scores || a.sample) {
       LaunchScope ls(c, "score_rows", 0, 4.0 * B * Nout + 8.0 * B * ((Nout + kScoreStrip - 1) / kScoreStrip));
-      launch_score_rows(d_logits, B, Nout, partials, s);
+      launch_score_rows(d_logits, B, Nout, partials, a.sample ? a.inv_t : 1.0f, s);
     }
   } else if (route.out == Out::Scores) {
     const double Md = B, Nd = Nout, Kd = E, strips = (Nout + kScoreStrip - 1) / kScoreStrip;
     LaunchScope ls(c, "dec_gemm_out_scores", 2.0 * Md * Nd * Kd, Md * Kd + Nd * Kd + 8.0 * Nd + 8.0 * Md + 8.0 * Md * strips);
-    if (launch_out_scores(out, map_oq, B, E, best, partials, c.num_sms, s)) {
+    if (launch_out_scores(out, map_oq, B, E, best, partials, a.sample ? a.inv_t : 1.0f, c.num_sms, s)) {
       set_error("output GEMM (scores): unsupported K " + std::to_string(E));
       return 1;
     }
@@ -1180,17 +1185,27 @@ int Pass::decode_step(int step) {
       return 1;
     }
   }
-  if (a.scores) {
+  if (a.scores || a.sample) {
     ScoreStepArgs k{};
     k.partials = partials, k.best = best, k.forced = d_forced, k.shortlist = use_sl ? d_sl : nullptr;
     k.oq = oq, k.w = out.w, k.c127 = out.c127, k.pb = out.pb, k.um = out.um;
     k.logits = route.out == Out::Logits ? d_logits : nullptr;
     k.B = B, k.N = Nout, k.K = E, k.step = step, k.scores = d_scores;
+    k.inv_t = a.inv_t, k.seed = a.seed, k.keys = d_keys;
     const double strips = (Nout + kScoreStrip - 1) / kScoreStrip;
-    LaunchScope ls(c, "score_step", 0, 8.0 * B * strips + 16.0 * B + (a.forced ? 2.0 * B * E : 0.0));
-    if (launch_score_step(k, s)) {
-      set_error("token scores: step kernel launch failed");
-      return 1;
+    if (a.sample) {
+      // the chosen strip's 64 columns are re-evaluated: 64 weight rows and the row's operand (or 64 tap logits)
+      LaunchScope ls(c, "sample_step", 0, 8.0 * B * strips + 24.0 * B + (k.logits ? 256.0 : 65.0 * E) * B);
+      if (launch_sample_step(k, s)) {
+        set_error("sampling: step kernel launch failed");
+        return 1;
+      }
+    } else {
+      LaunchScope ls(c, "score_step", 0, 8.0 * B * strips + 16.0 * B + (a.forced ? 2.0 * B * E : 0.0));
+      if (launch_score_step(k, s)) {
+        set_error("token scores: step kernel launch failed");
+        return 1;
+      }
     }
   }
   return 0;

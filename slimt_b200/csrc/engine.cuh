@@ -191,6 +191,13 @@ struct ForwardArgs {
   // [max_steps][B] log-probability of each step's chosen (or forced) word over the step's output columns; a device
   // pointer with device_io (score_partial.cuh)
   float* scores = nullptr;
+  // Sampling (include/slimt_b200.h, DESIGN §4.4b): each step's word drawn from softmax(fl32(y * inv_t)) with the
+  // uniform number of (seed, keys[b], step) instead of the greedy choice.  keys: [B], a device pointer with device_io;
+  // null = the row index.  The caller has checked the temperature and that forced is null.
+  bool sample = false;
+  float inv_t = 1.0f;
+  uint64_t seed = 0;
+  const uint64_t* keys = nullptr;
 };
 
 int model_forward(Model& m, ForwardArgs& a);

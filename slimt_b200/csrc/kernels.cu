@@ -7,6 +7,7 @@
 #include "exact_math.cuh"
 #include "packed_best.cuh"
 #include "ptx.cuh"
+#include "sample_rng.cuh"
 #include "score_partial.cuh"
 
 namespace sb {
@@ -236,8 +237,11 @@ __global__ void argmax_rows_kernel(const float* __restrict__ logits, int cols, u
 
 // ------------------------------------------------------------------ token scores
 // Logits tap: the partial (m, s) of every 64-column strip of every row, with the same strip_partial as the fused
-// scores epilogue.  Thread = (strip, row), rows fastest, so the partial stores are coalesced.
-__global__ void score_rows_kernel(const float* __restrict__ logits, int B, int N, float2* __restrict__ partials) {
+// scores epilogue.  Thread = (strip, row), rows fastest, so the partial stores are coalesced.  kTemper: the partials of
+// the tempered logits fl32(y * inv_t) (sampling at a temperature other than 1).
+template <bool kTemper>
+__global__ void score_rows_kernel(const float* __restrict__ logits, int B, int N, float2* __restrict__ partials,
+                                  float inv_t) {
   const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   const int n_strips = (N + kScoreStrip - 1) / kScoreStrip;
   if (i >= static_cast<size_t>(n_strips) * B) return;
@@ -253,14 +257,54 @@ __global__ void score_rows_kernel(const float* __restrict__ logits, int B, int N
     y0[j] = a.x, y0[j + 1] = a.y, y0[j + 2] = a.z, y0[j + 3] = a.w;
     y1[j] = c.x, y1[j + 1] = c.y, y1[j + 2] = c.z, y1[j + 3] = c.w;
   }
+  if constexpr (kTemper) temper64(y0, y1, inv_t);
   partials[i] = strip_partial(y0, y1);
 }
 
-// Block = 32 rows (lane = row) x 32 warps (warp = a contiguous group of strips).  LSE = M + log S with M = max_t m_t and
-// S = sum_t s_t * exp(m_t - M) summed in ascending strip order: each warp its group in double, the 32 group sums then
-// in ascending group order.  The chosen column's logit: the packed best word's value (greedy), or for a forced word its
-// column (binary search in the sorted shortlist) evaluated exactly from the int8 operands -- or read from the tap.
+// The exact logit of output column col for row b from the signed int8 operands (the fused GEMM's value, bit for bit).
+__device__ __forceinline__ float exact_logit(const ScoreStepArgs& a, int b, int col) {
+  const int4* q = reinterpret_cast<const int4*>(a.oq + static_cast<size_t>(b) * a.K);
+  const int4* wr = reinterpret_cast<const int4*>(a.w + static_cast<size_t>(col) * a.K);
+  int acc = 0;
+  for (int k = 0; k < a.K / 16; k++) {
+    const int4 x = q[k], v = wr[k];
+    acc = __dp4a(x.x, v.x, acc), acc = __dp4a(x.y, v.y, acc), acc = __dp4a(x.z, v.z, acc), acc = __dp4a(x.w, v.w, acc);
+  }
+  return dequant1(acc + a.c127[col], a.um, a.pb[col]);
+}
+
+// Block = 32 rows (lane = row) x 32 warps (warp = a contiguous group of strips).  Both step kernels reduce a row's
+// partials in this one order: M = max_t m_t, then group sum sm[w][lane] = sum over warp w's strips t0 <= t < t1, in
+// ascending order and in double, of s_t * exp(m_t - M).  The caller sums the 32 groups in ascending order: S, and
+// LSE = M + log S.  Returns M.
 constexpr int kScoreWarps = 32;
+__device__ __forceinline__ float reduce_partials(const float2* __restrict__ partials, int B, int N, int b, int lane,
+                                                 int w, float (&mx)[kScoreWarps][32], double (&sm)[kScoreWarps][32]) {
+  const float ninf = -__int_as_float(0x7f800000);
+  const int n_strips = (N + kScoreStrip - 1) / kScoreStrip;
+  const int per = (n_strips + kScoreWarps - 1) / kScoreWarps;
+  const int t0 = min(n_strips, w * per), t1 = min(n_strips, t0 + per);
+  float m = ninf;
+  if (b < B)
+    for (int t = t0; t < t1; t++) m = fmaxf(m, partials[static_cast<size_t>(t) * B + b].x);
+  mx[w][lane] = m;
+  __syncthreads();
+  float M = ninf;
+#pragma unroll 8
+  for (int k = 0; k < kScoreWarps; k++) M = fmaxf(M, mx[k][lane]);
+  double s = 0.0;
+  if (b < B)
+    for (int t = t0; t < t1; t++) {
+      const float2 p = partials[static_cast<size_t>(t) * B + b];
+      s += static_cast<double>(p.y) * static_cast<double>(score_exp(__fsub_rn(p.x, M)));
+    }
+  sm[w][lane] = s;
+  __syncthreads();
+  return M;
+}
+
+// The chosen column's logit: the packed best word's value (greedy), or for a forced word its column (binary search in
+// the sorted shortlist) evaluated exactly from the int8 operands -- or read from the tap.
 __global__ void __launch_bounds__(32 * kScoreWarps) score_step_kernel(ScoreStepArgs a) {
   __shared__ float mx[kScoreWarps][32];
   __shared__ double sm[kScoreWarps][32];
@@ -270,25 +314,7 @@ __global__ void __launch_bounds__(32 * kScoreWarps) score_step_kernel(ScoreStepA
   pdl_launch_dependents();
   pdl_wait();
   const float ninf = -__int_as_float(0x7f800000);
-  const int n_strips = (a.N + kScoreStrip - 1) / kScoreStrip;
-  const int per = (n_strips + kScoreWarps - 1) / kScoreWarps;
-  const int t0 = min(n_strips, w * per), t1 = min(n_strips, t0 + per);
-  float m = ninf;
-  if (b < B)
-    for (int t = t0; t < t1; t++) m = fmaxf(m, a.partials[static_cast<size_t>(t) * B + b].x);
-  mx[w][lane] = m;
-  __syncthreads();
-  float M = ninf;
-#pragma unroll 8
-  for (int k = 0; k < kScoreWarps; k++) M = fmaxf(M, mx[k][lane]);
-  double s = 0.0;
-  if (b < B)
-    for (int t = t0; t < t1; t++) {
-      const float2 p = a.partials[static_cast<size_t>(t) * B + b];
-      s += static_cast<double>(p.y) * static_cast<double>(score_exp(__fsub_rn(p.x, M)));
-    }
-  sm[w][lane] = s;
-  __syncthreads();
+  const float M = reduce_partials(a.partials, B, a.N, b, lane, w, mx, sm);
   if (w != 0 || b >= B) return;
   double S = 0.0;
   for (int k = 0; k < kScoreWarps; k++) S += sm[k][lane];
@@ -315,17 +341,94 @@ __global__ void __launch_bounds__(32 * kScoreWarps) score_step_kernel(ScoreStepA
     } else if (a.logits) {
       y = a.logits[static_cast<size_t>(b) * a.N + col];
     } else {
-      const int4* q = reinterpret_cast<const int4*>(a.oq + static_cast<size_t>(b) * a.K);
-      const int4* wr = reinterpret_cast<const int4*>(a.w + static_cast<size_t>(col) * a.K);
-      int acc = 0;
-      for (int k = 0; k < a.K / 16; k++) {
-        const int4 x = q[k], v = wr[k];
-        acc = __dp4a(x.x, v.x, acc), acc = __dp4a(x.y, v.y, acc), acc = __dp4a(x.z, v.z, acc), acc = __dp4a(x.w, v.w, acc);
-      }
-      y = dequant1(acc + a.c127[col], a.um, a.pb[col]);
+      y = exact_logit(a, b, col);
     }
   }
   a.scores[static_cast<size_t>(a.step) * B + b] = static_cast<float>(static_cast<double>(y) - lse);
+}
+
+// Sampling (include/slimt_b200.h, DESIGN §4.4b), same block shape.  Over the tempered partials: warp 0 (lane = row)
+// draws u and walks the cumulative sums towards u * S -- the 32 group sums, then the chosen group's strip terms, each in
+// the order and with the very terms reduce_partials summed -- to a strip; a strip whose running sum passes the target is
+// chosen, a term of 0 never is, and when rounding exhausts a level the last nonzero entry of that level is taken.  Every
+// warp then evaluates two of the 64 tempered logits z of each row's chosen strip (exactly from the int8 operands, or
+// from the tap), and warp 0 walks them in ascending order, accumulating score_exp(z_j - m_t), to the column.
+__global__ void __launch_bounds__(32 * kScoreWarps) sample_step_kernel(ScoreStepArgs a) {
+  __shared__ float mx[kScoreWarps][32];
+  __shared__ double sm[kScoreWarps][32];
+  __shared__ float z[32][kScoreStrip + 1];
+  __shared__ int strip_of[32];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int b = blockIdx.x * 32 + lane;
+  const int B = a.B;
+  pdl_launch_dependents();
+  pdl_wait();
+  const float ninf = -__int_as_float(0x7f800000);
+  const float M = reduce_partials(a.partials, B, a.N, b, lane, w, mx, sm);
+  const int n_strips = (a.N + kScoreStrip - 1) / kScoreStrip;
+  const int per = (n_strips + kScoreWarps - 1) / kScoreWarps;
+  double S = 0.0, r = 0.0;  // r: the target left over inside the chosen strip, in units of its exp(m_t - M)
+  float m_t = 0.0f;
+  if (w == 0) {
+    int t = -1;
+    if (b < B) {
+      for (int k = 0; k < kScoreWarps; k++) S += sm[k][lane];
+      const uint64_t key = a.keys ? a.keys[b] : static_cast<uint64_t>(b);
+      const double target = sample_uniform(a.seed, key, static_cast<uint32_t>(a.step)) * S;
+      double acc = 0.0, before = 0.0;
+      int g = -1;
+      for (int k = 0; k < kScoreWarps; k++) {
+        const double v = sm[k][lane];
+        if (v == 0.0) continue;
+        g = k, before = acc;
+        acc += v;
+        if (acc > target) break;
+      }
+      const double tg = target - before;
+      acc = 0.0, before = 0.0;
+      const int t0 = g * per, t1 = min(n_strips, t0 + per);
+      for (int tt = t0; tt < t1; tt++) {
+        const float2 p = a.partials[static_cast<size_t>(tt) * B + b];
+        const float e = score_exp(__fsub_rn(p.x, M));
+        const double v = static_cast<double>(p.y) * static_cast<double>(e);
+        if (v == 0.0) continue;
+        t = tt, before = acc, m_t = p.x;
+        r = static_cast<double>(e);
+        acc += v;
+        if (acc > tg) break;
+      }
+      r = (tg - before) / r;
+    }
+    strip_of[lane] = t;
+  }
+  __syncthreads();
+  {  // thread (w, lane): columns 2w and 2w + 1 of row lane's strip
+    const int t = strip_of[lane];
+    for (int j = 2 * w; j < 2 * w + 2; j++) {
+      const int col = t * kScoreStrip + j;
+      float v = ninf;
+      if (t >= 0 && col < a.N)
+        v = __fmul_rn(a.logits ? a.logits[static_cast<size_t>(b) * a.N + col] : exact_logit(a, b, col), a.inv_t);
+      z[lane][j] = v;
+    }
+  }
+  __syncthreads();
+  if (w != 0 || b >= B) return;
+  const int t = strip_of[lane];
+  double acc = 0.0;
+  int c = -1;
+  for (int j = 0; j < kScoreStrip; j++) {
+    const float e = score_exp(__fsub_rn(z[lane][j], m_t));
+    if (e == 0.0f) continue;
+    c = j;
+    acc += static_cast<double>(e);
+    if (acc > r) break;
+  }
+  const float zc = z[lane][c];
+  a.best[b] = pack_best(zc, static_cast<uint32_t>(t * kScoreStrip + c));
+  if (a.scores)
+    a.scores[static_cast<size_t>(a.step) * B + b] =
+        static_cast<float>(static_cast<double>(zc) - (static_cast<double>(M) + log(S)));
 }
 
 }  // namespace
@@ -410,15 +513,22 @@ void launch_argmax_rows(const float* logits, int rows, int cols, unsigned long l
   argmax_rows_kernel<<<rows, 256, 0, stream>>>(logits, cols, best);
 }
 
-void launch_score_rows(const float* logits, int B, int N, float2* partials, cudaStream_t stream) {
+void launch_score_rows(const float* logits, int B, int N, float2* partials, float inv_t, cudaStream_t stream) {
   const size_t n = static_cast<size_t>((N + kScoreStrip - 1) / kScoreStrip) * B;
   if (n == 0) return;
-  score_rows_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, stream>>>(logits, B, N, partials);
+  const unsigned grid = static_cast<unsigned>((n + 255) / 256);
+  if (inv_t == 1.0f) score_rows_kernel<false><<<grid, 256, 0, stream>>>(logits, B, N, partials, inv_t);
+  else score_rows_kernel<true><<<grid, 256, 0, stream>>>(logits, B, N, partials, inv_t);
 }
 
 int launch_score_step(const ScoreStepArgs& a, cudaStream_t stream) {
   if (a.B == 0) return 0;
   return launch_pdl(score_step_kernel, dim3((a.B + 31) / 32), dim3(32 * kScoreWarps), 0, stream, a) != cudaSuccess ? 1 : 0;
+}
+
+int launch_sample_step(const ScoreStepArgs& a, cudaStream_t stream) {
+  if (a.B == 0) return 0;
+  return launch_pdl(sample_step_kernel, dim3((a.B + 31) / 32), dim3(32 * kScoreWarps), 0, stream, a) != cudaSuccess ? 1 : 0;
 }
 
 }  // namespace sb

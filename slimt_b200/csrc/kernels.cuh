@@ -109,14 +109,17 @@ void launch_gather_rows(const int8_t* W, const float* pb, const int32_t* c127, c
 
 // Row-wise first-max over f32 logits (used when logits are materialised for parity taps).
 void launch_argmax_rows(const float* logits, int rows, int cols, unsigned long long* best, cudaStream_t stream);
-// Token scores (score_partial.cuh).  launch_score_rows: the strip partials [ceil(N / 64)][B] of tap logits [B][N].
-void launch_score_rows(const float* logits, int B, int N, float2* partials, cudaStream_t stream);
+// Token scores (score_partial.cuh).  launch_score_rows: the strip partials [ceil(N / 64)][B] of tap logits [B][N], or
+// of the tempered logits fl32(y * inv_t) when inv_t != 1.
+void launch_score_rows(const float* logits, int B, int N, float2* partials, float inv_t, cudaStream_t stream);
 // One decode step's scores[step][b] = y[c] - LSE(row b) from the strip partials, c the greedy choice in best[b] or the
 // column of forced[step][b] (-inf when the shortlist does not hold that word).  A forced column's logit is read from
 // `logits` when given (tap route), otherwise evaluated exactly from the signed int8 operands oq [B][K] and w [N][K].
+// launch_sample_step instead draws column c from the softmax of the tempered partials (sample_rng.cuh, DESIGN §4.4b),
+// writes best[b] = pack_best(z[c], c) and, when scores is set, scores[step][b] = z[c] - LSE(z).
 struct ScoreStepArgs {
   const float2* partials;
-  const unsigned long long* best;
+  unsigned long long* best;
   const uint32_t* forced;     // [max_steps][B] or null
   const uint32_t* shortlist;  // [N] sorted, or null
   const int8_t* oq;           // [B][K] signed
@@ -126,9 +129,14 @@ struct ScoreStepArgs {
   const float* logits;        // [B][N] or null
   float um;
   int B, N, K, step;
-  float* scores;              // [max_steps][B]
+  float* scores;              // [max_steps][B] (sampling: or null)
+  // sampling only
+  float inv_t;                // 1 / temperature
+  uint64_t seed;
+  const uint64_t* keys;       // [B] or null: the row index
 };
 int launch_score_step(const ScoreStepArgs& a, cudaStream_t stream);
+int launch_sample_step(const ScoreStepArgs& a, cudaStream_t stream);
 // dst[c][r] = src[r][c] for r < rows, c < cols (dst rows are dst_stride apart): step-major token matrix -> sentence-major
 void launch_transpose_u32(const uint32_t* src, int rows, int cols, uint32_t* dst, int dst_stride, cudaStream_t stream);
 

@@ -237,14 +237,18 @@ __device__ __forceinline__ void bounds_exact(const uint32_t (&v0)[32], const uin
 // Scores (both arithmetic modes): every column's exact logit.  The strip's partial (m, s) (score_partial.cuh) goes to
 // partials[strip][M]; its first maximum is published like the bound filter's, so the choice is the reference's first
 // strict maximum.  seen only spares an atomic that cannot raise the word: it decides nothing that is summed.
+// kTemper: the same over the tempered logits fl32(y * inv_t) (sampling at a temperature other than 1).
+template <bool kTemper>
 __device__ __forceinline__ void scores_exact(const uint32_t (&v0)[32], const uint32_t (&v1)[32], unsigned long long seen,
                                              int row, int nb0, int M, int N, const float* __restrict__ pb,
                                              const int32_t* __restrict__ c127, float um,
-                                             unsigned long long* __restrict__ best, float2* __restrict__ partials) {
+                                             unsigned long long* __restrict__ best, float2* __restrict__ partials,
+                                             float inv_t) {
   if (nb0 >= N) return;  // the whole warp: a strip past the last column has no partial
   float y0[32], y1[32];
   exact_logits32(v0, nb0, N, pb, c127, um, y0);
   exact_logits32(v1, nb0 + 32, N, pb, c127, um, y1);
+  if constexpr (kTemper) temper64(y0, y1, inv_t);
   const float2 p = strip_partial(y0, y1);
   if (row >= M) return;
   int idx = 63;
@@ -257,16 +261,16 @@ __device__ __forceinline__ void scores_exact(const uint32_t (&v0)[32], const uin
 
 // ------------------------------------------------------------------ the kernel
 // kDigits: the encoding; kFast: tolerance mode (digits only); kScores: the scores epilogue (kDigits = false: the weights
-// alone, no column table).
+// alone, no column table); kTemper: the scores epilogue over the tempered logits (sampling).
 // tma_e / dshift / inv_um are read by the digits only, c127 by the bound filter and the scores, dmax / eta by the bound
-// filter only, partials by the scores only.
-template <bool kDigits, int KB, bool kFast, bool kScores = false>  // K = 128 * KB bytes per row
+// filter only, partials by the scores only, inv_t by kTemper only.
+template <bool kDigits, int KB, bool kFast, bool kScores = false, bool kTemper = false>  // K = 128 * KB bytes per row
 __global__ void __launch_bounds__(kThreads, 1)
     out_argmax_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
                       const __grid_constant__ CUtensorMap tma_e, const float* __restrict__ pb,
                       const int32_t* __restrict__ dshift, float um, float inv_um, int M, int N,
                       unsigned long long* __restrict__ best, const int32_t* __restrict__ c127,
-                      const float* __restrict__ dmax, float eta, float2* __restrict__ partials) {
+                      const float* __restrict__ dmax, float eta, float2* __restrict__ partials, float inv_t) {
   using L = Smem<kDigits, KB>;
   constexpr int kStages = L::kStages;
   constexpr int kABytes = kBM * kBK;
@@ -440,7 +444,7 @@ __global__ void __launch_bounds__(kThreads, 1)
       if (lane == 0) mbar_arrive(&tmem_empty[buf]);  // accumulators are in registers: release the buffer
 
       if constexpr (kScores) {
-        scores_exact(v0, v1, seen, row, nb0, M, N, pb, c127, um, best, partials);
+        scores_exact<kTemper>(v0, v1, seen, row, nb0, M, N, pb, c127, um, best, partials, inv_t);
       } else if constexpr (kDigits) {
         int g[8];
         const int mx = digit_groups(v0, v1, nb0, N, g);
@@ -536,7 +540,7 @@ int launch_out_argmax(const OutColumns& c, const CUtensorMap& tma_a, bool fast, 
   auto go = [&](auto kern, size_t smem) {
     if (ensure_dyn_smem(kern, smem) != cudaSuccess) return 1;
     return launch_pdl(kern, dim3(grid), dim3(kThreads), smem, stream, tma_a, c.map_w, c.map_ext, c.pb, c.dshift, c.um,
-                      inv_um, M, N, best, c.c127, c.dmax, c.eta, static_cast<float2*>(nullptr)) != cudaSuccess ? 1 : 0;
+                      inv_um, M, N, best, c.c127, c.dmax, c.eta, static_cast<float2*>(nullptr), 1.0f) != cudaSuccess ? 1 : 0;
   };
   if (!c.digits) {
     if (KB == 2) return go(out_argmax_kernel<false, 2, false>, Smem<false, 2>::total);
@@ -549,7 +553,7 @@ int launch_out_argmax(const OutColumns& c, const CUtensorMap& tma_a, bool fast, 
 }
 
 int launch_out_scores(const OutColumns& c, const CUtensorMap& tma_a, int M, int K, unsigned long long* best,
-                      float2* partials, int num_sms, cudaStream_t stream) {
+                      float2* partials, float inv_t, int num_sms, cudaStream_t stream) {
   const int KB = K / kBK, N = c.N;
   const long tiles = static_cast<long>((M + kBM - 1) / kBM) * ((N + kBN - 1) / kBN);
   const int grid = static_cast<int>(tiles < num_sms ? tiles : num_sms);
@@ -558,10 +562,16 @@ int launch_out_scores(const OutColumns& c, const CUtensorMap& tma_a, int M, int 
     if (ensure_dyn_smem(kern, smem) != cudaSuccess) return 1;
     return launch_pdl(kern, dim3(grid), dim3(kThreads), smem, stream, tma_a, c.map_w, c.map_w, c.pb,
                       static_cast<const int32_t*>(nullptr), c.um, 0.0f, M, N, best, c.c127,
-                      static_cast<const float*>(nullptr), 0.0f, partials) != cudaSuccess ? 1 : 0;
+                      static_cast<const float*>(nullptr), 0.0f, partials, inv_t) != cudaSuccess ? 1 : 0;
   };
-  if (KB == 2) return go(out_argmax_kernel<false, 2, false, true>, Smem<false, 2>::total);
-  if (KB == 4) return go(out_argmax_kernel<false, 4, false, true>, Smem<false, 4>::total);
+  // temperature 1: z = y bit for bit, so the untempered epilogue serves
+  const bool temper = inv_t != 1.0f;
+  if (KB == 2)
+    return temper ? go(out_argmax_kernel<false, 2, false, true, true>, Smem<false, 2>::total)
+                  : go(out_argmax_kernel<false, 2, false, true>, Smem<false, 2>::total);
+  if (KB == 4)
+    return temper ? go(out_argmax_kernel<false, 4, false, true, true>, Smem<false, 4>::total)
+                  : go(out_argmax_kernel<false, 4, false, true>, Smem<false, 4>::total);
   return 1;
 }
 

@@ -61,8 +61,9 @@ int launch_out_argmax(const OutColumns& c, const CUtensorMap& tma_a, bool fast, 
 // The same GEMM with the scores epilogue, in either encoding and arithmetic mode (it reads c.w, c.pb, c.c127 and
 // c.map_w, none of the encoding's tables): every logit is evaluated exactly, best[M] (pre-zeroed) receives each row's
 // first maximum of them, and partials[ceil(N / 64)][M] each 64-column strip's (max, sum of exp) in the order of
-// score_partial.cuh.  Returns nonzero for an unsupported K.
+// score_partial.cuh.  inv_t != 1: the partials (and the maximum) are of the tempered logits fl32(y * inv_t), for
+// sampling.  Returns nonzero for an unsupported K.
 int launch_out_scores(const OutColumns& c, const CUtensorMap& tma_a, int M, int K, unsigned long long* best,
-                      float2* partials, int num_sms, cudaStream_t stream);
+                      float2* partials, float inv_t, int num_sms, cudaStream_t stream);
 
 }  // namespace sb

@@ -50,4 +50,11 @@ __device__ __forceinline__ float2 strip_partial(const float (&y0)[32], const flo
   return make_float2(m, s);
 }
 
+// Sampling at a temperature other than 1 (DESIGN §4.4b): the strip's tempered logits z = fl32(y * inv_t), in place.
+// inv_t > 0, so -inf stays -inf.
+__device__ __forceinline__ void temper64(float (&y0)[32], float (&y1)[32], float inv_t) {
+#pragma unroll
+  for (int j = 0; j < 32; j++) y0[j] = __fmul_rn(y0[j], inv_t), y1[j] = __fmul_rn(y1[j], inv_t);
+}
+
 }  // namespace sb

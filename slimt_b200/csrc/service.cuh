@@ -45,7 +45,15 @@ struct Batcher {
 }  // namespace sb
 
 struct slimt_b200_translate_io;
+struct slimt_b200_sampling;
 namespace sb {
 // exhaust() over one request with the batches dealt to the replicas' lanes (translate.cu)
-int translate_multi(Model* const* models, size_t n_replicas, slimt_b200_translate_io* io);
+int translate_multi(Model* const* models, size_t n_replicas, slimt_b200_translate_io* io,
+                    const slimt_b200_sampling* sampling);
+
+// Sampling arguments of the C ABI: nonzero (and the error set) for a temperature that is not finite or lies outside
+// [1e-3, 1e3]; sampling = null (greedy) passes.
+int check_sampling(const slimt_b200_sampling* sampling);
+// inv_t = (float)(1.0 / (double)temperature)
+inline float sampling_inv_t(float temperature) { return static_cast<float>(1.0 / static_cast<double>(temperature)); }
 }  // namespace sb

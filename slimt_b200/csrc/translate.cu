@@ -71,7 +71,17 @@ Context* Model::lane(size_t i) {
   return lanes[i - 1].get();
 }
 
-int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io* io) {
+int check_sampling(const slimt_b200_sampling* sampling) {
+  if (sampling == nullptr) return 0;
+  const float t = sampling->temperature;
+  if (!(t >= 1e-3f && t <= 1e3f)) {  // also NaN
+    set_error("sampling: temperature must be finite and in [1e-3, 1e3], got " + std::to_string(t));
+    return 1;
+  }
+  return 0;
+}
+
+int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io* io, const slimt_b200_sampling* sampling) {
   if (n_rep == 0 || models == nullptr || models[0] == nullptr) {
     set_error("translate: no model replica given");
     return 1;
@@ -172,12 +182,13 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
       const size_t B = p.ids.size(), width = p.width;
       const size_t stride = static_cast<size_t>(forward_max_steps(io->limit_factor, width));
       // staging: [padded tokens][lengths] | [sentence-major step tokens][recorded lengths] | [alignment rows] |
-      // [step-major scores]
+      // [step-major scores] | [sampling keys]
       const size_t in_bytes = (4 * (B * width + B) + 255) & ~size_t(255);
       const size_t tok_bytes = (4 * (stride + 1) * B + 255) & ~size_t(255);
       const size_t al_bytes = want_align ? 4 * stride * B * width : 0;
       const size_t sc_bytes = want_scores ? 4 * stride * B : 0;
-      char* stage = c.staging_reserve(in_bytes + tok_bytes + al_bytes + sc_bytes + 256);
+      const size_t key_off = (in_bytes + tok_bytes + al_bytes + sc_bytes + 7) & ~size_t(7);
+      char* stage = c.staging_reserve(in_bytes + tok_bytes + al_bytes + sc_bytes + (sampling ? 8 * B + 8 : 0) + 256);
       if (!stage) {
         st.error = last_error();
         failed = true;
@@ -210,6 +221,12 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
       a.sentence_tokens = rows, a.row_stride = stride, a.target_lengths = lens;
       a.alignment = align;
       a.scores = scores;
+      if (sampling) {
+        // each sentence's own key (default: its index in the request), wherever the Batcher put it
+        uint64_t* keys = reinterpret_cast<uint64_t*>(stage + key_off);
+        for (size_t r = 0; r < B; r++) keys[r] = sampling->keys ? sampling->keys[p.ids[r]] : static_cast<uint64_t>(p.ids[r]);
+        a.sample = true, a.inv_t = sampling_inv_t(sampling->temperature), a.seed = sampling->seed, a.keys = keys;
+      }
       if (!timed) {
         cudaEventCreate(&e0), cudaEventCreate(&e1);
         cudaEventRecord(e0, c.stream);

@@ -210,6 +210,55 @@ int slimt_b200_model_forward_sampled(slimt_b200_model* model, slimt_b200_forward
 int slimt_b200_translate_sampled(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_translate_io* io,
                                  const slimt_b200_sampling* sampling);
 
+/* ---- scoring: the log-probability of each word of a GIVEN translation ----
+ * For sentence pair i (source tokens[offsets[i] .. offsets[i + 1]), EOS included, non-empty; target
+ * targets[target_offsets[i] .. target_offsets[i + 1]), any length including 0) and each target position j, the score of
+ * t_j is y[c] - log sum_n exp(y[n]), where
+ *  - y is the logits of the decoder fed the zero embedding at j = 0 and t_{j-1} after that -- the decode steps' own
+ *    inputs, the position-0 signal included at every step (Transformer.cc:133-160) -- so exactly the token_scores that
+ *    slimt_b200_model_forward returns at step j with forced = the target;
+ *  - c is t_j's column: over the vocabulary, or over the batch's shortlist when one is given (a word outside the
+ *    shortlist scores -inf).
+ * Every given token is scored: EOS is a word like any other, scoring neither stops at it nor requires it, and no
+ * limit_factor applies.  Scoring the out_tokens of slimt_b200_translate (EOS included) reproduces its out_scores, and
+ * out_alignments, bit for bit: the sentences form the same batches (the Batcher over the source lengths) and so the same
+ * shortlist unions.
+ * Arithmetic: scoring always runs the bit-exact arithmetic, whatever slimt_b200_ctx_set_math says; reproducible numbers
+ * are what reranking, filtering and quality estimation need.
+ * Errors, each reported before any GPU work (the model stays usable): offsets that decrease; a target word >= the
+ * vocabulary size; a source or target longer than the smallest slimt_b200_model_max_length current over the replicas;
+ * an output capacity too small.
+ * Device workspace: about 25 * E bytes per target position of a batch (the longest target times the batch's sentences),
+ * plus 4 * source width per position with alignments. */
+typedef struct slimt_b200_score_io {
+  const uint32_t* tokens;          /* sources, ragged like slimt_b200_translate_io */
+  const uint64_t* offsets;         /* [n_sentences + 1] */
+  size_t n_sentences;
+  const uint32_t* targets;         /* targets, ragged */
+  const uint64_t* target_offsets;  /* [n_sentences + 1] */
+  size_t max_words;                /* Config::max_words: batches are formed over the source lengths */
+  const void* shortlist_bin;       /* as in slimt_b200_translate_io */
+  size_t shortlist_bytes;
+  int32_t shortlist_check;
+  int32_t shortlist_shared;
+  /* outputs */
+  float* out_scores;               /* ragged by target_offsets (rebased to 0) */
+  size_t out_capacity;             /* floats; at least the total number of target tokens */
+  /* optional (NULL = not wanted): head 0 of the last decoder layer's cross-attention, [target_len_i][source_len_i]
+   * floats for sentence i at out_alignments[out_align_offsets[i] ..), as in slimt_b200_translate_io */
+  float* out_alignments;
+  size_t align_capacity;           /* floats */
+  uint64_t* out_align_offsets;     /* [n_sentences + 1] */
+  uint64_t batches;                /* out */
+  double device_ms;                /* out: CUDA-event time of the passes (the longest replica's) */
+  uint64_t kernel_launches;        /* out */
+  uint64_t h2d_bytes;              /* out */
+  uint64_t d2h_bytes;              /* out */
+} slimt_b200_score_io;
+
+/* Scores io's targets with one or more replicas of one model (as slimt_b200_translate_multi serves a request). */
+int slimt_b200_score(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_score_io* io);
+
 /* Host-only pieces of the same path, callable without a GPU (used by the CPU test-suite):
  * ShortlistGenerator::generate (Shortlist.cc:115-175) and Batcher::generate (Batcher.cc:95-120). */
 int slimt_b200_shortlist_generate(const void* shortlist_bin, size_t shortlist_bytes, const uint32_t* words,

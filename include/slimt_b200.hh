@@ -673,6 +673,53 @@ class Blocking {
     WordsResponse pivot_to_target = translate(second, source_to_pivot.target, options);
     return combine(std::move(source_to_pivot), std::move(pivot_to_target));
   }
+  // Scores given translations (slimt_b200_score): for sources[i] and targets[i], the log-probability of every word of
+  // targets[i] in scores[i], and with Options::alignment each word's distribution over sources[i].  The pairs are
+  // scored as given -- no wrapping, EOS like any other word -- and never through the translation cache, which holds
+  // translations, not scores.  Options::sample and Options::html do not apply and are refused.
+  WordsResponse score(const Ptr<Model> &model, const Sentences &sources, const Sentences &targets,
+                      const Options &options = Options()) {
+    if (options.sample) throw std::invalid_argument("Blocking::score: Options::sample does not apply to scoring");
+    if (options.html) throw std::invalid_argument("Blocking::score: Options::html does not apply to scoring");
+    if (sources.size() != targets.size()) throw std::invalid_argument("Blocking::score: one target per source");
+    std::vector<uint32_t> tokens, words;
+    std::vector<uint64_t> offsets(1, 0), target_offsets(1, 0), align_offsets(sources.size() + 1, 0);
+    size_t n_align = 0;
+    for (size_t i = 0; i < sources.size(); i++) {
+      tokens.insert(tokens.end(), sources[i].begin(), sources[i].end());
+      words.insert(words.end(), targets[i].begin(), targets[i].end());
+      offsets.push_back(tokens.size()), target_offsets.push_back(words.size());
+      n_align += sources[i].size() * targets[i].size();
+    }
+    std::vector<float> scores(std::max<size_t>(1, words.size())), align;
+    slimt_b200_score_io io;
+    std::memset(&io, 0, sizeof(io));
+    io.tokens = tokens.data(), io.offsets = offsets.data(), io.n_sentences = sources.size();
+    io.targets = words.data(), io.target_offsets = target_offsets.data(), io.max_words = config_.max_words;
+    const std::vector<char> &sl = model->shortlist_image();
+    io.shortlist_bin = sl.empty() ? nullptr : sl.data(), io.shortlist_bytes = sl.size();
+    io.out_scores = scores.data(), io.out_capacity = words.size();
+    if (options.alignment) {
+      align.resize(std::max<size_t>(1, n_align));
+      io.out_alignments = align.data(), io.align_capacity = n_align, io.out_align_offsets = align_offsets.data();
+    }
+    const std::vector<slimt_b200_model *> &replicas = model->replicas();
+    detail::check(slimt_b200_score(replicas.data(), replicas.size(), &io), "slimt_b200_score");
+    WordsResponse response;
+    response.source = sources, response.target = targets;
+    for (size_t i = 0; i <= sources.size(); i++) response.sentence_begin.push_back(i);
+    for (size_t i = 0; i < sources.size(); i++) {
+      response.scores.emplace_back(scores.begin() + target_offsets[i], scores.begin() + target_offsets[i + 1]);
+      if (options.alignment) {
+        const size_t S = sources[i].size();
+        const float *p = align.data() + align_offsets[i];
+        Alignment a;
+        for (size_t t = 0; t < targets[i].size(); t++) a.emplace_back(p + t * S, p + (t + 1) * S);
+        response.alignments.push_back(std::move(a));
+      }
+    }
+    return response;
+  }
   size_t cache_hits() const { return cache_hits_; }
 
  private:

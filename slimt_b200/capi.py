@@ -27,7 +27,7 @@ EXPORTS = [
     "slimt_b200_shortlist_generate", "slimt_b200_batcher_plan", "slimt_b200_profile_enable", "slimt_b200_profile_read",
     "slimt_b200_translate_multi", "slimt_b200_shortlist_check", "slimt_b200_ctx_set_math", "slimt_b200_ctx_get_math",
     "slimt_b200_model_set_max_length", "slimt_b200_model_max_length", "slimt_b200_model_forward_sampled",
-    "slimt_b200_translate_sampled",
+    "slimt_b200_translate_sampled", "slimt_b200_score",
 ]
 
 
@@ -53,6 +53,16 @@ class TranslateIO(C.Structure):
                 ("target_tokens", C.c_uint64), ("batches", C.c_uint64),
                 ("device_ms", C.c_double), ("kernel_launches", C.c_uint64), ("h2d_bytes", C.c_uint64),
                 ("d2h_bytes", C.c_uint64), ("out_scores", C.c_void_p)]
+
+
+class ScoreIO(C.Structure):
+    _fields_ = [("tokens", C.c_void_p), ("offsets", C.c_void_p), ("n_sentences", C.c_size_t),
+                ("targets", C.c_void_p), ("target_offsets", C.c_void_p), ("max_words", C.c_size_t),
+                ("shortlist_bin", C.c_void_p), ("shortlist_bytes", C.c_size_t), ("shortlist_check", C.c_int32),
+                ("shortlist_shared", C.c_int32), ("out_scores", C.c_void_p), ("out_capacity", C.c_size_t),
+                ("out_alignments", C.c_void_p), ("align_capacity", C.c_size_t), ("out_align_offsets", C.c_void_p),
+                ("batches", C.c_uint64), ("device_ms", C.c_double), ("kernel_launches", C.c_uint64),
+                ("h2d_bytes", C.c_uint64), ("d2h_bytes", C.c_uint64)]
 
 
 class Sampling(C.Structure):
@@ -106,6 +116,7 @@ def lib() -> C.CDLL:
         L.slimt_b200_model_forward_sampled.argtypes = [C.c_void_p, C.POINTER(ForwardIO), C.POINTER(Sampling)]
         L.slimt_b200_translate_sampled.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.POINTER(TranslateIO),
                                                    C.POINTER(Sampling)]
+        L.slimt_b200_score.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.POINTER(ScoreIO)]
         L.slimt_b200_shortlist_check.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t]
         L.slimt_b200_shortlist_generate.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p,
                                                     C.c_size_t, C.POINTER(C.c_size_t)]
@@ -157,6 +168,45 @@ def batcher_plan(lengths, max_words: int):
     _check(lib().slimt_b200_batcher_plan(_ptr(lengths), n, max_words, _ptr(ids), _ptr(offs), _ptr(widths), C.byref(nb)),
            "slimt_b200_batcher_plan")
     return [(ids[int(offs[i]):int(offs[i + 1])].astype(np.int64), int(widths[i])) for i in range(nb.value)]
+
+
+def score_flat(replicas, tokens: np.ndarray, offsets: np.ndarray, targets: np.ndarray, target_offsets: np.ndarray,
+               max_words: int, shortlist_bin: Optional[bytes] = None, want_alignments: bool = False,
+               shortlist_check: bool = False, shortlist_shared: bool = False,
+               out_capacity: Optional[int] = None, align_capacity: Optional[int] = None):
+    """slimt_b200_score over `replicas` (Models, or raw model handles) on host buffers: ragged sources and targets in,
+    one log-probability per target token out (ragged like the targets).  Returns (scores, stats); stats["alignments"] /
+    ["align_offsets"] when want_alignments.  The capacities default to exactly what the request needs."""
+    tokens = np.ascontiguousarray(tokens, dtype=np.uint32)
+    offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+    targets = np.ascontiguousarray(targets, dtype=np.uint32)
+    target_offsets = np.ascontiguousarray(target_offsets, dtype=np.uint64)
+    n = len(offsets) - 1
+    tl = np.diff(target_offsets.astype(np.int64)) if n > 0 else np.zeros(0, np.int64)
+    sl = np.diff(offsets.astype(np.int64)) if n > 0 else np.zeros(0, np.int64)
+    n_tgt = int(tl.sum()) if n > 0 else 0
+    cap = n_tgt if out_capacity is None else out_capacity
+    scores = np.zeros(max(1, cap), dtype=np.float32)
+    align = align_offs = None
+    if want_alignments:
+        acap = int((np.maximum(tl, 0) * np.maximum(sl, 0)).sum()) if align_capacity is None else align_capacity
+        align = np.zeros(max(1, acap), dtype=np.float32)
+        align_offs = np.zeros(n + 1, dtype=np.uint64)
+    slbuf = None
+    if shortlist_bin is not None:
+        slbuf = shortlist_bin if isinstance(shortlist_bin, C.Array) else (C.c_char * len(shortlist_bin)).from_buffer_copy(shortlist_bin)
+    io = ScoreIO(_ptr(tokens), _ptr(offsets), n, _ptr(targets), _ptr(target_offsets), max_words,
+                 C.cast(slbuf, C.c_void_p) if slbuf is not None else None, 0 if slbuf is None else len(slbuf),
+                 int(shortlist_check), int(shortlist_shared), _ptr(scores), cap,
+                 _ptr(align), 0 if align is None else (acap if align_capacity is None else align_capacity),
+                 _ptr(align_offs), 0, 0.0, 0, 0, 0)
+    hs = (C.c_void_p * max(1, len(replicas)))(*[getattr(r, "h", r) for r in replicas])
+    _check(lib().slimt_b200_score(hs, len(replicas), C.byref(io)), "slimt_b200_score")
+    stats = {"batches": int(io.batches), "device_ms": io.device_ms, "kernel_launches": int(io.kernel_launches),
+             "h2d_bytes": int(io.h2d_bytes), "d2h_bytes": int(io.d2h_bytes)}
+    if want_alignments:
+        stats["alignments"], stats["align_offsets"] = align, align_offs
+    return scores[:n_tgt], stats
 
 
 def _err() -> str:
@@ -380,6 +430,26 @@ class Model:
         if want_scores:
             stats["scores"] = out_scores
         return out_tokens, out_offsets, stats
+
+    def score(self, sources, targets, max_words: int, shortlist_bin: Optional[bytes] = None, replicas=None,
+              want_alignments: bool = False, **kw):
+        """slimt_b200_score of targets[i] given sources[i] (lists of word ids): returns (scores, stats) with scores[i]
+        one log-probability per token of targets[i]; stats["alignments"][i] is [len(targets[i])][len(sources[i])]."""
+        def ragged(seqs):
+            offs = np.zeros(len(seqs) + 1, dtype=np.uint64)
+            offs[1:] = np.cumsum([len(s) for s in seqs])
+            flat = np.concatenate([np.asarray(s, dtype=np.uint32) for s in seqs]) if len(seqs) else np.zeros(0, np.uint32)
+            return flat, offs
+        tok, off = ragged(sources)
+        tg, toff = ragged(targets)
+        sc, stats = score_flat(replicas or [self], tok, off, tg, toff, max_words, shortlist_bin,
+                               want_alignments=want_alignments, **kw)
+        outs = [sc[int(toff[i]):int(toff[i + 1])].copy() for i in range(len(targets))]
+        if want_alignments:
+            al, ao = stats.pop("alignments"), stats.pop("align_offsets")
+            stats["alignments"] = [al[int(ao[i]):int(ao[i + 1])].reshape(len(targets[i]), len(sources[i])).copy()
+                                   for i in range(len(targets))]
+        return outs, stats
 
     def translate(self, sentences, max_words: int, limit_factor: float = 1.5, shortlist_bin: Optional[bytes] = None,
                   replicas=None, want_alignments: bool = False, want_scores: bool = False,

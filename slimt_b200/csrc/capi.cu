@@ -214,6 +214,16 @@ int slimt_b200_translate_sampled(slimt_b200_model* const* replicas, size_t n_rep
   return sb::translate_multi(ms.data(), n_replicas, io, sampling);
 }
 
+int slimt_b200_score(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_score_io* io) {
+  if (io == nullptr) {
+    sb::set_error("score: io is NULL");
+    return 1;
+  }
+  std::vector<sb::Model*> ms(n_replicas);
+  for (size_t i = 0; i < n_replicas; i++) ms[i] = replicas && replicas[i] ? &replicas[i]->m : nullptr;
+  return sb::score_multi(ms.data(), n_replicas, io);
+}
+
 uint64_t slimt_b200_kernel_launches(const slimt_b200_ctx* ctx) { return ctx->c.launches; }
 
 int slimt_b200_shortlist_generate(const void* shortlist_bin, size_t shortlist_bytes, const uint32_t* words,

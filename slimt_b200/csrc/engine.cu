@@ -492,6 +492,9 @@ void Model::destroy() {
 // ------------------------------------------------------------------ workspace
 namespace {
 
+// Rows of the scoring pass's output layer per launch: bounds its strip partials to ceil(N / 64) * 16 k * 8 bytes.
+constexpr int kScoreChunk = 16384;
+
 // The device buffers of one call, each listed once: add() records where a buffer's pointer goes and how many elements
 // it holds; carve() reserves the sum in the context's arena and hands out the pointers in list order, each buffer
 // starting on a 256-byte boundary.
@@ -739,6 +742,9 @@ struct Pass {
   int B, T, R, E, F, H, dh, Le, Ld, max_steps, Nout;  // Nout: with a lazy shortlist the vocabulary until its callback
   double src_tokens;
   bool lazy_sl, use_sl;
+  // scoring pass (a.targets set): Tt target positions per sentence, M = B * Tt decoder rows, always bit-exact arithmetic
+  bool scoring, fast;
+  int Tt, M;
   Routes route;
   // batch inputs and outputs: workspace copies with host buffers, the caller's buffers with device_io
   uint32_t *d_tokens, *d_lengths, *d_steps, *d_forced, *d_sl, *d_rows, *tgt_len;
@@ -748,6 +754,10 @@ struct Pass {
   int8_t *qa[4], *attn_q, *ffn_q;
   // decoder state (Model.cc:111-185); counters: [0] n_done, [1] step counter, [2] ticket
   float *xd, *hb, *qd, *zb, *state[2], *d_logits, *d_align_all;  // zb: the first of two decoder layers' output
+  // scoring pass: the targets, the SSRU's two projections of all rows, h's u8 copy (Wq's operand)
+  uint32_t* d_tgt;
+  float *Fb, *Wx;
+  int8_t* hq;
   float* d_scores;    // [max_steps][B]
   float2* partials;   // [ceil(Nout / 64)][B] strip partials of the step's scores
   int8_t *xq[2], *zq[2], *caq, *oq;
@@ -759,7 +769,7 @@ struct Pass {
   CUtensorMap map_qa[3], map_qa32[3], mapK[2], mapV[2];
   CUtensorMap map_xq[2], map_zq[2], map_caq;  // u8 activation operands of the row-tile kernels, box {128 B, 32 rows}
   CUtensorMap map_oq;
-  int plan(), encode(), prepare_cross(), prepare_output(), decode_step(int step), decode();
+  int plan(), encode(), prepare_cross(), prepare_output(), decode_step(int step), decode(), score();
 };
 
 // Checks the request, chooses the routes and plans the workspace: each buffer is listed once, under the condition in
@@ -774,6 +784,13 @@ int Pass::plan() {
   }
   if (Ld < 1 || 2 * Ld > kMaxQuantOut) {
     set_error("decoder_layers must be 1 or 2");
+    return 1;
+  }
+  scoring = a.targets != nullptr;
+  fast = c.fast && !scoring;
+  Tt = static_cast<int>(a.target_T), M = B * Tt;
+  if (scoring && Tt > m.max_len()) {
+    set_error("target length " + std::to_string(Tt) + " exceeds the supported maximum of " + std::to_string(m.max_len()));
     return 1;
   }
   // Model.cc:160: size_t max_seq_length = limit_factor * source_sequence_length (float product, truncated).  The first
@@ -799,7 +816,12 @@ int Pass::plan() {
     set_error("shortlist size must be a multiple of 8");
     return 1;
   }
-  route = choose_routes(m, T, B, c.fast, a.logits != nullptr, a.scores != nullptr || a.sample);
+  route = choose_routes(m, T, B, fast, a.logits != nullptr, a.scores != nullptr || a.sample);
+  if (scoring) {
+    // T_target queries read each layer's cross K/V: projected once (Cached); every logit evaluated exactly (Scores)
+    route.cross = Cross::Cached;
+    route.out = Out::Scores;
+  }
 
   const size_t RE = static_cast<size_t>(R) * E, BE = static_cast<size_t>(B) * E;
   const size_t SB = static_cast<size_t>(max_steps) * B, N = static_cast<size_t>(Nout);
@@ -814,13 +836,23 @@ int Pass::plan() {
   ws.add(attn_q, RE);
   if (route.ffn == EncFfn::Gemm) ws.add(ffn_q, static_cast<size_t>(R) * F);
   for (int l = 0; l < Ld && route.cross == Cross::Cached; l++) ws.add(Kc[l], RE), ws.add(Vc[l], RE);
-  ws.add(xd, BE), ws.add(hb, BE), ws.add(qd, BE), ws.add(zb, BE);
-  for (int l = 0; l < Ld; l++) ws.add(state[l], BE);
-  ws.add(xq[0], BE), ws.add(xq[1], BE), ws.add(zq[0], BE), ws.add(zq[1], BE), ws.add(caq, BE), ws.add(oq, BE);
-  ws.add(best, B), ws.add(done, B), ws.add(tgt_len, B), ws.add(counters, 64);
-  if (!a.device_io) {
-    ws.add(d_steps, SB);
-    if (a.forced) ws.add(d_forced, SB);
+  if (scoring) {
+    // one row per (sentence, target position); the layer input xd is rewritten in place by each layer's FFN
+    const size_t ME = static_cast<size_t>(M) * E, rows = std::min(M, kScoreChunk);
+    ws.add(d_tgt, M);
+    ws.add(xd, ME), ws.add(Fb, ME), ws.add(Wx, ME), ws.add(hb, ME), ws.add(qd, ME);
+    ws.add(xq[0], ME), ws.add(xq[1], ME), ws.add(hq, ME), ws.add(caq, ME), ws.add(oq, ME);
+    ws.add(d_scores, M), ws.add(best, rows), ws.add(partials, (N + kScoreStrip - 1) / kScoreStrip * rows);
+    if (a.alignment) ws.add(d_align_all, ME / E * T);
+  } else {
+    ws.add(xd, BE), ws.add(hb, BE), ws.add(qd, BE), ws.add(zb, BE);
+    for (int l = 0; l < Ld; l++) ws.add(state[l], BE);
+    ws.add(xq[0], BE), ws.add(xq[1], BE), ws.add(zq[0], BE), ws.add(zq[1], BE), ws.add(caq, BE), ws.add(oq, BE);
+    ws.add(best, B), ws.add(done, B), ws.add(tgt_len, B), ws.add(counters, 64);
+    if (!a.device_io) {
+      ws.add(d_steps, SB);
+      if (a.forced) ws.add(d_forced, SB);
+    }
   }
   if (use_sl) {
     if (!a.device_io) ws.add(d_sl, N);
@@ -829,12 +861,14 @@ int Pass::plan() {
     if (route.out == Out::Argmax) out.tables([&ws](auto*& p, size_t n) { ws.add(p, n); });
   }
   if (route.out == Out::Logits) ws.add(d_logits, static_cast<size_t>(B) * N);
-  if (a.scores && !a.device_io) ws.add(d_scores, SB);
-  if (a.scores || a.sample) ws.add(partials, (N + kScoreStrip - 1) / kScoreStrip * static_cast<size_t>(B));
-  if (a.sample && a.keys && !a.device_io) ws.add(d_keys, B);
-  // head-0 probabilities of every step stay on the device and come back in one copy after the loop
-  if (a.alignment) ws.add(d_align_all, SB * T);
-  if (!a.device_io && a.sentence_tokens) ws.add(d_rows, SB);
+  if (!scoring) {
+    if (a.scores && !a.device_io) ws.add(d_scores, SB);
+    if (a.scores || a.sample) ws.add(partials, (N + kScoreStrip - 1) / kScoreStrip * static_cast<size_t>(B));
+    if (a.sample && a.keys && !a.device_io) ws.add(d_keys, B);
+    // head-0 probabilities of every step stay on the device and come back in one copy after the loop
+    if (a.alignment) ws.add(d_align_all, SB * T);
+    if (!a.device_io && a.sentence_tokens) ws.add(d_rows, SB);
+  }
   if (ws.carve(c)) return 1;
   if (a.device_io) {
     d_tokens = const_cast<uint32_t*>(a.tokens), d_lengths = const_cast<uint32_t*>(a.lengths), d_steps = a.step_tokens;
@@ -854,6 +888,7 @@ int Pass::plan() {
   if (route.self == SelfAttn::Fused)
     for (int i = 0; i < 3; i++)
       if (c.make_map(&map_qa[i], qa[i], R, E, 128) || c.make_map(&map_qa32[i], qa[i], R, E, 32)) return 1;
+  if (scoring) return c.make_map(&map_caq, caq, M, E, kRowTile);  // the output operand's maps are made per row chunk
   for (int i = 0; i < 2; i++)
     if (c.make_map(&map_xq[i], xq[i], B, E, kRowTile) || c.make_map(&map_zq[i], zq[i], B, E, kRowTile)) return 1;
   if (c.make_map(&map_caq, caq, B, E, kRowTile) || c.make_map(&map_oq, oq, B, E, kBM)) return 1;
@@ -952,7 +987,7 @@ int Pass::encode() {
       LaunchScope ls(c, "enc_wo_ffn_fused", 2.0 * Rd * (Ed * Ed + 2.0 * Ed * Fd),
                      Ed * Ed + 2.0 * Ed * Fd + Rd * Ed * (1.0 + 4.0 + 4.0 + k.n_zq));  // u8 in, residual, f32 out, u8 copies
       // (the y rows this variant parks in global memory and reads back are overhead, not algorithmic bytes)
-      if (launch_rows_ffn(k, E, F, 128, c.fast, s)) {
+      if (launch_rows_ffn(k, E, F, 128, fast, s)) {
         set_error("fused encoder FFN kernel launch failed");
         return 1;
       }
@@ -1087,7 +1122,7 @@ int Pass::decode_step(int step) {
       k.h_out = hb, k.q_out = qd, k.M = B;
       const double Bd = B, Ed = E;
       LaunchScope ls(c, "dec_ssru_q_fused", 2.0 * Bd * 3.0 * Ed * Ed, 3.0 * Ed * Ed + Bd * Ed * (2.0 + 4.0 * 5.0));
-      if (launch_dec_ssru(k, E, c.fast, s)) {
+      if (launch_dec_ssru(k, E, fast, s)) {
         set_error("fused SSRU kernel: unsupported embedding size " + std::to_string(E));
         return 1;
       }
@@ -1107,7 +1142,7 @@ int Pass::decode_step(int step) {
       const bool rcl = route.cross == Cross::Rcl;
       LaunchScope ls(c, "dec_cross_attention_rc", 2.0 * (rcl ? src_tokens : Bd * (T > 32 ? 64.0 : 32.0)) * Ed * 2.0 * Ed,
                      2.0 * src_tokens * Ed + 2.0 * Ed * Ed + 5.0 * Bd * Ed);  // valid keys only
-      if (rcl ? launch_cross_attention_rcl(k, c.num_sms, s) : launch_cross_attention_rc(k, c.num_sms, c.fast, s)) {
+      if (rcl ? launch_cross_attention_rcl(k, c.num_sms, s) : launch_cross_attention_rc(k, c.num_sms, fast, s)) {
         set_error("recompute cross-attention launch failed");
         return 1;
       }
@@ -1146,7 +1181,7 @@ int Pass::decode_step(int step) {
       const double Bd = B, Ed = E, Fd = F;
       LaunchScope ls(c, "dec_wo_ffn_fused", 2.0 * Bd * (Ed * Ed + 2.0 * Ed * Fd),
                      Ed * Ed + 2.0 * Ed * Fd + Bd * Ed * (1.0 + 4.0 + (last ? 1.0 : 6.0)));
-      if (launch_rows_ffn(k, E, F, kRowTile, c.fast, s)) {
+      if (launch_rows_ffn(k, E, F, kRowTile, fast, s)) {
         set_error("fused FFN kernel: unsupported sizes E=" + std::to_string(E) + " F=" + std::to_string(F));
         return 1;
       }
@@ -1180,7 +1215,7 @@ int Pass::decode_step(int step) {
   } else {
     const double Md = B, Nd = Nout, Kd = E;
     LaunchScope ls(c, "dec_gemm_out_argmax", 2.0 * Md * Nd * Kd, Md * Kd + Nd * Kd + 4.0 * Nd + 8.0 * Md);
-    if (launch_out_argmax(out, map_oq, c.fast, B, E, best, c.num_sms, s)) {
+    if (launch_out_argmax(out, map_oq, fast, B, E, best, c.num_sms, s)) {
       set_error("output GEMM: unsupported K " + std::to_string(E));
       return 1;
     }
@@ -1313,6 +1348,136 @@ int Pass::decode() {
   return 0;
 }
 
+// The scoring pass (DESIGN §4.4c): every decoder input is known, so each layer runs over all M = B * Tt rows at once --
+// one GEMM for the SSRU's two projections, the scan that is left sequential, one GEMM for Wq, the multi-query
+// cross-attention, the Wo/FFN row-tile kernel of the step path -- and the output layer scores the rows in chunks.
+// Row (b, j) sees exactly the operands decode step j sees under teacher forcing, so its score is the same bits.
+int Pass::score() {
+  SB_CUDA(cudaMemcpyAsync(d_tgt, a.targets, 4ul * M, cudaMemcpyHostToDevice, s));
+  c.h2d_bytes += 4ul * M;
+  const double Md = M, Ed = E, Fd = F;
+  {  // decoder inputs: zero embedding at j = 0, then the previous target word, each + the position-0 signal (quirk Q1)
+    QuantOuts q = qouts();
+    qadd(q, xq[0], m.dec[0].rnn_wf.aq), qadd(q, xq[1], m.dec[0].rnn_w.aq);
+    LaunchScope ls(c, "score_embed", 0, Md * 4.0 + Md * Ed * (1.0 + 4.0 + 4.0 + 2.0));
+    launch_embed(d_tgt, m.emb_q, m.inv_qm, m.sqrt_e, m.pos, M, Tt, E, 0, 0, xd, q, s, 1);
+  }
+  for (int l = 0; l < Ld; l++) {
+    const DecLayerW& L = m.dec[l];
+    const bool last = (l + 1 == Ld);
+    {  // Wf x + bf and W x of every row (Modules.cc:190-235)
+      GemmCall g(&c, "score_gemm_ssru_f32", M, E, E, EPI_F32, 2);
+      GemmProblem* pf = g.add(xq[0], L.rnn_wf);
+      GemmProblem* pw = g.add(xq[1], L.rnn_w);
+      if (!pf || !pw) return 1;
+      pf->out = Fb, pw->out = Wx;
+      pf->ldo = pw->ldo = E;
+      if (g.launch()) return 1;
+    }
+    {
+      DecSsruScanArgs k{};
+      k.f = Fb, k.wx = Wx, k.x = xd;
+      k.ln_scale = L.rnn_ln.scale, k.ln_bias = L.rnn_ln.bias, k.eps = 1e-6f;
+      k.aq_q = L.ctx.q.aq, k.h_out = hb, k.hq = reinterpret_cast<uint8_t*>(hq);
+      k.B = B, k.T = Tt;
+      LaunchScope ls(c, "score_ssru_scan", 0, Md * Ed * (3.0 * 4.0 + 4.0 + 1.0));
+      if (launch_dec_ssru_scan(k, E, s)) {
+        set_error("SSRU scan kernel: unsupported embedding size " + std::to_string(E));
+        return 1;
+      }
+    }
+    {
+      GemmCall g(&c, "score_gemm_q_f32", M, E, E, EPI_F32);
+      GemmProblem* p = g.add(hq, L.ctx.q);
+      if (!p) return 1;
+      p->out = qd, p->ldo = E;
+      if (g.launch()) return 1;
+    }
+    {  // Tt queries per sentence against its cached K/V; head 0 of the last layer is the alignment
+      QuantOuts q = qouts();
+      qadd(q, caq, L.ctx.o.aq);
+      float* al = last ? d_align_all : nullptr;
+      const bool tiled = self_attention_tiled_supported(T, dh);
+      LaunchScope ls(c, "score_cross_attention", 4.0 * Md * (src_tokens / B) * Ed,
+                     Md * Ed * 5.0 + 2.0 * src_tokens * Ed * 4.0 + (al ? 4.0 * Md * T : 0.0));
+      const int rc = tiled ? launch_self_attention_tiled(qd, Kc[l], Vc[l], d_lengths, B, T, H, dh, q, s, Tt, al)
+                           : launch_self_attention_long(qd, Kc[l], Vc[l], d_lengths, B, T, H, dh, q, s, Tt, al);
+      if (rc) {
+        set_error("scoring cross-attention: no kernel for head size " + std::to_string(dh) + " over " +
+                  std::to_string(T) + " source tokens");
+        return 1;
+      }
+    }
+    {  // Wo + residual + LN, FFN: the step path's row-tile kernel over M rows
+      RowsFfnArgs k{};
+      k.map_a = map_caq;
+      k.map_wo = L.ctx.o.map128, k.map_w1 = L.ffn.w1.map128, k.map_w2 = L.ffn.w2.map128;
+      k.pb_o = L.ctx.o.pb, k.pb_1 = L.ffn.w1.pb, k.pb_2 = L.ffn.w2.pb;
+      k.um_o = L.ctx.o.um, k.um_1 = L.ffn.w1.um, k.um_2 = L.ffn.w2.um;
+      k.aq_1 = L.ffn.w1.aq, k.aq_2 = L.ffn.w2.aq;
+      k.res = hb;
+      k.ln1_scale = L.ctx.ln.scale, k.ln1_bias = L.ctx.ln.bias;
+      k.ln2_scale = L.ffn.ln.scale, k.ln2_bias = L.ffn.ln.bias, k.eps = 1e-6f;
+      if (last) {
+        k.z_out = nullptr;
+        k.zq[0] = reinterpret_cast<uint8_t*>(oq), k.zaq[0] = m.out.aq, k.n_zq = 1;
+        k.zq_signed = 1;
+      } else {
+        k.z_out = xd;
+        k.zq[0] = reinterpret_cast<uint8_t*>(xq[0]), k.zaq[0] = m.dec[l + 1].rnn_wf.aq;
+        k.zq[1] = reinterpret_cast<uint8_t*>(xq[1]), k.zaq[1] = m.dec[l + 1].rnn_w.aq;
+        k.n_zq = 2;
+      }
+      k.M = M;
+      LaunchScope ls(c, "score_wo_ffn_fused", 2.0 * Md * (Ed * Ed + 2.0 * Ed * Fd),
+                     Ed * Ed + 2.0 * Ed * Fd + Md * Ed * (1.0 + 4.0 + (last ? 1.0 : 6.0)));
+      if (launch_rows_ffn(k, E, F, kRowTile, false, s)) {
+        set_error("fused FFN kernel: unsupported sizes E=" + std::to_string(E) + " F=" + std::to_string(F));
+        return 1;
+      }
+    }
+  }
+  // output layer in row chunks, so that the strip partials [ceil(N / 64)][rows] stay bounded; each chunk is one "step"
+  // of score_step with the targets as the forced words
+  const double strips = (Nout + kScoreStrip - 1) / kScoreStrip;
+  for (int r0 = 0; r0 < M; r0 += kScoreChunk) {
+    const int rows = std::min(kScoreChunk, M - r0);
+    CUtensorMap map;
+    if (c.make_map(&map, oq + static_cast<size_t>(r0) * E, rows, E, kBM)) return 1;
+    SB_CUDA(cudaMemsetAsync(best, 0, 8ul * rows, s));
+    {
+      const double Rd = rows, Nd = Nout;
+      LaunchScope ls(c, "score_gemm_out_scores", 2.0 * Rd * Nd * Ed, Rd * Ed + Nd * Ed + 8.0 * Nd + 8.0 * Rd + 8.0 * Rd * strips);
+      if (launch_out_scores(out, map, rows, E, best, partials, 1.0f, c.num_sms, s)) {
+        set_error("output GEMM (scores): unsupported K " + std::to_string(E));
+        return 1;
+      }
+    }
+    ScoreStepArgs k{};
+    k.partials = partials, k.best = best, k.forced = d_tgt + r0, k.shortlist = use_sl ? d_sl : nullptr;
+    k.oq = oq + static_cast<size_t>(r0) * E, k.w = out.w, k.c127 = out.c127, k.pb = out.pb, k.um = out.um;
+    k.B = rows, k.N = Nout, k.K = E, k.step = 0, k.scores = d_scores + r0, k.inv_t = 1.0f;
+    LaunchScope ls(c, "score_step", 0, 8.0 * rows * strips + 16.0 * rows + 2.0 * rows * E);
+    if (launch_score_step(k, s)) {
+      set_error("token scores: step kernel launch failed");
+      return 1;
+    }
+  }
+  SB_CUDA(cudaMemcpyAsync(a.scores, d_scores, 4ul * M, cudaMemcpyDeviceToHost, s));
+  c.d2h_bytes += 4ul * M;
+  if (d_align_all) {
+    SB_CUDA(cudaMemcpyAsync(a.alignment, d_align_all, 4ul * M * T, cudaMemcpyDeviceToHost, s));
+    c.d2h_bytes += 4ul * M * T;
+  }
+  SB_CUDA(cudaStreamSynchronize(s));
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) {
+    set_error(std::string("scoring pass failed: ") + cudaGetErrorString(e));
+    return 1;
+  }
+  return 0;
+}
+
 }  // namespace
 
 int model_forward(Model& m, ForwardArgs& a) { return model_forward_on(m, *m.ctx, a); }
@@ -1329,6 +1494,22 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
   if (a.B == 0 || a.T == 0) return 0;
   Pass p{m, c, a, c.stream};
   return p.plan() || p.encode() || p.prepare_cross() || p.prepare_output() || p.decode() ? 1 : 0;
+}
+
+int model_score_on(Model& m, Context& c, ForwardArgs& a) {
+  std::lock_guard<std::recursive_mutex> ctx_lock(c.mu);
+  if (c.device != m.ctx->device) {
+    set_error("model_score: the lane context and the model live on different devices");
+    return 1;
+  }
+  if (a.targets == nullptr || a.scores == nullptr || a.forced || a.sample || a.logits || a.device_io) {
+    set_error("model_score: targets and scores on host buffers, and none of forced, sampling, logits or device_io");
+    return 1;
+  }
+  SB_CUDA(cudaSetDevice(c.device));
+  if (a.B == 0 || a.T == 0 || a.target_T == 0) return 0;
+  Pass p{m, c, a, c.stream};
+  return p.plan() || p.encode() || p.prepare_cross() || p.prepare_output() || p.score() ? 1 : 0;
 }
 
 }  // namespace sb

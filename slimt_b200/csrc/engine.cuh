@@ -198,12 +198,19 @@ struct ForwardArgs {
   float inv_t = 1.0f;
   uint64_t seed = 0;
   const uint64_t* keys = nullptr;
+  // Scoring pass (model_score_on, DESIGN §4.4c): the given targets [B][target_T] (host, padded), scored at every
+  // position into scores [B][target_T]; alignment, when set, receives [B][target_T][T].
+  const uint32_t* targets = nullptr;
+  size_t target_T = 0;
 };
 
 int model_forward(Model& m, ForwardArgs& a);
 // The same pass with stream, workspace and staging taken from `lane` instead of the model's own context: weights are
 // read-only, so several lanes on the model's device can run batches of one model concurrently (translate.cu).
 int model_forward_on(Model& m, Context& lane, ForwardArgs& a);
+// Teacher-forced scoring of a.targets in one time-parallel pass (bit-exact arithmetic whatever lane.fast says): the
+// scores and alignments model_forward would give with forced = the targets, at every target position.
+int model_score_on(Model& m, Context& lane, ForwardArgs& a);
 
 // Decoder steps Model::decode may run for a batch of width T: the first step is unconditional (Model.cc:145-157), the
 // loop that follows runs while i < size_t(limit_factor * T) (Model.cc:160-161).

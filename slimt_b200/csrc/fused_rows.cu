@@ -282,6 +282,51 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
   if (warp == 2) tmem_dealloc<512>(tmem);
 }
 
+// =====================================================================================================
+// SSRU scan of the scoring pass (DecSsruScanArgs)
+// =====================================================================================================
+// One CTA per sentence, thread = feature: the thread carries its feature's cell state c through the positions in order.
+// A tile of kScanRows positions is scanned into shared memory first, so that the LayerNorm statistics -- a sequential
+// E-long chain per row -- run one row per thread of the first warp instead of one chain per position.  Padded positions
+// (beyond the target's length) are computed and discarded by the caller; the scan is causal, so they affect no valid row.
+constexpr int kScanRows = 32;
+
+template <int E>
+__global__ void __launch_bounds__(E) dec_ssru_scan_kernel(const DecSsruScanArgs a) {
+  constexpr int XS = E + 1;
+  extern __shared__ float scan_sm[];
+  float* xs = scan_sm;                       // [kScanRows][E + 1]
+  float* stats = xs + kScanRows * XS;        // mean [kScanRows], sigma [kScanRows]
+  __shared__ uint64_t exp_tab[32];
+  const int f = threadIdx.x;
+  if (f < 32) exp_tab[f] = kExp2fTab[f];
+  __syncthreads();
+  const int T = a.T;
+  const size_t row0 = static_cast<size_t>(blockIdx.x) * T;
+  const float g = a.ln_scale[f], bias = a.ln_bias[f];
+  float c = 0.0f;  // Decoder::start_states
+  for (int j0 = 0; j0 < T; j0 += kScanRows) {
+    const int nr = min(kScanRows, T - j0);
+#pragma unroll 4
+    for (int r = 0; r < nr; r++) {
+      const size_t o = (row0 + j0 + r) * E + f;
+      const float sg = sigmoid_ref_tab(a.f[o], exp_tab);
+      c = __fadd_rn(__fmul_rn(sg, c), __fmul_rn(__fsub_rn(1.0f, sg), a.wx[o]));
+      xs[r * XS + f] = __fadd_rn(a.x[o], c > 0.0f ? c : 0.0f);
+    }
+    __syncthreads();
+    if (f < nr) ln_stats_row<E>(xs + f * XS, &stats[f], &stats[kScanRows + f], a.eps);
+    __syncthreads();
+    for (int r = 0; r < nr; r++) {
+      const size_t o = (row0 + j0 + r) * E + f;
+      const float y = ln_apply(xs[r * XS + f], stats[r], stats[kScanRows + r], g, bias);
+      a.h_out[o] = y;
+      a.hq[o] = static_cast<uint8_t>(quantize1(y, a.aq_q));
+    }
+    __syncthreads();
+  }
+}
+
 template <class Kern, class Args>
 int launch_rows(Kern kern, const Args& a, size_t smem, cudaStream_t stream) {
   const int tiles = (a.M + kR - 1) / kR;
@@ -308,6 +353,19 @@ int launch_ssru_e(const DecSsruArgs& a, bool fast, cudaStream_t stream) {
 int launch_dec_ssru(const DecSsruArgs& a, int E, bool fast, cudaStream_t stream) {
   if (E == 256) return launch_ssru_e<256>(a, fast, stream);
   if (E == 512) return launch_ssru_e<512>(a, fast, stream);
+  return 1;
+}
+
+int launch_dec_ssru_scan(const DecSsruScanArgs& a, int E, cudaStream_t stream) {
+  if (a.B == 0 || a.T == 0) return 0;
+  const size_t smem = (static_cast<size_t>(kScanRows) * (E + 1) + 2 * kScanRows) * sizeof(float);
+  auto go = [&](auto kern) {
+    if (ensure_dyn_smem(kern, smem) != cudaSuccess) return 1;
+    kern<<<a.B, E, smem, stream>>>(a);
+    return cudaGetLastError() != cudaSuccess ? 1 : 0;
+  };
+  if (E == 256) return go(dec_ssru_scan_kernel<256>);
+  if (E == 512) return go(dec_ssru_scan_kernel<512>);
   return 1;
 }
 

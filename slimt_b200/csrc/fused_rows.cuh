@@ -80,9 +80,27 @@ struct DecSsruArgs {
   float aq_xf, aq_xw;                  // a_quant of Wf / W (quantise x)
 };
 
+// The SSRU cell of the scoring pass, where every decoder input of a sentence is known before the first position: the
+// projections Wf x + bf and W x of all B * T rows come from one GEMM, and this kernel runs what remains sequential --
+// c_j = sg_j * c_{j-1} + (1 - sg_j) * (W x)_j from c_{-1} = 0 -- then h = LN(x + relu(c)) and h's u8 copy for Wq.  Rows
+// are b * T + j; the arithmetic is dec_ssru_kernel's bit-exact branch, so each row equals the step path's row at step j.
+struct DecSsruScanArgs {
+  const float* f;                      // f32 [B * T][E]: Wf x + bf
+  const float* wx;                     // f32 [B * T][E]: W x
+  const float* x;                      // f32 [B * T][E]: the layer's input
+  const float* ln_scale;
+  const float* ln_bias;
+  float eps;
+  float aq_q;                          // a_quant of Wq (quantises h)
+  float* h_out;                        // f32 [B * T][E]
+  uint8_t* hq;                         // u8 [B * T][E]
+  int B, T;
+};
+
 // E = 256, F = 1536 (tiny) and E = 512, F = 2048 (base) are built.  Returns nonzero when unsupported.
 // rows_per_tile: 32 (decoder step) or 128 (encoder; E = 256 only).
 int launch_rows_ffn(const RowsFfnArgs& a, int E, int F, int rows_per_tile, bool fast, cudaStream_t stream);
 int launch_dec_ssru(const DecSsruArgs& a, int E, bool fast, cudaStream_t stream);
+int launch_dec_ssru_scan(const DecSsruScanArgs& a, int E, cudaStream_t stream);
 
 }  // namespace sb

@@ -25,15 +25,15 @@ __device__ __forceinline__ void store_quant4(const QuantOuts& q, size_t off, con
 // ------------------------------------------------------------------ embedding
 __global__ void embed_kernel(const uint32_t* __restrict__ tokens, const int8_t* __restrict__ emb_q, float inv_qm,
                              float sqrt_e, const float* __restrict__ pos, int rows, int T, int E, int pos_from_row,
-                             int zero_embed, float* __restrict__ x, QuantOuts q) {
+                             int zero_embed, int shift, float* __restrict__ x, QuantOuts q) {
   const int per_row = E >> 2;
   const size_t gid = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (gid >= static_cast<size_t>(rows) * per_row) return;
   const int r = static_cast<int>(gid / per_row);
   const int e = static_cast<int>(gid % per_row) * 4;
   float w[4] = {0.0f, 0.0f, 0.0f, 0.0f};
-  if (!zero_embed) {
-    const uint32_t tok = tokens[r];
+  if (!zero_embed && !(shift && r % T == 0)) {
+    const uint32_t tok = tokens[shift ? r - 1 : r];
     const char4 c = *reinterpret_cast<const char4*>(emb_q + static_cast<size_t>(tok) * E + e);
     w[0] = __fmul_rn(static_cast<float>(c.x), inv_qm);
     w[1] = __fmul_rn(static_cast<float>(c.y), inv_qm);
@@ -434,11 +434,11 @@ __global__ void __launch_bounds__(32 * kScoreWarps) sample_step_kernel(ScoreStep
 }  // namespace
 
 void launch_embed(const uint32_t* tokens, const int8_t* emb_q, float inv_qm, float sqrt_e, const float* pos, int rows,
-                  int T, int E, int pos_from_row, int zero_embed, float* x, QuantOuts q, cudaStream_t stream) {
+                  int T, int E, int pos_from_row, int zero_embed, float* x, QuantOuts q, cudaStream_t stream, int shift) {
   const size_t n = static_cast<size_t>(rows) * (E / 4);
   if (n == 0) return;
   embed_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, stream>>>(tokens, emb_q, inv_qm, sqrt_e, pos, rows, T, E,
-                                                                         pos_from_row, zero_embed, x, q);
+                                                                         pos_from_row, zero_embed, shift, x, q);
 }
 
 void launch_quantize(const float* x, size_t n, QuantOuts q, cudaStream_t stream) {

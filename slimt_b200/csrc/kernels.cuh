@@ -18,9 +18,11 @@ struct QuantOuts {
 
 // x[r] = float(emb_q[tok[r]]) * inv_qm * sqrt_e + pos[(r % T) or 0]   (index_select + transform_embedding,
 // slimt/TensorOps.cc:227-243, Transformer.cc:24-49, Io.cc:275-283).  zero_embed=1 is decoder step 0.
+// shift=1 is the teacher-forced decoder input of the scoring pass: row r = b * T + j takes the zero embedding at j = 0
+// and tokens[r - 1] after that, the inputs the decode steps 0 .. T - 1 would see.
 void launch_embed(const uint32_t* tokens, const int8_t* emb_q, float inv_qm, float sqrt_e, const float* pos,
                   int rows, int T, int E, int pos_from_row, int zero_embed, float* x, QuantOuts q,
-                  cudaStream_t stream);
+                  cudaStream_t stream, int shift = 0);
 
 // f32 -> int8 copies (PrepareA as a standalone op, for the qmm:: operator API).
 void launch_quantize(const float* x, size_t n, QuantOuts q, cudaStream_t stream);
@@ -35,14 +37,20 @@ int launch_self_attention(const float* Q, const float* K, const float* V, const 
 // one place, choose_routes in engine.cu.
 // Returns nonzero when the shape does not fit: head sizes 32 and 64, T up to 556 (head size 32) or 400 (64), which
 // self_attention_tiled_supported tells without launching.
+// Tq > 0 makes it the decoder cross-attention of the scoring pass: Q is [B][Tq][E], every row a query, against the T
+// keys of K, V [B][T][E] masked by lengths; attn_head0 (optional) then receives head 0's probabilities [B][Tq][T].  The
+// bound is on T alone.
 int launch_self_attention_tiled(const float* Q, const float* K, const float* V, const uint32_t* lengths, int B, int T,
-                                int H, int dh, QuantOuts q, cudaStream_t stream);
+                                int H, int dh, QuantOuts q, cudaStream_t stream, int Tq = 0,
+                                float* attn_head0 = nullptr);
 bool self_attention_tiled_supported(int T, int dh);
 
 // The same operation for sentences the tiled kernel cannot hold (self_attention_long.cu): 32 query rows per block, K
-// and V streamed in 128-key tiles, the same chains and so the same bits.  Head sizes 32 and 64, T up to 1024.
+// and V streamed in 128-key tiles, the same chains and so the same bits.  Head sizes 32 and 64, T up to 1024.  Tq and
+// attn_head0 as for the tiled kernel.
 int launch_self_attention_long(const float* Q, const float* K, const float* V, const uint32_t* lengths, int B, int T,
-                               int H, int dh, QuantOuts q, cudaStream_t stream);
+                               int H, int dh, QuantOuts q, cudaStream_t stream, int Tq = 0,
+                               float* attn_head0 = nullptr);
 bool self_attention_long_supported(int T, int dh);
 
 // Decoder cross-attention for one query row per sentence over cached K,V [B][S][E] (cross_attention.cu).

@@ -14,6 +14,8 @@
 //            the V tiles.
 // Masked keys (>= the sentence's length) are skipped; padded query rows produce quantize(0).
 // Bound: the score block is [32][round_up(T, 128) + 4] floats, which fits the 220 KB budget up to T = 1024.
+// With Tq > 0 the kernel is the scoring pass's decoder cross-attention, like the tiled kernel's (self_attention_tiled.cu):
+// Tq live query rows per sentence against its T encoder keys; the bound is on the keys only.
 #include <stdio.h>
 
 #include "exact_math.cuh"
@@ -38,7 +40,8 @@ size_t long_smem_bytes(int T, int dh) {
 template <int DH>
 __global__ void __launch_bounds__(kLThreads, 1) self_attention_long_kernel(
     const float* __restrict__ Q, const float* __restrict__ K, const float* __restrict__ V,
-    const uint32_t* __restrict__ lengths, int T, int H, int n_qb, float dk, QuantOuts qo) {
+    const uint32_t* __restrict__ lengths, int T, int Tq, int cross, int H, int n_qb, float dk, QuantOuts qo,
+    float* __restrict__ attn_head0) {
   extern __shared__ __align__(16) float sm[];
   __shared__ uint64_t exp_tab[32];
   const int tid = threadIdx.x;
@@ -57,7 +60,8 @@ __global__ void __launch_bounds__(kLThreads, 1) self_attention_long_kernel(
   if (tid < 32) exp_tab[tid] = kExp2fTab[tid];
 
   const size_t base = static_cast<size_t>(b) * T * E + static_cast<size_t>(h) * DH;
-  const int rows_here = max(0, min(kLQB, len - i0));
+  const size_t base_q = static_cast<size_t>(b) * Tq * E + static_cast<size_t>(h) * DH;
+  const int rows_here = max(0, min(kLQB, (cross ? Tq : len) - i0));
   // V tile staging: keys jb .. jb + 127 below len, row-major [key][DH]
   auto stage_v = [&](int jb, int t0, int nt) {
     const int nk = min(kLKT, len - jb);
@@ -81,7 +85,7 @@ __global__ void __launch_bounds__(kLThreads, 1) self_attention_long_kernel(
     for (int i = tid; i < kLQB * (DH / 4); i += kLThreads) {
       const int r = i / (DH / 4), c = (i % (DH / 4)) * 4;
       float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (r < rows_here) v = *reinterpret_cast<const float4*>(Q + base + static_cast<size_t>(i0 + r) * E + c);
+      if (r < rows_here) v = *reinterpret_cast<const float4*>(Q + base_q + static_cast<size_t>(i0 + r) * E + c);
       Qt[(c + 0) * kLSQ + r] = v.x, Qt[(c + 1) * kLSQ + r] = v.y, Qt[(c + 2) * kLSQ + r] = v.z, Qt[(c + 3) * kLSQ + r] = v.w;
     }
 
@@ -165,6 +169,13 @@ __global__ void __launch_bounds__(kLThreads, 1) self_attention_long_kernel(
       }
     }
     __syncthreads();
+    if (attn_head0 != nullptr && h == 0) {  // alignment: head 0's probabilities over all T key slots, masked ones 0
+      const int r = tid >> 3, part = tid & 7;
+      if (r < rows_here) {
+        float* dst = attn_head0 + (static_cast<size_t>(b) * Tq + i0 + r) * T;
+        for (int j = part; j < T; j += 8) dst[j] = j < len ? S[r * SK + j] : 0.0f;
+      }
+    }
 
     // ---- P V, one 128-key V tile at a time (tile 0 is already staged)
     for (int jb = 0; jb < len; jb += kLKT) {
@@ -209,11 +220,11 @@ __global__ void __launch_bounds__(kLThreads, 1) self_attention_long_kernel(
 
   // ---- outputs: padded query rows carry zeros
   const int i = i0 + pr;
-  if (i >= T) return;
+  if (i >= Tq) return;
   const bool live = pr < rows_here;
 #pragma unroll
   for (int g = 0; g < NG; g++) {
-    const size_t off = base + static_cast<size_t>(i) * E + 32 * g + 4 * dg;
+    const size_t off = base_q + static_cast<size_t>(i) * E + 32 * g + 4 * dg;
     float y[4];
 #pragma unroll
     for (int k = 0; k < 4; k++) y[k] = live ? acc[g][k] : 0.0f;
@@ -231,21 +242,23 @@ bool self_attention_long_supported(int T, int dh) {
 }
 
 int launch_self_attention_long(const float* Q, const float* K, const float* V, const uint32_t* lengths, int B, int T, int H,
-                               int dh, QuantOuts q, cudaStream_t stream) {
+                               int dh, QuantOuts q, cudaStream_t stream, int Tq, float* attn_head0) {
   if (B == 0) return 0;
   if (!self_attention_long_supported(T, dh)) return 1;
   // 1/sqrt(dim_head) evaluated in double then narrowed, as `1.0F / std::sqrt(size_t)` does (Modules.cc:43)
   const float dk = static_cast<float>(1.0 / std::sqrt(static_cast<double>(dh)));
-  const int n_qb = (T + kLQB - 1) / kLQB;
+  const int cross = Tq > 0 ? 1 : 0;
+  if (!cross) Tq = T;
+  const int n_qb = (Tq + kLQB - 1) / kLQB;
   const size_t smem = long_smem_bytes(T, dh);
   const long blocks = static_cast<long>(B) * H * n_qb;
   if (blocks > 0x7fffffffL) return 1;
   if (dh == 32) {
     if (ensure_dyn_smem(self_attention_long_kernel<32>, smem) != cudaSuccess) return 1;
-    self_attention_long_kernel<32><<<static_cast<unsigned>(blocks), kLThreads, smem, stream>>>(Q, K, V, lengths, T, H, n_qb, dk, q);
+    self_attention_long_kernel<32><<<static_cast<unsigned>(blocks), kLThreads, smem, stream>>>(Q, K, V, lengths, T, Tq, cross, H, n_qb, dk, q, attn_head0);
   } else {
     if (ensure_dyn_smem(self_attention_long_kernel<64>, smem) != cudaSuccess) return 1;
-    self_attention_long_kernel<64><<<static_cast<unsigned>(blocks), kLThreads, smem, stream>>>(Q, K, V, lengths, T, H, n_qb, dk, q);
+    self_attention_long_kernel<64><<<static_cast<unsigned>(blocks), kLThreads, smem, stream>>>(Q, K, V, lengths, T, Tq, cross, H, n_qb, dk, q, attn_head0);
   }
   return 0;
 }

@@ -18,6 +18,9 @@
 //   P V      thread = 2 queries x 4 dims (x 8 for head size 64), one fma chain per output over the keys in order.
 // Masked keys (>= the sentence's length) contribute exactly +0 in the reference (exp(-99999999 + s) underflows to 0), so
 // they are skipped; padded query rows produce quantize(0) like the row-wise kernel.
+// The same chain serves the scoring pass's decoder cross-attention (Tq > 0): Q then holds Tq query rows per sentence,
+// every one of them live, against the sentence's T encoder keys; the chain per query row is the one the step path's
+// cross_attention_kernel runs for its single row, so the results are the same bits.
 #include <stdio.h>
 
 #include "exact_math.cuh"
@@ -34,7 +37,8 @@ constexpr int kTThreads = 256;
 template <int DH>
 __global__ void __launch_bounds__(kTThreads) self_attention_tiled_kernel(
     const float* __restrict__ Q, const float* __restrict__ K, const float* __restrict__ V,
-    const uint32_t* __restrict__ lengths, int T, int H, int n_qb, float dk, QuantOuts qo) {
+    const uint32_t* __restrict__ lengths, int T, int Tq, int cross, int H, int n_qb, float dk, QuantOuts qo,
+    float* __restrict__ attn_head0) {
   extern __shared__ __align__(16) float sm[];
   __shared__ uint64_t exp_tab[32];
   const int tid = threadIdx.x, lane = tid & 31;
@@ -56,14 +60,15 @@ __global__ void __launch_bounds__(kTThreads) self_attention_tiled_kernel(
   if (tid < 32) exp_tab[tid] = kExp2fTab[tid];
 
   const size_t base = static_cast<size_t>(b) * T * E + static_cast<size_t>(h) * DH;
-  const int rows_here = max(0, min(kQB, len - i0));  // valid query rows of this block
+  const size_t base_q = static_cast<size_t>(b) * Tq * E + static_cast<size_t>(h) * DH;
+  const int rows_here = max(0, min(kQB, (cross ? Tq : len) - i0));  // valid query rows of this block
 
   if (rows_here > 0) {
     // ---- stage Q (this block's rows) and K (the sentence's valid keys), transposed; zero beyond the valid range
     for (int i = tid; i < kQB * (DH / 4); i += kTThreads) {
       const int r = i / (DH / 4), c = (i % (DH / 4)) * 4;
       float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (r < rows_here) v = *reinterpret_cast<const float4*>(Q + base + static_cast<size_t>(i0 + r) * E + c);
+      if (r < rows_here) v = *reinterpret_cast<const float4*>(Q + base_q + static_cast<size_t>(i0 + r) * E + c);
       Qt[(c + 0) * SQ + r] = v.x, Qt[(c + 1) * SQ + r] = v.y, Qt[(c + 2) * SQ + r] = v.z, Qt[(c + 3) * SQ + r] = v.w;
     }
     const int kcap = (len + 127) & ~127;  // keys the score loop touches: whole 128-key tiles (capped by Tk below)
@@ -162,6 +167,13 @@ __global__ void __launch_bounds__(kTThreads) self_attention_tiled_kernel(
       }
     }
     __syncthreads();
+    if (attn_head0 != nullptr && h == 0) {  // alignment: head 0's probabilities over all T key slots, masked ones 0
+      const int r = tid >> 2, part = tid & 3;
+      if (r < rows_here) {
+        float* dst = attn_head0 + (static_cast<size_t>(b) * Tq + i0 + r) * T;
+        for (int j = part; j < T; j += 4) dst[j] = j < len ? S[r * SK + j] : 0.0f;
+      }
+    }
   }
 
   // ---- P V: thread = 2 queries x (DH / 8) dims... laid out as 32 query pairs x 8 dim groups
@@ -193,9 +205,9 @@ __global__ void __launch_bounds__(kTThreads) self_attention_tiled_kernel(
 #pragma unroll
     for (int u = 0; u < 2; u++) {
       const int i = i0 + r0 + u;
-      if (i >= T) continue;
+      if (i >= Tq) continue;
       const bool live = r0 + u < rows_here;  // padded query rows (and a row pair's odd tail) carry zeros
-      const size_t off = base + static_cast<size_t>(i) * E + d0;
+      const size_t off = base_q + static_cast<size_t>(i) * E + d0;
 #pragma unroll
       for (int w = 0; w < DG; w += 4) {
         float y[4];
@@ -227,20 +239,22 @@ bool self_attention_tiled_supported(int T, int dh) {
 }
 
 int launch_self_attention_tiled(const float* Q, const float* K, const float* V, const uint32_t* lengths, int B, int T, int H,
-                                int dh, QuantOuts q, cudaStream_t stream) {
+                                int dh, QuantOuts q, cudaStream_t stream, int Tq, float* attn_head0) {
   if (B == 0) return 0;
   // 1/sqrt(dim_head) evaluated in double then narrowed, as `1.0F / std::sqrt(size_t)` does (Modules.cc:43)
   const float dk = static_cast<float>(1.0 / std::sqrt(static_cast<double>(dh)));
-  const int n_qb = (T + kQB - 1) / kQB;
+  const int cross = Tq > 0 ? 1 : 0;
+  if (!cross) Tq = T;
+  const int n_qb = (Tq + kQB - 1) / kQB;
   const size_t smem = tiled_smem_bytes(T, dh);
   const long blocks = static_cast<long>(B) * H * n_qb;
   if (!self_attention_tiled_supported(T, dh) || blocks > 0x7fffffffL) return 1;
   if (dh == 32) {
     if (ensure_dyn_smem(self_attention_tiled_kernel<32>, smem) != cudaSuccess) return 1;
-    self_attention_tiled_kernel<32><<<static_cast<unsigned>(blocks), kTThreads, smem, stream>>>(Q, K, V, lengths, T, H, n_qb, dk, q);
+    self_attention_tiled_kernel<32><<<static_cast<unsigned>(blocks), kTThreads, smem, stream>>>(Q, K, V, lengths, T, Tq, cross, H, n_qb, dk, q, attn_head0);
   } else if (dh == 64) {
     if (ensure_dyn_smem(self_attention_tiled_kernel<64>, smem) != cudaSuccess) return 1;
-    self_attention_tiled_kernel<64><<<static_cast<unsigned>(blocks), kTThreads, smem, stream>>>(Q, K, V, lengths, T, H, n_qb, dk, q);
+    self_attention_tiled_kernel<64><<<static_cast<unsigned>(blocks), kTThreads, smem, stream>>>(Q, K, V, lengths, T, Tq, cross, H, n_qb, dk, q, attn_head0);
   } else {
     return 1;
   }

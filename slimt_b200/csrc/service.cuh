@@ -45,11 +45,14 @@ struct Batcher {
 }  // namespace sb
 
 struct slimt_b200_translate_io;
+struct slimt_b200_score_io;
 struct slimt_b200_sampling;
 namespace sb {
 // exhaust() over one request with the batches dealt to the replicas' lanes (translate.cu)
 int translate_multi(Model* const* models, size_t n_replicas, slimt_b200_translate_io* io,
                     const slimt_b200_sampling* sampling);
+// The same batches and lanes scoring given targets with the time-parallel pass (engine.cu: model_score_on)
+int score_multi(Model* const* models, size_t n_replicas, slimt_b200_score_io* io);
 
 // Sampling arguments of the C ABI: nonzero (and the error set) for a temperature that is not finite or lies outside
 // [1e-3, 1e3]; sampling = null (greedy) passes.

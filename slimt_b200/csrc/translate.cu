@@ -1,4 +1,5 @@
-// The service half of the path: one request -> Batcher -> batches -> replicas -> ragged targets.
+// The service half of the path: one request -> Batcher -> batches -> replicas -> ragged targets (translate_multi) or
+// ragged scores of given targets (score_multi); both share the batching and the lanes (Service).
 //
 // Reference: exhaust() (slimt/Frontend.cc:42-60) inside Blocking::translate (:91-145), and Async's worker threads
 // pulling batches from one batcher queue (Frontend.cc:207-227, Batcher.hh:203-259).  Here one host thread per *lane*
@@ -52,9 +53,188 @@ struct Done {
 
 struct LaneStats {
   double device_ms = 0;
-  uint64_t launches = 0, h2d = 0, d2h = 0, target_tokens = 0;
+  uint64_t launches = 0, h2d = 0, d2h = 0;
   std::string error;
 };
+
+// What translate_multi and score_multi share: one request's replicas, its shortlist generator, the Batcher's batches
+// over the source lengths, and the lanes that serve them.
+struct Service {
+  Model* const* models;
+  size_t n_rep;
+  const char* what;  // the entry point, for error messages
+  ShortlistGenerator gen;
+  bool use_sl = false;
+  std::vector<Plan> plan;
+  // counters of run(): device_ms is the longest lane's time
+  double device_ms = 0;
+  uint64_t launches = 0, h2d = 0, d2h = 0;
+
+  int check_replicas() const {
+    if (n_rep == 0 || models == nullptr || models[0] == nullptr) {
+      set_error(std::string(what) + ": no model replica given");
+      return 1;
+    }
+    const Model& m0 = *models[0];
+    for (size_t r = 1; r < n_rep; r++) {
+      if (models[r] == nullptr || models[r]->V != m0.V || models[r]->E != m0.E || models[r]->F != m0.F ||
+          models[r]->eos_id != m0.eos_id || models[r]->pad_id != m0.pad_id) {
+        set_error(std::string(what) + ": replicas must be copies of one model");
+        return 1;
+      }
+    }
+    return 0;
+  }
+  // The smallest length bound over the replicas: any replica may serve any batch.
+  int max_len() const {
+    int n = models[0]->max_len();
+    for (size_t r = 1; r < n_rep; r++) n = std::min(n, models[r]->max_len());
+    return n;
+  }
+  int load_shortlist(const void* bin, size_t bytes, int32_t check, int32_t shared) {
+    use_sl = bin != nullptr && bytes > 0;
+    if (!use_sl) return 0;
+    if (gen.load(bin, bytes, static_cast<size_t>(models[0]->V), check != 0)) return 1;
+    gen.shared_vocabulary = shared != 0;
+    return 0;
+  }
+  // The Batcher's batches, in the order it forms them (Batcher::generate, Batcher.cc:95-120).  Nothing has touched a
+  // GPU yet: a sentence no kernel can take fails the request as a whole, before any batch ran.
+  int make_plan(const uint64_t* offsets, size_t n, size_t max_words) {
+    Batcher batcher(max_words);
+    for (size_t i = 0; i < n; i++) {
+      if (offsets[i + 1] < offsets[i]) {
+        set_error(std::string(what) + ": offsets must be non-decreasing");
+        return 1;
+      }
+      if (offsets[i + 1] == offsets[i]) {
+        set_error(std::string(what) +
+                  ": empty sentences are not valid input (every segment ends in EOS, TextProcessor.cc:132-143)");
+        return 1;
+      }
+      batcher.enqueue(i, offsets[i + 1] - offsets[i]);
+    }
+    for (;;) {
+      Plan p;
+      p.ids = batcher.generate(&p.width);
+      if (p.ids.empty()) break;
+      plan.push_back(std::move(p));
+    }
+    const int bound = max_len();
+    for (const Plan& p : plan) {
+      if (p.width > static_cast<size_t>(bound)) {
+        set_error(std::string(what) + ": a sentence of " + std::to_string(p.width) +
+                  " tokens exceeds the supported maximum of " + std::to_string(bound) +
+                  " (wrap longer input first: TextProcessor's wrap_length)");
+        return 1;
+      }
+    }
+    return 0;
+  }
+  // Deals the batches to the lanes: one host thread per lane takes the next unserved batch as soon as it is free.
+  // serve(m, c, bi) runs batch bi on lane context c (whose lock is held) and returns nonzero with the error set.
+  template <class Serve>
+  int run(Serve serve) {
+    size_t lanes_per = 1;
+    if (const char* e = getenv("SLIMT_B200_LANES")) lanes_per = std::max(1, atoi(e));
+    else if (plan.size() >= 2 * n_rep) lanes_per = 2;
+    struct Lane {
+      Model* m;
+      Context* c;
+    };
+    std::vector<Lane> lanes;
+    for (size_t l = 0; l < lanes_per; l++)
+      for (size_t r = 0; r < n_rep; r++) {
+        Context* c = models[r]->lane(l);
+        if (!c) return 1;
+        lanes.push_back(Lane{models[r], c});
+      }
+    if (lanes.size() > plan.size()) lanes.resize(std::max<size_t>(1, plan.size()));
+    std::vector<LaneStats> stats(lanes.size());
+    std::atomic<size_t> next{0};
+    std::atomic<bool> failed{false};
+
+    auto lane_loop = [&](size_t li) {
+      Lane& lane = lanes[li];
+      Context& c = *lane.c;
+      LaneStats& st = stats[li];
+      std::lock_guard<std::recursive_mutex> ctx_lock(c.mu);  // the lane's staging block is ours for the whole request
+      const uint64_t l0 = c.launches, h0 = c.h2d_bytes, d0 = c.d2h_bytes;
+      cudaSetDevice(c.device);
+      cudaEvent_t e0 = nullptr, e1 = nullptr;
+      bool timed = false;
+      for (;;) {
+        const size_t bi = next.fetch_add(1);
+        if (bi >= plan.size() || failed.load()) break;
+        if (!timed) {
+          cudaEventCreate(&e0), cudaEventCreate(&e1);
+          cudaEventRecord(e0, c.stream);
+          timed = true;
+        }
+        if (serve(*lane.m, c, bi)) {
+          st.error = last_error();
+          failed = true;
+          break;
+        }
+      }
+      if (timed) {
+        cudaEventRecord(e1, c.stream);
+        cudaEventSynchronize(e1);
+        float ms = 0;
+        cudaEventElapsedTime(&ms, e0, e1);
+        st.device_ms = ms;
+        cudaEventDestroy(e0), cudaEventDestroy(e1);
+      }
+      st.launches = c.launches - l0, st.h2d = c.h2d_bytes - h0, st.d2h = c.d2h_bytes - d0;
+    };
+
+    if (lanes.size() == 1) {
+      lane_loop(0);
+    } else {
+      std::vector<std::thread> threads;
+      for (size_t li = 0; li < lanes.size(); li++) threads.emplace_back(lane_loop, li);
+      for (std::thread& t : threads) t.join();
+    }
+    for (const LaneStats& st : stats) {
+      if (!st.error.empty()) {
+        set_error(st.error);  // the worker's message, re-raised on the calling thread
+        return 1;
+      }
+      device_ms = std::max(device_ms, st.device_ms);
+      launches += st.launches, h2d += st.h2d, d2h += st.d2h;
+    }
+    return 0;
+  }
+};
+
+// convert(): Batch -> padded Input (Frontend.cc:30-40; Input.cc:20-47), and the batch's source words for the shortlist
+void pack_sources(const uint32_t* src, const uint64_t* offsets, const Plan& p, uint32_t pad_id, uint32_t* tokens,
+                  uint32_t* lengths, std::vector<uint32_t>* words) {
+  const size_t width = p.width;
+  words->clear();
+  words->reserve(p.ids.size() * width);
+  for (size_t r = 0; r < p.ids.size(); r++) {
+    const size_t s = p.ids[r];
+    const size_t len = offsets[s + 1] - offsets[s];
+    memcpy(tokens + r * width, src + offsets[s], 4 * len);
+    for (size_t t = len; t < width; t++) tokens[r * width + t] = pad_id;
+    lengths[r] = static_cast<uint32_t>(len);
+    words->insert(words->end(), src + offsets[s], src + offsets[s + 1]);
+  }
+}
+
+// Copies each batch's per-sentence results (back to back in batch row order, `n(s)` values for sentence s) to their
+// places in the request's ragged output.
+template <class T, class Get, class N>
+void scatter(const std::vector<Plan>& plan, Get per_batch, const std::vector<uint64_t>& off, N n, T* out) {
+  for (size_t bi = 0; bi < plan.size(); bi++) {
+    size_t pos = 0;
+    for (size_t s : plan[bi].ids) {
+      memcpy(out + off[s], per_batch(bi).data() + pos, sizeof(T) * n(s));
+      pos += n(s);
+    }
+  }
+}
 
 }  // namespace
 
@@ -82,246 +262,104 @@ int check_sampling(const slimt_b200_sampling* sampling) {
 }
 
 int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io* io, const slimt_b200_sampling* sampling) {
-  if (n_rep == 0 || models == nullptr || models[0] == nullptr) {
-    set_error("translate: no model replica given");
-    return 1;
-  }
-  Model& m0 = *models[0];
-  for (size_t r = 1; r < n_rep; r++) {
-    if (models[r] == nullptr || models[r]->V != m0.V || models[r]->E != m0.E || models[r]->F != m0.F ||
-        models[r]->eos_id != m0.eos_id || models[r]->pad_id != m0.pad_id) {
-      set_error("translate: replicas must be copies of one model");
-      return 1;
-    }
-  }
+  Service sv{models, n_rep, "translate"};
+  if (sv.check_replicas()) return 1;
   io->target_tokens = 0, io->batches = 0, io->device_ms = 0;
   io->kernel_launches = 0, io->h2d_bytes = 0, io->d2h_bytes = 0;
   const size_t n_sent = io->n_sentences;
   const bool want_align = io->out_alignments != nullptr;
   const bool want_scores = io->out_scores != nullptr;
-
-  ShortlistGenerator gen;
-  const bool use_sl = io->shortlist_bin != nullptr && io->shortlist_bytes > 0;
-  if (use_sl) {
-    if (gen.load(io->shortlist_bin, io->shortlist_bytes, static_cast<size_t>(m0.V), io->shortlist_check != 0)) return 1;
-    gen.shared_vocabulary = io->shortlist_shared != 0;
-  }
-
-  // ---- the Batcher's batches, in the order it forms them (Batcher::generate, Batcher.cc:95-120)
-  std::vector<Plan> plan;
-  {
-    Batcher batcher(io->max_words);
-    for (size_t i = 0; i < n_sent; i++) {
-      if (io->offsets[i + 1] < io->offsets[i]) {
-        set_error("translate: offsets must be non-decreasing");
-        return 1;
-      }
-      if (io->offsets[i + 1] == io->offsets[i]) {
-        set_error("translate: empty sentences are not valid input (every segment ends in EOS, TextProcessor.cc:132-143)");
-        return 1;
-      }
-      batcher.enqueue(i, io->offsets[i + 1] - io->offsets[i]);
-    }
-    for (;;) {
-      Plan p;
-      p.ids = batcher.generate(&p.width);
-      if (p.ids.empty()) break;
-      plan.push_back(std::move(p));
-    }
-  }
-  // nothing has touched a GPU yet: a sentence no kernel can take fails the request as a whole, before any batch ran.
-  // Any replica may serve any batch, so the smallest bound of them all applies.
-  int max_len = m0.max_len();
-  for (size_t r = 1; r < n_rep; r++) max_len = std::min(max_len, models[r]->max_len());
-  for (const Plan& p : plan) {
-    if (p.width > static_cast<size_t>(max_len)) {
-      set_error("translate: a sentence of " + std::to_string(p.width) + " tokens exceeds the supported maximum of " +
-                std::to_string(max_len) + " (wrap longer input first: TextProcessor's wrap_length)");
-      return 1;
-    }
-  }
+  if (sv.load_shortlist(io->shortlist_bin, io->shortlist_bytes, io->shortlist_check, io->shortlist_shared)) return 1;
+  if (sv.make_plan(io->offsets, n_sent, io->max_words)) return 1;
+  const std::vector<Plan>& plan = sv.plan;
 
   std::vector<Done> done(plan.size());
   std::vector<uint32_t> out_len(n_sent, 0);
-
-  // ---- lanes
-  size_t lanes_per = 1;
-  if (const char* e = getenv("SLIMT_B200_LANES")) lanes_per = std::max(1, atoi(e));
-  else if (plan.size() >= 2 * n_rep) lanes_per = 2;
-  struct Lane {
-    Model* m;
-    Context* c;
-  };
-  std::vector<Lane> lanes;
-  for (size_t l = 0; l < lanes_per; l++)
-    for (size_t r = 0; r < n_rep; r++) {
-      Context* c = models[r]->lane(l);
-      if (!c) return 1;
-      lanes.push_back(Lane{models[r], c});
-    }
-  if (lanes.size() > plan.size()) lanes.resize(std::max<size_t>(1, plan.size()));
-  std::vector<LaneStats> stats(lanes.size());
-  std::atomic<size_t> next{0};
-  std::atomic<bool> failed{false};
-
-  auto serve = [&](size_t li) {
-    Lane& lane = lanes[li];
-    Context& c = *lane.c;
-    Model& m = *lane.m;
-    LaneStats& st = stats[li];
-    std::lock_guard<std::recursive_mutex> ctx_lock(c.mu);  // the lane's staging block is ours for the whole request
-    const uint64_t l0 = c.launches, h0 = c.h2d_bytes, d0 = c.d2h_bytes;
-    cudaSetDevice(c.device);
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    bool timed = false;
+  auto serve = [&](Model& m, Context& c, size_t bi) -> int {
+    const Plan& p = plan[bi];
+    const size_t B = p.ids.size(), width = p.width;
+    const size_t stride = static_cast<size_t>(forward_max_steps(io->limit_factor, width));
+    // staging: [padded tokens][lengths] | [sentence-major step tokens][recorded lengths] | [alignment rows] |
+    // [step-major scores] | [sampling keys]
+    const size_t in_bytes = (4 * (B * width + B) + 255) & ~size_t(255);
+    const size_t tok_bytes = (4 * (stride + 1) * B + 255) & ~size_t(255);
+    const size_t al_bytes = want_align ? 4 * stride * B * width : 0;
+    const size_t sc_bytes = want_scores ? 4 * stride * B : 0;
+    const size_t key_off = (in_bytes + tok_bytes + al_bytes + sc_bytes + 7) & ~size_t(7);
+    char* stage = c.staging_reserve(in_bytes + tok_bytes + al_bytes + sc_bytes + (sampling ? 8 * B + 8 : 0) + 256);
+    if (!stage) return 1;
+    uint32_t* tokens = reinterpret_cast<uint32_t*>(stage);
+    uint32_t* lengths = tokens + B * width;
     std::vector<uint32_t> words;
-    for (;;) {
-      const size_t bi = next.fetch_add(1);
-      if (bi >= plan.size() || failed.load()) break;
-      const Plan& p = plan[bi];
-      const size_t B = p.ids.size(), width = p.width;
-      const size_t stride = static_cast<size_t>(forward_max_steps(io->limit_factor, width));
-      // staging: [padded tokens][lengths] | [sentence-major step tokens][recorded lengths] | [alignment rows] |
-      // [step-major scores] | [sampling keys]
-      const size_t in_bytes = (4 * (B * width + B) + 255) & ~size_t(255);
-      const size_t tok_bytes = (4 * (stride + 1) * B + 255) & ~size_t(255);
-      const size_t al_bytes = want_align ? 4 * stride * B * width : 0;
-      const size_t sc_bytes = want_scores ? 4 * stride * B : 0;
-      const size_t key_off = (in_bytes + tok_bytes + al_bytes + sc_bytes + 7) & ~size_t(7);
-      char* stage = c.staging_reserve(in_bytes + tok_bytes + al_bytes + sc_bytes + (sampling ? 8 * B + 8 : 0) + 256);
-      if (!stage) {
-        st.error = last_error();
-        failed = true;
-        break;
-      }
-      // convert(): Batch -> padded Input (Frontend.cc:30-40; Input.cc:20-47)
-      uint32_t* tokens = reinterpret_cast<uint32_t*>(stage);
-      uint32_t* lengths = tokens + B * width;
-      words.clear();
-      words.reserve(B * width);
-      for (size_t r = 0; r < B; r++) {
-        const size_t s = p.ids[r];
-        const size_t len = io->offsets[s + 1] - io->offsets[s];
-        memcpy(tokens + r * width, io->tokens + io->offsets[s], 4 * len);
-        for (size_t t = len; t < width; t++) tokens[r * width + t] = m.pad_id;
-        lengths[r] = static_cast<uint32_t>(len);
-        words.insert(words.end(), io->tokens + io->offsets[s], io->tokens + io->offsets[s + 1]);
-      }
-      // Model::decode builds the candidate set before its first step (Model.cc:116-120); here the host does it
-      // while the GPU runs the encoder (the callback fires once the encoder kernels are queued)
-      LazyShortlist lazy{&gen, &words, static_cast<size_t>(m.V), {}};
-      uint32_t* rows = reinterpret_cast<uint32_t*>(stage + in_bytes);
-      uint32_t* lens = rows + stride * B;
-      float* align = want_align ? reinterpret_cast<float*>(stage + in_bytes + tok_bytes) : nullptr;
-      float* scores = want_scores ? reinterpret_cast<float*>(stage + in_bytes + tok_bytes + al_bytes) : nullptr;
-      ForwardArgs a;
-      a.tokens = tokens, a.lengths = lengths, a.B = B, a.T = width;
-      a.limit_factor = io->limit_factor;
-      if (use_sl) a.shortlist_cb = lazy_shortlist_cb, a.shortlist_user = &lazy;
-      a.sentence_tokens = rows, a.row_stride = stride, a.target_lengths = lens;
-      a.alignment = align;
-      a.scores = scores;
-      if (sampling) {
-        // each sentence's own key (default: its index in the request), wherever the Batcher put it
-        uint64_t* keys = reinterpret_cast<uint64_t*>(stage + key_off);
-        for (size_t r = 0; r < B; r++) keys[r] = sampling->keys ? sampling->keys[p.ids[r]] : static_cast<uint64_t>(p.ids[r]);
-        a.sample = true, a.inv_t = sampling_inv_t(sampling->temperature), a.seed = sampling->seed, a.keys = keys;
-      }
-      if (!timed) {
-        cudaEventCreate(&e0), cudaEventCreate(&e1);
-        cudaEventRecord(e0, c.stream);
-        timed = true;
-      }
-      if (model_forward_on(m, c, a)) {
-        st.error = last_error();
-        failed = true;
-        break;
-      }
-      Done& d = done[bi];
-      size_t kept_total = 0, align_total = 0;
-      for (size_t r = 0; r < B; r++) {
-        out_len[p.ids[r]] = lens[r];
-        kept_total += lens[r];
-        align_total += static_cast<size_t>(lens[r]) * lengths[r];
-      }
-      d.kept.resize(kept_total);
-      size_t pos = 0;
-      for (size_t r = 0; r < B; r++) {
-        memcpy(d.kept.data() + pos, rows + r * stride, 4ul * lens[r]);
-        pos += lens[r];
-      }
-      if (want_align) {  // update_alignment (Model.cc:84-108): one distribution over the sentence's own source tokens per target token
-        d.align.resize(align_total);
-        size_t ap = 0;
-        for (size_t r = 0; r < B; r++)
-          for (size_t s = 0; s < lens[r]; s++) {
-            memcpy(d.align.data() + ap, align + (s * B + r) * width, 4ul * lengths[r]);
-            ap += lengths[r];
-          }
-      }
-      if (want_scores) {  // the scores of the recorded steps, sentence by sentence in batch row order like kept
-        d.scores.resize(kept_total);
-        size_t sp = 0;
-        for (size_t r = 0; r < B; r++)
-          for (size_t s = 0; s < lens[r]; s++) d.scores[sp++] = scores[s * B + r];
-      }
-      st.target_tokens += a.target_tokens;
+    pack_sources(io->tokens, io->offsets, p, m.pad_id, tokens, lengths, &words);
+    // Model::decode builds the candidate set before its first step (Model.cc:116-120); here the host does it
+    // while the GPU runs the encoder (the callback fires once the encoder kernels are queued)
+    LazyShortlist lazy{&sv.gen, &words, static_cast<size_t>(m.V), {}};
+    uint32_t* rows = reinterpret_cast<uint32_t*>(stage + in_bytes);
+    uint32_t* lens = rows + stride * B;
+    float* align = want_align ? reinterpret_cast<float*>(stage + in_bytes + tok_bytes) : nullptr;
+    float* scores = want_scores ? reinterpret_cast<float*>(stage + in_bytes + tok_bytes + al_bytes) : nullptr;
+    ForwardArgs a;
+    a.tokens = tokens, a.lengths = lengths, a.B = B, a.T = width;
+    a.limit_factor = io->limit_factor;
+    if (sv.use_sl) a.shortlist_cb = lazy_shortlist_cb, a.shortlist_user = &lazy;
+    a.sentence_tokens = rows, a.row_stride = stride, a.target_lengths = lens;
+    a.alignment = align;
+    a.scores = scores;
+    if (sampling) {
+      // each sentence's own key (default: its index in the request), wherever the Batcher put it
+      uint64_t* keys = reinterpret_cast<uint64_t*>(stage + key_off);
+      for (size_t r = 0; r < B; r++) keys[r] = sampling->keys ? sampling->keys[p.ids[r]] : static_cast<uint64_t>(p.ids[r]);
+      a.sample = true, a.inv_t = sampling_inv_t(sampling->temperature), a.seed = sampling->seed, a.keys = keys;
     }
-    if (timed) {
-      cudaEventRecord(e1, c.stream);
-      cudaEventSynchronize(e1);
-      float ms = 0;
-      cudaEventElapsedTime(&ms, e0, e1);
-      st.device_ms = ms;
-      cudaEventDestroy(e0), cudaEventDestroy(e1);
+    if (model_forward_on(m, c, a)) return 1;
+    Done& d = done[bi];
+    size_t kept_total = 0, align_total = 0;
+    for (size_t r = 0; r < B; r++) {
+      out_len[p.ids[r]] = lens[r];
+      kept_total += lens[r];
+      align_total += static_cast<size_t>(lens[r]) * lengths[r];
     }
-    st.launches = c.launches - l0, st.h2d = c.h2d_bytes - h0, st.d2h = c.d2h_bytes - d0;
+    d.kept.resize(kept_total);
+    size_t pos = 0;
+    for (size_t r = 0; r < B; r++) {
+      memcpy(d.kept.data() + pos, rows + r * stride, 4ul * lens[r]);
+      pos += lens[r];
+    }
+    if (want_align) {  // update_alignment (Model.cc:84-108): one distribution over the sentence's own source tokens per target token
+      d.align.resize(align_total);
+      size_t ap = 0;
+      for (size_t r = 0; r < B; r++)
+        for (size_t s = 0; s < lens[r]; s++) {
+          memcpy(d.align.data() + ap, align + (s * B + r) * width, 4ul * lengths[r]);
+          ap += lengths[r];
+        }
+    }
+    if (want_scores) {  // the scores of the recorded steps, sentence by sentence in batch row order like kept
+      d.scores.resize(kept_total);
+      size_t sp = 0;
+      for (size_t r = 0; r < B; r++)
+        for (size_t s = 0; s < lens[r]; s++) d.scores[sp++] = scores[s * B + r];
+    }
+    return 0;
   };
-
-  if (lanes.size() == 1) {
-    serve(0);
-  } else {
-    std::vector<std::thread> threads;
-    for (size_t li = 0; li < lanes.size(); li++) threads.emplace_back(serve, li);
-    for (std::thread& t : threads) t.join();
-  }
-  for (const LaneStats& st : stats) {
-    if (!st.error.empty()) {
-      set_error(st.error);  // the worker's message, re-raised on the calling thread
-      return 1;
-    }
-    io->device_ms = std::max(io->device_ms, st.device_ms);
-    io->kernel_launches += st.launches, io->h2d_bytes += st.h2d, io->d2h_bytes += st.d2h;
-    io->target_tokens += st.target_tokens;
-  }
+  if (sv.run(serve)) return 1;
+  io->device_ms = sv.device_ms;
+  io->kernel_launches = sv.launches, io->h2d_bytes = sv.h2d, io->d2h_bytes = sv.d2h;
   io->batches = plan.size();
 
   // ---- ragged outputs
   std::vector<uint64_t> out_off(n_sent + 1, 0);
   for (size_t i = 0; i < n_sent; i++) out_off[i + 1] = out_off[i] + out_len[i];
+  io->target_tokens = out_off[n_sent];
   if ((io->out_tokens || want_scores) && out_off[n_sent] > io->out_capacity) {
     set_error(io->out_tokens ? "out_tokens capacity too small" : "out_scores capacity too small");
     return 1;
   }
   if (io->out_offsets) memcpy(io->out_offsets, out_off.data(), 8 * (n_sent + 1));
-  if (io->out_tokens) {
-    for (size_t bi = 0; bi < plan.size(); bi++) {
-      size_t pos = 0;
-      for (size_t s : plan[bi].ids) {
-        memcpy(io->out_tokens + out_off[s], done[bi].kept.data() + pos, 4ul * out_len[s]);
-        pos += out_len[s];
-      }
-    }
-  }
-  if (want_scores) {
-    for (size_t bi = 0; bi < plan.size(); bi++) {
-      size_t pos = 0;
-      for (size_t s : plan[bi].ids) {
-        memcpy(io->out_scores + out_off[s], done[bi].scores.data() + pos, 4ul * out_len[s]);
-        pos += out_len[s];
-      }
-    }
-  }
+  auto n_out = [&](size_t s) { return static_cast<size_t>(out_len[s]); };
+  if (io->out_tokens) scatter(plan, [&](size_t bi) -> const auto& { return done[bi].kept; }, out_off, n_out, io->out_tokens);
+  if (want_scores) scatter(plan, [&](size_t bi) -> const auto& { return done[bi].scores; }, out_off, n_out, io->out_scores);
   if (want_align) {
     std::vector<uint64_t> al_off(n_sent + 1, 0);
     for (size_t i = 0; i < n_sent; i++) al_off[i + 1] = al_off[i] + static_cast<uint64_t>(out_len[i]) * (io->offsets[i + 1] - io->offsets[i]);
@@ -330,14 +368,135 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
       return 1;
     }
     if (io->out_align_offsets) memcpy(io->out_align_offsets, al_off.data(), 8 * (n_sent + 1));
-    for (size_t bi = 0; bi < plan.size(); bi++) {
-      size_t pos = 0;
-      for (size_t s : plan[bi].ids) {
-        const size_t n = static_cast<size_t>(al_off[s + 1] - al_off[s]);
-        memcpy(io->out_alignments + al_off[s], done[bi].align.data() + pos, 4ul * n);
-        pos += n;
+    scatter(plan, [&](size_t bi) -> const auto& { return done[bi].align; }, al_off,
+            [&](size_t s) { return static_cast<size_t>(al_off[s + 1] - al_off[s]); }, io->out_alignments);
+  }
+  return 0;
+}
+
+int score_multi(Model* const* models, size_t n_rep, slimt_b200_score_io* io) {
+  io->batches = 0, io->device_ms = 0, io->kernel_launches = 0, io->h2d_bytes = 0, io->d2h_bytes = 0;
+  const size_t n_sent = io->n_sentences;
+  const uint64_t* so = io->offsets;
+  const uint64_t* to = io->target_offsets;
+  const bool want_align = io->out_alignments != nullptr;
+  // the request's shape, checked before anything else (no model is needed for it)
+  if (n_sent > 0 && (so == nullptr || to == nullptr || io->tokens == nullptr)) {
+    set_error("score: tokens, offsets and target_offsets are required");
+    return 1;
+  }
+  for (size_t i = 0; i < n_sent; i++) {
+    if (so[i + 1] < so[i] || to[i + 1] < to[i]) {
+      set_error("score: offsets must be non-decreasing");
+      return 1;
+    }
+  }
+  const uint64_t n_tgt = n_sent ? to[n_sent] - to[0] : 0;
+  if (n_tgt > 0 && (io->targets == nullptr || io->out_scores == nullptr)) {
+    set_error("score: targets and out_scores are required");
+    return 1;
+  }
+  if (n_tgt > io->out_capacity) {
+    set_error("score: out_scores capacity too small (" + std::to_string(n_tgt) + " target tokens)");
+    return 1;
+  }
+  std::vector<uint64_t> al_off(n_sent + 1, 0);
+  for (size_t i = 0; i < n_sent; i++) al_off[i + 1] = al_off[i] + (to[i + 1] - to[i]) * (so[i + 1] - so[i]);
+  if (want_align && al_off[n_sent] > io->align_capacity) {
+    set_error("score: out_alignments capacity too small");
+    return 1;
+  }
+  Service sv{models, n_rep, "score"};
+  if (sv.check_replicas()) return 1;
+  const int bound = sv.max_len();
+  const uint32_t V = static_cast<uint32_t>(models[0]->V);
+  for (size_t i = 0; i < n_sent; i++) {
+    if (to[i + 1] - to[i] > static_cast<uint64_t>(bound)) {
+      set_error("score: target " + std::to_string(i) + " of " + std::to_string(to[i + 1] - to[i]) +
+                " tokens exceeds the supported maximum of " + std::to_string(bound));
+      return 1;
+    }
+    for (uint64_t k = to[i]; k < to[i + 1]; k++)
+      if (io->targets[k] >= V) {
+        set_error("score: target word " + std::to_string(io->targets[k]) + " is outside the vocabulary of " +
+                  std::to_string(V));
+        return 1;
+      }
+  }
+  if (sv.load_shortlist(io->shortlist_bin, io->shortlist_bytes, io->shortlist_check, io->shortlist_shared)) return 1;
+  if (sv.make_plan(so, n_sent, io->max_words)) return 1;
+  const std::vector<Plan>& plan = sv.plan;
+
+  std::vector<std::vector<float>> scores(plan.size()), align(plan.size());
+  auto serve = [&](Model& m, Context& c, size_t bi) -> int {
+    const Plan& p = plan[bi];
+    const size_t B = p.ids.size(), width = p.width;
+    size_t Tt = 0, n_scores = 0, n_align = 0;
+    for (size_t s : p.ids) {
+      const size_t tl = to[s + 1] - to[s];
+      Tt = std::max(Tt, tl), n_scores += tl, n_align += tl * (so[s + 1] - so[s]);
+    }
+    if (Tt == 0) return 0;  // every target of the batch is empty: nothing to score
+    // staging: [padded tokens][lengths] | [padded targets] | [scores] | [alignments]
+    const size_t in_bytes = (4 * (B * width + B) + 255) & ~size_t(255);
+    const size_t tg_bytes = (4 * B * Tt + 255) & ~size_t(255);
+    const size_t al_bytes = want_align ? 4 * B * Tt * width : 0;
+    char* stage = c.staging_reserve(in_bytes + 2 * tg_bytes + al_bytes + 256);
+    if (!stage) return 1;
+    uint32_t* tokens = reinterpret_cast<uint32_t*>(stage);
+    uint32_t* lengths = tokens + B * width;
+    std::vector<uint32_t> words;
+    pack_sources(io->tokens, so, p, m.pad_id, tokens, lengths, &words);
+    uint32_t* targets = reinterpret_cast<uint32_t*>(stage + in_bytes);
+    float* sc = reinterpret_cast<float*>(stage + in_bytes + tg_bytes);
+    float* al = want_align ? reinterpret_cast<float*>(stage + in_bytes + 2 * tg_bytes) : nullptr;
+    for (size_t r = 0; r < B; r++) {
+      const size_t s = p.ids[r], tl = to[s + 1] - to[s];
+      memcpy(targets + r * Tt, io->targets + to[s], 4 * tl);
+      for (size_t j = tl; j < Tt; j++) targets[r * Tt + j] = m.pad_id;  // computed and discarded
+    }
+    LazyShortlist lazy{&sv.gen, &words, static_cast<size_t>(m.V), {}};
+    ForwardArgs a;
+    a.tokens = tokens, a.lengths = lengths, a.B = B, a.T = width;
+    if (sv.use_sl) a.shortlist_cb = lazy_shortlist_cb, a.shortlist_user = &lazy;
+    a.targets = targets, a.target_T = Tt, a.scores = sc, a.alignment = al;
+    if (model_score_on(m, c, a)) return 1;
+    // each sentence's valid positions, back to back in batch row order
+    std::vector<float>& ds = scores[bi];
+    ds.resize(n_scores);
+    size_t sp = 0;
+    for (size_t r = 0; r < B; r++) {
+      const size_t tl = to[p.ids[r] + 1] - to[p.ids[r]];
+      memcpy(ds.data() + sp, sc + r * Tt, 4 * tl);
+      sp += tl;
+    }
+    if (want_align) {
+      std::vector<float>& da = align[bi];
+      da.resize(n_align);
+      size_t ap = 0;
+      for (size_t r = 0; r < B; r++) {
+        const size_t tl = to[p.ids[r] + 1] - to[p.ids[r]];
+        for (size_t j = 0; j < tl; j++) {
+          memcpy(da.data() + ap, al + (r * Tt + j) * width, 4ul * lengths[r]);
+          ap += lengths[r];
+        }
       }
     }
+    return 0;
+  };
+  if (sv.run(serve)) return 1;
+  io->device_ms = sv.device_ms;
+  io->kernel_launches = sv.launches, io->h2d_bytes = sv.h2d, io->d2h_bytes = sv.d2h;
+  io->batches = plan.size();
+
+  std::vector<uint64_t> out_off(n_sent + 1, 0);
+  for (size_t i = 0; i < n_sent; i++) out_off[i + 1] = out_off[i] + (to[i + 1] - to[i]);
+  auto n_out = [&](size_t s) { return static_cast<size_t>(to[s + 1] - to[s]); };
+  if (n_tgt > 0) scatter(plan, [&](size_t bi) -> const auto& { return scores[bi]; }, out_off, n_out, io->out_scores);
+  if (want_align) {
+    if (io->out_align_offsets) memcpy(io->out_align_offsets, al_off.data(), 8 * (n_sent + 1));
+    scatter(plan, [&](size_t bi) -> const auto& { return align[bi]; }, al_off, [&](size_t s) { return static_cast<size_t>(al_off[s + 1] - al_off[s]); },
+            io->out_alignments);
   }
   return 0;
 }

@@ -593,6 +593,21 @@ void padd(GemmProblem* p, int8_t* ptr, float aq) {
   p->n_qout++;
 }
 
+// The row-tile kernel's arguments for one layer's Wo + residual + LN and FFN + residual + LN over M rows: the weights,
+// biases, multipliers and LayerNorms of `att` and `ffn`.  The caller adds the A operand's map, y_park and the outputs.
+RowsFfnArgs rows_ffn_args(const AttnW& att, const FfnW& ffn, const float* res, int M) {
+  RowsFfnArgs k{};
+  k.map_wo = att.o.map128, k.map_w1 = ffn.w1.map128, k.map_w2 = ffn.w2.map128;
+  k.pb_o = att.o.pb, k.pb_1 = ffn.w1.pb, k.pb_2 = ffn.w2.pb;
+  k.um_o = att.o.um, k.um_1 = ffn.w1.um, k.um_2 = ffn.w2.um;
+  k.aq_1 = ffn.w1.aq, k.aq_2 = ffn.w2.aq;
+  k.res = res;
+  k.ln1_scale = att.ln.scale, k.ln1_bias = att.ln.bias;
+  k.ln2_scale = ffn.ln.scale, k.ln2_bias = ffn.ln.bias, k.eps = 1e-6f;
+  k.M = M;
+  return k;
+}
+
 }  // namespace
 
 // ------------------------------------------------------------------ operator API
@@ -769,11 +784,15 @@ struct Pass {
   CUtensorMap map_qa[3], map_qa32[3], mapK[2], mapV[2];
   CUtensorMap map_xq[2], map_zq[2], map_caq;  // u8 activation operands of the row-tile kernels, box {128 B, 32 rows}
   CUtensorMap map_oq;
-  int plan(), encode(), prepare_cross(), prepare_output(), decode_step(int step), decode(), score();
+  int plan(), plan_step(Workspace& ws), plan_score(Workspace& ws), carve(const Workspace& ws);
+  int encode(), prepare_cross(), prepare_output(), decode_step(int step), decode(), score();
+  QuantOuts enc_inputs(int i);
+  void dec_layer_out(RowsFfnArgs& k, int l, float* z, int8_t* xf, int8_t* xw) const;
+  ScoreStepArgs score_step_args(int rows, const int8_t* oq_rows, const uint32_t* forced, int step, float* scores) const;
 };
 
 // Checks the request, chooses the routes and plans the workspace: each buffer is listed once, under the condition in
-// which the chosen routes read it.
+// which the chosen routes read it.  The buffers both paths share are listed here, the rest by plan_step / plan_score.
 int Pass::plan() {
   B = static_cast<int>(a.B), T = static_cast<int>(a.T), E = m.E, F = m.F, H = m.H, dh = m.dh;
   R = B * T;
@@ -784,13 +803,6 @@ int Pass::plan() {
   }
   if (Ld < 1 || 2 * Ld > kMaxQuantOut) {
     set_error("decoder_layers must be 1 or 2");
-    return 1;
-  }
-  scoring = a.targets != nullptr;
-  fast = c.fast && !scoring;
-  Tt = static_cast<int>(a.target_T), M = B * Tt;
-  if (scoring && Tt > m.max_len()) {
-    set_error("target length " + std::to_string(Tt) + " exceeds the supported maximum of " + std::to_string(m.max_len()));
     return 1;
   }
   // Model.cc:160: size_t max_seq_length = limit_factor * source_sequence_length (float product, truncated).  The first
@@ -816,6 +828,8 @@ int Pass::plan() {
     set_error("shortlist size must be a multiple of 8");
     return 1;
   }
+  scoring = a.targets != nullptr;
+  fast = c.fast && !scoring;
   route = choose_routes(m, T, B, fast, a.logits != nullptr, a.scores != nullptr || a.sample);
   if (scoring) {
     // T_target queries read each layer's cross K/V: projected once (Cached); every logit evaluated exactly (Scores)
@@ -823,8 +837,7 @@ int Pass::plan() {
     route.out = Out::Scores;
   }
 
-  const size_t RE = static_cast<size_t>(R) * E, BE = static_cast<size_t>(B) * E;
-  const size_t SB = static_cast<size_t>(max_steps) * B, N = static_cast<size_t>(Nout);
+  const size_t RE = static_cast<size_t>(R) * E, N = static_cast<size_t>(Nout);
   // the output layer's columns are the model's unless the shortlist's are listed below; a subset of the columns fits
   // the model's encoding and its eta
   out = m.vocab;
@@ -836,47 +849,18 @@ int Pass::plan() {
   ws.add(attn_q, RE);
   if (route.ffn == EncFfn::Gemm) ws.add(ffn_q, static_cast<size_t>(R) * F);
   for (int l = 0; l < Ld && route.cross == Cross::Cached; l++) ws.add(Kc[l], RE), ws.add(Vc[l], RE);
-  if (scoring) {
-    // one row per (sentence, target position); the layer input xd is rewritten in place by each layer's FFN
-    const size_t ME = static_cast<size_t>(M) * E, rows = std::min(M, kScoreChunk);
-    ws.add(d_tgt, M);
-    ws.add(xd, ME), ws.add(Fb, ME), ws.add(Wx, ME), ws.add(hb, ME), ws.add(qd, ME);
-    ws.add(xq[0], ME), ws.add(xq[1], ME), ws.add(hq, ME), ws.add(caq, ME), ws.add(oq, ME);
-    ws.add(d_scores, M), ws.add(best, rows), ws.add(partials, (N + kScoreStrip - 1) / kScoreStrip * rows);
-    if (a.alignment) ws.add(d_align_all, ME / E * T);
-  } else {
-    ws.add(xd, BE), ws.add(hb, BE), ws.add(qd, BE), ws.add(zb, BE);
-    for (int l = 0; l < Ld; l++) ws.add(state[l], BE);
-    ws.add(xq[0], BE), ws.add(xq[1], BE), ws.add(zq[0], BE), ws.add(zq[1], BE), ws.add(caq, BE), ws.add(oq, BE);
-    ws.add(best, B), ws.add(done, B), ws.add(tgt_len, B), ws.add(counters, 64);
-    if (!a.device_io) {
-      ws.add(d_steps, SB);
-      if (a.forced) ws.add(d_forced, SB);
-    }
-  }
   if (use_sl) {
     if (!a.device_io) ws.add(d_sl, N);
     out.N = Nout;
     ws.add(out.w, N * E), ws.add(out.pb, N), ws.add(out.c127, N);
     if (route.out == Out::Argmax) out.tables([&ws](auto*& p, size_t n) { ws.add(p, n); });
   }
-  if (route.out == Out::Logits) ws.add(d_logits, static_cast<size_t>(B) * N);
-  if (!scoring) {
-    if (a.scores && !a.device_io) ws.add(d_scores, SB);
-    if (a.scores || a.sample) ws.add(partials, (N + kScoreStrip - 1) / kScoreStrip * static_cast<size_t>(B));
-    if (a.sample && a.keys && !a.device_io) ws.add(d_keys, B);
-    // head-0 probabilities of every step stay on the device and come back in one copy after the loop
-    if (a.alignment) ws.add(d_align_all, SB * T);
-    if (!a.device_io && a.sentence_tokens) ws.add(d_rows, SB);
-  }
-  if (ws.carve(c)) return 1;
-  if (a.device_io) {
-    d_tokens = const_cast<uint32_t*>(a.tokens), d_lengths = const_cast<uint32_t*>(a.lengths), d_steps = a.step_tokens;
-    d_forced = const_cast<uint32_t*>(a.forced), d_sl = use_sl ? const_cast<uint32_t*>(a.shortlist) : nullptr;
-    d_scores = a.scores;
-    d_keys = const_cast<uint64_t*>(a.keys);
-  }
+  return scoring ? plan_score(ws) : plan_step(ws);
+}
 
+// Reserves the workspace once a path has listed its buffers, and makes the encoder's tensor maps.
+int Pass::carve(const Workspace& ws) {
+  if (ws.carve(c)) return 1;
   // cross-attention K/V operands: projected once (Cross::Cached), or the u8 encoder output the recompute kernels read
   const uint32_t box_rows = static_cast<uint32_t>(cross_attention_box_rows(T));
   for (int l = 0; l < Ld; l++)
@@ -888,11 +872,93 @@ int Pass::plan() {
   if (route.self == SelfAttn::Fused)
     for (int i = 0; i < 3; i++)
       if (c.make_map(&map_qa[i], qa[i], R, E, 128) || c.make_map(&map_qa32[i], qa[i], R, E, 32)) return 1;
-  if (scoring) return c.make_map(&map_caq, caq, M, E, kRowTile);  // the output operand's maps are made per row chunk
+  return 0;
+}
+
+// The decode loop's buffers and the row-tile kernels' operand maps: one row per sentence.
+int Pass::plan_step(Workspace& ws) {
+  const size_t BE = static_cast<size_t>(B) * E, SB = static_cast<size_t>(max_steps) * B;
+  ws.add(xd, BE), ws.add(hb, BE), ws.add(qd, BE), ws.add(zb, BE);
+  for (int l = 0; l < Ld; l++) ws.add(state[l], BE);
+  ws.add(xq[0], BE), ws.add(xq[1], BE), ws.add(zq[0], BE), ws.add(zq[1], BE), ws.add(caq, BE), ws.add(oq, BE);
+  ws.add(best, B), ws.add(done, B), ws.add(tgt_len, B), ws.add(counters, 64);
+  if (!a.device_io) {
+    ws.add(d_steps, SB);
+    if (a.forced) ws.add(d_forced, SB);
+  }
+  if (route.out == Out::Logits) ws.add(d_logits, static_cast<size_t>(B) * Nout);
+  if (a.scores && !a.device_io) ws.add(d_scores, SB);
+  if (a.scores || a.sample) ws.add(partials, (Nout + kScoreStrip - 1) / kScoreStrip * static_cast<size_t>(B));
+  if (a.sample && a.keys && !a.device_io) ws.add(d_keys, B);
+  // head-0 probabilities of every step stay on the device and come back in one copy after the loop
+  if (a.alignment) ws.add(d_align_all, SB * T);
+  if (!a.device_io && a.sentence_tokens) ws.add(d_rows, SB);
+  if (carve(ws)) return 1;
+  if (a.device_io) {
+    d_tokens = const_cast<uint32_t*>(a.tokens), d_lengths = const_cast<uint32_t*>(a.lengths), d_steps = a.step_tokens;
+    d_forced = const_cast<uint32_t*>(a.forced), d_sl = use_sl ? const_cast<uint32_t*>(a.shortlist) : nullptr;
+    d_scores = a.scores;
+    d_keys = const_cast<uint64_t*>(a.keys);
+  }
   for (int i = 0; i < 2; i++)
     if (c.make_map(&map_xq[i], xq[i], B, E, kRowTile) || c.make_map(&map_zq[i], zq[i], B, E, kRowTile)) return 1;
-  if (c.make_map(&map_caq, caq, B, E, kRowTile) || c.make_map(&map_oq, oq, B, E, kBM)) return 1;
-  return 0;
+  return c.make_map(&map_caq, caq, B, E, kRowTile) || c.make_map(&map_oq, oq, B, E, kBM);
+}
+
+// The scoring pass's buffers: one row per (sentence, target position); the layer input xd is rewritten in place by each
+// layer's FFN.  The output operand's maps are made per row chunk.
+int Pass::plan_score(Workspace& ws) {
+  Tt = static_cast<int>(a.target_T), M = B * Tt;
+  if (Tt > m.max_len()) {
+    set_error("target length " + std::to_string(Tt) + " exceeds the supported maximum of " + std::to_string(m.max_len()));
+    return 1;
+  }
+  const size_t ME = static_cast<size_t>(M) * E, rows = std::min(M, kScoreChunk);
+  ws.add(d_tgt, M);
+  ws.add(xd, ME), ws.add(Fb, ME), ws.add(Wx, ME), ws.add(hb, ME), ws.add(qd, ME);
+  ws.add(xq[0], ME), ws.add(xq[1], ME), ws.add(hq, ME), ws.add(caq, ME), ws.add(oq, ME);
+  ws.add(d_scores, M), ws.add(best, rows), ws.add(partials, (Nout + kScoreStrip - 1) / kScoreStrip * rows);
+  if (a.alignment) ws.add(d_align_all, ME / E * T);
+  return carve(ws) || c.make_map(&map_caq, caq, M, E, kRowTile);
+}
+
+// The u8 operands quantised from the input of encoder layer i: its q/k/v projections', or for i == Le every decoder
+// layer's cross K/V projections'.
+QuantOuts Pass::enc_inputs(int i) {
+  QuantOuts q = qouts();
+  if (i < Le) {
+    const AttnW& A = m.enc[i].self;
+    qadd(q, qa[0], A.q.aq), qadd(q, qa[1], A.k.aq), qadd(q, qa[2], A.v.aq);
+  } else {
+    for (int l = 0; l < Ld; l++) qadd(q, qa[2 * l], m.dec[l].ctx.k.aq), qadd(q, qa[2 * l + 1], m.dec[l].ctx.v.aq);
+  }
+  return q;
+}
+
+// Where decoder layer l's output goes: after the last layer only into the output operand (signed for the fused GEMMs,
+// u8 for the logits tap's generic GEMM); after an earlier layer into z and the next layer's SSRU operands xf and xw.
+void Pass::dec_layer_out(RowsFfnArgs& k, int l, float* z, int8_t* xf, int8_t* xw) const {
+  if (l + 1 == Ld) {
+    k.zq[0] = reinterpret_cast<uint8_t*>(oq), k.zaq[0] = m.out.aq, k.n_zq = 1;
+    k.zq_signed = route.out == Out::Logits ? 0 : 1;
+  } else {
+    k.z_out = z;
+    k.zq[0] = reinterpret_cast<uint8_t*>(xf), k.zaq[0] = m.dec[l + 1].rnn_wf.aq;
+    k.zq[1] = reinterpret_cast<uint8_t*>(xw), k.zaq[1] = m.dec[l + 1].rnn_w.aq;
+    k.n_zq = 2;
+  }
+}
+
+// score_step's arguments for `rows` output rows whose operands start at oq_rows; forced and scores are [step][rows].
+// The sampling fields, which only sample_step reads, are the decode step's to set.
+ScoreStepArgs Pass::score_step_args(int rows, const int8_t* oq_rows, const uint32_t* forced, int step,
+                                    float* scores) const {
+  ScoreStepArgs k{};
+  k.partials = partials, k.best = best, k.forced = forced, k.shortlist = use_sl ? d_sl : nullptr;
+  k.oq = oq_rows, k.w = out.w, k.c127 = out.c127, k.pb = out.pb, k.um = out.um;
+  k.logits = route.out == Out::Logits ? d_logits : nullptr;
+  k.B = rows, k.N = Nout, k.K = E, k.step = step, k.scores = scores;
+  return k;
 }
 
 int Pass::encode() {
@@ -903,10 +969,7 @@ int Pass::encode() {
   }
   // ---- embedding (Model.cc:195-197)
   {
-    QuantOuts q = qouts();
-    if (Le > 0) {
-      qadd(q, qa[0], m.enc[0].self.q.aq), qadd(q, qa[1], m.enc[0].self.k.aq), qadd(q, qa[2], m.enc[0].self.v.aq);
-    }
+    const QuantOuts q = Le > 0 ? enc_inputs(0) : qouts();
     LaunchScope ls(c, "enc_embed", 0, (1.0 + 4.0 + q.n) * R * E);
     launch_embed(d_tokens, m.emb_q, m.inv_qm, m.sqrt_e, m.pos, R, T, E, 1, 0, x0, q, s);
   }
@@ -959,30 +1022,12 @@ int Pass::encode() {
         return 1;
       }
     }
+    const QuantOuts next = enc_inputs(i + 1);
     if (route.ffn == EncFfn::Rows) {
-      RowsFfnArgs k{};
-      k.map_a = map_attn_q;
-      k.map_wo = L.self.o.map128, k.map_w1 = L.ffn.w1.map128, k.map_w2 = L.ffn.w2.map128;
-      k.pb_o = L.self.o.pb, k.pb_1 = L.ffn.w1.pb, k.pb_2 = L.ffn.w2.pb;
-      k.um_o = L.self.o.um, k.um_1 = L.ffn.w1.um, k.um_2 = L.ffn.w2.um;
-      k.aq_1 = L.ffn.w1.aq, k.aq_2 = L.ffn.w2.aq;
-      k.res = x0, k.y_park = x1, k.z_out = x0;
-      k.ln1_scale = L.self.ln.scale, k.ln1_bias = L.self.ln.bias;
-      k.ln2_scale = L.ffn.ln.scale, k.ln2_bias = L.ffn.ln.bias, k.eps = 1e-6f;
-      if (i + 1 < Le) {
-        const EncLayerW& Nx = m.enc[i + 1];
-        k.zq[0] = reinterpret_cast<uint8_t*>(qa[0]), k.zaq[0] = Nx.self.q.aq;
-        k.zq[1] = reinterpret_cast<uint8_t*>(qa[1]), k.zaq[1] = Nx.self.k.aq;
-        k.zq[2] = reinterpret_cast<uint8_t*>(qa[2]), k.zaq[2] = Nx.self.v.aq;
-        k.n_zq = 3;
-      } else {
-        for (int l = 0; l < Ld; l++) {
-          k.zq[2 * l] = reinterpret_cast<uint8_t*>(qa[2 * l]), k.zaq[2 * l] = m.dec[l].ctx.k.aq;
-          k.zq[2 * l + 1] = reinterpret_cast<uint8_t*>(qa[2 * l + 1]), k.zaq[2 * l + 1] = m.dec[l].ctx.v.aq;
-        }
-        k.n_zq = 2 * Ld;
-      }
-      k.M = R;
+      RowsFfnArgs k = rows_ffn_args(L.self, L.ffn, x0, R);
+      k.map_a = map_attn_q, k.y_park = x1, k.z_out = x0;
+      for (int j = 0; j < next.n; j++) k.zq[j] = reinterpret_cast<uint8_t*>(next.ptr[j]), k.zaq[j] = next.aq[j];
+      k.n_zq = next.n;
       const double Rd = R, Ed = E, Fd = F;
       LaunchScope ls(c, "enc_wo_ffn_fused", 2.0 * Rd * (Ed * Ed + 2.0 * Ed * Fd),
                      Ed * Ed + 2.0 * Ed * Fd + Rd * Ed * (1.0 + 4.0 + 4.0 + k.n_zq));  // u8 in, residual, f32 out, u8 copies
@@ -1016,18 +1061,12 @@ int Pass::encode() {
       if (!p) return 1;
       p->residual = x1, p->ln_scale = L.ffn.ln.scale, p->ln_bias = L.ffn.ln.bias;
       p->out = x0;
-      if (i + 1 < Le) {
-        const EncLayerW& Nx = m.enc[i + 1];
-        padd(p, qa[0], Nx.self.q.aq), padd(p, qa[1], Nx.self.k.aq), padd(p, qa[2], Nx.self.v.aq);
-      } else {
-        for (int l = 0; l < Ld; l++) padd(p, qa[2 * l], m.dec[l].ctx.k.aq), padd(p, qa[2 * l + 1], m.dec[l].ctx.v.aq);
-      }
+      for (int j = 0; j < next.n; j++) padd(p, next.ptr[j], next.aq[j]);
       if (g.launch()) return 1;
     }
   }
   if (Le == 0) {  // degenerate: quantize the embedding for the decoder's K/V projections
-    QuantOuts q = qouts();
-    for (int l = 0; l < Ld; l++) qadd(q, qa[2 * l], m.dec[l].ctx.k.aq), qadd(q, qa[2 * l + 1], m.dec[l].ctx.v.aq);
+    const QuantOuts q = enc_inputs(0);
     LaunchScope ls(c, "quantize", 0, (4.0 + q.n) * R * E);
     launch_quantize(x0, static_cast<size_t>(R) * E, q, s);
   }
@@ -1158,26 +1197,9 @@ int Pass::decode_step(int step) {
       }
     }
     {  // Wo + residual + LN, FFN1 + ReLU, FFN2 + residual + LN in one row-tile kernel (Modules.cc:308-316, 251-257)
-      RowsFfnArgs k{};
+      RowsFfnArgs k = rows_ffn_args(L.ctx, L.ffn, hb, B);
       k.map_a = map_caq;
-      k.map_wo = L.ctx.o.map128, k.map_w1 = L.ffn.w1.map128, k.map_w2 = L.ffn.w2.map128;
-      k.pb_o = L.ctx.o.pb, k.pb_1 = L.ffn.w1.pb, k.pb_2 = L.ffn.w2.pb;
-      k.um_o = L.ctx.o.um, k.um_1 = L.ffn.w1.um, k.um_2 = L.ffn.w2.um;
-      k.aq_1 = L.ffn.w1.aq, k.aq_2 = L.ffn.w2.aq;
-      k.res = hb;
-      k.ln1_scale = L.ctx.ln.scale, k.ln1_bias = L.ctx.ln.bias;
-      k.ln2_scale = L.ffn.ln.scale, k.ln2_bias = L.ffn.ln.bias, k.eps = 1e-6f;
-      if (last) {
-        k.z_out = nullptr;
-        k.zq[0] = reinterpret_cast<uint8_t*>(oq), k.zaq[0] = m.out.aq, k.n_zq = 1;
-        k.zq_signed = route.out == Out::Logits ? 0 : 1;  // the fused argmax GEMMs take the signed qa
-      } else {
-        k.z_out = zb;
-        k.zq[0] = reinterpret_cast<uint8_t*>(zq[0]), k.zaq[0] = m.dec[l + 1].rnn_wf.aq;
-        k.zq[1] = reinterpret_cast<uint8_t*>(zq[1]), k.zaq[1] = m.dec[l + 1].rnn_w.aq;
-        k.n_zq = 2;
-      }
-      k.M = B;
+      dec_layer_out(k, l, zb, zq[0], zq[1]);
       const double Bd = B, Ed = E, Fd = F;
       LaunchScope ls(c, "dec_wo_ffn_fused", 2.0 * Bd * (Ed * Ed + 2.0 * Ed * Fd),
                      Ed * Ed + 2.0 * Ed * Fd + Bd * Ed * (1.0 + 4.0 + (last ? 1.0 : 6.0)));
@@ -1221,11 +1243,7 @@ int Pass::decode_step(int step) {
     }
   }
   if (a.scores || a.sample) {
-    ScoreStepArgs k{};
-    k.partials = partials, k.best = best, k.forced = d_forced, k.shortlist = use_sl ? d_sl : nullptr;
-    k.oq = oq, k.w = out.w, k.c127 = out.c127, k.pb = out.pb, k.um = out.um;
-    k.logits = route.out == Out::Logits ? d_logits : nullptr;
-    k.B = B, k.N = Nout, k.K = E, k.step = step, k.scores = d_scores;
+    ScoreStepArgs k = score_step_args(B, oq, d_forced, step, d_scores);
     k.inv_t = a.inv_t, k.seed = a.seed, k.keys = d_keys;
     const double strips = (Nout + kScoreStrip - 1) / kScoreStrip;
     if (a.sample) {
@@ -1409,26 +1427,9 @@ int Pass::score() {
       }
     }
     {  // Wo + residual + LN, FFN: the step path's row-tile kernel over M rows
-      RowsFfnArgs k{};
+      RowsFfnArgs k = rows_ffn_args(L.ctx, L.ffn, hb, M);
       k.map_a = map_caq;
-      k.map_wo = L.ctx.o.map128, k.map_w1 = L.ffn.w1.map128, k.map_w2 = L.ffn.w2.map128;
-      k.pb_o = L.ctx.o.pb, k.pb_1 = L.ffn.w1.pb, k.pb_2 = L.ffn.w2.pb;
-      k.um_o = L.ctx.o.um, k.um_1 = L.ffn.w1.um, k.um_2 = L.ffn.w2.um;
-      k.aq_1 = L.ffn.w1.aq, k.aq_2 = L.ffn.w2.aq;
-      k.res = hb;
-      k.ln1_scale = L.ctx.ln.scale, k.ln1_bias = L.ctx.ln.bias;
-      k.ln2_scale = L.ffn.ln.scale, k.ln2_bias = L.ffn.ln.bias, k.eps = 1e-6f;
-      if (last) {
-        k.z_out = nullptr;
-        k.zq[0] = reinterpret_cast<uint8_t*>(oq), k.zaq[0] = m.out.aq, k.n_zq = 1;
-        k.zq_signed = 1;
-      } else {
-        k.z_out = xd;
-        k.zq[0] = reinterpret_cast<uint8_t*>(xq[0]), k.zaq[0] = m.dec[l + 1].rnn_wf.aq;
-        k.zq[1] = reinterpret_cast<uint8_t*>(xq[1]), k.zaq[1] = m.dec[l + 1].rnn_w.aq;
-        k.n_zq = 2;
-      }
-      k.M = M;
+      dec_layer_out(k, l, xd, xq[0], xq[1]);
       LaunchScope ls(c, "score_wo_ffn_fused", 2.0 * Md * (Ed * Ed + 2.0 * Ed * Fd),
                      Ed * Ed + 2.0 * Ed * Fd + Md * Ed * (1.0 + 4.0 + (last ? 1.0 : 6.0)));
       if (launch_rows_ffn(k, E, F, kRowTile, false, s)) {
@@ -1453,10 +1454,7 @@ int Pass::score() {
         return 1;
       }
     }
-    ScoreStepArgs k{};
-    k.partials = partials, k.best = best, k.forced = d_tgt + r0, k.shortlist = use_sl ? d_sl : nullptr;
-    k.oq = oq + static_cast<size_t>(r0) * E, k.w = out.w, k.c127 = out.c127, k.pb = out.pb, k.um = out.um;
-    k.B = rows, k.N = Nout, k.K = E, k.step = 0, k.scores = d_scores + r0, k.inv_t = 1.0f;
+    const ScoreStepArgs k = score_step_args(rows, oq + static_cast<size_t>(r0) * E, d_tgt + r0, 0, d_scores + r0);
     LaunchScope ls(c, "score_step", 0, 8.0 * rows * strips + 16.0 * rows + 2.0 * rows * E);
     if (launch_score_step(k, s)) {
       set_error("token scores: step kernel launch failed");
@@ -1478,38 +1476,36 @@ int Pass::score() {
   return 0;
 }
 
+// One call on context c (`name` prefixes its errors): an empty request does nothing; otherwise the encoder and the
+// output layer's set-up, then `decoder` (Pass::decode or Pass::score).
+int run_pass(Model& m, Context& c, ForwardArgs& a, const char* name, bool empty, int (Pass::*decoder)()) {
+  std::lock_guard<std::recursive_mutex> ctx_lock(c.mu);
+  if (c.device != m.ctx->device) {
+    set_error(std::string(name) + ": the lane context and the model live on different devices");
+    return 1;
+  }
+  SB_CUDA(cudaSetDevice(c.device));
+  if (empty) return 0;
+  Pass p{m, c, a, c.stream};
+  return p.plan() || p.encode() || p.prepare_cross() || p.prepare_output() || (p.*decoder)() ? 1 : 0;
+}
+
 }  // namespace
 
 int model_forward(Model& m, ForwardArgs& a) { return model_forward_on(m, *m.ctx, a); }
 
 int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
-  std::lock_guard<std::recursive_mutex> ctx_lock(c.mu);
-  if (c.device != m.ctx->device) {
-    set_error("model_forward: the lane context and the model live on different devices");
-    return 1;
-  }
-  SB_CUDA(cudaSetDevice(c.device));
   a.steps = 0;
   a.target_tokens = 0;
-  if (a.B == 0 || a.T == 0) return 0;
-  Pass p{m, c, a, c.stream};
-  return p.plan() || p.encode() || p.prepare_cross() || p.prepare_output() || p.decode() ? 1 : 0;
+  return run_pass(m, c, a, "model_forward", a.B == 0 || a.T == 0, &Pass::decode);
 }
 
 int model_score_on(Model& m, Context& c, ForwardArgs& a) {
-  std::lock_guard<std::recursive_mutex> ctx_lock(c.mu);
-  if (c.device != m.ctx->device) {
-    set_error("model_score: the lane context and the model live on different devices");
-    return 1;
-  }
   if (a.targets == nullptr || a.scores == nullptr || a.forced || a.sample || a.logits || a.device_io) {
     set_error("model_score: targets and scores on host buffers, and none of forced, sampling, logits or device_io");
     return 1;
   }
-  SB_CUDA(cudaSetDevice(c.device));
-  if (a.B == 0 || a.T == 0 || a.target_T == 0) return 0;
-  Pass p{m, c, a, c.stream};
-  return p.plan() || p.encode() || p.prepare_cross() || p.prepare_output() || p.score() ? 1 : 0;
+  return run_pass(m, c, a, "model_score", a.B == 0 || a.T == 0 || a.target_T == 0, &Pass::score);
 }
 
 }  // namespace sb

@@ -159,8 +159,7 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
               was_done = a.done[bk];
               len_before = a.tgt_len[bk];
               const uint32_t forced = a.forced ? a.forced[static_cast<size_t>(a.prev_step) * a.M + bk] : 0u;
-              const uint32_t idx = best_index(packed);
-              word = a.shortlist ? a.shortlist[idx] : idx;
+              word = best_word(packed, a.shortlist);
               tok = a.forced ? forced : word;
             }
             s_tok[et] = tok;
@@ -180,8 +179,7 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
 #pragma unroll
             for (int r = 0; r < 8; r++) {
               const int row = rq * 8 + r;
-              const float w = static_cast<float>(a.emb_q[static_cast<size_t>(s_tok[row]) * E + f]);
-              const float y = __fadd_rn(__fmul_rn(__fmul_rn(w, a.inv_qm), a.sqrt_e), ps);
+              const float y = embed1(a.emb_q[static_cast<size_t>(s_tok[row]) * E + f], a.inv_qm, a.sqrt_e, ps);
               xv[mb][r] = y;
               const uint32_t off = static_cast<uint32_t>(mb * kOpK + row * 128) + xo[r];  // row & 7 == r: rq * 8 is a multiple of 8
               opnd_xf[off] = static_cast<uint8_t>(quantize1(y, a.aq_xf));
@@ -191,17 +189,9 @@ __global__ void __launch_bounds__(kThreads, 1) dec_ssru_kernel(const __grid_cons
           fence_proxy_async();
           __syncwarp();
           if (lane == 0) mbar_arrive(x_full);
-          if (et < kR && bk < a.M) {  // record(): append unless already finished; re-arm the packed best
-            a.step_tokens[static_cast<size_t>(a.prev_step) * a.M + bk] = word;
-            if (!was_done) {
-              a.tgt_len[bk] = len_before + 1;
-              if (word == a.eos_id) {
-                a.done[bk] = 1;
-                atomicAdd(a.n_done, 1);
-              }
-            }
-            a.best[bk] = 0ull;
-          }
+          if (et < kR && bk < a.M)
+            record_word(word, was_done, len_before, a.eos_id, a.prev_step, a.M, bk, a.step_tokens, a.done, a.tgt_len,
+                        a.n_done, a.best);
         }
 #pragma unroll
         for (int mb = 0; mb < EM; mb++) {

@@ -31,22 +31,15 @@ __global__ void embed_kernel(const uint32_t* __restrict__ tokens, const int8_t* 
   if (gid >= static_cast<size_t>(rows) * per_row) return;
   const int r = static_cast<int>(gid / per_row);
   const int e = static_cast<int>(gid % per_row) * 4;
-  float w[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+  char4 c = make_char4(0, 0, 0, 0);
   if (!zero_embed && !(shift && r % T == 0)) {
     const uint32_t tok = tokens[shift ? r - 1 : r];
-    const char4 c = *reinterpret_cast<const char4*>(emb_q + static_cast<size_t>(tok) * E + e);
-    w[0] = __fmul_rn(static_cast<float>(c.x), inv_qm);
-    w[1] = __fmul_rn(static_cast<float>(c.y), inv_qm);
-    w[2] = __fmul_rn(static_cast<float>(c.z), inv_qm);
-    w[3] = __fmul_rn(static_cast<float>(c.w), inv_qm);
+    c = *reinterpret_cast<const char4*>(emb_q + static_cast<size_t>(tok) * E + e);
   }
   const int p = pos_from_row ? (r % T) : 0;
   const float4 ps = *reinterpret_cast<const float4*>(pos + static_cast<size_t>(p) * E + e);
-  float y[4];
-  y[0] = __fadd_rn(__fmul_rn(w[0], sqrt_e), ps.x);
-  y[1] = __fadd_rn(__fmul_rn(w[1], sqrt_e), ps.y);
-  y[2] = __fadd_rn(__fmul_rn(w[2], sqrt_e), ps.z);
-  y[3] = __fadd_rn(__fmul_rn(w[3], sqrt_e), ps.w);
+  const float y[4] = {embed1(c.x, inv_qm, sqrt_e, ps.x), embed1(c.y, inv_qm, sqrt_e, ps.y),
+                      embed1(c.z, inv_qm, sqrt_e, ps.z), embed1(c.w, inv_qm, sqrt_e, ps.w)};
   const size_t off = static_cast<size_t>(r) * E + e;
   if (x) *reinterpret_cast<float4*>(x + off) = make_float4(y[0], y[1], y[2], y[3]);
   store_quant4(q, off, y);
@@ -180,29 +173,16 @@ __global__ void __launch_bounds__(256) finalize_step_kernel(
   if (b >= B) return;
   uint32_t tok = 0;
   if (lane == 0) {
-    const unsigned long long packed = best[b];
-    const uint32_t idx = best_index(packed);
-    const uint32_t word = shortlist ? shortlist[idx] : idx;
-    step_tokens[static_cast<size_t>(step) * B + b] = word;
-    if (!done[b]) {  // record(), slimt/Model.cc:127-137: append unless already finished
-      tgt_len[b] += 1;
-      if (word == eos_id) {
-        done[b] = 1;
-        atomicAdd(n_done, 1);
-      }
-    }
-    best[b] = 0ull;
+    const uint32_t word = best_word(best[b], shortlist);
+    record_word(word, done[b], tgt_len[b], eos_id, step, B, b, step_tokens, done, tgt_len, n_done, best);
     tok = forced ? forced[static_cast<size_t>(step) * B + b] : word;
   }
   tok = __shfl_sync(0xffffffffu, tok, 0);
   for (int e = lane * 4; e < E; e += 128) {
     const char4 c = *reinterpret_cast<const char4*>(emb_q + static_cast<size_t>(tok) * E + e);
     const float4 ps = *reinterpret_cast<const float4*>(pos0 + e);
-    float y[4];
-    y[0] = __fadd_rn(__fmul_rn(__fmul_rn(static_cast<float>(c.x), inv_qm), sqrt_e), ps.x);
-    y[1] = __fadd_rn(__fmul_rn(__fmul_rn(static_cast<float>(c.y), inv_qm), sqrt_e), ps.y);
-    y[2] = __fadd_rn(__fmul_rn(__fmul_rn(static_cast<float>(c.z), inv_qm), sqrt_e), ps.z);
-    y[3] = __fadd_rn(__fmul_rn(__fmul_rn(static_cast<float>(c.w), inv_qm), sqrt_e), ps.w);
+    const float y[4] = {embed1(c.x, inv_qm, sqrt_e, ps.x), embed1(c.y, inv_qm, sqrt_e, ps.y),
+                        embed1(c.z, inv_qm, sqrt_e, ps.z), embed1(c.w, inv_qm, sqrt_e, ps.w)};
     const size_t off = static_cast<size_t>(b) * E + e;
     *reinterpret_cast<float4*>(x + off) = make_float4(y[0], y[1], y[2], y[3]);
     store_quant4(q, off, y);

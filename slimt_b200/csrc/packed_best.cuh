@@ -39,4 +39,28 @@ __device__ __forceinline__ int best_proxy(unsigned long long packed) {
   return static_cast<int>(static_cast<uint32_t>(packed >> 32) ^ 0x80000000u);
 }
 
+// The vocabulary word of a packed candidate: its column, through the shortlist when one is given.
+__device__ __forceinline__ uint32_t best_word(unsigned long long packed, const uint32_t* shortlist) {
+  const uint32_t idx = best_index(packed);
+  return shortlist ? shortlist[idx] : idx;
+}
+
+// record() (slimt/Model.cc:127-137) of row b's word at one step, then re-arm the row's packed best.  The word is
+// written to step_tokens; a row not yet finished grows by one and finishes at EOS.  was_done and len_before are
+// done[b] and tgt_len[b] as the caller loaded them: this helper loads nothing, so a caller can issue those loads early
+// and run the record off its critical path.
+__device__ __forceinline__ void record_word(uint32_t word, uint32_t was_done, uint32_t len_before, uint32_t eos_id,
+                                            int step, int B, int b, uint32_t* step_tokens, uint8_t* done,
+                                            uint32_t* tgt_len, int* n_done, unsigned long long* best) {
+  step_tokens[static_cast<size_t>(step) * B + b] = word;
+  if (!was_done) {
+    tgt_len[b] = len_before + 1;
+    if (word == eos_id) {
+      done[b] = 1;
+      atomicAdd(n_done, 1);
+    }
+  }
+  best[b] = 0ull;
+}
+
 }  // namespace sb

@@ -259,6 +259,47 @@ typedef struct slimt_b200_score_io {
 /* Scores io's targets with one or more replicas of one model (as slimt_b200_translate_multi serves a request). */
 int slimt_b200_score(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_score_io* io);
 
+/* ---- beam search: K hypotheses per sentence instead of one (marian's --beam-size, --n-best, --normalize) ----
+ * The batches are slimt_b200_translate's (the Batcher over the source lengths), so the shortlist unions and the step
+ * limit max_steps = max(1, (size_t)(limit_factor * width)) are greedy's.  Sentence b's slots are its decoder rows
+ * b * K + k; it starts with one live slot (slot 0) holding the empty hypothesis with cumulative score cum = 0, and a
+ * width w = K of hypotheses still to finish.  At step s, for each live slot with exact logits y over the output columns:
+ *  - its candidates are its first K columns ordered by (y descending, column ascending) -- for K = 1 the greedy choice;
+ *  - a candidate's token score is sc = (float)((double)y[c] - LSE(y)), LSE formed exactly as token_scores forms it,
+ *    and its total t = fl32(cum + sc);
+ *  - the sentence takes the first w candidates over its live slots, ordered by (t descending, slot ascending,
+ *    candidate rank ascending).  A chosen candidate whose word (through the shortlist) is EOS becomes a finished
+ *    hypothesis, EOS included; the others become the live slots 0, 1, ... in the order they were chosen, and w drops
+ *    by the number of EOS choices (marian's shrinking beam).  At step max_steps - 1 every chosen candidate finishes as
+ *    it stands.  A sentence is done when w reaches 0; decoding stops when every sentence is done.
+ * Every sentence so ends with exactly K finished hypotheses.  Each is ranked by normalized = (double)total /
+ * pow(len, length_penalty), len counting EOS; ties go to the earlier finishing step, then the earlier choice.  total
+ * is the float sum of the token scores in order.  So K = 1 is greedy decoding, bit for bit (tokens, scores,
+ * alignments), and slimt_b200_score of a returned hypothesis reproduces its token scores bit for bit.
+ * Arithmetic: beam search always runs the bit-exact arithmetic, whatever slimt_b200_ctx_set_math says.
+ * Errors, each reported before any GPU work (the model stays usable): beam_size outside 1..8, nbest outside
+ * 1..beam_size, a length penalty that is negative or not finite, an n-best capacity below n_sentences * nbest *
+ * max_steps of the sentence's batch.
+ * Device workspace: greedy's with K rows per sentence, plus 12 * K bytes per sentence and step of step records (and
+ * 4 * K * source width per sentence and step with alignments). */
+typedef struct slimt_b200_beam {
+  int32_t beam_size;          /* K, 1..8 */
+  int32_t nbest;              /* 1..K hypotheses per sentence in the n-best outputs */
+  float length_penalty;       /* alpha: finite, >= 0 */
+  /* optional (NULL = not wanted): hypothesis h of sentence i is entry i * nbest + h, best first */
+  uint32_t* nbest_tokens;     /* ragged by nbest_offsets, EOS included */
+  float* nbest_token_scores;  /* ragged like nbest_tokens */
+  size_t nbest_capacity;      /* tokens */
+  uint64_t* nbest_offsets;    /* [n_sentences * nbest + 1] */
+  float* nbest_totals;        /* [n_sentences * nbest] */
+  double* nbest_normalized;   /* [n_sentences * nbest] */
+  uint64_t steps;             /* out: decoder steps executed, summed over the batches */
+} slimt_b200_beam;
+/* Beam search over a request: io's out_tokens, out_scores and out_alignments receive each sentence's best hypothesis
+ * (as slimt_b200_translate_multi returns the greedy one), beam's n-best outputs the first nbest hypotheses. */
+int slimt_b200_translate_beam(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_translate_io* io,
+                              slimt_b200_beam* beam);
+
 /* Host-only pieces of the same path, callable without a GPU (used by the CPU test-suite):
  * ShortlistGenerator::generate (Shortlist.cc:115-175) and Batcher::generate (Batcher.cc:95-120). */
 int slimt_b200_shortlist_generate(const void* shortlist_bin, size_t shortlist_bytes, const uint32_t* words,

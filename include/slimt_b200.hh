@@ -768,12 +768,14 @@ class Blocking {
   }
 
   // cache prefill (Request.cc:58-78): a segment this model has translated before is not batched again.  A record
-  // stored by a request that did not ask for alignments (or scores) cannot answer one that does.  A sampled segment is
-  // neither looked up nor stored: the cache holds greedy translations.  The rest: run().
+  // stored by a request that did not ask for alignments (or scores) cannot answer one that does.  A sampled or beam
+  // segment is neither looked up nor stored: the cache holds greedy translations.  The rest: run().
   Histories serve(const Ptr<Model> &model, const Sentences &segments, const Options &options) {
+    if (options.sample && options.beam_size > 1)
+      throw std::invalid_argument("Options: sample and beam_size > 1 exclude each other");
     Histories histories(segments.size());
     std::vector<size_t> todo;
-    const bool cached = cache_ && !options.sample;
+    const bool cached = cache_ && !options.sample && options.beam_size == 1;
     for (size_t i = 0; i < segments.size(); i++) {
       if (cached) {
         auto [found, history] = cache_->find(cache_key(model->id(), segments[i]));
@@ -833,8 +835,15 @@ class Blocking {
       sampling.keys = keys.data();
     }
     const std::vector<slimt_b200_model *> &replicas = model->replicas();
-    detail::check(slimt_b200_translate_sampled(replicas.data(), replicas.size(), &io, options.sample ? &sampling : nullptr),
-                  "slimt_b200_translate_sampled");
+    if (options.beam_size > 1) {
+      slimt_b200_beam beam;
+      std::memset(&beam, 0, sizeof(beam));
+      beam.beam_size = options.beam_size, beam.nbest = 1, beam.length_penalty = options.length_penalty;
+      detail::check(slimt_b200_translate_beam(replicas.data(), replicas.size(), &io, &beam), "slimt_b200_translate_beam");
+    } else {
+      detail::check(slimt_b200_translate_sampled(replicas.data(), replicas.size(), &io, options.sample ? &sampling : nullptr),
+                    "slimt_b200_translate_sampled");
+    }
     for (size_t k = 0; k < todo.size(); k++) {
       auto h = std::make_shared<Hypothesis>();
       h->target.assign(out.begin() + out_offsets[k], out.begin() + out_offsets[k + 1]);
@@ -957,7 +966,8 @@ class Async {
   static bool poolable(const Job &a, const Job &b) {
     return !a.second && !b.second && a.first == b.first && a.is_text == b.is_text && a.options.alignment == b.options.alignment &&
            a.options.html == b.options.html && a.options.scores == b.options.scores && a.options.sample == b.options.sample &&
-           (!a.options.sample || (a.options.temperature == b.options.temperature && a.options.seed == b.options.seed));
+           (!a.options.sample || (a.options.temperature == b.options.temperature && a.options.seed == b.options.seed)) &&
+           a.options.beam_size == b.options.beam_size && a.options.length_penalty == b.options.length_penalty;
   }
   void work() {
     Config one = config_;

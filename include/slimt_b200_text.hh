@@ -1311,6 +1311,12 @@ struct Options {
   bool sample = false;
   float temperature = 1.0f;  // finite, in [1e-3, 1e3]
   uint64_t seed = 0;
+  // Beam search with beam_size hypotheses per segment (marian's --beam-size / --normalize; slimt_b200_translate_beam):
+  // the best hypothesis by total / len^length_penalty is returned, its scores and alignments with it.  beam_size = 1 is
+  // the greedy call; beam_size > 1 together with sample is std::invalid_argument.  Beam segments bypass the translation
+  // cache.
+  int beam_size = 1;  // 1 .. 8
+  float length_penalty = 0.0f;  // finite, >= 0
 };
 
 struct Response {

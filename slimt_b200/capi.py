@@ -27,7 +27,7 @@ EXPORTS = [
     "slimt_b200_shortlist_generate", "slimt_b200_batcher_plan", "slimt_b200_profile_enable", "slimt_b200_profile_read",
     "slimt_b200_translate_multi", "slimt_b200_shortlist_check", "slimt_b200_ctx_set_math", "slimt_b200_ctx_get_math",
     "slimt_b200_model_set_max_length", "slimt_b200_model_max_length", "slimt_b200_model_forward_sampled",
-    "slimt_b200_translate_sampled", "slimt_b200_score",
+    "slimt_b200_translate_sampled", "slimt_b200_score", "slimt_b200_translate_beam",
 ]
 
 
@@ -67,6 +67,13 @@ class ScoreIO(C.Structure):
 
 class Sampling(C.Structure):
     _fields_ = [("temperature", C.c_float), ("seed", C.c_uint64), ("keys", C.c_void_p)]
+
+
+class Beam(C.Structure):
+    _fields_ = [("beam_size", C.c_int32), ("nbest", C.c_int32), ("length_penalty", C.c_float),
+                ("nbest_tokens", C.c_void_p), ("nbest_token_scores", C.c_void_p), ("nbest_capacity", C.c_size_t),
+                ("nbest_offsets", C.c_void_p), ("nbest_totals", C.c_void_p), ("nbest_normalized", C.c_void_p),
+                ("steps", C.c_uint64)]
 
 
 class KernelStat(C.Structure):
@@ -117,6 +124,7 @@ def lib() -> C.CDLL:
         L.slimt_b200_translate_sampled.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.POINTER(TranslateIO),
                                                    C.POINTER(Sampling)]
         L.slimt_b200_score.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.POINTER(ScoreIO)]
+        L.slimt_b200_translate_beam.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.POINTER(TranslateIO), C.POINTER(Beam)]
         L.slimt_b200_shortlist_check.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t]
         L.slimt_b200_shortlist_generate.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p,
                                                     C.c_size_t, C.POINTER(C.c_size_t)]
@@ -450,6 +458,67 @@ class Model:
             stats["alignments"] = [al[int(ao[i]):int(ao[i + 1])].reshape(len(targets[i]), len(sources[i])).copy()
                                    for i in range(len(targets))]
         return outs, stats
+
+    def translate_beam(self, sentences, max_words: int, beam_size: int, nbest: int = 1, length_penalty: float = 0.0,
+                       limit_factor: float = 1.5, shortlist_bin: Optional[bytes] = None, replicas=None,
+                       want_alignments: bool = False, shortlist_check: bool = False, shortlist_shared: bool = False,
+                       nbest_capacity: Optional[int] = None):
+        """slimt_b200_translate_beam over one request (sentences: lists of word ids).  Returns (nbest, stats):
+        nbest[i] is sentence i's list of its first `nbest` hypotheses, best first, each a dict(tokens, scores, total,
+        normalized).  stats holds the best hypotheses as translate returns them ("tokens", "scores", and "alignments"
+        when want_alignments), "steps" (decoder steps executed over all batches) and the call's counters."""
+        n = len(sentences)
+        offsets = np.zeros(n + 1, dtype=np.uint64)
+        offsets[1:] = np.cumsum([len(s) for s in sentences])
+        tokens = np.concatenate([np.asarray(s, dtype=np.uint32) for s in sentences]) if n else np.zeros(0, np.uint32)
+        lens = np.diff(offsets.astype(np.int64))
+        per = max(1, int(np.float32(limit_factor) * np.float32(int(lens.max()) if n else 0)))
+        out_tokens = np.zeros(max(1, n * per), dtype=np.uint32)
+        out_scores = np.zeros(len(out_tokens), dtype=np.float32)
+        out_offsets = np.zeros(n + 1, dtype=np.uint64)
+        align = align_offs = None
+        if want_alignments:
+            align = np.zeros(max(1, per * int(lens.sum())), dtype=np.float32)
+            align_offs = np.zeros(n + 1, dtype=np.uint64)
+        cap = n * max(1, nbest) * per if nbest_capacity is None else nbest_capacity
+        nb_tokens = np.zeros(max(1, cap), dtype=np.uint32)
+        nb_scores = np.zeros(max(1, cap), dtype=np.float32)
+        nb_offsets = np.zeros(n * max(1, nbest) + 1, dtype=np.uint64)
+        nb_totals = np.zeros(max(1, n * nbest), dtype=np.float32)
+        nb_norm = np.zeros(max(1, n * nbest), dtype=np.float64)
+        slbuf = None
+        if shortlist_bin is not None:
+            slbuf = shortlist_bin if isinstance(shortlist_bin, C.Array) else (C.c_char * len(shortlist_bin)).from_buffer_copy(shortlist_bin)
+        io = TranslateIO(_ptr(tokens), _ptr(offsets), n, max_words, limit_factor,
+                         C.cast(slbuf, C.c_void_p) if slbuf is not None else None,
+                         0 if slbuf is None else len(slbuf), int(shortlist_check), int(shortlist_shared),
+                         _ptr(out_tokens), len(out_tokens), _ptr(out_offsets),
+                         _ptr(align), 0 if align is None else len(align), _ptr(align_offs), 0, 0, 0.0, 0, 0, 0,
+                         _ptr(out_scores))
+        bm = Beam(int(beam_size), int(nbest), float(length_penalty), _ptr(nb_tokens), _ptr(nb_scores), cap,
+                  _ptr(nb_offsets), _ptr(nb_totals), _ptr(nb_norm), 0)
+        reps = replicas or [self]
+        hs = (C.c_void_p * len(reps))(*[r.h for r in reps])
+        _check(lib().slimt_b200_translate_beam(hs, len(hs), C.byref(io), C.byref(bm)), "slimt_b200_translate_beam")
+        out = []
+        for i in range(n):
+            hyps = []
+            for h in range(nbest):
+                e = i * nbest + h
+                a, b = int(nb_offsets[e]), int(nb_offsets[e + 1])
+                hyps.append({"tokens": nb_tokens[a:b].copy(), "scores": nb_scores[a:b].copy(),
+                             "total": np.float32(nb_totals[e]), "normalized": float(nb_norm[e])})
+            out.append(hyps)
+        stats = {"target_tokens": int(io.target_tokens), "batches": int(io.batches), "device_ms": io.device_ms,
+                 "kernel_launches": int(io.kernel_launches), "h2d_bytes": int(io.h2d_bytes),
+                 "d2h_bytes": int(io.d2h_bytes), "steps": int(bm.steps),
+                 "tokens": [out_tokens[int(out_offsets[i]):int(out_offsets[i + 1])].copy() for i in range(n)],
+                 "scores": [out_scores[int(out_offsets[i]):int(out_offsets[i + 1])].copy() for i in range(n)],
+                 "out_offsets": out_offsets}
+        if want_alignments:
+            stats["alignments"] = [align[int(align_offs[i]):int(align_offs[i + 1])].reshape(
+                int(out_offsets[i + 1] - out_offsets[i]), len(sentences[i])).copy() for i in range(n)]
+        return out, stats
 
     def translate(self, sentences, max_words: int, limit_factor: float = 1.5, shortlist_bin: Optional[bytes] = None,
                   replicas=None, want_alignments: bool = False, want_scores: bool = False,

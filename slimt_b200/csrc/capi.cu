@@ -214,6 +214,17 @@ int slimt_b200_translate_sampled(slimt_b200_model* const* replicas, size_t n_rep
   return sb::translate_multi(ms.data(), n_replicas, io, sampling);
 }
 
+int slimt_b200_translate_beam(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_translate_io* io,
+                              slimt_b200_beam* beam) {
+  if (beam == nullptr) {
+    sb::set_error("translate_beam: beam is NULL");
+    return 1;
+  }
+  std::vector<sb::Model*> ms(n_replicas);
+  for (size_t i = 0; i < n_replicas; i++) ms[i] = replicas && replicas[i] ? &replicas[i]->m : nullptr;
+  return sb::translate_multi(ms.data(), n_replicas, io, nullptr, beam);
+}
+
 int slimt_b200_score(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_score_io* io) {
   if (io == nullptr) {
     sb::set_error("score: io is NULL");

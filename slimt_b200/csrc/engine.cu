@@ -757,9 +757,10 @@ struct Pass {
   int B, T, R, E, F, H, dh, Le, Ld, max_steps, Nout;  // Nout: with a lazy shortlist the vocabulary until its callback
   double src_tokens;
   bool lazy_sl, use_sl;
-  // scoring pass (a.targets set): Tt target positions per sentence, M = B * Tt decoder rows, always bit-exact arithmetic
+  // scoring pass (a.targets set): Tt target positions per sentence, M = B * Tt decoder rows, always bit-exact arithmetic.
+  // Decode loop: M = B * K decoder rows, K = a.beam for beam search (bit-exact arithmetic too), else 1.
   bool scoring, fast;
-  int Tt, M;
+  int Tt, M, K;
   Routes route;
   // batch inputs and outputs: workspace copies with host buffers, the caller's buffers with device_io
   uint32_t *d_tokens, *d_lengths, *d_steps, *d_forced, *d_sl, *d_rows, *tgt_len;
@@ -769,6 +770,14 @@ struct Pass {
   int8_t *qa[4], *attn_q, *ffn_q;
   // decoder state (Model.cc:111-185); counters: [0] n_done, [1] step counter, [2] ticket
   float *xd, *hb, *qd, *zb, *state[2], *d_logits, *d_align_all;  // zb: the first of two decoder layers' output
+  // beam search: the other half of each layer's state ping-pong, the step's candidates, the slots' cumulative scores,
+  // each sentence's width, the step records and the finished hypotheses (kernels.cuh)
+  float* state_nx[2];
+  BeamCand* cand;
+  float* cum;
+  uint8_t* width;
+  BeamRec* d_rec;
+  BeamFin* d_fin;
   // scoring pass: the targets, the SSRU's two projections of all rows, h's u8 copy (Wq's operand)
   uint32_t* d_tgt;
   float *Fb, *Wx;
@@ -785,7 +794,8 @@ struct Pass {
   CUtensorMap map_xq[2], map_zq[2], map_caq;  // u8 activation operands of the row-tile kernels, box {128 B, 32 rows}
   CUtensorMap map_oq;
   int plan(), plan_step(Workspace& ws), plan_score(Workspace& ws), carve(const Workspace& ws);
-  int encode(), prepare_cross(), prepare_output(), decode_step(int step), decode(), score();
+  int encode(), prepare_cross(), prepare_output(), decode_step(int step), decode(), score(), beam_search();
+  int poll_done(int step, bool* all_done);
   QuantOuts enc_inputs(int i);
   void dec_layer_out(RowsFfnArgs& k, int l, float* z, int8_t* xf, int8_t* xw) const;
   ScoreStepArgs score_step_args(int rows, const int8_t* oq_rows, const uint32_t* forced, int step, float* scores) const;
@@ -829,10 +839,11 @@ int Pass::plan() {
     return 1;
   }
   scoring = a.targets != nullptr;
-  fast = c.fast && !scoring;
+  K = a.beam > 0 ? a.beam : 1;
+  fast = c.fast && !scoring && a.beam == 0;
   route = choose_routes(m, T, B, fast, a.logits != nullptr, a.scores != nullptr || a.sample);
-  if (scoring) {
-    // T_target queries read each layer's cross K/V: projected once (Cached); every logit evaluated exactly (Scores)
+  if (scoring || a.beam > 0) {
+    // T_target (or K) queries read each layer's cross K/V: projected once (Cached); every logit evaluated exactly (Scores)
     route.cross = Cross::Cached;
     route.out = Out::Scores;
   }
@@ -875,14 +886,21 @@ int Pass::carve(const Workspace& ws) {
   return 0;
 }
 
-// The decode loop's buffers and the row-tile kernels' operand maps: one row per sentence.
+// The decode loop's buffers and the row-tile kernels' operand maps: one row per sentence, or K with beam search.
 int Pass::plan_step(Workspace& ws) {
-  const size_t BE = static_cast<size_t>(B) * E, SB = static_cast<size_t>(max_steps) * B;
+  M = B * K;
+  const size_t BE = static_cast<size_t>(M) * E, SB = static_cast<size_t>(max_steps) * B;
   ws.add(xd, BE), ws.add(hb, BE), ws.add(qd, BE), ws.add(zb, BE);
   for (int l = 0; l < Ld; l++) ws.add(state[l], BE);
   ws.add(xq[0], BE), ws.add(xq[1], BE), ws.add(zq[0], BE), ws.add(zq[1], BE), ws.add(caq, BE), ws.add(oq, BE);
-  ws.add(best, B), ws.add(done, B), ws.add(tgt_len, B), ws.add(counters, 64);
-  if (!a.device_io) {
+  ws.add(best, M), ws.add(done, B), ws.add(tgt_len, B), ws.add(counters, 64);
+  if (a.beam > 0) {
+    for (int l = 0; l < Ld; l++) ws.add(state_nx[l], BE);
+    ws.add(cand, static_cast<size_t>(M) * K), ws.add(cum, M), ws.add(width, B);
+    ws.add(d_rec, static_cast<size_t>(max_steps) * M), ws.add(d_fin, M);
+    ws.add(partials, (Nout + kScoreStrip - 1) / kScoreStrip * static_cast<size_t>(M));
+  }
+  if (!a.device_io && a.beam == 0) {
     ws.add(d_steps, SB);
     if (a.forced) ws.add(d_forced, SB);
   }
@@ -891,7 +909,7 @@ int Pass::plan_step(Workspace& ws) {
   if (a.scores || a.sample) ws.add(partials, (Nout + kScoreStrip - 1) / kScoreStrip * static_cast<size_t>(B));
   if (a.sample && a.keys && !a.device_io) ws.add(d_keys, B);
   // head-0 probabilities of every step stay on the device and come back in one copy after the loop
-  if (a.alignment) ws.add(d_align_all, SB * T);
+  if (a.alignment) ws.add(d_align_all, SB * K * T);
   if (!a.device_io && a.sentence_tokens) ws.add(d_rows, SB);
   if (carve(ws)) return 1;
   if (a.device_io) {
@@ -901,8 +919,8 @@ int Pass::plan_step(Workspace& ws) {
     d_keys = const_cast<uint64_t*>(a.keys);
   }
   for (int i = 0; i < 2; i++)
-    if (c.make_map(&map_xq[i], xq[i], B, E, kRowTile) || c.make_map(&map_zq[i], zq[i], B, E, kRowTile)) return 1;
-  return c.make_map(&map_caq, caq, B, E, kRowTile) || c.make_map(&map_oq, oq, B, E, kBM);
+    if (c.make_map(&map_xq[i], xq[i], M, E, kRowTile) || c.make_map(&map_zq[i], zq[i], M, E, kRowTile)) return 1;
+  return c.make_map(&map_caq, caq, M, E, kRowTile) || c.make_map(&map_oq, oq, M, E, kBM);
 }
 
 // The scoring pass's buffers: one row per (sentence, target position); the layer input xd is rewritten in place by each
@@ -1135,9 +1153,11 @@ int Pass::prepare_output() {
   return 0;
 }
 
-// One decoder step: the decoder layers and the output projection with the greedy choice.
+// One decoder step over the M decoder rows: the decoder layers and the output projection with the greedy choice, or
+// with beam search the candidates of every live slot and each sentence's merge.
 int Pass::decode_step(int step) {
-  float* d_align = d_align_all ? d_align_all + static_cast<size_t>(step) * B * T : nullptr;
+  const bool beam = a.beam > 0;
+  float* d_align = d_align_all ? d_align_all + static_cast<size_t>(step) * M * T : nullptr;
   for (int l = 0; l < Ld; l++) {
     const DecLayerW& L = m.dec[l];
     const bool last = (l + 1 == Ld);
@@ -1150,7 +1170,7 @@ int Pass::decode_step(int step) {
       k.um_f = L.rnn_wf.um, k.um_w = L.rnn_w.um, k.um_q = L.ctx.q.um;
       k.aq_q = L.ctx.q.aq;
       k.x = l == 0 ? xd : zb, k.state = state[l];
-      if (l == 0 && step > 0) {  // close the previous step and embed its words in this kernel's front
+      if (l == 0 && step > 0 && !beam) {  // close the previous step and embed its words in this kernel's front
         k.embed = 1, k.prev_step = step - 1;
         k.best = best, k.shortlist = d_sl, k.forced = d_forced, k.step_tokens = d_steps;
         k.done = done, k.tgt_len = tgt_len, k.n_done = counters, k.eos_id = m.eos_id;
@@ -1158,15 +1178,30 @@ int Pass::decode_step(int step) {
         k.aq_xf = L.rnn_wf.aq, k.aq_xw = L.rnn_w.aq;
       }
       k.ln_scale = L.rnn_ln.scale, k.ln_bias = L.rnn_ln.bias, k.eps = 1e-6f;
-      k.h_out = hb, k.q_out = qd, k.M = B;
-      const double Bd = B, Ed = E;
+      k.h_out = hb, k.q_out = qd, k.M = M;
+      const double Bd = M, Ed = E;
       LaunchScope ls(c, "dec_ssru_q_fused", 2.0 * Bd * 3.0 * Ed * Ed, 3.0 * Ed * Ed + Bd * Ed * (2.0 + 4.0 * 5.0));
       if (launch_dec_ssru(k, E, fast, s)) {
         set_error("fused SSRU kernel: unsupported embedding size " + std::to_string(E));
         return 1;
       }
     }
-    if (route.cross != Cross::Cached) {
+    if (beam) {  // K queries per sentence against its cached K/V, as the scoring pass runs them
+      QuantOuts q = qouts();
+      qadd(q, caq, L.ctx.o.aq);
+      float* al = last ? d_align : nullptr;
+      const double Md = M, Ed = E;
+      LaunchScope ls(c, "beam_cross_attention", 4.0 * Md * (src_tokens / B) * Ed,
+                     Md * Ed * 5.0 + 2.0 * src_tokens * Ed * 4.0 + (al ? 4.0 * Md * T : 0.0));
+      const int rc = self_attention_tiled_supported(T, dh)
+                         ? launch_self_attention_tiled(qd, Kc[l], Vc[l], d_lengths, B, T, H, dh, q, s, K, al)
+                         : launch_self_attention_long(qd, Kc[l], Vc[l], d_lengths, B, T, H, dh, q, s, K, al);
+      if (rc) {
+        set_error("beam cross-attention: no kernel for head size " + std::to_string(dh) + " over " + std::to_string(T) +
+                  " source tokens");
+        return 1;
+      }
+    } else if (route.cross != Cross::Cached) {
       CrossRcArgs k{};
       k.map_ak = mapK[l], k.map_av = mapV[l];
       k.map_wk = L.ctx.k.map128, k.map_wv = L.ctx.v.map128;
@@ -1197,10 +1232,10 @@ int Pass::decode_step(int step) {
       }
     }
     {  // Wo + residual + LN, FFN1 + ReLU, FFN2 + residual + LN in one row-tile kernel (Modules.cc:308-316, 251-257)
-      RowsFfnArgs k = rows_ffn_args(L.ctx, L.ffn, hb, B);
+      RowsFfnArgs k = rows_ffn_args(L.ctx, L.ffn, hb, M);
       k.map_a = map_caq;
       dec_layer_out(k, l, zb, zq[0], zq[1]);
-      const double Bd = B, Ed = E, Fd = F;
+      const double Bd = M, Ed = E, Fd = F;
       LaunchScope ls(c, "dec_wo_ffn_fused", 2.0 * Bd * (Ed * Ed + 2.0 * Ed * Fd),
                      Ed * Ed + 2.0 * Ed * Fd + Bd * Ed * (1.0 + 4.0 + (last ? 1.0 : 6.0)));
       if (launch_rows_ffn(k, E, F, kRowTile, fast, s)) {
@@ -1228,9 +1263,9 @@ int Pass::decode_step(int step) {
       launch_score_rows(d_logits, B, Nout, partials, a.sample ? a.inv_t : 1.0f, s);
     }
   } else if (route.out == Out::Scores) {
-    const double Md = B, Nd = Nout, Kd = E, strips = (Nout + kScoreStrip - 1) / kScoreStrip;
+    const double Md = M, Nd = Nout, Kd = E, strips = (Nout + kScoreStrip - 1) / kScoreStrip;
     LaunchScope ls(c, "dec_gemm_out_scores", 2.0 * Md * Nd * Kd, Md * Kd + Nd * Kd + 8.0 * Nd + 8.0 * Md + 8.0 * Md * strips);
-    if (launch_out_scores(out, map_oq, B, E, best, partials, a.sample ? a.inv_t : 1.0f, c.num_sms, s)) {
+    if (launch_out_scores(out, map_oq, M, E, best, partials, a.sample ? a.inv_t : 1.0f, c.num_sms, s)) {
       set_error("output GEMM (scores): unsupported K " + std::to_string(E));
       return 1;
     }
@@ -1241,6 +1276,34 @@ int Pass::decode_step(int step) {
       set_error("output GEMM: unsupported K " + std::to_string(E));
       return 1;
     }
+  }
+  if (beam) {
+    BeamStepArgs k{};
+    k.s = score_step_args(M, oq, nullptr, step, nullptr);
+    k.beam = K, k.n_sent = B, k.step = step, k.last_step = max_steps - 1;
+    k.cand = cand, k.cum = cum, k.width = width, k.rec = d_rec, k.fin = d_fin, k.n_done = counters;
+    for (int l = 0; l < Ld; l++) k.state_cur[l] = state[l], k.state_nxt[l] = state_nx[l];
+    k.Ld = Ld, k.E = E, k.eos_id = m.eos_id;
+    k.emb_q = m.emb_q, k.inv_qm = m.inv_qm, k.sqrt_e = m.sqrt_e, k.pos0 = m.pos, k.x = xd;
+    k.q = qouts();
+    qadd(k.q, xq[0], m.dec[0].rnn_wf.aq), qadd(k.q, xq[1], m.dec[0].rnn_w.aq);
+    const double Md = M, strips = (Nout + kScoreStrip - 1) / kScoreStrip;
+    {  // the K strips of largest maximum are re-evaluated: 64 K weight rows and the row's operand
+      LaunchScope ls(c, "beam_topk", 0, 8.0 * Md * strips * 2.0 + 8.0 * Md * K + 65.0 * K * E * Md);
+      if (launch_beam_topk(k, s)) {
+        set_error("beam search: candidate kernel launch failed");
+        return 1;
+      }
+    }
+    {
+      LaunchScope ls(c, "beam_merge", 0, 8.0 * Md * K + 16.0 * Md + Md * E * (8.0 * Ld + 4.0 + 2.0 + 1.0));
+      if (launch_beam_merge(k, s)) {
+        set_error("beam search: merge kernel launch failed");
+        return 1;
+      }
+    }
+    for (int l = 0; l < Ld; l++) std::swap(state[l], state_nx[l]);
+    return 0;
   }
   if (a.scores || a.sample) {
     ScoreStepArgs k = score_step_args(B, oq, d_forced, step, d_scores);
@@ -1259,6 +1322,26 @@ int Pass::decode_step(int step) {
         set_error("token scores: step kernel launch failed");
         return 1;
       }
+    }
+  }
+  return 0;
+}
+
+// Model.cc:161: the loop stops once every sentence has produced EOS.  Every second step the done-counter is copied to a
+// pinned slot behind an event and the host looks at the previous copy, so the stream always holds a few queued steps
+// and is never drained (extra steps only produce discarded tokens); the steps in between stay chained by programmatic
+// dependent launch.
+int Pass::poll_done(int step, bool* all_done) {
+  if ((step & 1) == 1) {
+    constexpr int kSlots = 8;
+    const int poll = step >> 1;
+    SB_CUDA(cudaMemcpyAsync(&c.done_slots[poll % kSlots], counters, 4, cudaMemcpyDeviceToHost, s));
+    SB_CUDA(cudaEventRecord(c.done_events[poll % kSlots], s));
+    c.d2h_bytes += 4;
+    if (poll >= 1) {
+      const int old = (poll - 1) % kSlots;
+      SB_CUDA(cudaEventSynchronize(c.done_events[old]));
+      *all_done = c.done_slots[old] >= B;
     }
   }
   return 0;
@@ -1287,22 +1370,9 @@ int Pass::decode() {
     // FRONT of the next step's first kernel (dec_ssru_kernel with embed set); the last executed step is closed by the
     // stand-alone kernel after the loop.
     executed = step + 1;
-    // Model.cc:161: the loop stops once every sentence has produced EOS.  Every second step the done-counter is copied
-    // to a pinned slot behind an event and the host looks at the previous copy, so the stream always holds a few
-    // queued steps and is never drained (extra steps only produce discarded tokens); the steps in between stay
-    // chained by programmatic dependent launch.
-    if ((step & 1) == 1) {
-      constexpr int kSlots = 8;
-      const int poll = step >> 1;
-      SB_CUDA(cudaMemcpyAsync(&c.done_slots[poll % kSlots], counters, 4, cudaMemcpyDeviceToHost, s));
-      SB_CUDA(cudaEventRecord(c.done_events[poll % kSlots], s));
-      c.d2h_bytes += 4;
-      if (poll >= 1) {
-        const int old = (poll - 1) % kSlots;
-        SB_CUDA(cudaEventSynchronize(c.done_events[old]));
-        if (c.done_slots[old] >= B) break;
-      }
-    }
+    bool all_done = false;
+    if (poll_done(step, &all_done)) return 1;
+    if (all_done) break;
   }
   if (executed > 0) {
     {
@@ -1478,6 +1548,45 @@ int Pass::score() {
 
 // One call on context c (`name` prefixes its errors): an empty request does nothing; otherwise the encoder and the
 // output layer's set-up, then `decoder` (Pass::decode or Pass::score).
+// Beam search (DESIGN §4.4d): the decode loop over B * K rows, each step closed by the candidate and merge kernels.  The
+// step records and finished hypotheses come back to the host, which does the backtrace and the ranking.
+int Pass::beam_search() {
+  for (int l = 0; l < Ld; l++) SB_CUDA(cudaMemsetAsync(state[l], 0, 4ul * M * E, s));
+  SB_CUDA(cudaMemsetAsync(best, 0, 8ul * M, s));
+  SB_CUDA(cudaMemsetAsync(cum, 0, 4ul * M, s));
+  SB_CUDA(cudaMemsetAsync(width, K, B, s));
+  SB_CUDA(cudaMemsetAsync(counters, 0, 256, s));
+  {  // step 0 input of every slot: zero embedding + position-0 signal
+    QuantOuts q = qouts();
+    qadd(q, xq[0], m.dec[0].rnn_wf.aq), qadd(q, xq[1], m.dec[0].rnn_w.aq);
+    LaunchScope ls(c, "dec_embed0", 0, 6.0 * M * E);
+    launch_embed(nullptr, m.emb_q, m.inv_qm, m.sqrt_e, m.pos, M, 1, E, 0, 1, xd, q, s);
+  }
+  int executed = 0;
+  for (int step = 0; step < max_steps; step++) {
+    if (decode_step(step)) return 1;
+    executed = step + 1;
+    bool all_done = false;
+    if (poll_done(step, &all_done)) return 1;
+    if (all_done) break;
+  }
+  SB_CUDA(cudaMemcpyAsync(a.beam_steps, d_rec, sizeof(BeamRec) * executed * M, cudaMemcpyDeviceToHost, s));
+  SB_CUDA(cudaMemcpyAsync(a.beam_finished, d_fin, sizeof(BeamFin) * M, cudaMemcpyDeviceToHost, s));
+  c.d2h_bytes += sizeof(BeamRec) * executed * M + sizeof(BeamFin) * M;
+  if (d_align_all) {
+    SB_CUDA(cudaMemcpyAsync(a.alignment, d_align_all, 4ul * executed * M * T, cudaMemcpyDeviceToHost, s));
+    c.d2h_bytes += 4ul * executed * M * T;
+  }
+  SB_CUDA(cudaStreamSynchronize(s));
+  a.steps = static_cast<size_t>(executed);
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) {
+    set_error(std::string("beam search failed: ") + cudaGetErrorString(e));
+    return 1;
+  }
+  return 0;
+}
+
 int run_pass(Model& m, Context& c, ForwardArgs& a, const char* name, bool empty, int (Pass::*decoder)()) {
   std::lock_guard<std::recursive_mutex> ctx_lock(c.mu);
   if (c.device != m.ctx->device) {
@@ -1498,6 +1607,18 @@ int model_forward_on(Model& m, Context& c, ForwardArgs& a) {
   a.steps = 0;
   a.target_tokens = 0;
   return run_pass(m, c, a, "model_forward", a.B == 0 || a.T == 0, &Pass::decode);
+}
+
+int model_beam_on(Model& m, Context& c, ForwardArgs& a) {
+  a.steps = 0;
+  a.target_tokens = 0;
+  if (a.beam < 1 || a.beam > kMaxBeam || a.beam_steps == nullptr || a.beam_finished == nullptr || a.targets || a.forced ||
+      a.sample || a.logits || a.scores || a.device_io) {
+    set_error("model_beam: a beam of 1 .. 8, host buffers for the records, and none of targets, forced, sampling, "
+              "logits, scores or device_io");
+    return 1;
+  }
+  return run_pass(m, c, a, "model_beam", a.B == 0 || a.T == 0, &Pass::beam_search);
 }
 
 int model_score_on(Model& m, Context& c, ForwardArgs& a) {

@@ -202,6 +202,12 @@ struct ForwardArgs {
   // position into scores [B][target_T]; alignment, when set, receives [B][target_T][T].
   const uint32_t* targets = nullptr;
   size_t target_T = 0;
+  // Beam search (model_beam_on, DESIGN §4.4d): `beam` hypotheses per sentence in decoder rows b * beam + k.  Host
+  // buffers: beam_steps [max_steps][B * beam] receives each step's surviving hypotheses, beam_finished [B][beam] every
+  // sentence's finished ones; alignment, when set, receives [max_steps][B * beam][T].  steps = the steps executed.
+  int beam = 0;
+  BeamRec* beam_steps = nullptr;
+  BeamFin* beam_finished = nullptr;
 };
 
 int model_forward(Model& m, ForwardArgs& a);
@@ -211,6 +217,9 @@ int model_forward_on(Model& m, Context& lane, ForwardArgs& a);
 // Teacher-forced scoring of a.targets in one time-parallel pass (bit-exact arithmetic whatever lane.fast says): the
 // scores and alignments model_forward would give with forced = the targets, at every target position.
 int model_score_on(Model& m, Context& lane, ForwardArgs& a);
+// Beam search over a.beam slots per sentence (bit-exact arithmetic whatever lane.fast says): the records from which the
+// host rebuilds and ranks each sentence's hypotheses.
+int model_beam_on(Model& m, Context& lane, ForwardArgs& a);
 
 // Decoder steps Model::decode may run for a batch of width T: the first step is unconditional (Model.cc:145-157), the
 // loop that follows runs while i < size_t(limit_factor * T) (Model.cc:160-161).

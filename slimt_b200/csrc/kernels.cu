@@ -411,6 +411,165 @@ __global__ void __launch_bounds__(32 * kScoreWarps) sample_step_kernel(ScoreStep
         static_cast<float>(static_cast<double>(zc) - (static_cast<double>(M) + log(S)));
 }
 
+// ------------------------------------------------------------------ beam search
+// Candidates are packed as in packed_best.cuh, so a larger key ranks first and equal values go to the lower index.
+// top[0..7] holds the largest keys seen, descending (0 = empty); keys are distinct.
+__device__ __forceinline__ void top8_insert(unsigned long long (&top)[kMaxBeam], unsigned long long key) {
+#pragma unroll
+  for (int i = kMaxBeam - 1; i >= 0; i--) {
+    const unsigned long long prev = i > 0 ? top[i - 1] : ~0ull;
+    if (key > top[i]) top[i] = key < prev ? key : prev;
+  }
+}
+
+__device__ __forceinline__ unsigned long long warp_max_u64(unsigned long long v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const unsigned long long u = __shfl_xor_sync(0xffffffffu, v, o);
+    v = u > v ? u : v;
+  }
+  return v;
+}
+
+// The warp's largest key over every lane's top list, removed from the list that held it.
+__device__ __forceinline__ unsigned long long top8_pop(unsigned long long (&top)[kMaxBeam]) {
+  const unsigned long long m = warp_max_u64(top[0]);
+  if (m != 0ull && top[0] == m) {
+#pragma unroll
+    for (int i = 0; i + 1 < kMaxBeam; i++) top[i] = top[i + 1];
+    top[kMaxBeam - 1] = 0ull;
+  }
+  return m;
+}
+
+// Block = 32 rows x 32 warps, reduce_partials' shape; then warp w takes row w of the block.
+__global__ void __launch_bounds__(32 * kScoreWarps) beam_topk_kernel(BeamStepArgs a) {
+  __shared__ float mx[kScoreWarps][32];
+  __shared__ double sm[kScoreWarps][32];
+  __shared__ double lse_of[32];
+  const ScoreStepArgs& s = a.s;
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int rows = s.B, K = a.beam;
+  pdl_launch_dependents();
+  pdl_wait();
+  const float M = reduce_partials(s.partials, rows, s.N, blockIdx.x * 32 + lane, lane, w, mx, sm);
+  if (w == 0) {
+    double S = 0.0;
+    for (int k = 0; k < kScoreWarps; k++) S += sm[k][lane];
+    lse_of[lane] = static_cast<double>(M) + log(S);
+    if (blockIdx.x * 32 + lane < rows) s.best[blockIdx.x * 32 + lane] = 0ull;  // the output GEMM's greedy slot, unused
+  }
+  __syncthreads();
+  const int row = blockIdx.x * 32 + w;
+  if (row >= rows) return;
+  const int b = row / K, slot = row % K;
+  if (slot >= (a.step == 0 ? 1 : static_cast<int>(a.width[b]))) return;
+  // the K strips of largest (max, -strip)
+  const int n_strips = (s.N + kScoreStrip - 1) / kScoreStrip;
+  unsigned long long top[kMaxBeam];
+#pragma unroll
+  for (int i = 0; i < kMaxBeam; i++) top[i] = 0ull;
+  for (int t = lane; t < n_strips; t += 32)
+    top8_insert(top, pack_best(s.partials[static_cast<size_t>(t) * rows + row].x, static_cast<uint32_t>(t)));
+  int my_strip = -1;  // lane r < K: the r-th strip
+  for (int r = 0; r < K; r++) {
+    const unsigned long long m = top8_pop(top);
+    if (lane == r && m != 0ull) my_strip = static_cast<int>(best_index(m));
+  }
+  // their 64 * K logits, exactly: lane takes columns lane and lane + 32 of each strip
+  const float ninf = -__int_as_float(0x7f800000);
+#pragma unroll
+  for (int i = 0; i < kMaxBeam; i++) top[i] = 0ull;
+  for (int i = 0; i < 2 * K; i++) {
+    const int t = __shfl_sync(0xffffffffu, my_strip, i >> 1);
+    if (t < 0) break;
+    const int col = t * kScoreStrip + lane + 32 * (i & 1);
+    top8_insert(top, pack_best(col < s.N ? exact_logit(s, row, col) : ninf, static_cast<uint32_t>(col)));
+  }
+  const double lse = lse_of[w];
+  for (int r = 0; r < K; r++) {
+    const unsigned long long m = top8_pop(top);
+    if (lane == 0)
+      a.cand[static_cast<size_t>(row) * K + r] =
+          BeamCand{best_index(m), static_cast<float>(static_cast<double>(best_value(m)) - lse)};
+  }
+}
+
+// Warp = one sentence, eight per block.  Every lane computes the same choices; lane 0 writes the records.
+__global__ void __launch_bounds__(256) beam_merge_kernel(BeamStepArgs a) {
+  const int lane = threadIdx.x & 31;
+  const int b = blockIdx.x * 8 + (threadIdx.x >> 5);
+  pdl_launch_dependents();
+  pdl_wait();
+  if (b >= a.n_sent) return;
+  const int K = a.beam, width = a.width[b];
+  if (width == 0) return;
+  const int live = a.step == 0 ? 1 : width, base = b * K;
+  // candidate i = slot * K + rank of the live slots: lanes hold i = lane and lane + 32
+  auto key_of = [&](int i) -> unsigned long long {
+    if (i >= live * K) return 0ull;
+    const float t = __fadd_rn(a.cum[base + i / K], a.cand[static_cast<size_t>(base) * K + i].score);
+    return pack_best(t, static_cast<uint32_t>(i));
+  };
+  unsigned long long k0 = key_of(lane), k1 = key_of(lane + 32);
+  int pick[kMaxBeam];
+  float total[kMaxBeam];
+#pragma unroll
+  for (int r = 0; r < kMaxBeam; r++) {
+    if (r >= width) break;
+    const unsigned long long m = warp_max_u64(k0 > k1 ? k0 : k1);
+    if (k0 == m) k0 = 0ull;
+    if (k1 == m) k1 = 0ull;
+    pick[r] = static_cast<int>(best_index(m));
+    total[r] = __fadd_rn(a.cum[base + pick[r] / K], a.cand[static_cast<size_t>(base) * K + pick[r]].score);
+  }
+  __syncwarp();  // every lane has read cum before it is rewritten
+  const size_t rows = static_cast<size_t>(a.n_sent) * K;
+  int n_live = 0, n_fin = K - width;
+  int parent[kMaxBeam];
+  uint32_t word[kMaxBeam];
+#pragma unroll
+  for (int r = 0; r < kMaxBeam; r++) {
+    if (r >= width) break;
+    const int k = pick[r] / K;
+    const BeamCand c = a.cand[static_cast<size_t>(base) * K + pick[r]];
+    const uint32_t wd = a.s.shortlist ? a.s.shortlist[c.col] : c.col;
+    if (wd == a.eos_id || a.step == a.last_step) {
+      if (lane == 0)
+        a.fin[base + n_fin] = BeamFin{static_cast<uint32_t>(a.step), static_cast<uint32_t>(k), wd, c.score, total[r]};
+      n_fin++;
+    } else {
+      if (lane == 0) {
+        a.rec[static_cast<size_t>(a.step) * rows + base + n_live] = BeamRec{wd, static_cast<uint32_t>(k), c.score};
+        a.cum[base + n_live] = total[r];
+      }
+      parent[n_live] = k, word[n_live] = wd;
+      n_live++;
+    }
+  }
+  if (lane == 0) {
+    a.width[b] = static_cast<uint8_t>(n_live);
+    if (n_live == 0) atomicAdd(a.n_done, 1);
+  }
+  const int E = a.E;
+#pragma unroll
+  for (int n = 0; n < kMaxBeam; n++) {
+    if (n >= n_live) break;
+    const size_t dst = static_cast<size_t>(base + n) * E, src = static_cast<size_t>(base + parent[n]) * E;
+    for (int l = 0; l < a.Ld; l++)
+      for (int e = lane * 4; e < E; e += 128)
+        *reinterpret_cast<float4*>(a.state_nxt[l] + dst + e) = *reinterpret_cast<const float4*>(a.state_cur[l] + src + e);
+    for (int e = lane * 4; e < E; e += 128) {
+      const char4 c = *reinterpret_cast<const char4*>(a.emb_q + static_cast<size_t>(word[n]) * E + e);
+      const float4 ps = *reinterpret_cast<const float4*>(a.pos0 + e);
+      const float y[4] = {embed1(c.x, a.inv_qm, a.sqrt_e, ps.x), embed1(c.y, a.inv_qm, a.sqrt_e, ps.y),
+                          embed1(c.z, a.inv_qm, a.sqrt_e, ps.z), embed1(c.w, a.inv_qm, a.sqrt_e, ps.w)};
+      *reinterpret_cast<float4*>(a.x + dst + e) = make_float4(y[0], y[1], y[2], y[3]);
+      store_quant4(a.q, dst + e, y);
+    }
+  }
+}
+
 }  // namespace
 
 void launch_embed(const uint32_t* tokens, const int8_t* emb_q, float inv_qm, float sqrt_e, const float* pos, int rows,
@@ -509,6 +668,18 @@ int launch_score_step(const ScoreStepArgs& a, cudaStream_t stream) {
 int launch_sample_step(const ScoreStepArgs& a, cudaStream_t stream) {
   if (a.B == 0) return 0;
   return launch_pdl(sample_step_kernel, dim3((a.B + 31) / 32), dim3(32 * kScoreWarps), 0, stream, a) != cudaSuccess ? 1 : 0;
+}
+
+int launch_beam_topk(const BeamStepArgs& a, cudaStream_t stream) {
+  if (a.s.B == 0) return 0;
+  if (a.beam < 1 || a.beam > kMaxBeam || a.Ld > 2) return 1;
+  return launch_pdl(beam_topk_kernel, dim3((a.s.B + 31) / 32), dim3(32 * kScoreWarps), 0, stream, a) != cudaSuccess ? 1 : 0;
+}
+
+int launch_beam_merge(const BeamStepArgs& a, cudaStream_t stream) {
+  if (a.n_sent == 0) return 0;
+  if (a.beam < 1 || a.beam > kMaxBeam || a.Ld > 2) return 1;
+  return launch_pdl(beam_merge_kernel, dim3((a.n_sent + 7) / 8), dim3(256), 0, stream, a) != cudaSuccess ? 1 : 0;
 }
 
 }  // namespace sb

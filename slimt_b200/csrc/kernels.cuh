@@ -145,6 +145,53 @@ struct ScoreStepArgs {
 };
 int launch_score_step(const ScoreStepArgs& a, cudaStream_t stream);
 int launch_sample_step(const ScoreStepArgs& a, cudaStream_t stream);
+
+// Beam search (include/slimt_b200.h, DESIGN §4.4d).  Sentence b owns decoder rows b * beam + k (slot k); width[b] is
+// the number of hypotheses it still has to finish (beam - finished), and its live slots are 0 .. width[b] - 1 (slot 0
+// alone at step 0).
+constexpr int kMaxBeam = 8;
+struct BeamCand {  // one of a row's candidates: its output column and token score y[c] - LSE
+  uint32_t col;
+  float score;
+};
+struct BeamRec {  // the hypothesis a step put into a slot: its last word, the slot it extends, that word's score
+  uint32_t word;
+  uint32_t parent;
+  float score;
+};
+struct BeamFin {  // a finished hypothesis: the step of its last word, the slot it extends, the word, its score, the total
+  uint32_t step;
+  uint32_t parent;
+  uint32_t word;
+  float score;
+  float total;
+};
+struct BeamStepArgs {
+  ScoreStepArgs s;                // the output layer's rows (s.B = n_sent * beam), partials and operands; s.step unused
+  int beam, n_sent, step, last_step;
+  BeamCand* cand;                 // [rows][beam]
+  float* cum;                     // [rows] cumulative score of each live slot
+  uint8_t* width;                 // [n_sent]
+  BeamRec* rec;                   // [max_steps][rows]
+  BeamFin* fin;                   // [n_sent][beam], in the order the hypotheses finished
+  int* n_done;                    // sentences whose width reached 0
+  const float* state_cur[2];      // each decoder layer's SSRU state after this step [rows][E] ...
+  float* state_nxt[2];            // ... gathered by parent into the next step's state
+  int Ld, E;
+  uint32_t eos_id;
+  const int8_t* emb_q;            // next input: embedding * sqrt(E) + position-0 signal, as finalize_step builds it
+  float inv_qm, sqrt_e;
+  const float* pos0;
+  float* x;                       // [rows][E]
+  QuantOuts q;                    // its u8 copies (layer 0's SSRU operands)
+};
+// Per row (32 rows per block): the row's LSE exactly as score_step forms it, the `beam` strips of largest maximum (every
+// top-beam column lies in one of them), their logits re-evaluated exactly, and the row's first `beam` columns ordered by
+// (logit descending, column ascending) into cand.  Rows of dead slots are skipped.
+int launch_beam_topk(const BeamStepArgs& a, cudaStream_t stream);
+// Per sentence (one warp): the merge of its live slots' candidates by (cum + score descending, slot ascending, rank
+// ascending), the step record, finished hypotheses, the state gather and the next step's input.
+int launch_beam_merge(const BeamStepArgs& a, cudaStream_t stream);
 // dst[c][r] = src[r][c] for r < rows, c < cols (dst rows are dst_stride apart): step-major token matrix -> sentence-major
 void launch_transpose_u32(const uint32_t* src, int rows, int cols, uint32_t* dst, int dst_stride, cudaStream_t stream);
 

@@ -47,10 +47,12 @@ struct Batcher {
 struct slimt_b200_translate_io;
 struct slimt_b200_score_io;
 struct slimt_b200_sampling;
+struct slimt_b200_beam;
 namespace sb {
-// exhaust() over one request with the batches dealt to the replicas' lanes (translate.cu)
+// exhaust() over one request with the batches dealt to the replicas' lanes (translate.cu); with beam set, each batch
+// runs beam search (engine.cu: model_beam_on) and io receives every sentence's best hypothesis
 int translate_multi(Model* const* models, size_t n_replicas, slimt_b200_translate_io* io,
-                    const slimt_b200_sampling* sampling);
+                    const slimt_b200_sampling* sampling, slimt_b200_beam* beam = nullptr);
 // The same batches and lanes scoring given targets with the time-parallel pass (engine.cu: model_score_on)
 int score_multi(Model* const* models, size_t n_replicas, slimt_b200_score_io* io);
 

@@ -7,6 +7,7 @@
 // free, so N replicas on N GPUs are fed from ONE process by ONE Batcher; two lanes per replica let batch i + 1's
 // packing, shortlist generation and H2D copy overlap batch i on the GPU.  Sentences are independent and batch
 // composition is decided by the Batcher alone, so the result does not depend on which lane served which batch.
+#include <math.h>
 #include <string.h>
 
 #include <algorithm>
@@ -223,6 +224,40 @@ void pack_sources(const uint32_t* src, const uint64_t* offsets, const Plan& p, u
   }
 }
 
+// One hypothesis of beam search, rebuilt on the host from the step records: its words and their scores, and for each
+// word the slot whose row computed it (where its alignment row is).
+struct Hyp {
+  std::vector<uint32_t> tokens;
+  std::vector<float> scores;
+  std::vector<uint32_t> slots;
+  float total = 0;
+  double normalized = 0;
+};
+
+// Sentence r's K finished hypotheses (fin[r * K ..], in the order they finished), ranked by normalized score; ties keep
+// the finishing order.  rec: [steps][B * K].
+std::vector<Hyp> beam_hypotheses(const BeamRec* rec, const BeamFin* fin, size_t r, size_t B, int K, float alpha) {
+  std::vector<Hyp> hs(K);
+  for (int f = 0; f < K; f++) {
+    const BeamFin& e = fin[r * K + f];
+    const size_t len = e.step + 1;
+    Hyp& h = hs[f];
+    h.tokens.resize(len), h.scores.resize(len), h.slots.resize(len);
+    h.tokens[e.step] = e.word, h.scores[e.step] = e.score, h.slots[e.step] = e.parent;
+    uint32_t p = e.parent;
+    for (size_t st = e.step; st-- > 0;) {
+      const BeamRec& x = rec[st * B * K + r * K + p];
+      h.tokens[st] = x.word, h.scores[st] = x.score;
+      p = x.parent;
+      h.slots[st] = p;
+    }
+    h.total = e.total;
+    h.normalized = static_cast<double>(e.total) / std::pow(static_cast<double>(len), static_cast<double>(alpha));
+  }
+  std::stable_sort(hs.begin(), hs.end(), [](const Hyp& x, const Hyp& y) { return x.normalized > y.normalized; });
+  return hs;
+}
+
 // Copies each batch's per-sentence results (back to back in batch row order, `n(s)` values for sentence s) to their
 // places in the request's ragged output.
 template <class T, class Get, class N>
@@ -261,8 +296,27 @@ int check_sampling(const slimt_b200_sampling* sampling) {
   return 0;
 }
 
-int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io* io, const slimt_b200_sampling* sampling) {
-  Service sv{models, n_rep, "translate"};
+int check_beam(const slimt_b200_beam* beam) {
+  if (beam == nullptr) return 0;
+  if (beam->beam_size < 1 || beam->beam_size > kMaxBeam) {
+    set_error("beam: beam_size must be in 1 .. " + std::to_string(kMaxBeam) + ", got " + std::to_string(beam->beam_size));
+    return 1;
+  }
+  if (beam->nbest < 1 || beam->nbest > beam->beam_size) {
+    set_error("beam: nbest must be in 1 .. beam_size, got " + std::to_string(beam->nbest));
+    return 1;
+  }
+  if (!(beam->length_penalty >= 0.0f && beam->length_penalty <= 3.402823466e38f)) {  // also NaN
+    set_error("beam: length_penalty must be finite and >= 0, got " + std::to_string(beam->length_penalty));
+    return 1;
+  }
+  return 0;
+}
+
+int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io* io, const slimt_b200_sampling* sampling,
+                    slimt_b200_beam* beam) {
+  if (check_beam(beam)) return 1;
+  Service sv{models, n_rep, beam ? "translate_beam" : "translate"};
   if (sv.check_replicas()) return 1;
   io->target_tokens = 0, io->batches = 0, io->device_ms = 0;
   io->kernel_launches = 0, io->h2d_bytes = 0, io->d2h_bytes = 0;
@@ -272,10 +326,68 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
   if (sv.load_shortlist(io->shortlist_bin, io->shortlist_bytes, io->shortlist_check, io->shortlist_shared)) return 1;
   if (sv.make_plan(io->offsets, n_sent, io->max_words)) return 1;
   const std::vector<Plan>& plan = sv.plan;
+  const int K = beam ? beam->beam_size : 0;
+  const bool want_nbest = beam && (beam->nbest_tokens || beam->nbest_token_scores);
+  if (want_nbest) {  // every hypothesis has at most its batch's max_steps tokens
+    uint64_t bound = 0;
+    for (const Plan& p : plan)
+      bound += static_cast<uint64_t>(p.ids.size()) * beam->nbest * forward_max_steps(io->limit_factor, p.width);
+    if (beam->nbest_capacity < bound) {
+      set_error("translate_beam: nbest_capacity of " + std::to_string(beam->nbest_capacity) + " tokens is below the " +
+                std::to_string(bound) + " that nbest hypotheses of max_steps tokens per sentence can take");
+      return 1;
+    }
+  }
 
   std::vector<Done> done(plan.size());
   std::vector<uint32_t> out_len(n_sent, 0);
+  std::vector<std::vector<Hyp>> nbest(beam ? n_sent : 0);  // each sentence's first nbest hypotheses
+  std::atomic<uint64_t> beam_steps{0};
+  auto serve_beam = [&](Model& m, Context& c, size_t bi) -> int {
+    const Plan& p = plan[bi];
+    const size_t B = p.ids.size(), width = p.width, M = B * K;
+    const size_t stride = static_cast<size_t>(forward_max_steps(io->limit_factor, width));
+    // staging: [padded tokens][lengths] | [step records] | [finished hypotheses] | [alignment rows]
+    const size_t in_bytes = (4 * (B * width + B) + 255) & ~size_t(255);
+    const size_t rec_bytes = (sizeof(BeamRec) * stride * M + 255) & ~size_t(255);
+    const size_t fin_bytes = (sizeof(BeamFin) * M + 255) & ~size_t(255);
+    const size_t al_bytes = want_align ? 4 * stride * M * width : 0;
+    char* stage = c.staging_reserve(in_bytes + rec_bytes + fin_bytes + al_bytes + 256);
+    if (!stage) return 1;
+    uint32_t* tokens = reinterpret_cast<uint32_t*>(stage);
+    uint32_t* lengths = tokens + B * width;
+    std::vector<uint32_t> words;
+    pack_sources(io->tokens, io->offsets, p, m.pad_id, tokens, lengths, &words);
+    LazyShortlist lazy{&sv.gen, &words, static_cast<size_t>(m.V), {}};
+    BeamRec* rec = reinterpret_cast<BeamRec*>(stage + in_bytes);
+    BeamFin* fin = reinterpret_cast<BeamFin*>(stage + in_bytes + rec_bytes);
+    float* align = want_align ? reinterpret_cast<float*>(stage + in_bytes + rec_bytes + fin_bytes) : nullptr;
+    ForwardArgs a;
+    a.tokens = tokens, a.lengths = lengths, a.B = B, a.T = width;
+    a.limit_factor = io->limit_factor;
+    if (sv.use_sl) a.shortlist_cb = lazy_shortlist_cb, a.shortlist_user = &lazy;
+    a.beam = K, a.beam_steps = rec, a.beam_finished = fin, a.alignment = align;
+    if (model_beam_on(m, c, a)) return 1;
+    beam_steps += a.steps;
+    Done& d = done[bi];
+    for (size_t r = 0; r < B; r++) {
+      std::vector<Hyp> hs = beam_hypotheses(rec, fin, r, B, K, beam->length_penalty);
+      const Hyp& h = hs[0];
+      out_len[p.ids[r]] = static_cast<uint32_t>(h.tokens.size());
+      d.kept.insert(d.kept.end(), h.tokens.begin(), h.tokens.end());
+      if (want_scores) d.scores.insert(d.scores.end(), h.scores.begin(), h.scores.end());
+      if (want_align)  // the row that computed word s: slot h.slots[s] of step s
+        for (size_t st = 0; st < h.tokens.size(); st++) {
+          const float* row = align + (st * M + r * K + h.slots[st]) * width;
+          d.align.insert(d.align.end(), row, row + lengths[r]);
+        }
+      hs.resize(beam->nbest);
+      nbest[p.ids[r]] = std::move(hs);
+    }
+    return 0;
+  };
   auto serve = [&](Model& m, Context& c, size_t bi) -> int {
+    if (beam) return serve_beam(m, c, bi);
     const Plan& p = plan[bi];
     const size_t B = p.ids.size(), width = p.width;
     const size_t stride = static_cast<size_t>(forward_max_steps(io->limit_factor, width));
@@ -370,6 +482,23 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
     if (io->out_align_offsets) memcpy(io->out_align_offsets, al_off.data(), 8 * (n_sent + 1));
     scatter(plan, [&](size_t bi) -> const auto& { return done[bi].align; }, al_off,
             [&](size_t s) { return static_cast<size_t>(al_off[s + 1] - al_off[s]); }, io->out_alignments);
+  }
+  if (beam) {
+    beam->steps = beam_steps.load();
+    const size_t nb = static_cast<size_t>(beam->nbest);
+    uint64_t pos = 0;
+    for (size_t i = 0; i < n_sent; i++)
+      for (size_t h = 0; h < nb; h++) {
+        const Hyp& x = nbest[i][h];
+        const size_t e = i * nb + h;
+        if (beam->nbest_offsets) beam->nbest_offsets[e] = pos;
+        if (beam->nbest_tokens) memcpy(beam->nbest_tokens + pos, x.tokens.data(), 4 * x.tokens.size());
+        if (beam->nbest_token_scores) memcpy(beam->nbest_token_scores + pos, x.scores.data(), 4 * x.scores.size());
+        if (beam->nbest_totals) beam->nbest_totals[e] = x.total;
+        if (beam->nbest_normalized) beam->nbest_normalized[e] = x.normalized;
+        pos += x.tokens.size();
+      }
+    if (beam->nbest_offsets) beam->nbest_offsets[n_sent * nb] = pos;
   }
   return 0;
 }

@@ -210,6 +210,31 @@ int slimt_b200_model_forward_sampled(slimt_b200_model* model, slimt_b200_forward
 int slimt_b200_translate_sampled(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_translate_io* io,
                                  const slimt_b200_sampling* sampling);
 
+/* ---- top-k sampling: each step's word drawn from the k most likely columns only (marian's --output-sampling topk) ----
+ * For decode step s and row b, with y[n] the step's exact logits over the N output columns (as for sampling above) and
+ * k = top_k:
+ *  - the set S_k is the first min(k, N) columns ordered by (y descending, column ascending): ties go to the lower
+ *    column, so S_1 is the greedy choice.
+ *  - z[n] = fl32(y[n] * inv_t) as above; M = max z over S_k; each column c of S_k has the term
+ *    e_c = exp(z[c] - M), evaluated as the token scores evaluate it (ex2.approx of one rounded product), and S is the
+ *    sum of the terms in ascending column order, in double.
+ *  - u as above (the same Philox stream, keys and defaults); the word is the first column of S_k, in ascending column
+ *    order, whose running sum exceeds u * S.  A zero term is never chosen; if rounding exhausts the set, the last
+ *    column with a nonzero term is taken.
+ *  - token_scores / out_scores, when asked for, hold (float)((double)z[c] - ((double)M + log S)): the word's
+ *    log-probability under the distribution it was drawn from (slimt_b200_score gives the full-vocabulary one).
+ *  - everything after the draw is as for sampling: EOS handling, recorded tokens, alignments, the step limit, batching.
+ * k = 1 is greedy decoding in the bit-exact arithmetic, with every score 0; k >= N draws from every column.  Both
+ * arithmetic modes draw from the step's exact logits.  Errors, each reported before any GPU work (the model stays
+ * usable): top_k < 0 or > 256; top_k > 0 with sampling = NULL; and sampling's own errors (temperature, `forced`).
+ * top_k = 0 is the _sampled call.
+ * Device workspace: with top_k > 0 every step's logits are materialised, 4 * B * N bytes per batch (N the shortlist's
+ * or the vocabulary's width). */
+int slimt_b200_model_forward_topk(slimt_b200_model* model, slimt_b200_forward_io* io,
+                                  const slimt_b200_sampling* sampling, int32_t top_k);
+int slimt_b200_translate_topk(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_translate_io* io,
+                              const slimt_b200_sampling* sampling, int32_t top_k);
+
 /* ---- scoring: the log-probability of each word of a GIVEN translation ----
  * For sentence pair i (source tokens[offsets[i] .. offsets[i + 1]), EOS included, non-empty; target
  * targets[target_offsets[i] .. target_offsets[i + 1]), any length including 0) and each target position j, the score of

@@ -676,10 +676,11 @@ class Blocking {
   // Scores given translations (slimt_b200_score): for sources[i] and targets[i], the log-probability of every word of
   // targets[i] in scores[i], and with Options::alignment each word's distribution over sources[i].  The pairs are
   // scored as given -- no wrapping, EOS like any other word -- and never through the translation cache, which holds
-  // translations, not scores.  Options::sample and Options::html do not apply and are refused.
+  // translations, not scores.  Options::sample, top_k and html do not apply and are refused.
   WordsResponse score(const Ptr<Model> &model, const Sentences &sources, const Sentences &targets,
                       const Options &options = Options()) {
     if (options.sample) throw std::invalid_argument("Blocking::score: Options::sample does not apply to scoring");
+    if (options.top_k != 0) throw std::invalid_argument("Blocking::score: Options::top_k does not apply to scoring");
     if (options.html) throw std::invalid_argument("Blocking::score: Options::html does not apply to scoring");
     if (sources.size() != targets.size()) throw std::invalid_argument("Blocking::score: one target per source");
     std::vector<uint32_t> tokens, words;
@@ -771,6 +772,11 @@ class Blocking {
   // stored by a request that did not ask for alignments (or scores) cannot answer one that does.  A sampled or beam
   // segment is neither looked up nor stored: the cache holds greedy translations.  The rest: run().
   Histories serve(const Ptr<Model> &model, const Sentences &segments, const Options &options) {
+    if (options.top_k < 0 || options.top_k > 256)
+      throw std::invalid_argument("Options: top_k must be in 0 .. 256, got " + std::to_string(options.top_k));
+    if (options.top_k > 0 && !options.sample) throw std::invalid_argument("Options: top_k > 0 needs sample");
+    if (options.top_k > 0 && options.beam_size > 1)
+      throw std::invalid_argument("Options: top_k and beam_size > 1 exclude each other");
     if (options.sample && options.beam_size > 1)
       throw std::invalid_argument("Options: sample and beam_size > 1 exclude each other");
     Histories histories(segments.size());
@@ -841,8 +847,9 @@ class Blocking {
       beam.beam_size = options.beam_size, beam.nbest = 1, beam.length_penalty = options.length_penalty;
       detail::check(slimt_b200_translate_beam(replicas.data(), replicas.size(), &io, &beam), "slimt_b200_translate_beam");
     } else {
-      detail::check(slimt_b200_translate_sampled(replicas.data(), replicas.size(), &io, options.sample ? &sampling : nullptr),
-                    "slimt_b200_translate_sampled");
+      detail::check(slimt_b200_translate_topk(replicas.data(), replicas.size(), &io, options.sample ? &sampling : nullptr,
+                                              options.top_k),
+                    "slimt_b200_translate_topk");
     }
     for (size_t k = 0; k < todo.size(); k++) {
       auto h = std::make_shared<Hypothesis>();
@@ -967,6 +974,7 @@ class Async {
     return !a.second && !b.second && a.first == b.first && a.is_text == b.is_text && a.options.alignment == b.options.alignment &&
            a.options.html == b.options.html && a.options.scores == b.options.scores && a.options.sample == b.options.sample &&
            (!a.options.sample || (a.options.temperature == b.options.temperature && a.options.seed == b.options.seed)) &&
+           a.options.top_k == b.options.top_k &&
            a.options.beam_size == b.options.beam_size && a.options.length_penalty == b.options.length_penalty;
   }
   void work() {

@@ -1311,6 +1311,10 @@ struct Options {
   bool sample = false;
   float temperature = 1.0f;  // finite, in [1e-3, 1e3]
   uint64_t seed = 0;
+  // With sample: draw each word from the top_k most likely words only (marian's --output-sampling topk;
+  // slimt_b200_translate_topk).  0 = from every word; 1 .. 256 otherwise.  top_k > 0 without sample, with
+  // beam_size > 1, or out of range is std::invalid_argument.
+  int top_k = 0;
   // Beam search with beam_size hypotheses per segment (marian's --beam-size / --normalize; slimt_b200_translate_beam):
   // the best hypothesis by total / len^length_penalty is returned, its scores and alignments with it.  beam_size = 1 is
   // the greedy call; beam_size > 1 together with sample is std::invalid_argument.  Beam segments bypass the translation

@@ -27,7 +27,8 @@ EXPORTS = [
     "slimt_b200_shortlist_generate", "slimt_b200_batcher_plan", "slimt_b200_profile_enable", "slimt_b200_profile_read",
     "slimt_b200_translate_multi", "slimt_b200_shortlist_check", "slimt_b200_ctx_set_math", "slimt_b200_ctx_get_math",
     "slimt_b200_model_set_max_length", "slimt_b200_model_max_length", "slimt_b200_model_forward_sampled",
-    "slimt_b200_translate_sampled", "slimt_b200_score", "slimt_b200_translate_beam",
+    "slimt_b200_translate_sampled", "slimt_b200_score", "slimt_b200_translate_beam", "slimt_b200_model_forward_topk",
+    "slimt_b200_translate_topk",
 ]
 
 
@@ -123,6 +124,9 @@ def lib() -> C.CDLL:
         L.slimt_b200_model_forward_sampled.argtypes = [C.c_void_p, C.POINTER(ForwardIO), C.POINTER(Sampling)]
         L.slimt_b200_translate_sampled.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.POINTER(TranslateIO),
                                                    C.POINTER(Sampling)]
+        L.slimt_b200_model_forward_topk.argtypes = [C.c_void_p, C.POINTER(ForwardIO), C.POINTER(Sampling), C.c_int32]
+        L.slimt_b200_translate_topk.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.POINTER(TranslateIO),
+                                                C.POINTER(Sampling), C.c_int32]
         L.slimt_b200_score.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.POINTER(ScoreIO)]
         L.slimt_b200_translate_beam.argtypes = [C.POINTER(C.c_void_p), C.c_size_t, C.POINTER(TranslateIO), C.POINTER(Beam)]
         L.slimt_b200_shortlist_check.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t]
@@ -348,7 +352,8 @@ class Model:
                 want_scores: bool = False, sampling: Optional[dict] = None):
         """Model::forward on host buffers. Returns dict(step_tokens [steps,B], steps, target_tokens, ...); "scores"
         [steps,B] holds each step's log-probability of its chosen (or forced) word when want_scores.  sampling =
-        dict(temperature, seed, keys [B] or None) draws each word from the model's distribution (slimt_b200.h)."""
+        dict(temperature, seed, keys [B] or None) draws each word from the model's distribution (slimt_b200.h); with
+        "top_k" (0 .. 256) it calls slimt_b200_model_forward_topk, which draws from the top_k most likely words."""
         tokens = np.ascontiguousarray(tokens, dtype=np.uint32)
         lengths = np.ascontiguousarray(lengths, dtype=np.uint32)
         B, T = tokens.shape
@@ -383,6 +388,10 @@ class Model:
     def _forward(self, io: ForwardIO, sampling: Optional[dict], device_keys: bool = False):
         if sampling is None:
             _check(lib().slimt_b200_model_forward(self.h, C.byref(io)), "slimt_b200_model_forward")
+        elif "top_k" in sampling:
+            sp, _keys = _sampling(sampling, device_keys)
+            _check(lib().slimt_b200_model_forward_topk(self.h, C.byref(io), C.byref(sp), int(sampling["top_k"])),
+                   "slimt_b200_model_forward_topk")
         else:
             sp, _keys = _sampling(sampling, device_keys)
             _check(lib().slimt_b200_model_forward_sampled(self.h, C.byref(io), C.byref(sp)),
@@ -397,7 +406,8 @@ class Model:
         ragged sentences in (tokens, offsets), ragged targets out (out_tokens, out_offsets).  This is the C-ABI call a
         host integration makes; nothing is repacked.  want_scores: stats["scores"] is ragged like out_tokens (one
         log-probability per target token, EOS included); out_scores, when given, is that buffer.  sampling =
-        dict(temperature, seed, keys [n] or None): slimt_b200_translate_sampled, one key per sentence."""
+        dict(temperature, seed, keys [n] or None): slimt_b200_translate_sampled, one key per sentence; with "top_k",
+        slimt_b200_translate_topk."""
         n = len(offsets) - 1
         lens = np.diff(offsets.astype(np.int64))
         max_len = int(lens.max()) if n else 0
@@ -424,7 +434,12 @@ class Model:
         if sampling is not None:
             sp, _keys = _sampling(sampling)
             hs = (C.c_void_p * len(replicas or [self]))(*[r.h for r in (replicas or [self])])
-            _check(lib().slimt_b200_translate_sampled(hs, len(hs), C.byref(io), C.byref(sp)), "slimt_b200_translate_sampled")
+            if "top_k" in sampling:
+                _check(lib().slimt_b200_translate_topk(hs, len(hs), C.byref(io), C.byref(sp), int(sampling["top_k"])),
+                       "slimt_b200_translate_topk")
+            else:
+                _check(lib().slimt_b200_translate_sampled(hs, len(hs), C.byref(io), C.byref(sp)),
+                       "slimt_b200_translate_sampled")
         elif replicas is None:
             _check(lib().slimt_b200_translate(self.h, C.byref(io)), "slimt_b200_translate")
         else:

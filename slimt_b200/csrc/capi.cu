@@ -177,7 +177,12 @@ int slimt_b200_model_forward(slimt_b200_model* model, slimt_b200_forward_io* io)
 
 int slimt_b200_model_forward_sampled(slimt_b200_model* model, slimt_b200_forward_io* io,
                                      const slimt_b200_sampling* sampling) {
-  if (sb::check_sampling(sampling)) return 1;
+  return slimt_b200_model_forward_topk(model, io, sampling, 0);
+}
+
+int slimt_b200_model_forward_topk(slimt_b200_model* model, slimt_b200_forward_io* io,
+                                  const slimt_b200_sampling* sampling, int32_t top_k) {
+  if (sb::check_sampling(sampling) || sb::check_top_k(sampling, top_k)) return 1;
   if (sampling && io->forced) {
     sb::set_error("sampling: teacher forcing (forced) and sampling exclude each other");
     return 1;
@@ -191,6 +196,7 @@ int slimt_b200_model_forward_sampled(slimt_b200_model* model, slimt_b200_forward
   a.encoder_out = io->encoder_out, a.logits = io->logits, a.alignment = io->alignment;
   a.scores = io->token_scores;
   if (sampling) a.sample = true, a.inv_t = sb::sampling_inv_t(sampling->temperature), a.seed = sampling->seed, a.keys = sampling->keys;
+  a.top_k = top_k;
   int rc = sb::model_forward(model->m, a);
   io->steps = a.steps;
   io->target_tokens = a.target_tokens;
@@ -208,10 +214,15 @@ int slimt_b200_translate_multi(slimt_b200_model* const* replicas, size_t n_repli
 
 int slimt_b200_translate_sampled(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_translate_io* io,
                                  const slimt_b200_sampling* sampling) {
-  if (sb::check_sampling(sampling)) return 1;
+  return slimt_b200_translate_topk(replicas, n_replicas, io, sampling, 0);
+}
+
+int slimt_b200_translate_topk(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_translate_io* io,
+                              const slimt_b200_sampling* sampling, int32_t top_k) {
+  if (sb::check_sampling(sampling) || sb::check_top_k(sampling, top_k)) return 1;
   std::vector<sb::Model*> ms(n_replicas);
   for (size_t i = 0; i < n_replicas; i++) ms[i] = replicas && replicas[i] ? &replicas[i]->m : nullptr;
-  return sb::translate_multi(ms.data(), n_replicas, io, sampling);
+  return sb::translate_multi(ms.data(), n_replicas, io, sampling, nullptr, top_k);
 }
 
 int slimt_b200_translate_beam(slimt_b200_model* const* replicas, size_t n_replicas, slimt_b200_translate_io* io,

@@ -690,9 +690,10 @@ enum class Cross { Cached, Rc, Rcl };
 const char* const kSelfAttnName[] = {"Fused", "Rowwise", "Tiled", "Long"};  // indexed by SelfAttn
 
 enum class EncFfn { Rows, Gemm };
-// output: the fused argmax GEMM (out_argmax.cu, in the encoding Model::load chose), logits tap + argmax_rows, or the
-// scores GEMM (the fused GEMM with every logit evaluated exactly) + score_step or sample_step
-enum class Out { Argmax, Logits, Scores };
+// output: the fused argmax GEMM (out_argmax.cu, in the encoding Model::load chose), logits tap + argmax_rows, the
+// scores GEMM (the fused GEMM with every logit evaluated exactly) + score_step or sample_step, or the logits GEMM alone +
+// topk_sample (top-k sampling, which needs every logit of a row)
+enum class Out { Argmax, Logits, Scores, TopK };
 
 struct Routes {
   SelfAttn self;
@@ -703,7 +704,7 @@ struct Routes {
 
 // Which kernel runs each stage of one forward call that has more than one.  The two environment variables are read on
 // every call, so that tests can switch kernels between calls; a value not listed below means the default.
-Routes choose_routes(const Model& m, int T, int B, bool fast, bool logits, bool scores) {
+Routes choose_routes(const Model& m, int T, int B, bool fast, bool logits, bool scores, bool topk) {
   const int E = m.E, H = m.H, dh = m.dh;
   auto env_is = [](const char* env, const char* v) { return env != nullptr && strcmp(env, v) == 0; };
   Routes r{};
@@ -741,8 +742,9 @@ Routes choose_routes(const Model& m, int T, int B, bool fast, bool logits, bool 
   r.ffn = E == 256 && m.F == 1536 ? EncFfn::Rows : EncFfn::Gemm;
 
   // a caller that wants the logits gets them from the tap (and scores or samples, when asked for, from them); scores
-  // or samples alone come from the scores epilogue of the fused GEMM
-  r.out = logits ? Out::Logits : scores ? Out::Scores : Out::Argmax;
+  // or samples alone come from the scores epilogue of the fused GEMM.  Top-k sampling reads the tap's logits, whether
+  // or not the caller wants a copy.
+  r.out = topk ? Out::TopK : logits ? Out::Logits : scores ? Out::Scores : Out::Argmax;
   return r;
 }
 
@@ -841,7 +843,7 @@ int Pass::plan() {
   scoring = a.targets != nullptr;
   K = a.beam > 0 ? a.beam : 1;
   fast = c.fast && !scoring && a.beam == 0;
-  route = choose_routes(m, T, B, fast, a.logits != nullptr, a.scores != nullptr || a.sample);
+  route = choose_routes(m, T, B, fast, a.logits != nullptr, a.scores != nullptr || a.sample, a.top_k > 0);
   if (scoring || a.beam > 0) {
     // T_target (or K) queries read each layer's cross K/V: projected once (Cached); every logit evaluated exactly (Scores)
     route.cross = Cross::Cached;
@@ -904,9 +906,10 @@ int Pass::plan_step(Workspace& ws) {
     ws.add(d_steps, SB);
     if (a.forced) ws.add(d_forced, SB);
   }
-  if (route.out == Out::Logits) ws.add(d_logits, static_cast<size_t>(B) * Nout);
+  if (route.out == Out::Logits || route.out == Out::TopK) ws.add(d_logits, static_cast<size_t>(B) * Nout);
   if (a.scores && !a.device_io) ws.add(d_scores, SB);
-  if (a.scores || a.sample) ws.add(partials, (Nout + kScoreStrip - 1) / kScoreStrip * static_cast<size_t>(B));
+  if ((a.scores || a.sample) && route.out != Out::TopK)
+    ws.add(partials, (Nout + kScoreStrip - 1) / kScoreStrip * static_cast<size_t>(B));
   if (a.sample && a.keys && !a.device_io) ws.add(d_keys, B);
   // head-0 probabilities of every step stay on the device and come back in one copy after the loop
   if (a.alignment) ws.add(d_align_all, SB * K * T);
@@ -954,11 +957,12 @@ QuantOuts Pass::enc_inputs(int i) {
 }
 
 // Where decoder layer l's output goes: after the last layer only into the output operand (signed for the fused GEMMs,
-// u8 for the logits tap's generic GEMM); after an earlier layer into z and the next layer's SSRU operands xf and xw.
+// u8 for the generic logits GEMM of the tap and of top-k); after an earlier layer into z and the next layer's SSRU
+// operands xf and xw.
 void Pass::dec_layer_out(RowsFfnArgs& k, int l, float* z, int8_t* xf, int8_t* xw) const {
   if (l + 1 == Ld) {
     k.zq[0] = reinterpret_cast<uint8_t*>(oq), k.zaq[0] = m.out.aq, k.n_zq = 1;
-    k.zq_signed = route.out == Out::Logits ? 0 : 1;
+    k.zq_signed = route.out == Out::Logits || route.out == Out::TopK ? 0 : 1;
   } else {
     k.z_out = z;
     k.zq[0] = reinterpret_cast<uint8_t*>(xf), k.zaq[0] = m.dec[l + 1].rnn_wf.aq;
@@ -974,7 +978,7 @@ ScoreStepArgs Pass::score_step_args(int rows, const int8_t* oq_rows, const uint3
   ScoreStepArgs k{};
   k.partials = partials, k.best = best, k.forced = forced, k.shortlist = use_sl ? d_sl : nullptr;
   k.oq = oq_rows, k.w = out.w, k.c127 = out.c127, k.pb = out.pb, k.um = out.um;
-  k.logits = route.out == Out::Logits ? d_logits : nullptr;
+  k.logits = route.out == Out::Logits || route.out == Out::TopK ? d_logits : nullptr;
   k.B = rows, k.N = Nout, k.K = E, k.step = step, k.scores = scores;
   return k;
 }
@@ -1245,20 +1249,22 @@ int Pass::decode_step(int step) {
     }
   }
   // output projection (+ shortlist) and greedy choice (Transformer.cc:176-182, 279-339)
-  if (route.out == Out::Logits) {
+  if (route.out == Out::Logits || route.out == Out::TopK) {
     GemmCall g(&c, "dec_gemm_out_logits", B, Nout, E, EPI_F32);
     GemmProblem* p = g.add(oq, out.w, out.pb, out.um);
     if (!p) return 1;
     p->out = d_logits, p->ldo = Nout;
     if (g.launch()) return 1;
-    {
+    if (route.out == Out::Logits) {
       LaunchScope ls(c, "argmax_rows", 0, 4.0 * B * Nout);
       launch_argmax_rows(d_logits, B, Nout, best, s);
     }
-    SB_CUDA(cudaMemcpyAsync(a.logits + static_cast<size_t>(step) * B * Nout, d_logits, 4ul * B * Nout,
-                            cudaMemcpyDeviceToHost, s));
-    c.d2h_bytes += 4ul * B * Nout;
-    if (a.scores || a.sample) {
+    if (a.logits) {
+      SB_CUDA(cudaMemcpyAsync(a.logits + static_cast<size_t>(step) * B * Nout, d_logits, 4ul * B * Nout,
+                              cudaMemcpyDeviceToHost, s));
+      c.d2h_bytes += 4ul * B * Nout;
+    }
+    if ((a.scores || a.sample) && route.out == Out::Logits) {
       LaunchScope ls(c, "score_rows", 0, 4.0 * B * Nout + 8.0 * B * ((Nout + kScoreStrip - 1) / kScoreStrip));
       launch_score_rows(d_logits, B, Nout, partials, a.sample ? a.inv_t : 1.0f, s);
     }
@@ -1309,7 +1315,14 @@ int Pass::decode_step(int step) {
     ScoreStepArgs k = score_step_args(B, oq, d_forced, step, d_scores);
     k.inv_t = a.inv_t, k.seed = a.seed, k.keys = d_keys;
     const double strips = (Nout + kScoreStrip - 1) / kScoreStrip;
-    if (a.sample) {
+    if (route.out == Out::TopK) {
+      // the row's logits, read twice (the first digit's histogram, then the columns it stages)
+      LaunchScope ls(c, "topk_sample", 0, 8.0 * B * Nout + 24.0 * B);
+      if (launch_topk_sample(k, a.top_k, s)) {
+        set_error("top-k sampling: step kernel launch failed");
+        return 1;
+      }
+    } else if (a.sample) {
       // the chosen strip's 64 columns are re-evaluated: 64 weight rows and the row's operand (or 64 tap logits)
       LaunchScope ls(c, "sample_step", 0, 8.0 * B * strips + 24.0 * B + (k.logits ? 256.0 : 65.0 * E) * B);
       if (launch_sample_step(k, s)) {

@@ -198,6 +198,9 @@ struct ForwardArgs {
   float inv_t = 1.0f;
   uint64_t seed = 0;
   const uint64_t* keys = nullptr;
+  // Top-k sampling (DESIGN §4.4e), with sample set: each step's word drawn from the first top_k (1 .. 256) columns by
+  // (logit descending, column ascending) of the logits GEMM's output; 0 = from every column, as above.
+  int top_k = 0;
   // Scoring pass (model_score_on, DESIGN §4.4c): the given targets [B][target_T] (host, padded), scored at every
   // position into scores [B][target_T]; alignment, when set, receives [B][target_T][T].
   const uint32_t* targets = nullptr;

@@ -411,6 +411,232 @@ __global__ void __launch_bounds__(32 * kScoreWarps) sample_step_kernel(ScoreStep
         static_cast<float>(static_cast<double>(zc) - (static_cast<double>(M) + log(S)));
 }
 
+// ------------------------------------------------------------------ top-k sampling
+// One block per row over the row's logits [N] (include/slimt_b200.h, DESIGN §4.4e).  S_k, the first min(k, N) columns
+// by (y descending, column ascending), is the set of columns whose 32-bit order key (pack_best's high word) lies above
+// a threshold key, plus the first columns equal to it.  The threshold comes from a radix select over the key in three
+// digits (12, 10, 10 bits); each digit's histogram is built with shared-memory atomics, whose counts do not depend on
+// their order.  After the first digit, every column at or above the boundary bin is compacted, in column order, into a
+// shared buffer when it fits there, and the later digits and the final compaction read that buffer instead of the row.
+constexpr int kTopkThreads = 512;
+constexpr int kTopkStage = 2048;  // staged columns
+constexpr int kTopkBins = 4096;   // bins of the first digit
+
+__device__ __forceinline__ uint32_t order_key(float y) { return static_cast<uint32_t>(pack_best(y, 0u) >> 32); }
+
+// Exclusive prefix sum of v over the block's threads in thread order; total receives the block's sum.  Every thread
+// calls it.
+__device__ __forceinline__ int block_exclusive_scan(int v, int* ws, int& total) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = kTopkThreads / 32;
+  int x = v;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int y = __shfl_up_sync(0xffffffffu, x, o);
+    if (lane >= o) x += y;
+  }
+  if (lane == 31) ws[w] = x;
+  __syncthreads();
+  if (w == 0) {
+    int s = lane < nw ? ws[lane] : 0;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int y = __shfl_up_sync(0xffffffffu, s, o);
+      if (lane >= o) s += y;
+    }
+    ws[lane] = s;
+  }
+  __syncthreads();
+  const int before = (w > 0 ? ws[w - 1] : 0) + x - v;
+  total = ws[nw - 1];
+  __syncthreads();
+  return before;
+}
+
+// The row's columns in ascending order: four consecutive columns per thread and round, float4 loads (N % 8 == 0).
+struct TopkRow {
+  const float* y;
+  int n;
+  __device__ __forceinline__ void load4(int i, float (&v)[4], uint32_t (&c)[4]) const {
+    const float4 q = *reinterpret_cast<const float4*>(y + i);
+    v[0] = q.x, v[1] = q.y, v[2] = q.z, v[3] = q.w;
+#pragma unroll
+    for (int j = 0; j < 4; j++) c[j] = static_cast<uint32_t>(i + j);
+  }
+};
+// The staged columns, still in ascending order.
+struct TopkStaged {
+  const float* y;
+  const uint32_t* col;
+  int n;
+  __device__ __forceinline__ void load4(int i, float (&v)[4], uint32_t (&c)[4]) const {
+#pragma unroll
+    for (int j = 0; j < 4; j++) v[j] = i + j < n ? y[i + j] : 0.0f, c[j] = i + j < n ? col[i + j] : 0u;
+  }
+};
+
+// Calls f(valid, value, column, key) for every element of src, four per thread and round, every thread the same
+// number of times (so f may hold block barriers).
+template <class Src, class F>
+__device__ __forceinline__ void topk_rounds(const Src& src, F&& f) {
+  for (int base = 0; base < src.n; base += 4 * kTopkThreads) {
+    const int i = base + 4 * static_cast<int>(threadIdx.x);
+    float v[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+    uint32_t c[4] = {0u, 0u, 0u, 0u};
+    if (i < src.n) src.load4(i, v, c);
+    bool ok[4];
+    uint32_t key[4];
+#pragma unroll
+    for (int j = 0; j < 4; j++) ok[j] = i + j < src.n, key[j] = order_key(v[j]);
+    f(ok, v, c, key);
+  }
+}
+
+struct TopkSelect {
+  uint32_t prefix, mask;  // the candidates: keys with (key & mask) == prefix
+  int need;               // how many of the candidates belong to S_k
+};
+
+// One digit of the radix select: the histogram of bits [shift, shift + log2(bins)) over the candidates, and the bin in
+// which the need-th largest candidate lies.  The candidates in higher bins all belong to S_k.
+template <class Src>
+__device__ void topk_digit(const Src& src, int shift, int bins, TopkSelect& s, int* hist, int* ws, int* found) {
+  for (int i = threadIdx.x; i < bins; i += kTopkThreads) hist[i] = 0;
+  __syncthreads();
+  const uint32_t prefix = s.prefix, mask = s.mask, dmask = static_cast<uint32_t>(bins - 1);
+  topk_rounds(src, [&](const bool (&ok)[4], const float (&)[4], const uint32_t (&)[4], const uint32_t (&key)[4]) {
+#pragma unroll
+    for (int j = 0; j < 4; j++)
+      if (ok[j] && (key[j] & mask) == prefix) atomicAdd(&hist[(key[j] >> shift) & dmask], 1);
+  });
+  __syncthreads();
+  // thread t owns the chunk of bins kTopkThreads - 1 - t, so its exclusive scan is the count in higher bins
+  const int per = bins / kTopkThreads, first = (kTopkThreads - 1 - static_cast<int>(threadIdx.x)) * per;
+  int local = 0;
+  for (int k = 0; k < per; k++) local += hist[first + k];
+  int total;
+  int above = block_exclusive_scan(local, ws, total);
+  if (above < s.need && above + local >= s.need)
+    for (int k = per - 1; k >= 0; k--) {
+      if (above + hist[first + k] >= s.need) {
+        found[0] = first + k, found[1] = above;
+        break;
+      }
+      above += hist[first + k];
+    }
+  __syncthreads();
+  s.prefix |= static_cast<uint32_t>(found[0]) << shift, s.mask |= dmask << shift, s.need -= found[1];
+  __syncthreads();
+}
+
+// The last two digits over src, then S_k in ascending column order into (sy, sc): every column whose key is above
+// the threshold, and the first `need` columns equal to it.  Returns |S_k|.
+template <class Src>
+__device__ int topk_finish(const Src& src, TopkSelect s, int* hist, int* ws, int* found, float* sy, uint32_t* sc) {
+  topk_digit(src, 10, 1024, s, hist, ws, found);
+  topk_digit(src, 0, 1024, s, hist, ws, found);
+  const uint32_t thr = s.prefix;
+  int eq_before = 0, out_before = 0;
+  topk_rounds(src, [&](const bool (&ok)[4], const float (&v)[4], const uint32_t (&c)[4], const uint32_t (&key)[4]) {
+    int n_eq = 0;
+#pragma unroll
+    for (int j = 0; j < 4; j++) n_eq += ok[j] && key[j] == thr;
+    int eq_total;
+    int rank = eq_before + block_exclusive_scan(n_eq, ws, eq_total);
+    bool in[4];
+    int n_in = 0;
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+      const bool eq = ok[j] && key[j] == thr;
+      in[j] = ok[j] && (key[j] > thr || (eq && rank < s.need));
+      rank += eq;
+      n_in += in[j];
+    }
+    int in_total;
+    int pos = out_before + block_exclusive_scan(n_in, ws, in_total);
+#pragma unroll
+    for (int j = 0; j < 4; j++)
+      if (in[j]) sy[pos] = v[j], sc[pos] = c[j], pos++;
+    eq_before += eq_total, out_before += in_total;
+  });
+  return out_before;
+}
+
+// Per row: S_k (above), then warp 0 tempers its logits and their maximum M, every thread one term score_exp(z - M), and
+// thread 0 sums the terms in ascending column order in double, draws u * S and walks the running sum to the word.
+__global__ void __launch_bounds__(kTopkThreads) topk_sample_kernel(ScoreStepArgs a, int top_k) {
+  __shared__ int hist[kTopkBins];
+  __shared__ float stage_y[kTopkStage];
+  __shared__ uint32_t stage_c[kTopkStage];
+  __shared__ float sy[kMaxTopK], se[kMaxTopK];
+  __shared__ uint32_t sc[kMaxTopK];
+  __shared__ int ws[32], found[2];
+  __shared__ float m_all;
+  const int b = blockIdx.x, N = a.N;
+  pdl_launch_dependents();
+  pdl_wait();
+  const TopkRow row{a.logits + static_cast<size_t>(b) * N, N};
+  TopkSelect s{0u, 0u, min(top_k, N)};
+  topk_digit(row, 20, kTopkBins, s, hist, ws, found);
+  // the columns in bins at or above the boundary: those above it and the boundary bin's own
+  const int first_bin = static_cast<int>(s.prefix >> 20);
+  int staged = 0;
+  for (int i = threadIdx.x; i < kTopkBins; i += kTopkThreads) staged += i >= first_bin ? hist[i] : 0;
+  int n_stage;
+  block_exclusive_scan(staged, ws, n_stage);
+  int n;
+  if (n_stage <= kTopkStage) {
+    int out_before = 0;
+    topk_rounds(row, [&](const bool (&ok)[4], const float (&v)[4], const uint32_t (&c)[4], const uint32_t (&key)[4]) {
+      bool in[4];
+      int n_in = 0;
+#pragma unroll
+      for (int j = 0; j < 4; j++) in[j] = ok[j] && static_cast<int>(key[j] >> 20) >= first_bin, n_in += in[j];
+      int in_total;
+      int pos = out_before + block_exclusive_scan(n_in, ws, in_total);
+#pragma unroll
+      for (int j = 0; j < 4; j++)
+        if (in[j]) stage_y[pos] = v[j], stage_c[pos] = c[j], pos++;
+      out_before += in_total;
+    });
+    __syncthreads();
+    n = topk_finish(TopkStaged{stage_y, stage_c, n_stage}, s, hist, ws, found, sy, sc);
+  } else {  // many equal or nearly equal logits: the later digits read the row again
+    n = topk_finish(row, s, hist, ws, found, sy, sc);
+  }
+  __syncthreads();
+  const int t = threadIdx.x;
+  const float z = t < n ? __fmul_rn(sy[t], a.inv_t) : -__int_as_float(0x7f800000);
+  if (t < 32) {
+    float m = z;
+    for (int i = t + 32; i < n; i += 32) m = fmaxf(m, __fmul_rn(sy[i], a.inv_t));
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+    if (t == 0) m_all = m;
+  }
+  __syncthreads();
+  const float M = m_all;
+  if (t < n) se[t] = score_exp(__fsub_rn(z, M));
+  __syncthreads();
+  if (t != 0) return;
+  double S = 0.0;
+  for (int i = 0; i < n; i++) S += static_cast<double>(se[i]);
+  const uint64_t key = a.keys ? a.keys[b] : static_cast<uint64_t>(b);
+  const double target = sample_uniform(a.seed, key, static_cast<uint32_t>(a.step)) * S;
+  double acc = 0.0;
+  int c = -1;
+  for (int i = 0; i < n; i++) {
+    if (se[i] == 0.0f) continue;
+    c = i;
+    acc += static_cast<double>(se[i]);
+    if (acc > target) break;
+  }
+  const float zc = __fmul_rn(sy[c], a.inv_t);
+  a.best[b] = pack_best(zc, sc[c]);
+  if (a.scores)
+    a.scores[static_cast<size_t>(a.step) * a.B + b] =
+        static_cast<float>(static_cast<double>(zc) - (static_cast<double>(M) + log(S)));
+}
+
 // ------------------------------------------------------------------ beam search
 // Candidates are packed as in packed_best.cuh, so a larger key ranks first and equal values go to the lower index.
 // top[0..7] holds the largest keys seen, descending (0 = empty); keys are distinct.
@@ -668,6 +894,12 @@ int launch_score_step(const ScoreStepArgs& a, cudaStream_t stream) {
 int launch_sample_step(const ScoreStepArgs& a, cudaStream_t stream) {
   if (a.B == 0) return 0;
   return launch_pdl(sample_step_kernel, dim3((a.B + 31) / 32), dim3(32 * kScoreWarps), 0, stream, a) != cudaSuccess ? 1 : 0;
+}
+
+int launch_topk_sample(const ScoreStepArgs& a, int top_k, cudaStream_t stream) {
+  if (a.B == 0) return 0;
+  if (top_k < 1 || top_k > kMaxTopK || a.logits == nullptr) return 1;
+  return launch_pdl(topk_sample_kernel, dim3(a.B), dim3(kTopkThreads), 0, stream, a, top_k) != cudaSuccess ? 1 : 0;
 }
 
 int launch_beam_topk(const BeamStepArgs& a, cudaStream_t stream) {

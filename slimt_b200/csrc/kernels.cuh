@@ -145,6 +145,12 @@ struct ScoreStepArgs {
 };
 int launch_score_step(const ScoreStepArgs& a, cudaStream_t stream);
 int launch_sample_step(const ScoreStepArgs& a, cudaStream_t stream);
+// Top-k sampling (include/slimt_b200.h, DESIGN §4.4e) over the tap logits a.logits [B][N], one block per row: the word
+// is drawn from the first min(top_k, N) columns by (logit descending, column ascending), tempered, with their terms
+// summed in ascending column order; best[b] = pack_best(z[c], c) and, when scores is set, scores[step][b] = z[c] -
+// log-sum of the set.  Returns nonzero for top_k outside 1 .. kMaxTopK or without logits.
+constexpr int kMaxTopK = 256;
+int launch_topk_sample(const ScoreStepArgs& a, int top_k, cudaStream_t stream);
 
 // Beam search (include/slimt_b200.h, DESIGN §4.4d).  Sentence b owns decoder rows b * beam + k (slot k); width[b] is
 // the number of hypotheses it still has to finish (beam - finished), and its live slots are 0 .. width[b] - 1 (slot 0

@@ -51,14 +51,17 @@ struct slimt_b200_beam;
 namespace sb {
 // exhaust() over one request with the batches dealt to the replicas' lanes (translate.cu); with beam set, each batch
 // runs beam search (engine.cu: model_beam_on) and io receives every sentence's best hypothesis
+// run beam search; with sampling and top_k > 0, each batch samples from the top_k columns of every step
 int translate_multi(Model* const* models, size_t n_replicas, slimt_b200_translate_io* io,
-                    const slimt_b200_sampling* sampling, slimt_b200_beam* beam = nullptr);
+                    const slimt_b200_sampling* sampling, slimt_b200_beam* beam = nullptr, int top_k = 0);
 // The same batches and lanes scoring given targets with the time-parallel pass (engine.cu: model_score_on)
 int score_multi(Model* const* models, size_t n_replicas, slimt_b200_score_io* io);
 
 // Sampling arguments of the C ABI: nonzero (and the error set) for a temperature that is not finite or lies outside
 // [1e-3, 1e3]; sampling = null (greedy) passes.
 int check_sampling(const slimt_b200_sampling* sampling);
+// Top-k arguments of the C ABI: nonzero (and the error set) for top_k outside 0 .. 256, or top_k > 0 without sampling.
+int check_top_k(const slimt_b200_sampling* sampling, int top_k);
 // inv_t = (float)(1.0 / (double)temperature)
 inline float sampling_inv_t(float temperature) { return static_cast<float>(1.0 / static_cast<double>(temperature)); }
 }  // namespace sb

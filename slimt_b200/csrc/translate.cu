@@ -296,6 +296,18 @@ int check_sampling(const slimt_b200_sampling* sampling) {
   return 0;
 }
 
+int check_top_k(const slimt_b200_sampling* sampling, int top_k) {
+  if (top_k < 0 || top_k > kMaxTopK) {
+    set_error("top-k sampling: top_k must be in 0 .. " + std::to_string(kMaxTopK) + ", got " + std::to_string(top_k));
+    return 1;
+  }
+  if (top_k > 0 && sampling == nullptr) {
+    set_error("top-k sampling: top_k > 0 needs sampling parameters (temperature, seed, keys)");
+    return 1;
+  }
+  return 0;
+}
+
 int check_beam(const slimt_b200_beam* beam) {
   if (beam == nullptr) return 0;
   if (beam->beam_size < 1 || beam->beam_size > kMaxBeam) {
@@ -314,7 +326,7 @@ int check_beam(const slimt_b200_beam* beam) {
 }
 
 int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io* io, const slimt_b200_sampling* sampling,
-                    slimt_b200_beam* beam) {
+                    slimt_b200_beam* beam, int top_k) {
   if (check_beam(beam)) return 1;
   Service sv{models, n_rep, beam ? "translate_beam" : "translate"};
   if (sv.check_replicas()) return 1;
@@ -423,6 +435,7 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
       uint64_t* keys = reinterpret_cast<uint64_t*>(stage + key_off);
       for (size_t r = 0; r < B; r++) keys[r] = sampling->keys ? sampling->keys[p.ids[r]] : static_cast<uint64_t>(p.ids[r]);
       a.sample = true, a.inv_t = sampling_inv_t(sampling->temperature), a.seed = sampling->seed, a.keys = keys;
+      a.top_k = top_k;
     }
     if (model_forward_on(m, c, a)) return 1;
     Done& d = done[bi];

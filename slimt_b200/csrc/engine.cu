@@ -495,29 +495,6 @@ namespace {
 // Rows of the scoring pass's output layer per launch: bounds its strip partials to ceil(N / 64) * 16 k * 8 bytes.
 constexpr int kScoreChunk = 16384;
 
-// The device buffers of one call, each listed once: add() records where a buffer's pointer goes and how many elements
-// it holds; carve() reserves the sum in the context's arena and hands out the pointers in list order, each buffer
-// starting on a 256-byte boundary.
-// Margin behind the last buffer: not every kernel has been shown to keep its loads inside its buffer (the output GEMMs
-// index per-column arrays by 256-column tile), so the arena keeps ending with 16 KB that no buffer owns.
-constexpr size_t kTailPad = 64 * 256;
-
-struct Workspace {
-  size_t bytes = kTailPad;
-  std::vector<std::pair<void**, size_t>> bufs;
-  template <class T>
-  void add(T*& slot, size_t count) {
-    bufs.emplace_back(reinterpret_cast<void**>(&slot), (count * sizeof(T) + 255) & ~size_t(255));
-    bytes += bufs.back().second;
-  }
-  int carve(Context& c) const {
-    if (c.reserve(bytes)) return 1;
-    char* p = c.arena;
-    for (const auto& b : bufs) *b.first = p, p += b.second;
-    return 0;
-  }
-};
-
 }  // namespace
 
 // ------------------------------------------------------------------ GEMM helpers
@@ -796,10 +773,12 @@ struct Pass {
   CUtensorMap map_xq[2], map_zq[2], map_caq;  // u8 activation operands of the row-tile kernels, box {128 B, 32 rows}
   CUtensorMap map_oq;
   int plan(), plan_step(Workspace& ws), plan_score(Workspace& ws), carve(const Workspace& ws);
-  int encode(), prepare_cross(), prepare_output(), decode_step(int step), decode(), score(), beam_search();
+  int encode(), prepare_cross(), prepare_output(), decode_step(int step), decode(), score();
   int poll_done(int step, bool* all_done);
   QuantOuts enc_inputs(int i);
-  void dec_layer_out(RowsFfnArgs& k, int l, float* z, int8_t* xf, int8_t* xw) const;
+  int cross_attention_mq(int l, int queries, float* al, const char* tag, const char* what);
+  int wo_ffn(int l, float* z, int8_t* xf, int8_t* xw, const char* tag);
+  int scores_gemm(const CUtensorMap& map, int rows, const char* tag);
   ScoreStepArgs score_step_args(int rows, const int8_t* oq_rows, const uint32_t* forced, int step, float* scores) const;
 };
 
@@ -956,11 +935,36 @@ QuantOuts Pass::enc_inputs(int i) {
   return q;
 }
 
-// Where decoder layer l's output goes: after the last layer only into the output operand (signed for the fused GEMMs,
-// u8 for the generic logits GEMM of the tap and of top-k); after an earlier layer into z and the next layer's SSRU
-// operands xf and xw.
-void Pass::dec_layer_out(RowsFfnArgs& k, int l, float* z, int8_t* xf, int8_t* xw) const {
-  if (l + 1 == Ld) {
+// Multi-query cross-attention of decoder layer l against its cached K/V, `queries` consecutive rows per sentence (beam
+// search's K slots, the scoring pass's Tt target positions); head 0's probabilities go to al when it is set.  `what`
+// names the path in the error.
+int Pass::cross_attention_mq(int l, int queries, float* al, const char* tag, const char* what) {
+  QuantOuts q = qouts();
+  qadd(q, caq, m.dec[l].ctx.o.aq);
+  const double Md = M, Ed = E;
+  LaunchScope ls(c, tag, 4.0 * Md * (src_tokens / B) * Ed,
+                 Md * Ed * 5.0 + 2.0 * src_tokens * Ed * 4.0 + (al ? 4.0 * Md * T : 0.0));
+  const int rc = self_attention_tiled_supported(T, dh)
+                     ? launch_self_attention_tiled(qd, Kc[l], Vc[l], d_lengths, B, T, H, dh, q, s, queries, al)
+                     : launch_self_attention_long(qd, Kc[l], Vc[l], d_lengths, B, T, H, dh, q, s, queries, al);
+  if (rc) {
+    set_error(std::string(what) + " cross-attention: no kernel for head size " + std::to_string(dh) + " over " +
+              std::to_string(T) + " source tokens");
+    return 1;
+  }
+  return 0;
+}
+
+// Wo + residual + LN, FFN1 + ReLU, FFN2 + residual + LN of decoder layer l over the M rows in one row-tile kernel
+// (Modules.cc:308-316, 251-257).  After the last layer the output goes only into the output operand (signed for the
+// fused GEMMs, u8 for the generic logits GEMM of the tap and of top-k); after an earlier layer into z and the next
+// layer's SSRU operands xf and xw.
+int Pass::wo_ffn(int l, float* z, int8_t* xf, int8_t* xw, const char* tag) {
+  const DecLayerW& L = m.dec[l];
+  const bool last = l + 1 == Ld;
+  RowsFfnArgs k = rows_ffn_args(L.ctx, L.ffn, hb, M);
+  k.map_a = map_caq;
+  if (last) {
     k.zq[0] = reinterpret_cast<uint8_t*>(oq), k.zaq[0] = m.out.aq, k.n_zq = 1;
     k.zq_signed = route.out == Out::Logits || route.out == Out::TopK ? 0 : 1;
   } else {
@@ -969,6 +973,26 @@ void Pass::dec_layer_out(RowsFfnArgs& k, int l, float* z, int8_t* xf, int8_t* xw
     k.zq[1] = reinterpret_cast<uint8_t*>(xw), k.zaq[1] = m.dec[l + 1].rnn_w.aq;
     k.n_zq = 2;
   }
+  const double Md = M, Ed = E, Fd = F;
+  LaunchScope ls(c, tag, 2.0 * Md * (Ed * Ed + 2.0 * Ed * Fd),
+                 Ed * Ed + 2.0 * Ed * Fd + Md * Ed * (1.0 + 4.0 + (last ? 1.0 : 6.0)));
+  if (launch_rows_ffn(k, E, F, kRowTile, fast, s)) {
+    set_error("fused FFN kernel: unsupported sizes E=" + std::to_string(E) + " F=" + std::to_string(F));
+    return 1;
+  }
+  return 0;
+}
+
+// The output GEMM with the scores epilogue over `rows` rows of the operand `map`: every logit evaluated exactly, each
+// row's best column into best and its strip partials (of the logits tempered by inv_t when sampling) into partials.
+int Pass::scores_gemm(const CUtensorMap& map, int rows, const char* tag) {
+  const double Rd = rows, Nd = Nout, Kd = E, strips = (Nout + kScoreStrip - 1) / kScoreStrip;
+  LaunchScope ls(c, tag, 2.0 * Rd * Nd * Kd, Rd * Kd + Nd * Kd + 8.0 * Nd + 8.0 * Rd + 8.0 * Rd * strips);
+  if (launch_out_scores(out, map, rows, E, best, partials, a.sample ? a.inv_t : 1.0f, c.num_sms, s)) {
+    set_error("output GEMM (scores): unsupported K " + std::to_string(E));
+    return 1;
+  }
+  return 0;
 }
 
 // score_step's arguments for `rows` output rows whose operands start at oq_rows; forced and scores are [step][rows].
@@ -1191,20 +1215,7 @@ int Pass::decode_step(int step) {
       }
     }
     if (beam) {  // K queries per sentence against its cached K/V, as the scoring pass runs them
-      QuantOuts q = qouts();
-      qadd(q, caq, L.ctx.o.aq);
-      float* al = last ? d_align : nullptr;
-      const double Md = M, Ed = E;
-      LaunchScope ls(c, "beam_cross_attention", 4.0 * Md * (src_tokens / B) * Ed,
-                     Md * Ed * 5.0 + 2.0 * src_tokens * Ed * 4.0 + (al ? 4.0 * Md * T : 0.0));
-      const int rc = self_attention_tiled_supported(T, dh)
-                         ? launch_self_attention_tiled(qd, Kc[l], Vc[l], d_lengths, B, T, H, dh, q, s, K, al)
-                         : launch_self_attention_long(qd, Kc[l], Vc[l], d_lengths, B, T, H, dh, q, s, K, al);
-      if (rc) {
-        set_error("beam cross-attention: no kernel for head size " + std::to_string(dh) + " over " + std::to_string(T) +
-                  " source tokens");
-        return 1;
-      }
+      if (cross_attention_mq(l, K, last ? d_align : nullptr, "beam_cross_attention", "beam")) return 1;
     } else if (route.cross != Cross::Cached) {
       CrossRcArgs k{};
       k.map_ak = mapK[l], k.map_av = mapV[l];
@@ -1235,18 +1246,7 @@ int Pass::decode_step(int step) {
         return 1;
       }
     }
-    {  // Wo + residual + LN, FFN1 + ReLU, FFN2 + residual + LN in one row-tile kernel (Modules.cc:308-316, 251-257)
-      RowsFfnArgs k = rows_ffn_args(L.ctx, L.ffn, hb, M);
-      k.map_a = map_caq;
-      dec_layer_out(k, l, zb, zq[0], zq[1]);
-      const double Bd = M, Ed = E, Fd = F;
-      LaunchScope ls(c, "dec_wo_ffn_fused", 2.0 * Bd * (Ed * Ed + 2.0 * Ed * Fd),
-                     Ed * Ed + 2.0 * Ed * Fd + Bd * Ed * (1.0 + 4.0 + (last ? 1.0 : 6.0)));
-      if (launch_rows_ffn(k, E, F, kRowTile, fast, s)) {
-        set_error("fused FFN kernel: unsupported sizes E=" + std::to_string(E) + " F=" + std::to_string(F));
-        return 1;
-      }
-    }
+    if (wo_ffn(l, zb, zq[0], zq[1], "dec_wo_ffn_fused")) return 1;
   }
   // output projection (+ shortlist) and greedy choice (Transformer.cc:176-182, 279-339)
   if (route.out == Out::Logits || route.out == Out::TopK) {
@@ -1269,12 +1269,7 @@ int Pass::decode_step(int step) {
       launch_score_rows(d_logits, B, Nout, partials, a.sample ? a.inv_t : 1.0f, s);
     }
   } else if (route.out == Out::Scores) {
-    const double Md = M, Nd = Nout, Kd = E, strips = (Nout + kScoreStrip - 1) / kScoreStrip;
-    LaunchScope ls(c, "dec_gemm_out_scores", 2.0 * Md * Nd * Kd, Md * Kd + Nd * Kd + 8.0 * Nd + 8.0 * Md + 8.0 * Md * strips);
-    if (launch_out_scores(out, map_oq, M, E, best, partials, a.sample ? a.inv_t : 1.0f, c.num_sms, s)) {
-      set_error("output GEMM (scores): unsupported K " + std::to_string(E));
-      return 1;
-    }
+    if (scores_gemm(map_oq, M, "dec_gemm_out_scores")) return 1;
   } else {
     const double Md = B, Nd = Nout, Kd = E;
     LaunchScope ls(c, "dec_gemm_out_argmax", 2.0 * Md * Nd * Kd, Md * Kd + Nd * Kd + 4.0 * Nd + 8.0 * Md);
@@ -1360,90 +1355,98 @@ int Pass::poll_done(int step, bool* all_done) {
   return 0;
 }
 
-// The decode loop (Model.cc:111-185) with its early exit, the kernel that closes the last step, and the result copies.
+// The decode loop (Model.cc:111-185) over the M decoder rows with its early exit, then the result copies: greedy
+// decoding closes its last step with one more kernel and returns the step matrix, lengths and scores; beam search
+// (DESIGN §4.4d) returns the step records and finished hypotheses from which the host rebuilds and ranks each
+// sentence's hypotheses.
 int Pass::decode() {
-  int executed = 0, host_done = 0;
-  for (int l = 0; l < Ld; l++) SB_CUDA(cudaMemsetAsync(state[l], 0, 4ul * B * E, s));  // Decoder::start_states
-  SB_CUDA(cudaMemsetAsync(best, 0, 8ul * B, s));
-  SB_CUDA(cudaMemsetAsync(done, 0, B, s));
-  SB_CUDA(cudaMemsetAsync(tgt_len, 0, 4ul * B, s));
+  const bool beam = a.beam > 0;
+  for (int l = 0; l < Ld; l++) SB_CUDA(cudaMemsetAsync(state[l], 0, 4ul * M * E, s));  // Decoder::start_states
+  SB_CUDA(cudaMemsetAsync(best, 0, 8ul * M, s));
+  if (beam) {
+    SB_CUDA(cudaMemsetAsync(cum, 0, 4ul * M, s));
+    SB_CUDA(cudaMemsetAsync(width, K, B, s));
+  } else {
+    SB_CUDA(cudaMemsetAsync(done, 0, B, s));
+    SB_CUDA(cudaMemsetAsync(tgt_len, 0, 4ul * B, s));
+  }
   SB_CUDA(cudaMemsetAsync(counters, 0, 256, s));
 
-  // step 0 input: zero embedding + position-0 signal (Transformer.cc:133-160)
+  // step 0 input of every row: zero embedding + position-0 signal (Transformer.cc:133-160)
   QuantOuts q = qouts();
   qadd(q, xq[0], m.dec[0].rnn_wf.aq), qadd(q, xq[1], m.dec[0].rnn_w.aq);
   {
-    LaunchScope ls(c, "dec_embed0", 0, 6.0 * B * E);
-    launch_embed(nullptr, m.emb_q, m.inv_qm, m.sqrt_e, m.pos, B, 1, E, 0, 1, xd, q, s);
+    LaunchScope ls(c, "dec_embed0", 0, 6.0 * M * E);
+    launch_embed(nullptr, m.emb_q, m.inv_qm, m.sqrt_e, m.pos, M, 1, E, 0, 1, xd, q, s);
   }
 
+  int executed = 0;
   for (int step = 0; step < max_steps; step++) {
     if (decode_step(step)) return 1;
-    // The step's bookkeeping (argmax -> word, record(), EOS flags) and the next step's input embedding are done by the
-    // FRONT of the next step's first kernel (dec_ssru_kernel with embed set); the last executed step is closed by the
-    // stand-alone kernel after the loop.
+    // Greedy: the step's bookkeeping (argmax -> word, record(), EOS flags) and the next step's input embedding are done
+    // by the FRONT of the next step's first kernel (dec_ssru_kernel with embed set); the last executed step is closed by
+    // the stand-alone kernel after the loop.
     executed = step + 1;
     bool all_done = false;
     if (poll_done(step, &all_done)) return 1;
     if (all_done) break;
   }
-  if (executed > 0) {
+
+  // ---- results
+  if (beam) {
+    SB_CUDA(cudaMemcpyAsync(a.beam_steps, d_rec, sizeof(BeamRec) * executed * M, cudaMemcpyDeviceToHost, s));
+    SB_CUDA(cudaMemcpyAsync(a.beam_finished, d_fin, sizeof(BeamFin) * M, cudaMemcpyDeviceToHost, s));
+    c.d2h_bytes += sizeof(BeamRec) * executed * M + sizeof(BeamFin) * M;
+    a.steps = static_cast<size_t>(executed);
+  } else {
     {
       LaunchScope ls(c, "dec_finalize_embed", 0, 7.0 * B * E + 20.0 * B);
       launch_finalize_step(best, d_sl, d_forced, executed - 1, d_steps, done, tgt_len, counters, m.eos_id, m.emb_q, m.inv_qm,
                            m.sqrt_e, m.pos, B, E, xd, q, s);
     }
+    std::vector<uint32_t> lens(B);
     SB_CUDA(cudaMemcpyAsync(&c.done_slots[0], counters, 4, cudaMemcpyDeviceToHost, s));
-    c.d2h_bytes += 4;
+    SB_CUDA(cudaMemcpyAsync(lens.data(), tgt_len, 4ul * B, cudaMemcpyDeviceToHost, s));
+    c.d2h_bytes += 4 + 4ul * B;
     SB_CUDA(cudaStreamSynchronize(s));
-    host_done = c.done_slots[0];
-  }
-
-  // ---- results
-  std::vector<uint32_t> lens(B);
-  SB_CUDA(cudaMemcpyAsync(lens.data(), tgt_len, 4ul * B, cudaMemcpyDeviceToHost, s));
-  if (d_align_all && executed > 0) {
-    SB_CUDA(cudaMemcpyAsync(a.alignment, d_align_all, 4ul * executed * B * T, cudaMemcpyDeviceToHost, s));
-    c.d2h_bytes += 4ul * executed * B * T;
-  }
-  if (!a.device_io && a.scores && executed > 0) {
-    SB_CUDA(cudaMemcpyAsync(a.scores, d_scores, 4ul * executed * B, cudaMemcpyDeviceToHost, s));
-    c.d2h_bytes += 4ul * executed * B;
-  }
-  if (!a.device_io && a.step_tokens && executed > 0) {
-    SB_CUDA(cudaMemcpyAsync(a.step_tokens, d_steps, 4ul * executed * B, cudaMemcpyDeviceToHost, s));
-    c.d2h_bytes += 4ul * executed * B;
-  }
-  if (!a.device_io && a.sentence_tokens && executed > 0) {
-    if (a.row_stride < static_cast<size_t>(executed)) {
-      set_error("sentence_tokens: row_stride smaller than the number of decode steps");
-      return 1;
+    if (a.target_lengths) memcpy(a.target_lengths, lens.data(), 4ul * B);
+    uint64_t total = 0;
+    uint32_t longest = 0;
+    for (uint32_t n : lens) total += n, longest = std::max(longest, n);
+    a.target_tokens = total;
+    // steps the reference would have run: up to the step where the last sentence finished
+    a.steps = c.done_slots[0] >= B ? longest : static_cast<size_t>(executed);
+    if (!a.device_io && a.scores) {
+      SB_CUDA(cudaMemcpyAsync(a.scores, d_scores, 4ul * executed * B, cudaMemcpyDeviceToHost, s));
+      c.d2h_bytes += 4ul * executed * B;
     }
-    // one row per sentence: the host then copies each sentence's recorded prefix without striding through the matrix
-    {
-      LaunchScope ls(c, "transpose_steps", 0, 8.0 * executed * B);
-      launch_transpose_u32(d_steps, executed, B, d_rows, executed, s);
+    if (!a.device_io && a.step_tokens) {
+      SB_CUDA(cudaMemcpyAsync(a.step_tokens, d_steps, 4ul * executed * B, cudaMemcpyDeviceToHost, s));
+      c.d2h_bytes += 4ul * executed * B;
     }
-    SB_CUDA(cudaMemcpy2DAsync(a.sentence_tokens, 4ul * a.row_stride, d_rows, 4ul * executed, 4ul * executed, B,
-                              cudaMemcpyDeviceToHost, s));
-    c.d2h_bytes += 4ul * executed * B;
+    if (!a.device_io && a.sentence_tokens) {
+      if (a.row_stride < static_cast<size_t>(executed)) {
+        set_error("sentence_tokens: row_stride smaller than the number of decode steps");
+        return 1;
+      }
+      // one row per sentence: the host then copies each sentence's recorded prefix without striding through the matrix
+      {
+        LaunchScope ls(c, "transpose_steps", 0, 8.0 * executed * B);
+        launch_transpose_u32(d_steps, executed, B, d_rows, executed, s);
+      }
+      SB_CUDA(cudaMemcpy2DAsync(a.sentence_tokens, 4ul * a.row_stride, d_rows, 4ul * executed, 4ul * executed, B,
+                                cudaMemcpyDeviceToHost, s));
+      c.d2h_bytes += 4ul * executed * B;
+    }
+  }
+  if (d_align_all) {
+    SB_CUDA(cudaMemcpyAsync(a.alignment, d_align_all, 4ul * executed * M * T, cudaMemcpyDeviceToHost, s));
+    c.d2h_bytes += 4ul * executed * M * T;
   }
   SB_CUDA(cudaStreamSynchronize(s));
-  if (a.target_lengths) memcpy(a.target_lengths, lens.data(), 4ul * B);
-  c.d2h_bytes += 4ul * B;
-  uint64_t total = 0;
-  uint32_t longest = 0;
-  bool all_done = host_done >= B;
-  for (int b = 0; b < B; b++) {
-    total += lens[b];
-    longest = std::max(longest, lens[b]);
-  }
-  a.target_tokens = total;
-  // steps the reference would have run: up to the step where the last sentence finished
-  a.steps = all_done ? longest : static_cast<size_t>(executed);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) {
-    set_error(std::string("forward failed: ") + cudaGetErrorString(e));
+    set_error(std::string(beam ? "beam search failed: " : "forward failed: ") + cudaGetErrorString(e));
     return 1;
   }
   return 0;
@@ -1456,7 +1459,7 @@ int Pass::decode() {
 int Pass::score() {
   SB_CUDA(cudaMemcpyAsync(d_tgt, a.targets, 4ul * M, cudaMemcpyHostToDevice, s));
   c.h2d_bytes += 4ul * M;
-  const double Md = M, Ed = E, Fd = F;
+  const double Md = M, Ed = E;
   {  // decoder inputs: zero embedding at j = 0, then the previous target word, each + the position-0 signal (quirk Q1)
     QuantOuts q = qouts();
     qadd(q, xq[0], m.dec[0].rnn_wf.aq), qadd(q, xq[1], m.dec[0].rnn_w.aq);
@@ -1494,32 +1497,9 @@ int Pass::score() {
       p->out = qd, p->ldo = E;
       if (g.launch()) return 1;
     }
-    {  // Tt queries per sentence against its cached K/V; head 0 of the last layer is the alignment
-      QuantOuts q = qouts();
-      qadd(q, caq, L.ctx.o.aq);
-      float* al = last ? d_align_all : nullptr;
-      const bool tiled = self_attention_tiled_supported(T, dh);
-      LaunchScope ls(c, "score_cross_attention", 4.0 * Md * (src_tokens / B) * Ed,
-                     Md * Ed * 5.0 + 2.0 * src_tokens * Ed * 4.0 + (al ? 4.0 * Md * T : 0.0));
-      const int rc = tiled ? launch_self_attention_tiled(qd, Kc[l], Vc[l], d_lengths, B, T, H, dh, q, s, Tt, al)
-                           : launch_self_attention_long(qd, Kc[l], Vc[l], d_lengths, B, T, H, dh, q, s, Tt, al);
-      if (rc) {
-        set_error("scoring cross-attention: no kernel for head size " + std::to_string(dh) + " over " +
-                  std::to_string(T) + " source tokens");
-        return 1;
-      }
-    }
-    {  // Wo + residual + LN, FFN: the step path's row-tile kernel over M rows
-      RowsFfnArgs k = rows_ffn_args(L.ctx, L.ffn, hb, M);
-      k.map_a = map_caq;
-      dec_layer_out(k, l, xd, xq[0], xq[1]);
-      LaunchScope ls(c, "score_wo_ffn_fused", 2.0 * Md * (Ed * Ed + 2.0 * Ed * Fd),
-                     Ed * Ed + 2.0 * Ed * Fd + Md * Ed * (1.0 + 4.0 + (last ? 1.0 : 6.0)));
-      if (launch_rows_ffn(k, E, F, kRowTile, false, s)) {
-        set_error("fused FFN kernel: unsupported sizes E=" + std::to_string(E) + " F=" + std::to_string(F));
-        return 1;
-      }
-    }
+    // Tt queries per sentence against its cached K/V; head 0 of the last layer is the alignment
+    if (cross_attention_mq(l, Tt, last ? d_align_all : nullptr, "score_cross_attention", "scoring")) return 1;
+    if (wo_ffn(l, xd, xq[0], xq[1], "score_wo_ffn_fused")) return 1;  // the step path's row-tile kernel over M rows
   }
   // output layer in row chunks, so that the strip partials [ceil(N / 64)][rows] stay bounded; each chunk is one "step"
   // of score_step with the targets as the forced words
@@ -1529,14 +1509,7 @@ int Pass::score() {
     CUtensorMap map;
     if (c.make_map(&map, oq + static_cast<size_t>(r0) * E, rows, E, kBM)) return 1;
     SB_CUDA(cudaMemsetAsync(best, 0, 8ul * rows, s));
-    {
-      const double Rd = rows, Nd = Nout;
-      LaunchScope ls(c, "score_gemm_out_scores", 2.0 * Rd * Nd * Ed, Rd * Ed + Nd * Ed + 8.0 * Nd + 8.0 * Rd + 8.0 * Rd * strips);
-      if (launch_out_scores(out, map, rows, E, best, partials, 1.0f, c.num_sms, s)) {
-        set_error("output GEMM (scores): unsupported K " + std::to_string(E));
-        return 1;
-      }
-    }
+    if (scores_gemm(map, rows, "score_gemm_out_scores")) return 1;
     const ScoreStepArgs k = score_step_args(rows, oq + static_cast<size_t>(r0) * E, d_tgt + r0, 0, d_scores + r0);
     LaunchScope ls(c, "score_step", 0, 8.0 * rows * strips + 16.0 * rows + 2.0 * rows * E);
     if (launch_score_step(k, s)) {
@@ -1561,45 +1534,6 @@ int Pass::score() {
 
 // One call on context c (`name` prefixes its errors): an empty request does nothing; otherwise the encoder and the
 // output layer's set-up, then `decoder` (Pass::decode or Pass::score).
-// Beam search (DESIGN §4.4d): the decode loop over B * K rows, each step closed by the candidate and merge kernels.  The
-// step records and finished hypotheses come back to the host, which does the backtrace and the ranking.
-int Pass::beam_search() {
-  for (int l = 0; l < Ld; l++) SB_CUDA(cudaMemsetAsync(state[l], 0, 4ul * M * E, s));
-  SB_CUDA(cudaMemsetAsync(best, 0, 8ul * M, s));
-  SB_CUDA(cudaMemsetAsync(cum, 0, 4ul * M, s));
-  SB_CUDA(cudaMemsetAsync(width, K, B, s));
-  SB_CUDA(cudaMemsetAsync(counters, 0, 256, s));
-  {  // step 0 input of every slot: zero embedding + position-0 signal
-    QuantOuts q = qouts();
-    qadd(q, xq[0], m.dec[0].rnn_wf.aq), qadd(q, xq[1], m.dec[0].rnn_w.aq);
-    LaunchScope ls(c, "dec_embed0", 0, 6.0 * M * E);
-    launch_embed(nullptr, m.emb_q, m.inv_qm, m.sqrt_e, m.pos, M, 1, E, 0, 1, xd, q, s);
-  }
-  int executed = 0;
-  for (int step = 0; step < max_steps; step++) {
-    if (decode_step(step)) return 1;
-    executed = step + 1;
-    bool all_done = false;
-    if (poll_done(step, &all_done)) return 1;
-    if (all_done) break;
-  }
-  SB_CUDA(cudaMemcpyAsync(a.beam_steps, d_rec, sizeof(BeamRec) * executed * M, cudaMemcpyDeviceToHost, s));
-  SB_CUDA(cudaMemcpyAsync(a.beam_finished, d_fin, sizeof(BeamFin) * M, cudaMemcpyDeviceToHost, s));
-  c.d2h_bytes += sizeof(BeamRec) * executed * M + sizeof(BeamFin) * M;
-  if (d_align_all) {
-    SB_CUDA(cudaMemcpyAsync(a.alignment, d_align_all, 4ul * executed * M * T, cudaMemcpyDeviceToHost, s));
-    c.d2h_bytes += 4ul * executed * M * T;
-  }
-  SB_CUDA(cudaStreamSynchronize(s));
-  a.steps = static_cast<size_t>(executed);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) {
-    set_error(std::string("beam search failed: ") + cudaGetErrorString(e));
-    return 1;
-  }
-  return 0;
-}
-
 int run_pass(Model& m, Context& c, ForwardArgs& a, const char* name, bool empty, int (Pass::*decoder)()) {
   std::lock_guard<std::recursive_mutex> ctx_lock(c.mu);
   if (c.device != m.ctx->device) {
@@ -1631,7 +1565,7 @@ int model_beam_on(Model& m, Context& c, ForwardArgs& a) {
               "logits, scores or device_io");
     return 1;
   }
-  return run_pass(m, c, a, "model_beam", a.B == 0 || a.T == 0, &Pass::beam_search);
+  return run_pass(m, c, a, "model_beam", a.B == 0 || a.T == 0, &Pass::decode);
 }
 
 int model_score_on(Model& m, Context& c, ForwardArgs& a) {

@@ -51,12 +51,13 @@ struct Context {
   CUresult (*encode_tiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                            const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                            CUtensorMapL2promotion, CUtensorMapFloatOOBfill) = nullptr;
-  // workspace arena (grown on demand, reused across calls; engine.cu's Workspace cuts it into buffers)
+  // workspace arena (grown on demand, reused across calls; Workspace cuts it into buffers)
   char* arena = nullptr;
   size_t arena_bytes = 0;
   char* flush_buf = nullptr;
   size_t flush_bytes = 0;
-  // pinned host staging of the service path (padded batch in, step tokens out): grown on demand, reused across calls
+  // pinned host staging of the service path (padded batch in, step tokens out): grown on demand, reused across calls;
+  // Workspace cuts it into buffers too
   char* staging = nullptr;
   size_t staging_bytes = 0;
   char* staging_reserve(size_t bytes);
@@ -83,6 +84,29 @@ struct Context {
   int make_map(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows);
   // f32 row-major [rows][cols] -> 2D tensor map, box = {32 floats (128 bytes), box_rows}, 128B swizzle
   int make_map_f32(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows);
+};
+
+// Margin behind the last buffer of the arena: not every kernel has been shown to keep its loads inside its buffer (the
+// output GEMMs index per-column arrays by 256-column tile), so the arena keeps ending with 16 KB that no buffer owns.
+constexpr size_t kTailPad = 64 * 256;
+
+// The buffers of one call, each listed once: add() records where a buffer's pointer goes and how many elements it
+// holds; carve() reserves the sum in the context's device arena, or with `staging` in its pinned host staging block, and
+// hands out the pointers in list order, each buffer starting on a 256-byte boundary.
+struct Workspace {
+  size_t bytes = 0;
+  std::vector<std::pair<void**, size_t>> bufs;
+  template <class T>
+  void add(T*& slot, size_t count) {
+    bufs.emplace_back(reinterpret_cast<void**>(&slot), (count * sizeof(T) + 255) & ~size_t(255));
+    bytes += bufs.back().second;
+  }
+  int carve(Context& c, bool staging = false) const {
+    char* p = staging ? c.staging_reserve(bytes) : c.reserve(bytes + kTailPad) ? nullptr : c.arena;
+    if (p == nullptr) return 1;
+    for (const auto& b : bufs) *b.first = p, p += b.second;
+    return 0;
+  }
 };
 
 // Counts a kernel launch and, in profiling mode, brackets it with events.  `ops` = algorithmic int8

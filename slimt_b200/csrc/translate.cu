@@ -33,13 +33,13 @@ struct Plan {
 
 struct LazyShortlist {
   const ShortlistGenerator* gen;
-  const std::vector<uint32_t>* words;
+  std::vector<uint32_t> words;
   size_t vocab;
   std::vector<uint32_t> out;
 };
 int lazy_shortlist_cb(void* user, const uint32_t** words, size_t* n) {
   auto* l = static_cast<LazyShortlist*>(user);
-  if (l->gen->generate(l->words->data(), l->words->size(), l->vocab, &l->out)) return 1;
+  if (l->gen->generate(l->words.data(), l->words.size(), l->vocab, &l->out)) return 1;
   *words = l->out.data();
   *n = l->out.size();
   return 0;
@@ -50,6 +50,12 @@ struct Done {
   std::vector<uint32_t> kept;
   std::vector<float> align;  // per sentence [target_len][source_len], back to back (only when asked for)
   std::vector<float> scores;  // like kept (only when asked for)
+};
+
+// One batch on its lane: its ForwardArgs and the shortlist that is built from its source words during the call.
+struct Batch {
+  ForwardArgs a;
+  LazyShortlist sl;
 };
 
 struct LaneStats {
@@ -132,6 +138,31 @@ struct Service {
     }
     return 0;
   }
+  // Sets up batch p on lane c: cuts the lane's staging block into the buffers the caller listed in `staging` and the
+  // padded sources, packs the sources (convert(), Frontend.cc:30-40; Input.cc:20-47) and fills the ForwardArgs fields
+  // every mode shares.  Model::decode builds the candidate set before its first step (Model.cc:116-120); here the host
+  // does it from the batch's words while the GPU runs the encoder (the callback fires once the encoder kernels are
+  // queued).
+  int stage(const Model& m, Context& c, const Plan& p, const uint32_t* src, const uint64_t* offsets, Workspace& staging,
+            Batch& b) const {
+    const size_t B = p.ids.size(), width = p.width;
+    uint32_t *tokens = nullptr, *lengths = nullptr;
+    staging.add(tokens, B * width), staging.add(lengths, B);
+    if (staging.carve(c, true)) return 1;
+    b.sl = LazyShortlist{&gen, {}, static_cast<size_t>(m.V), {}};
+    b.sl.words.reserve(B * width);
+    for (size_t r = 0; r < B; r++) {
+      const size_t s = p.ids[r];
+      const size_t len = offsets[s + 1] - offsets[s];
+      memcpy(tokens + r * width, src + offsets[s], 4 * len);
+      for (size_t t = len; t < width; t++) tokens[r * width + t] = m.pad_id;
+      lengths[r] = static_cast<uint32_t>(len);
+      b.sl.words.insert(b.sl.words.end(), src + offsets[s], src + offsets[s + 1]);
+    }
+    b.a.tokens = tokens, b.a.lengths = lengths, b.a.B = B, b.a.T = width;
+    if (use_sl) b.a.shortlist_cb = lazy_shortlist_cb, b.a.shortlist_user = &b.sl;
+    return 0;
+  }
   // Deals the batches to the lanes: one host thread per lane takes the next unserved batch as soon as it is free.
   // serve(m, c, bi) runs batch bi on lane context c (whose lock is held) and returns nonzero with the error set.
   template <class Serve>
@@ -208,22 +239,6 @@ struct Service {
   }
 };
 
-// convert(): Batch -> padded Input (Frontend.cc:30-40; Input.cc:20-47), and the batch's source words for the shortlist
-void pack_sources(const uint32_t* src, const uint64_t* offsets, const Plan& p, uint32_t pad_id, uint32_t* tokens,
-                  uint32_t* lengths, std::vector<uint32_t>* words) {
-  const size_t width = p.width;
-  words->clear();
-  words->reserve(p.ids.size() * width);
-  for (size_t r = 0; r < p.ids.size(); r++) {
-    const size_t s = p.ids[r];
-    const size_t len = offsets[s + 1] - offsets[s];
-    memcpy(tokens + r * width, src + offsets[s], 4 * len);
-    for (size_t t = len; t < width; t++) tokens[r * width + t] = pad_id;
-    lengths[r] = static_cast<uint32_t>(len);
-    words->insert(words->end(), src + offsets[s], src + offsets[s + 1]);
-  }
-}
-
 // One hypothesis of beam search, rebuilt on the host from the step records: its words and their scores, and for each
 // word the slot whose row computed it (where its alignment row is).
 struct Hyp {
@@ -258,15 +273,24 @@ std::vector<Hyp> beam_hypotheses(const BeamRec* rec, const BeamFin* fin, size_t 
   return hs;
 }
 
-// Copies each batch's per-sentence results (back to back in batch row order, `n(s)` values for sentence s) to their
-// places in the request's ragged output.
-template <class T, class Get, class N>
-void scatter(const std::vector<Plan>& plan, Get per_batch, const std::vector<uint64_t>& off, N n, T* out) {
+// The offsets of a ragged output whose sentence i holds n(i) values.
+template <class N>
+std::vector<uint64_t> ragged_offsets(size_t n_sent, N n) {
+  std::vector<uint64_t> off(n_sent + 1, 0);
+  for (size_t i = 0; i < n_sent; i++) off[i + 1] = off[i] + n(i);
+  return off;
+}
+
+// Copies one field of each batch's Done (per-sentence results back to back in batch row order) to the sentences'
+// places in the request's ragged output: sentence s's off[s + 1] - off[s] values go to out + off[s].
+template <class T>
+void scatter(const std::vector<Plan>& plan, const std::vector<Done>& done, std::vector<T> Done::*field,
+             const std::vector<uint64_t>& off, T* out) {
   for (size_t bi = 0; bi < plan.size(); bi++) {
-    size_t pos = 0;
+    const T* src = (done[bi].*field).data();
     for (size_t s : plan[bi].ids) {
-      memcpy(out + off[s], per_batch(bi).data() + pos, sizeof(T) * n(s));
-      pos += n(s);
+      memcpy(out + off[s], src, sizeof(T) * (off[s + 1] - off[s]));
+      src += off[s + 1] - off[s];
     }
   }
 }
@@ -359,25 +383,17 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
     const Plan& p = plan[bi];
     const size_t B = p.ids.size(), width = p.width, M = B * K;
     const size_t stride = static_cast<size_t>(forward_max_steps(io->limit_factor, width));
-    // staging: [padded tokens][lengths] | [step records] | [finished hypotheses] | [alignment rows]
-    const size_t in_bytes = (4 * (B * width + B) + 255) & ~size_t(255);
-    const size_t rec_bytes = (sizeof(BeamRec) * stride * M + 255) & ~size_t(255);
-    const size_t fin_bytes = (sizeof(BeamFin) * M + 255) & ~size_t(255);
-    const size_t al_bytes = want_align ? 4 * stride * M * width : 0;
-    char* stage = c.staging_reserve(in_bytes + rec_bytes + fin_bytes + al_bytes + 256);
-    if (!stage) return 1;
-    uint32_t* tokens = reinterpret_cast<uint32_t*>(stage);
-    uint32_t* lengths = tokens + B * width;
-    std::vector<uint32_t> words;
-    pack_sources(io->tokens, io->offsets, p, m.pad_id, tokens, lengths, &words);
-    LazyShortlist lazy{&sv.gen, &words, static_cast<size_t>(m.V), {}};
-    BeamRec* rec = reinterpret_cast<BeamRec*>(stage + in_bytes);
-    BeamFin* fin = reinterpret_cast<BeamFin*>(stage + in_bytes + rec_bytes);
-    float* align = want_align ? reinterpret_cast<float*>(stage + in_bytes + rec_bytes + fin_bytes) : nullptr;
-    ForwardArgs a;
-    a.tokens = tokens, a.lengths = lengths, a.B = B, a.T = width;
+    // staging: step records, finished hypotheses, alignment rows
+    Workspace staging;
+    BeamRec* rec = nullptr;
+    BeamFin* fin = nullptr;
+    float* align = nullptr;
+    staging.add(rec, stride * M), staging.add(fin, M);
+    if (want_align) staging.add(align, stride * M * width);
+    Batch b;
+    if (sv.stage(m, c, p, io->tokens, io->offsets, staging, b)) return 1;
+    ForwardArgs& a = b.a;
     a.limit_factor = io->limit_factor;
-    if (sv.use_sl) a.shortlist_cb = lazy_shortlist_cb, a.shortlist_user = &lazy;
     a.beam = K, a.beam_steps = rec, a.beam_finished = fin, a.alignment = align;
     if (model_beam_on(m, c, a)) return 1;
     beam_steps += a.steps;
@@ -391,7 +407,7 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
       if (want_align)  // the row that computed word s: slot h.slots[s] of step s
         for (size_t st = 0; st < h.tokens.size(); st++) {
           const float* row = align + (st * M + r * K + h.slots[st]) * width;
-          d.align.insert(d.align.end(), row, row + lengths[r]);
+          d.align.insert(d.align.end(), row, row + a.lengths[r]);
         }
       hs.resize(beam->nbest);
       nbest[p.ids[r]] = std::move(hs);
@@ -403,36 +419,24 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
     const Plan& p = plan[bi];
     const size_t B = p.ids.size(), width = p.width;
     const size_t stride = static_cast<size_t>(forward_max_steps(io->limit_factor, width));
-    // staging: [padded tokens][lengths] | [sentence-major step tokens][recorded lengths] | [alignment rows] |
-    // [step-major scores] | [sampling keys]
-    const size_t in_bytes = (4 * (B * width + B) + 255) & ~size_t(255);
-    const size_t tok_bytes = (4 * (stride + 1) * B + 255) & ~size_t(255);
-    const size_t al_bytes = want_align ? 4 * stride * B * width : 0;
-    const size_t sc_bytes = want_scores ? 4 * stride * B : 0;
-    const size_t key_off = (in_bytes + tok_bytes + al_bytes + sc_bytes + 7) & ~size_t(7);
-    char* stage = c.staging_reserve(in_bytes + tok_bytes + al_bytes + sc_bytes + (sampling ? 8 * B + 8 : 0) + 256);
-    if (!stage) return 1;
-    uint32_t* tokens = reinterpret_cast<uint32_t*>(stage);
-    uint32_t* lengths = tokens + B * width;
-    std::vector<uint32_t> words;
-    pack_sources(io->tokens, io->offsets, p, m.pad_id, tokens, lengths, &words);
-    // Model::decode builds the candidate set before its first step (Model.cc:116-120); here the host does it
-    // while the GPU runs the encoder (the callback fires once the encoder kernels are queued)
-    LazyShortlist lazy{&sv.gen, &words, static_cast<size_t>(m.V), {}};
-    uint32_t* rows = reinterpret_cast<uint32_t*>(stage + in_bytes);
-    uint32_t* lens = rows + stride * B;
-    float* align = want_align ? reinterpret_cast<float*>(stage + in_bytes + tok_bytes) : nullptr;
-    float* scores = want_scores ? reinterpret_cast<float*>(stage + in_bytes + tok_bytes + al_bytes) : nullptr;
-    ForwardArgs a;
-    a.tokens = tokens, a.lengths = lengths, a.B = B, a.T = width;
+    // staging: sentence-major step tokens, recorded lengths, alignment rows, step-major scores, sampling keys
+    Workspace staging;
+    uint32_t *rows = nullptr, *lens = nullptr;
+    float *align = nullptr, *scores = nullptr;
+    uint64_t* keys = nullptr;
+    staging.add(rows, stride * B), staging.add(lens, B);
+    if (want_align) staging.add(align, stride * B * width);
+    if (want_scores) staging.add(scores, stride * B);
+    if (sampling) staging.add(keys, B);
+    Batch b;
+    if (sv.stage(m, c, p, io->tokens, io->offsets, staging, b)) return 1;
+    ForwardArgs& a = b.a;
     a.limit_factor = io->limit_factor;
-    if (sv.use_sl) a.shortlist_cb = lazy_shortlist_cb, a.shortlist_user = &lazy;
     a.sentence_tokens = rows, a.row_stride = stride, a.target_lengths = lens;
     a.alignment = align;
     a.scores = scores;
     if (sampling) {
       // each sentence's own key (default: its index in the request), wherever the Batcher put it
-      uint64_t* keys = reinterpret_cast<uint64_t*>(stage + key_off);
       for (size_t r = 0; r < B; r++) keys[r] = sampling->keys ? sampling->keys[p.ids[r]] : static_cast<uint64_t>(p.ids[r]);
       a.sample = true, a.inv_t = sampling_inv_t(sampling->temperature), a.seed = sampling->seed, a.keys = keys;
       a.top_k = top_k;
@@ -443,7 +447,7 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
     for (size_t r = 0; r < B; r++) {
       out_len[p.ids[r]] = lens[r];
       kept_total += lens[r];
-      align_total += static_cast<size_t>(lens[r]) * lengths[r];
+      align_total += static_cast<size_t>(lens[r]) * a.lengths[r];
     }
     d.kept.resize(kept_total);
     size_t pos = 0;
@@ -456,8 +460,8 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
       size_t ap = 0;
       for (size_t r = 0; r < B; r++)
         for (size_t s = 0; s < lens[r]; s++) {
-          memcpy(d.align.data() + ap, align + (s * B + r) * width, 4ul * lengths[r]);
-          ap += lengths[r];
+          memcpy(d.align.data() + ap, align + (s * B + r) * width, 4ul * a.lengths[r]);
+          ap += a.lengths[r];
         }
     }
     if (want_scores) {  // the scores of the recorded steps, sentence by sentence in batch row order like kept
@@ -474,27 +478,24 @@ int translate_multi(Model* const* models, size_t n_rep, slimt_b200_translate_io*
   io->batches = plan.size();
 
   // ---- ragged outputs
-  std::vector<uint64_t> out_off(n_sent + 1, 0);
-  for (size_t i = 0; i < n_sent; i++) out_off[i + 1] = out_off[i] + out_len[i];
+  const std::vector<uint64_t> out_off = ragged_offsets(n_sent, [&](size_t i) { return out_len[i]; });
   io->target_tokens = out_off[n_sent];
   if ((io->out_tokens || want_scores) && out_off[n_sent] > io->out_capacity) {
     set_error(io->out_tokens ? "out_tokens capacity too small" : "out_scores capacity too small");
     return 1;
   }
   if (io->out_offsets) memcpy(io->out_offsets, out_off.data(), 8 * (n_sent + 1));
-  auto n_out = [&](size_t s) { return static_cast<size_t>(out_len[s]); };
-  if (io->out_tokens) scatter(plan, [&](size_t bi) -> const auto& { return done[bi].kept; }, out_off, n_out, io->out_tokens);
-  if (want_scores) scatter(plan, [&](size_t bi) -> const auto& { return done[bi].scores; }, out_off, n_out, io->out_scores);
+  if (io->out_tokens) scatter(plan, done, &Done::kept, out_off, io->out_tokens);
+  if (want_scores) scatter(plan, done, &Done::scores, out_off, io->out_scores);
   if (want_align) {
-    std::vector<uint64_t> al_off(n_sent + 1, 0);
-    for (size_t i = 0; i < n_sent; i++) al_off[i + 1] = al_off[i] + static_cast<uint64_t>(out_len[i]) * (io->offsets[i + 1] - io->offsets[i]);
+    const std::vector<uint64_t> al_off = ragged_offsets(
+        n_sent, [&](size_t i) { return static_cast<uint64_t>(out_len[i]) * (io->offsets[i + 1] - io->offsets[i]); });
     if (al_off[n_sent] > io->align_capacity) {
       set_error("out_alignments capacity too small");
       return 1;
     }
     if (io->out_align_offsets) memcpy(io->out_align_offsets, al_off.data(), 8 * (n_sent + 1));
-    scatter(plan, [&](size_t bi) -> const auto& { return done[bi].align; }, al_off,
-            [&](size_t s) { return static_cast<size_t>(al_off[s + 1] - al_off[s]); }, io->out_alignments);
+    scatter(plan, done, &Done::align, al_off, io->out_alignments);
   }
   if (beam) {
     beam->steps = beam_steps.load();
@@ -542,8 +543,8 @@ int score_multi(Model* const* models, size_t n_rep, slimt_b200_score_io* io) {
     set_error("score: out_scores capacity too small (" + std::to_string(n_tgt) + " target tokens)");
     return 1;
   }
-  std::vector<uint64_t> al_off(n_sent + 1, 0);
-  for (size_t i = 0; i < n_sent; i++) al_off[i + 1] = al_off[i] + (to[i + 1] - to[i]) * (so[i + 1] - so[i]);
+  const std::vector<uint64_t> al_off =
+      ragged_offsets(n_sent, [&](size_t i) { return (to[i + 1] - to[i]) * (so[i + 1] - so[i]); });
   if (want_align && al_off[n_sent] > io->align_capacity) {
     set_error("score: out_alignments capacity too small");
     return 1;
@@ -569,7 +570,7 @@ int score_multi(Model* const* models, size_t n_rep, slimt_b200_score_io* io) {
   if (sv.make_plan(so, n_sent, io->max_words)) return 1;
   const std::vector<Plan>& plan = sv.plan;
 
-  std::vector<std::vector<float>> scores(plan.size()), align(plan.size());
+  std::vector<Done> done(plan.size());
   auto serve = [&](Model& m, Context& c, size_t bi) -> int {
     const Plan& p = plan[bi];
     const size_t B = p.ids.size(), width = p.width;
@@ -579,48 +580,39 @@ int score_multi(Model* const* models, size_t n_rep, slimt_b200_score_io* io) {
       Tt = std::max(Tt, tl), n_scores += tl, n_align += tl * (so[s + 1] - so[s]);
     }
     if (Tt == 0) return 0;  // every target of the batch is empty: nothing to score
-    // staging: [padded tokens][lengths] | [padded targets] | [scores] | [alignments]
-    const size_t in_bytes = (4 * (B * width + B) + 255) & ~size_t(255);
-    const size_t tg_bytes = (4 * B * Tt + 255) & ~size_t(255);
-    const size_t al_bytes = want_align ? 4 * B * Tt * width : 0;
-    char* stage = c.staging_reserve(in_bytes + 2 * tg_bytes + al_bytes + 256);
-    if (!stage) return 1;
-    uint32_t* tokens = reinterpret_cast<uint32_t*>(stage);
-    uint32_t* lengths = tokens + B * width;
-    std::vector<uint32_t> words;
-    pack_sources(io->tokens, so, p, m.pad_id, tokens, lengths, &words);
-    uint32_t* targets = reinterpret_cast<uint32_t*>(stage + in_bytes);
-    float* sc = reinterpret_cast<float*>(stage + in_bytes + tg_bytes);
-    float* al = want_align ? reinterpret_cast<float*>(stage + in_bytes + 2 * tg_bytes) : nullptr;
+    // staging: padded targets, scores, alignments
+    Workspace staging;
+    uint32_t* targets = nullptr;
+    float *sc = nullptr, *al = nullptr;
+    staging.add(targets, B * Tt), staging.add(sc, B * Tt);
+    if (want_align) staging.add(al, B * Tt * width);
+    Batch b;
+    if (sv.stage(m, c, p, io->tokens, so, staging, b)) return 1;
     for (size_t r = 0; r < B; r++) {
       const size_t s = p.ids[r], tl = to[s + 1] - to[s];
       memcpy(targets + r * Tt, io->targets + to[s], 4 * tl);
       for (size_t j = tl; j < Tt; j++) targets[r * Tt + j] = m.pad_id;  // computed and discarded
     }
-    LazyShortlist lazy{&sv.gen, &words, static_cast<size_t>(m.V), {}};
-    ForwardArgs a;
-    a.tokens = tokens, a.lengths = lengths, a.B = B, a.T = width;
-    if (sv.use_sl) a.shortlist_cb = lazy_shortlist_cb, a.shortlist_user = &lazy;
+    ForwardArgs& a = b.a;
     a.targets = targets, a.target_T = Tt, a.scores = sc, a.alignment = al;
     if (model_score_on(m, c, a)) return 1;
     // each sentence's valid positions, back to back in batch row order
-    std::vector<float>& ds = scores[bi];
-    ds.resize(n_scores);
+    Done& d = done[bi];
+    d.scores.resize(n_scores);
     size_t sp = 0;
     for (size_t r = 0; r < B; r++) {
       const size_t tl = to[p.ids[r] + 1] - to[p.ids[r]];
-      memcpy(ds.data() + sp, sc + r * Tt, 4 * tl);
+      memcpy(d.scores.data() + sp, sc + r * Tt, 4 * tl);
       sp += tl;
     }
     if (want_align) {
-      std::vector<float>& da = align[bi];
-      da.resize(n_align);
+      d.align.resize(n_align);
       size_t ap = 0;
       for (size_t r = 0; r < B; r++) {
         const size_t tl = to[p.ids[r] + 1] - to[p.ids[r]];
         for (size_t j = 0; j < tl; j++) {
-          memcpy(da.data() + ap, al + (r * Tt + j) * width, 4ul * lengths[r]);
-          ap += lengths[r];
+          memcpy(d.align.data() + ap, al + (r * Tt + j) * width, 4ul * a.lengths[r]);
+          ap += a.lengths[r];
         }
       }
     }
@@ -631,14 +623,11 @@ int score_multi(Model* const* models, size_t n_rep, slimt_b200_score_io* io) {
   io->kernel_launches = sv.launches, io->h2d_bytes = sv.h2d, io->d2h_bytes = sv.d2h;
   io->batches = plan.size();
 
-  std::vector<uint64_t> out_off(n_sent + 1, 0);
-  for (size_t i = 0; i < n_sent; i++) out_off[i + 1] = out_off[i] + (to[i + 1] - to[i]);
-  auto n_out = [&](size_t s) { return static_cast<size_t>(to[s + 1] - to[s]); };
-  if (n_tgt > 0) scatter(plan, [&](size_t bi) -> const auto& { return scores[bi]; }, out_off, n_out, io->out_scores);
+  const std::vector<uint64_t> out_off = ragged_offsets(n_sent, [&](size_t i) { return to[i + 1] - to[i]; });
+  if (n_tgt > 0) scatter(plan, done, &Done::scores, out_off, io->out_scores);
   if (want_align) {
     if (io->out_align_offsets) memcpy(io->out_align_offsets, al_off.data(), 8 * (n_sent + 1));
-    scatter(plan, [&](size_t bi) -> const auto& { return align[bi]; }, al_off, [&](size_t s) { return static_cast<size_t>(al_off[s + 1] - al_off[s]); },
-            io->out_alignments);
+    scatter(plan, done, &Done::align, al_off, io->out_alignments);
   }
   return 0;
 }

@@ -711,7 +711,7 @@ Routes choose_routes(const Model& m, int T, int B, bool fast, bool logits, bool 
   const char* ca = getenv("SLIMT_B200_CROSS");
   if (env_is(ca, "cached") || (!env_is(ca, "rc") && static_cast<long>(B) * T <= 4096)) r.cross = Cross::Cached;
   else if (cross_attention_rc_supported(E, H, dh, T)) r.cross = Cross::Rc;
-  // long sentences (65 .. 256 tokens) take the sentence-at-a-time recompute kernel (cross_attention_rcl.cu; bit-exact mode)
+  // long sentences (65 .. 256 tokens) take the sentence-at-a-time recompute kernel (cross_attention_rc.cu; bit-exact mode)
   else if (!fast && cross_attention_rcl_supported(E, H, dh, T)) r.cross = Cross::Rcl;
   else r.cross = Cross::Cached;
 

@@ -79,7 +79,7 @@ struct CrossRcArgs {
 };
 bool cross_attention_rc_supported(int E, int H, int dh, int S);
 int launch_cross_attention_rc(const CrossRcArgs& a, int num_sms, bool fast, cudaStream_t stream);
-// The same for long source sentences (S <= 256), one sentence at a time (cross_attention_rcl.cu); bit-exact mode only.
+// The same for long source sentences (S <= 256), one sentence at a time (cross_attention_rc.cu); bit-exact mode only.
 bool cross_attention_rcl_supported(int E, int H, int dh, int S);
 int launch_cross_attention_rcl(const CrossRcArgs& a, int num_sms, cudaStream_t stream);
 

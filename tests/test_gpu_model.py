@@ -92,10 +92,10 @@ def test_cross_attention_recompute_equals_cached_path(tiny_gpu, shape, monkeypat
 
 @pytest.mark.parametrize("shape", [(5, 65), (3, 100), (4, 128), (3, 129), (2, 256), (150, 70), (6, 200), (9, 255)])
 def test_long_sentence_cross_attention_recompute_equals_cached_path(tiny_gpu, shape, monkeypatch):
-    """Batches of 65 .. 256 source tokens re-project K/V a sentence at a time (cross_attention_rcl.cu: one or two
-    128-key groups per sentence, softmax across the groups, one weighted-sum chain carried over them; ragged lengths
-    from 1 token up, more sentences than SMs).  Forcing the cached f32 K/V kernel must give the same bits, and both
-    must equal the oracle."""
+    """Batches of 65 .. 256 source tokens re-project K/V a sentence at a time (cross_attention_rcl_kernel in
+    cross_attention_rc.cu: one or two 128-key groups per sentence, softmax across the groups, one weighted-sum chain
+    carried over them; ragged lengths from 1 token up, more sentences than SMs).  Forcing the cached f32 K/V kernel
+    must give the same bits, and both must equal the oracle."""
     m, orc = tiny_gpu
     B, T = shape
     sents = synth.make_sentences(B, (1, T), seed=17 * B + T)
